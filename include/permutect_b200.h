@@ -269,15 +269,6 @@ int pmt_losses_backward(const PmtLossDesc* desc, const float* weights, const Pmt
                         float* d_logits_b, float* d_outlier_logits_b, float* d_features_be, float* d_weights,
                         void* workspace, size_t workspace_bytes, void* stream);
 
-/* Measurement hook (no reference counterpart): device buffer of 3 x 1024 int64 that CTA 0 of the next tensor-core
- * haplotype-CNN launches fills with (event id, clock64) pairs (profiles/trace_cnn.py); NULL disarms. */
-int pmt_set_cnn_trace(long long* device_buffer);
-/* Same for the tensor-core read kernel: 4 x 2048 int64 (two epilogue warps, the two MMA warps; profiles/trace_reads.py). */
-int pmt_set_reads_trace(long long* device_buffer);
-/* Same for the backward read kernel: 512 int64, [0] = record count (caller zeroes it), then (phase id, clock64) pairs of
- * CTA 0's third tile (profiles/trace_backward.py). */
-int pmt_set_backward_trace(long long* device_buffer);
-
 /* ---- flat optimiser step ---------------------------------------------------------------------------
  * Replaces misc_utils.backpropagate's clip_grad_norm_(max_norm=1.0) + AdamW.step (misc_utils.py:125-129;
  * optimiser built at model_training.py:68-72) for a model whose parameters are views of one flat fp32 buffer.

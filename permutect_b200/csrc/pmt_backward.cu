@@ -9,7 +9,6 @@
 //   hap_cnn_backward_kernel   DNASequenceConvolution
 //   reduce_partials_kernel    sum of the CTA-private buffers in CTA order (bitwise reproducible)
 //   skip_fix_kernel           DenseSkipBlock.alpha gradients and the alpha scaling of its last layer
-#include <cstdlib>
 #include <cstring>
 
 // The per-row phases are written for NPART = NTHREADS / TILE threads per tile row.  Measured on B200 (65 536 variants,
@@ -39,10 +38,7 @@ struct BwdArgs {
   long long long_scratch_stride;
   float* partials;            // per-CTA flat gradient buffers [grid][n_params]
   int n_claims;
-  long long* trace;           // measurement hook (pmt_set_backward_trace): phase clocks of CTA 0's third tile, or null
 };
-
-// trace[0] = number of records; record i = (phase id, clock64()) at trace[1 + 2i]  (PMT_TILE_TRACE)
 
 // The four activation buffers of a backward CTA, as (base, stride): an array of pointers would live in local memory,
 // and with nearly all of L1 carved out as shared memory every read of it is an L2 round trip.
@@ -67,14 +63,7 @@ __device__ __forceinline__ float* pick_free(const BufSet& bufs, const float* a, 
 static __device__ __noinline__ float* mlp_backward(const Plan& P, const PmtLinearOp* ops, int n_ops, int g0,
                                                    const float* scr, const int* scr_off, float* g, const BufSet& bufs,
                                                    Stage& stage, const float* wflat, float* part, int rows_used,
-                                                   bool need_input_grad, long long* trace = nullptr) {
-#define PMT_MLP_TRACE(id)                                                                                        \
-  do {                                                                                                           \
-    if (trace && threadIdx.x == 0) {                                                                             \
-      const long long n_ = trace[0];                                                                             \
-      if (n_ < 250) { trace[1 + 2 * n_] = (id); trace[2 + 2 * n_] = clock64(); trace[0] = n_ + 1; }             \
-    }                                                                                                            \
-  } while (0)
+                                                   bool need_input_grad) {
   float* gcur = g;
   int i = n_ops - 1;
   while (i >= 0) {
@@ -90,21 +79,15 @@ static __device__ __noinline__ float* mlp_backward(const Plan& P, const PmtLinea
         const GemmOp& gop = P.gemm[g0 + j];
         float* A = pick_free(bufs, gres, din, nullptr);
         __syncthreads();
-        PMT_MLP_TRACE(200);
         load_rows_async(A, lop.in_dim, scr + scr_off[j]);   // acquire() waits for every cp.async of the thread
         const float* imgT = stage.acquire(MAX_GEMM + g0 + j);
-        PMT_MLP_TRACE(201);
         if (j == j0) { selu_copy(A, A, lop.in_dim); __syncthreads(); }   // A = s0 = SELU(x)
         if (j > 0) stage.prefetch(MAX_GEMM + g0 + j - 1);
-        PMT_MLP_TRACE(202);
         wgrad_tile(smem_addr(din), lop.out_dim, smem_addr(A), lop.in_dim, part + lop.w_off, 0, rows_used);
-        PMT_MLP_TRACE(203);
         rowdot_tile(din, nullptr, lop.out_dim, part + lop.b_off, 0, rows_used);
-        PMT_MLP_TRACE(204);
         const float scale = (j == j1) ? alpha : 1.f;
         float* dnext = pick_free(bufs, gres, din, A);
         gemm_tile_T(din, gop, imgT, 0, dnext, EPI_DSELU, scale, A, rows_used);
-        PMT_MLP_TRACE(205);
         if (j == j0) {   // gres += dnext (the SELU(x) branch joins the identity branch)
           __syncthreads();
           for (int t = threadIdx.x; t < lop.in_dim * (TILE / 4); t += NTHREADS) {
@@ -177,7 +160,6 @@ struct BwdTile {
   float* small;         // [64] scratch for tiny reductions
   float* part;          // this CTA's flat gradient buffer
   int acc_cap;
-  bool tracing;
 };
 
 struct BwdSmem {
@@ -213,14 +195,6 @@ __device__ __forceinline__ void carve_bwd_smem(const Plan& P, float* smem, TileC
   C.M = reinterpret_cast<TileMeta*>((reinterpret_cast<uintptr_t>(C.HC + 1) + 15) & ~uintptr_t(15));
 }
 
-#define PMT_TILE_TRACE(id)                                                    \
-  do {                                                                        \
-    if (T.tracing && threadIdx.x == 0) {                                      \
-      const long long n_ = T.A.trace[0];                                      \
-      if (n_ < 250) { T.A.trace[1 + 2 * n_] = (id); T.A.trace[2 + 2 * n_] = clock64(); T.A.trace[0] = n_ + 1; } \
-    }                                                                         \
-  } while (0)
-
 // Reducer -> rotation -> clustering head (recompute, activations to `scr`), then their backward
 // (feature_clustering.py:82-135, euclidean_transformation.py:19-20, artifact_model.py:258-259).
 // C.X holds the reducer's input.  Returns the buffer holding dL/d(output of the last gated block).
@@ -240,7 +214,6 @@ static __device__ __forceinline__ float* bwd_tail(BwdTile& T, float* scr) {
   const PmtOutputs no_out{};
   float *Yb, *Fb;
   tile_tail(P, C, T.stage, no_out, false, scr, Yb, Fb);
-  PMT_TILE_TRACE(20);
   float* Lb = pick_free(T.bufs, Yb, Fb, T.bufs[3]);   // the third forward buffer (held the log-likelihoods)
   float* Xtra = T.bufs[3];
 
@@ -334,9 +307,7 @@ static __device__ __forceinline__ float* bwd_tail(BwdTile& T, float* scr) {
   }
   __syncthreads();
   rowdot_tile(Xtra, nullptr, E, part + D.translation, 0, rows_used);
-  PMT_TILE_TRACE(21);
   float* G = mlp_backward(P, D.red_ops, D.n_red_ops, P.red_g0, scr, P.scr_red, Xtra, T.bufs, T.stage, W, part, rows_used, true);
-  PMT_TILE_TRACE(22);
   return G;
 }
 
@@ -413,7 +384,6 @@ static __device__ __forceinline__ RowNorm bwd_block_gate(BwdTile& T, int blk, co
     Cz[(3 * H + f) * LD + row] = gate;
     Cz[(4 * H + f) * LD + row] = Cz[f * LD + row] * gate;   // u = z1 * gate
   }
-  PMT_TILE_TRACE(100 + blk * 10 + 0);
   // proj2: x_out = x + W2_s u + b2_s
   const float* imgT2 = T.stage.acquire(MAX_GEMM + g2);
   T.stage.prefetch(MAX_GEMM + g1);
@@ -423,7 +393,6 @@ static __device__ __forceinline__ RowNorm bwd_block_gate(BwdTile& T, int blk, co
   rowdot_tile(G, nullptr, Dm, part + BO.p2_alt_b, ref_pad, rows_used);
   gemm_tile_T(G, P.gemm[g2], imgT2, ref_pad, Cz + 5 * H * LD, EPI_STORE, 1.f, nullptr, rows_used);   // du
   __syncthreads();
-  PMT_TILE_TRACE(100 + blk * 10 + 1);
   {  // d z1 = du * gate ; d gate = du * z1 ; scalar gradients of the gate
     float s_alpha = 0.f, s_beta = 0.f, s_gamma = 0.f;
     for (int f = f_lo; f < f_hi; ++f) {
@@ -541,7 +510,6 @@ static __device__ __forceinline__ void bwd_block_finish(BwdTile& T, int blk, flo
     }
   }
   __syncthreads();
-  PMT_TILE_TRACE(100 + blk * 10 + 2);
   mul_dselu(Cz + 4 * H * LD, Cz, 2 * H);   // through z = SELU(proj1 n)
   // proj1: z_pre = W1_s n + b1_s
   const float* imgT1 = T.stage.acquire(MAX_GEMM + g1);
@@ -553,7 +521,6 @@ static __device__ __forceinline__ void bwd_block_finish(BwdTile& T, int blk, flo
   __syncthreads();
   gemm_tile_T(Cz + 4 * H * LD, P.gemm[g1], imgT1, ref_pad, Bn, EPI_STORE, 1.f, nullptr, rows_used);   // d n
   __syncthreads();
-  PMT_TILE_TRACE(100 + blk * 10 + 3);
   rowdot_tile(Bn, Ab, Dm, part + BO.ln_w, 0, rows_used);
   rowdot_tile(Bn, nullptr, Dm, part + BO.ln_b, 0, rows_used);
   {  // LayerNorm backward, added to the residual gradient
@@ -569,7 +536,6 @@ static __device__ __forceinline__ void bwd_block_finish(BwdTile& T, int blk, flo
     }
   }
   __syncthreads();
-  PMT_TILE_TRACE(100 + blk * 10 + 4);
 }
 
 // concat (artifact_model.py:246-251): d info_seq of each variant (added to it when the set spans several chunks), then
@@ -590,17 +556,8 @@ static __device__ __forceinline__ void bwd_embed(BwdTile& T, float* scr, float* 
       *o = accumulate ? *o + s : s;
     }
   }
-  PMT_TILE_TRACE(23);
-#ifdef PMT_GEMM_TRACE
-  if (T.tracing && threadIdx.x == 0) T.A.trace[511] = 1;
-#endif
-  mlp_backward(P, D.read_ops, D.n_read_ops, P.read_g0, scr, P.scr_read, G, T.bufs, T.stage, T.C.W, T.part, T.C.rows_used, false,
-               T.tracing ? T.A.trace : nullptr);
+  mlp_backward(P, D.read_ops, D.n_read_ops, P.read_g0, scr, P.scr_read, G, T.bufs, T.stage, T.C.W, T.part, T.C.rows_used, false);
   __syncthreads();
-#ifdef PMT_GEMM_TRACE
-  if (T.tracing && threadIdx.x == 0) T.A.trace[511] = 0;
-#endif
-  PMT_TILE_TRACE(24);
 }
 
 __global__ void __launch_bounds__(NTHREADS, 1)
@@ -628,10 +585,9 @@ reads_backward_kernel(const __grid_constant__ Plan Pparam, const __grid_constant
   __syncthreads();
   const long long total_ref = __ldg(A.batch.ref_off + B);
   float* scr = A.scratch + (long long)blockIdx.x * A.scratch_stride;
-  BwdTile T{P, A, C, stage, acc, S.bufs, S.dsums, S.wpart, S.small, A.partials + (long long)blockIdx.x * D.n_params, S.acc_cap, false};
+  BwdTile T{P, A, C, stage, acc, S.bufs, S.dsums, S.wpart, S.small, A.partials + (long long)blockIdx.x * D.n_params, S.acc_cap};
   const int claim = P.claim_variants;
 
-  int tile_no = 0;
   // static round-robin assignment of claims to CTAs: the summation order of every gradient is fixed
   for (int c = blockIdx.x; c < A.n_claims; c += gridDim.x) {
     const long long cv0 = (long long)c * claim;
@@ -641,14 +597,10 @@ reads_backward_kernel(const __grid_constant__ Plan Pparam, const __grid_constant
       const int nv = build_tile(A.batch, v_cur, cv1, total_ref, M);
       if (nv == 0) { v_cur += 1; continue; }   // a set longer than a tile: reads_backward_long_kernel
       v_cur += nv;
-      T.tracing = A.trace != nullptr && blockIdx.x == 0 && tile_no == 2;
-      tile_no += 1;
-      PMT_TILE_TRACE(0);
       C.rows_used = (M.rows + 3) & ~3;
 
       // ======================= forward recompute, activations to scratch =======================
       tile_embed(P, C, stage, A.batch, A.info_seq, scr);
-      PMT_TILE_TRACE(1);
       for (int blk = 0; blk < D.n_blocks; ++blk) {
         save_rows(C.X, Dm, scr + P.scr_x[blk]);
         block_phase_a(P, C, stage, blk, scr + P.scr_z[blk]);
@@ -656,7 +608,6 @@ reads_backward_kernel(const __grid_constant__ Plan Pparam, const __grid_constant
         __syncthreads();
         block_means(P, C, blk);
         block_phase_b(P, C, stage, blk, blk + 1 < D.n_blocks ? P.blk_g0 + 2 * blk + 2 : P.red_g0);
-        PMT_TILE_TRACE(2 + blk);
       }
       // ======================= backward =======================
       float* G = bwd_tail(T, scr);
@@ -702,7 +653,7 @@ reads_backward_long_kernel(const __grid_constant__ Plan Pparam, const __grid_con
   __syncthreads();
   const long long total_ref = __ldg(A.batch.ref_off + B);
   float* scr0 = A.long_scratch + (long long)blockIdx.x * A.long_scratch_stride;
-  BwdTile T{P, A, C, stage, acc, S.bufs, S.dsums, S.wpart, S.small, A.partials + (long long)blockIdx.x * D.n_params, S.acc_cap, false};
+  BwdTile T{P, A, C, stage, acc, S.bufs, S.dsums, S.wpart, S.small, A.partials + (long long)blockIdx.x * D.n_params, S.acc_cap};
   // per-chunk scratch: the recompute images of the tile kernel, then dL/dx [Dm] and the gate state [6H]
   const long long g_off = P.scratch_floats, cz_off = g_off + (long long)Dm * LD, chunk_stride = cz_off + 6LL * H * LD;
   float* const G = S.bufs[0];
@@ -1281,14 +1232,10 @@ static int long_bwd_grid(const Plan& P, const PmtBatch* batch) {
   if (grid > (size_t)batch->n_variants) grid = batch->n_variants;
   return grid < 1 ? 1 : (int)grid;
 }
-static long long* g_bwd_trace = nullptr;
-extern "C" int pmt_set_backward_trace(long long* device_buffer) {
-  g_bwd_trace = device_buffer;
-#ifdef PMT_GEMM_TRACE
-  cudaMemcpyToSymbol(pmt::g_gemm_trace, &device_buffer, sizeof(device_buffer));
-#endif
-  return 0;
-}
+// The backward kernels of a call: the tensor-core read-path and haplotype-CNN kernels (pmt_tc_bwd.cu, pmt_cnn_bwd.cu)
+// unless the FP32 mode is selected or the model is outside their envelope, the FP32 SIMT kernels otherwise.
+static bool bwd_reads_tc(const Plan& P) { return pmt_precision_mode() != PMT_PRECISION_FP32 && pmt_tc_supported(P); }
+static bool bwd_cnn_tc(const Plan& P) { return pmt_precision_mode() != PMT_PRECISION_FP32 && pmt_cnn_bwd_mma_supported(P); }
 
 size_t pmt_backward_workspace_bytes(const Plan& P, const PmtBatch* batch) {
   size_t bytes = 1024;
@@ -1305,10 +1252,8 @@ size_t pmt_backward_workspace_bytes(const Plan& P, const PmtBatch* batch) {
 extern "C" int pmt_backward_kernels(const PmtModelDesc* desc, int32_t* reads_tc, int32_t* cnn_tc) {
   Plan P;
   if (pmt_build_plan(desc, &P)) return 1;
-  const bool tc_mode = pmt_precision_mode() != PMT_PRECISION_FP32;
-  const char* cnn_env = getenv("PMT_CNN_BWD_SIMT");
-  if (reads_tc) *reads_tc = tc_mode && pmt_tc_supported(P) ? 1 : 0;
-  if (cnn_tc) *cnn_tc = tc_mode && pmt_cnn_bwd_mma_supported(P) && !(cnn_env && atoi(cnn_env) == 1) ? 1 : 0;
+  if (reads_tc) *reads_tc = bwd_reads_tc(P) ? 1 : 0;
+  if (cnn_tc) *cnn_tc = bwd_cnn_tc(P) ? 1 : 0;
   return 0;
 }
 
@@ -1338,15 +1283,12 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
   const int lgrid = long_bwd_grid(P, batch);
   const size_t long_floats = long_bwd_floats_per_cta(P, batch);
   float* long_scratch = reinterpret_cast<float*>(ws + off); off += (size_t)lgrid * long_floats * sizeof(float);
-  // Tile-sized sets go through the tensor-core backward (pmt_tc_bwd.cu) unless the FP32 mode is selected
-  const bool use_tc = pmt_precision_mode() != PMT_PRECISION_FP32 && pmt_tc_supported(P);
+  const bool use_tc = bwd_reads_tc(P);   // tile-sized sets; longer sets always take the SIMT long-set kernel
   off = (off + 255) & ~(size_t)255;
   unsigned char* tc_ws = reinterpret_cast<unsigned char*>(ws + off);
   const size_t tc_ws_bytes = use_tc ? pmt_tc_bwd_workspace_bytes(P, batch) + 1024 : 0;
   off += tc_ws_bytes;
-  // The haplotype CNN's backward follows the precision mode too: tensor-core kernel (pmt_cnn_bwd.cu) unless FP32 is selected
-  const char* cnn_env = getenv("PMT_CNN_BWD_SIMT");   // measurement: the FP32 SIMT kernel in every mode
-  const bool cnn_mma = pmt_precision_mode() != PMT_PRECISION_FP32 && pmt_cnn_bwd_mma_supported(P) && !(cnn_env && atoi(cnn_env) == 1);
+  const bool cnn_mma = bwd_cnn_tc(P);
   off = (off + 255) & ~(size_t)255;
   unsigned char* cnn_ws = reinterpret_cast<unsigned char*>(ws + off);
   const size_t cnn_ws_bytes = cnn_mma ? pmt_cnn_bwd_mma_workspace_bytes(P, batch) : 0;
@@ -1396,7 +1338,6 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
   A.d_info_seq = d_info_seq; A.scratch = scratch; A.scratch_stride = (long long)scr_floats; A.partials = partials;
   A.long_scratch = long_scratch; A.long_scratch_stride = (long long)long_floats;
   A.n_claims = (B + claim - 1) / claim;
-  A.trace = g_bwd_trace;
   int grid = A.n_claims < kBwdGrid ? A.n_claims : kBwdGrid;
   if (grid > n_sm) grid = n_sm;
   int tc_grid = 0;

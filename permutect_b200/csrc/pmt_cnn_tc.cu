@@ -107,11 +107,11 @@ struct Bars {
   int pad_;
 };
 
-template <int PASSES, bool TRACE, bool SAVE = false>
+template <int PASSES, bool SAVE>
 __global__ void __launch_bounds__(THREADS, 1)
 hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restrict__ image, const float* __restrict__ wflat,
                   const __grid_constant__ PmtModelDesc D, const void* __restrict__ haps, int hap_kind, long long hap_stride,
-                  int n_variants, float* __restrict__ info_seq, long long* __restrict__ trace,
+                  int n_variants, float* __restrict__ info_seq,
                   const __grid_constant__ SaveLayout SL, float* __restrict__ save) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   unsigned char* p = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -124,11 +124,6 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int lane = tid & 31;
   const int n_layers = TP.n_layers, n_items = TP.n_items, G = TP.G, L0 = TP.L0;
-  // optional cycle trace of CTA 0 (profiles/trace_cnn.py): entries of (event id, clock) per recording thread
-  int tr_n = 0;
-  const bool tr_on = trace != nullptr && blockIdx.x == 0 && lane == 0 && (warp == 0 || warp == 5 || warp == MMA_WARP);
-  long long* tr = trace + (warp == MMA_WARP ? 2 : (warp == 5 ? 1 : 0)) * 1024;
-  auto TR = [&](int id) { if (TRACE && tr_on && tr_n < 510) { tr[2 * tr_n] = id; tr[2 * tr_n + 1] = clock64(); ++tr_n; } };
 
   if (tid == 0) {
     for (int i = 0; i <= n_items; ++i) mbar_init(smem_addr(&S->done_bar[i]), EPI_WARPS);
@@ -180,10 +175,8 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
       int waited = 0;   // done_bar[0 .. waited) observed in this group
       for (int it = 0; it < n_items; ++it) {
         const ItemDev I = S->item[it];
-        TR(100 + it);
         for (; waited <= I.need; ++waited) mbar_wait(smem_addr(&S->done_bar[waited]), gpar);
         tc_fence_after();
-        TR(130 + it);
         if (elect_one()) {
           if (I.first) {
             if (I.N == 64) issue_first<64, PASSES>(I.count, I.d, I.a_hi, I.b);
@@ -194,7 +187,6 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
           mma_commit(smem_addr(&S->acc_bar[it]));
         }
         __syncwarp();
-        TR(160 + it);
       }
     }
   } else {
@@ -241,7 +233,6 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
     unsigned gpar = 0;
     for (int g = blockIdx.x; g < n_groups; g += gridDim.x, gpar ^= 1) {
       const int v0 = g * G, nv = min(G, n_variants - v0);
-      TR(1);
       // ---- im2col rows of the first conv (batch.py:115-130): zero this warp's rows, then scatter the ones ----
       for (int j = r_lo + lane; j < r_hi; j += 32) {
         const unsigned ra = act + j * 16;
@@ -250,7 +241,6 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
           if (pl < planes0) sts128(ra + pl * PLANE_BYTES, make_float4(0.f, 0.f, 0.f, 0.f));
       }
       __syncwarp();
-      TR(3);
 #pragma unroll
       for (int k = 0; k < MAX_TASKS; ++k) {
         if ((unsigned)codes[k] < 5u) {
@@ -258,11 +248,9 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
           sts_f32(t_row[k] + (col >> 2) * PLANE_BYTES + (col & 3) * 4, 1.f);
         }
       }
-      TR(4);
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_addr(&S->done_bar[0]));
-      TR(2);
       fetch_codes(g + gridDim.x);
 
       for (int it = 0; it < n_items; ++it) {
@@ -282,10 +270,8 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
         if (flags & F_POOL2) { valid = valid && !(pos & 1); pp = pos >> 1; }
         valid = valid && pp < L_pool;
         const float4 b0 = lds128(bias_a), b1 = lds128(bias_a + 16);
-        TR(200 + it);
         mbar_wait(smem_addr(&S->acc_bar[it]), gpar);
         tc_fence_after();
-        TR(230 + it);
         float x[8];
         {
           unsigned r[8], rl[8];
@@ -309,7 +295,6 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
             for (int i = 0; i < 8; ++i) x[i] = PASSES == 3 ? __uint_as_float(r[i]) + __uint_as_float(rl[i]) : __uint_as_float(r[i]);
           }
         }
-        TR(500 + it);
         tc_fence_before();   // the accumulator has been read: a later item may overwrite it once this warp has arrived
         if (flags & F_POOL2) {
 #pragma unroll
@@ -355,17 +340,13 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
               sts128(dst + BUF_BYTES + PLANE_BYTES, make_float4(x[4], x[5], x[6], x[7]));
             }
           }
-          TR(530 + it);
           asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-          TR(560 + it);
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(smem_addr(&S->done_bar[1 + it]));
-        TR(260 + it);
       }
     }
   }
-  if (TRACE && tr_on) tr[1022] = tr_n;
   tc_fence_before();
   __syncthreads();
   if (warp == MMA_WARP) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
@@ -553,15 +534,13 @@ size_t pmt_cnn_tc_image_bytes(const pmt::Plan& P) {
   return (size_t)T.image_bytes + 256;
 }
 
-template <int PASSES, bool TRACE>
-static int launch_cnn_tc(const cnntc::Plan& T, const unsigned char* image, const float* weights, const PmtModelDesc& D,
-                          const PmtBatch* batch, float* info_seq, int grid, long long* trace, cudaStream_t st) {
+template <int PASSES, bool SAVE>
+static int launch_cnn_tc(const cnntc::Plan& T, const unsigned char* image, const float* weights, const PmtModelDesc& D, const void* haps,
+                         const PmtBatch* batch, int n, float* info_seq, const SaveLayout& SL, float* save, int grid, cudaStream_t st) {
   const size_t smem = 2 * BUF_BYTES + T.image_bytes + MAX_LAYERS * 32 * sizeof(float) + sizeof(Bars) + 1024 + 64;
-  SaveLayout SL;
-  memset(&SL, 0, sizeof(SL));
-  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_tc_kernel<PASSES, TRACE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  hap_cnn_tc_kernel<PASSES, TRACE><<<grid, THREADS, smem, st>>>(T, image, weights, D, batch->haplotypes, batch->hap_kind, batch->hap_stride,
-                                                         batch->n_variants, info_seq, trace, SL, nullptr);
+  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_tc_kernel<PASSES, SAVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  hap_cnn_tc_kernel<PASSES, SAVE><<<grid, THREADS, smem, st>>>(T, image, weights, D, haps, batch->hap_kind, batch->hap_stride, n, info_seq,
+                                                               SL, save);
   return 0;
 }
 
@@ -584,7 +563,6 @@ void pmt_cnn_save_layout(const cnntc::Plan& T, SaveLayout* out) {
 // Training recompute: always the split-precision mode (the saved activations are the fp32-parity ones).
 int pmt_launch_cnn_tc_save(const pmt::Plan& P, const cnntc::Plan& T, const float* weights, const PmtBatch* batch, int v_first, int n,
                            float* info_seq, const unsigned char* image, float* save, int n_sm, cudaStream_t st) {
-  const size_t smem = 2 * BUF_BYTES + T.image_bytes + MAX_LAYERS * 32 * sizeof(float) + sizeof(Bars) + 1024 + 64;
   SaveLayout SL;
   pmt_cnn_save_layout(T, &SL);
   const int n_groups = (n + T.G - 1) / T.G;
@@ -592,10 +570,7 @@ int pmt_launch_cnn_tc_save(const pmt::Plan& P, const cnntc::Plan& T, const float
   const size_t esz = batch->hap_kind == PMT_I64 ? 8 : 2;
   const void* haps = reinterpret_cast<const unsigned char*>(batch->haplotypes) + (size_t)v_first * batch->hap_stride * esz;
   float* out = info_seq + (size_t)v_first * (P.d.d_info + P.d.d_seq);
-  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_tc_kernel<3, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  hap_cnn_tc_kernel<3, false, true><<<grid, THREADS, smem, st>>>(T, image, weights, P.d, haps, batch->hap_kind, batch->hap_stride, n, out,
-                                                                  nullptr, SL, save);
-  return 0;
+  return launch_cnn_tc<3, true>(T, image, weights, P.d, haps, batch, n, out, SL, save, grid, st);
 }
 
 int pmt_pack_cnn_tc_images(const pmt::Plan& P, const cnntc::Plan& T, const float* weights, unsigned char* image, cudaStream_t st) {
@@ -604,11 +579,6 @@ int pmt_pack_cnn_tc_images(const pmt::Plan& P, const cnntc::Plan& T, const float
 }
 
 // `image` is a 16-byte aligned device buffer of pmt_cnn_tc_image_bytes(P) bytes.
-static long long* g_cnn_trace = nullptr;
-// Measurement hook: device buffer of 3 x 1024 int64 that CTA 0 of the next tensor-core CNN launches fills with
-// (event, clock64) pairs; NULL disarms.
-extern "C" int pmt_set_cnn_trace(long long* device_buffer) { g_cnn_trace = device_buffer; return 0; }
-
 int pmt_launch_cnn_tc(const pmt::Plan& P, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
                       bool reuse_image, int n_sm, int mode, cudaStream_t st) {
   cnntc::Plan T;
@@ -616,12 +586,9 @@ int pmt_launch_cnn_tc(const pmt::Plan& P, const float* weights, const PmtBatch* 
   if (!reuse_image) pack_cnn_tc_kernel<<<dim3(T.n_layers, 16), 256, 0, st>>>(P.d, T, weights, image);
   const int n_groups = (batch->n_variants + T.G - 1) / T.G;
   const int grid = n_groups < n_sm ? n_groups : n_sm;
-  if (g_cnn_trace) {
-    if (mode == PMT_PRECISION_TF32) { if (launch_cnn_tc<1, true>(T, image, weights, P.d, batch, info_seq, grid, g_cnn_trace, st)) return 1; }
-    else { if (launch_cnn_tc<3, true>(T, image, weights, P.d, batch, info_seq, grid, g_cnn_trace, st)) return 1; }
-  } else {
-    if (mode == PMT_PRECISION_TF32) { if (launch_cnn_tc<1, false>(T, image, weights, P.d, batch, info_seq, grid, nullptr, st)) return 1; }
-    else { if (launch_cnn_tc<3, false>(T, image, weights, P.d, batch, info_seq, grid, nullptr, st)) return 1; }
-  }
-  return 0;
+  SaveLayout SL;
+  memset(&SL, 0, sizeof(SL));
+  return mode == PMT_PRECISION_TF32
+             ? launch_cnn_tc<1, false>(T, image, weights, P.d, batch->haplotypes, batch, batch->n_variants, info_seq, SL, nullptr, grid, st)
+             : launch_cnn_tc<3, false>(T, image, weights, P.d, batch->haplotypes, batch, batch->n_variants, info_seq, SL, nullptr, grid, st);
 }

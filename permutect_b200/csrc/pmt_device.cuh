@@ -159,26 +159,12 @@ struct Stage {
 enum EpilogueFlags { EPI_STORE = 0, EPI_SELU = 1, EPI_ACC = 2, EPI_DSELU = 4 };
 constexpr int EPI_RESIDUAL = EPI_ACC;
 
-#ifdef PMT_GEMM_TRACE   // experiment builds only: clocks of warp 0 inside the tile GEMM (ids 300..303)
-static __device__ long long* g_gemm_trace = nullptr;
-#define PMT_GEMM_TRACE_POINT(id)                                                                       \
-  do {                                                                                                 \
-    if (g_gemm_trace && threadIdx.x == 0 && blockIdx.x == 0 && g_gemm_trace[511] == 1) {                                  \
-      const long long n_ = g_gemm_trace[0];                                                            \
-      if (n_ < 250) { g_gemm_trace[1 + 2 * n_] = (id); g_gemm_trace[2 + 2 * n_] = clock64(); g_gemm_trace[0] = n_ + 1; } \
-    }                                                                                                  \
-  } while (0)
-#else
-#define PMT_GEMM_TRACE_POINT(id)
-#endif
-
 template <int NT>
 __device__ __noinline__ void gemm_tile_nt(unsigned x_s, int K, int N, int G, bool dual, int b_off, int b_alt_off,
                                           unsigned img_s, const float* __restrict__ wflat, int ref_rows_padded,
                                           unsigned y_s, int flags, float alpha, unsigned act_s, int rows_used) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int r0 = lane * 4;
-  PMT_GEMM_TRACE_POINT(300);
   if (r0 >= rows_used) return;
   const bool is_alt = dual && (r0 >= ref_rows_padded);
   const int wstride = G * GROUP_STRIDE * 4;  // bytes
@@ -194,7 +180,6 @@ __device__ __noinline__ void gemm_tile_nt(unsigned x_s, int K, int N, int G, boo
     }
     unsigned xp = x_s + r0 * 4;
     unsigned wp = wimg + g * GROUP_STRIDE * 4;
-    PMT_GEMM_TRACE_POINT(301);
 #pragma unroll 4
     for (int k = 0; k < K; ++k) {
       const float4 x = lds128(xp);
@@ -215,7 +200,6 @@ __device__ __noinline__ void gemm_tile_nt(unsigned x_s, int K, int N, int G, boo
         acc[3][j] = fmaf(x.w, w[j], acc[3][j]);
       }
     }
-    PMT_GEMM_TRACE_POINT(302);
 #pragma unroll
     for (int j = 0; j < NT; ++j) {
       const int n = g * NT + j;
@@ -237,7 +221,6 @@ __device__ __noinline__ void gemm_tile_nt(unsigned x_s, int K, int N, int G, boo
         sts128(y_s + off, v);
       }
     }
-    PMT_GEMM_TRACE_POINT(303);
   }
 }
 

@@ -51,10 +51,10 @@ __device__ __forceinline__ int ld_acquire_gpu(const int* p) {
   return v;
 }
 
-template <int PASSES, bool TRACE, bool SAVE, bool LONG = false>
+template <int PASSES, bool SAVE, bool LONG>
 __global__ void __launch_bounds__(FWD_THREADS, 1)
 reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_constant__ TcPlan TP, const __grid_constant__ TcArgs A,
-                        int n_stages, int stage_bytes, long long* __restrict__ trace) {
+                        int n_stages, int stage_bytes) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   // carve: [weight ring: n_stages x stage_bytes][xch 2 slots][sums 2 slots][pair exchange][block scalars][HeadConst][Shared]
   unsigned char* p = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -70,12 +70,6 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
   const int tid = threadIdx.x;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const float* W = A.wflat;
-  // optional cycle trace of CTA 0 (profiles/trace_reads.py): (event id, clock) pairs of four recording threads
-  int tr_n = 0;
-  const int tr_w = warp == 0 ? 0 : (warp == 8 ? 1 : (warp == MMA_WARP ? 2 : (warp == MMA_WARP + 1 ? 3 : -1)));
-  const bool tr_on = TRACE && trace != nullptr && blockIdx.x == 0 && (tid & 31) == 0 && tr_w >= 0;
-  long long* tr = trace + (tr_w < 0 ? 0 : tr_w) * 2048;
-  auto TR = [&](int id) { if (TRACE && tr_on && tr_n < 1020) { tr[2 * tr_n] = id; tr[2 * tr_n + 1] = clock64(); ++tr_n; } };
   if (tid == 0) {
     for (int s = 0; s < 2; ++s) {
       mbar_init(smem_addr(&S->bar_a[s]), 8); mbar_init(smem_addr(&S->bar_d[s]), 1);
@@ -310,11 +304,9 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
         const unsigned kb_stride16 = (unsigned)(oN * 128) >> 4;
         const bool lo_pass = step > 0 || l0_lo;
         const unsigned d = tb + (o_dst_x ? COL_X : COL_Z);
-        TR(100 + step);
         mbar_wait(smem_addr(&S->wfull[stage]), wparity);
         mbar_wait(bar_a, aparity);
         tc_fence_after();
-        TR(200 + step);
         if (elect_one()) {
           switch (oKS) {
             case 3: issue_chain<3, PASSES>(d, tb + COL_AHI, tb + COL_ALO, b_hi, b_lo, kb_stride16, idesc, o_dst_x, lo_pass); break;
@@ -325,7 +317,6 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
           mma_commit(smem_addr(&S->wfree[stage]));
         }
         __syncwarp();
-        TR(300 + step);
         aparity ^= 1;
         if (++stage == n_stages) { stage = 0; wparity ^= 1; }
       }
@@ -367,11 +358,9 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
       const int my_var = rv == 255 ? -1 : rv;
       const bool is_alt = row >= ref_pad;
 
-      TR(1);
       for (int step = 0; step < n_steps; ++step) {
         const int epi = TP.step[step].epi;
         unsigned char* const scr_op = (SAVE && scr) ? scr + TP.step[step].scr_off : nullptr;
-        TR(400 + step);
         switch (epi) {
           case EPI_DECODE: {   // batch.py:51-56, plain_text_data.py:510-511 (quirk Q2: the uint8 de-quantisation wraps)
             float v[32];
@@ -526,7 +515,6 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
               for (int i = 0; i < 16; ++i) z2s[i] = __uint_as_float(r2[i]);
             }
             // z1s[j] = z1[k0 + j] (j < 6), z2s[k] = z2[k] (k < 12; columns >= H are zero)
-            TR(800 + step);
             const int k0 = half * 6;
             float z2[12];
 #pragma unroll
@@ -561,9 +549,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
             float z1a[6];
 #pragma unroll
             for (int j = 0; j < 6; ++j) z1a[j] = SELU_SCALE * selu_u(z1s[j]);
-            TR(900 + step);
             named_barrier(slot_bar, 256);
-            TR(1000 + step);
             if (LONG) {   // mean fields of a set spread over many tiles (pmt_tc.cuh: LongTile)
               const float regw = lds_f32(bcs + BC_REGW * 4);
               const int blk = TP.step[step].blk, nb = D.n_blocks;
@@ -643,9 +629,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
                 }
               }
             }
-            TR(1100 + step);
             named_barrier(slot_bar, 256);
-            TR(1200 + step);
             // proj2 operand columns of this thread: [t_ref (6) | t_alt (6)]; the second thread's last two hidden
             // slots (k = 10 would be unit 11; MAXH = 11 -> slot 5 of half 1 is unit 11 < MAXH only if H = 11)
             // layout, half 0: [t_ref k 0..5 | t_alt k 0..5]; half 1: [t_ref k 6..10 | t_alt k 6..10 | is_ref, is_alt]
@@ -690,34 +674,28 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
           case EPI_COPY_X64: {
             float v[32];
             load_cols<32>((epi == EPI_ACT_Z64 ? t_z : t_x) + half * 32, v);
-            TR(1300 + step);
             if (epi != EPI_COPY_X64) {
 #pragma unroll
               for (int i = 0; i < 32; ++i) v[i] = selu_u(v[i]);
             }
             if (half == 0) v[31] = 1.f;
-            TR(1400 + step);
             if (SAVE && scr_op) save_operand<32>(scr_op, row, half * 32, v);
             store_operand<32, PASSES>(t_hi + half * 32, t_lo + half * 32, v, true);
           } break;
         }
         // ---- hand the operand to the MMA warp, wait for the accumulator ----
-        TR(500 + step);
         tmem_wait_st();
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(bar_a);
-        TR(600 + step);
         mbar_wait(bar_d, dparity);
         dparity ^= 1;
         tc_fence_after();
-        TR(700 + step);
       }
 
       // ---------------- clustering head (rotation folded into the last layer; feature_clustering.py:82-135) ----------------
       // Both threads of a row hold its features.  half 0: feature rows for the set means, the non-artifact term and the
       // even clusters; half 1: the outlier term and the odd clusters.
-      TR(2);
       float f[MAXE];
       load_cols<MAXE>(t_z, f);
       if (half == 0) {
@@ -755,9 +733,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
           sts_f32(xch + ((MAXE + 2 + k) * XCH_LD + row) * 4, ll_orth + ll_par);
         }
       }
-      TR(3);
       named_barrier(slot_bar, 256);
-      TR(4);
       // ---- per-variant sums and outputs (ragged_sets.py:144-158; artifact_model.py:291-292) ----
       if (LONG) {
         // This tile's raw sums (features of its side; for an alt tile also the K + 2 log-likelihood terms) go to its slot of
@@ -889,12 +865,10 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
         }
       }
       }   // !LONG
-      TR(5);
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_addr(&S->meta_free[slot][round & 1]));   // the tile's tables may be refilled
     }
   }
-  if (TRACE && tr_on) tr[2046] = tr_n;
   tc_fence_before();
   __syncthreads();
   if (warp == MMA_WARP) {
@@ -1377,11 +1351,6 @@ size_t pmt_tc_tiles_bytes(const PmtBatch* batch) {
   return tiles_bytes(B) + perm_bytes(B) + 256;
 }
 
-static long long* g_reads_trace = nullptr;
-// Measurement hook: device buffer of 4 x 2048 int64 that CTA 0 of the next tensor-core read-kernel launches fills
-// with (event, clock64) pairs; NULL disarms.
-extern "C" int pmt_set_reads_trace(long long* device_buffer) { g_reads_trace = device_buffer; return 0; }
-
 static int plan_claim_variants(int n_variants, int n_sm) {
   // planner claims: large enough that the partial last tile of a claim is a small loss, small enough that a small
   // batch is planned by many warps (each claim is walked sequentially)
@@ -1416,8 +1385,10 @@ int pmt_plan_tiles(const PmtBatch* batch, int max_variants, bool deterministic, 
   return 0;
 }
 
-template <int PASSES>
-static int launch_tc(const PmtModelDesc& D, const TcPlan& T, const TcArgs& A, int grid, cudaStream_t st) {
+// Sizes the weight ring (as many stages as fit next to the fixed carve, at most NS_MAX) and launches one instantiation
+// of the read kernel.
+template <int PASSES, bool SAVE, bool LONG>
+static int launch_reads_tc(const PmtModelDesc& D, const TcPlan& T, const TcArgs& A, int grid, cudaStream_t st) {
   const int stage_bytes = PASSES == 3 ? T.slot_bytes : T.slot_bytes / 2;
   const size_t fixed = 2 * XCH_ROWS * XCH_LD * sizeof(float) + 2 * SUMS_FLOATS * sizeof(float) + 2 * 2 * TILE * 2 * sizeof(float) +
                        PMT_MAX_BLOCKS * BC_STRIDE * sizeof(float) + sizeof(HeadConstTc) + sizeof(Shared) + 1024 + 64;
@@ -1425,13 +1396,8 @@ static int launch_tc(const PmtModelDesc& D, const TcPlan& T, const TcArgs& A, in
   if (n_stages > NS_MAX) n_stages = NS_MAX;
   PMT_CHECK(n_stages >= 2, "tensor-core forward: weight ring does not fit in shared memory");
   const size_t smem = fixed + (size_t)n_stages * stage_bytes;
-  if (g_reads_trace) {
-    PMT_CUDA(cudaFuncSetAttribute(reads_forward_tc_kernel<PASSES, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    reads_forward_tc_kernel<PASSES, true, false><<<grid, FWD_THREADS, smem, st>>>(D, T, A, n_stages, stage_bytes, g_reads_trace);
-  } else {
-    PMT_CUDA(cudaFuncSetAttribute(reads_forward_tc_kernel<PASSES, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    reads_forward_tc_kernel<PASSES, false, false><<<grid, FWD_THREADS, smem, st>>>(D, T, A, n_stages, stage_bytes, nullptr);
-  }
+  PMT_CUDA(cudaFuncSetAttribute(reads_forward_tc_kernel<PASSES, SAVE, LONG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  reads_forward_tc_kernel<PASSES, SAVE, LONG><<<grid, FWD_THREADS, smem, st>>>(D, T, A, n_stages, stage_bytes);
   return 0;
 }
 
@@ -1442,16 +1408,7 @@ int pmt_launch_pack_tc(const Plan& P, const TcPlan& T, const float* weights, uns
 
 // Training recompute (always the split-precision mode: the saved activations are the fp32-parity ones).
 int pmt_launch_reads_tc_save(const Plan& P, const TcPlan& T, const TcArgs& A, int grid, cudaStream_t st) {
-  const int stage_bytes = T.slot_bytes;
-  const size_t fixed = 2 * XCH_ROWS * XCH_LD * sizeof(float) + 2 * SUMS_FLOATS * sizeof(float) + 2 * 2 * TILE * 2 * sizeof(float) +
-                       PMT_MAX_BLOCKS * BC_STRIDE * sizeof(float) + sizeof(HeadConstTc) + sizeof(Shared) + 1024 + 64;
-  int n_stages = (int)((227 * 1024 - fixed) / stage_bytes);
-  if (n_stages > NS_MAX) n_stages = NS_MAX;
-  PMT_CHECK(n_stages >= 2, "tensor-core forward: weight ring does not fit in shared memory");
-  const size_t smem = fixed + (size_t)n_stages * stage_bytes;
-  PMT_CUDA(cudaFuncSetAttribute(reads_forward_tc_kernel<3, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  reads_forward_tc_kernel<3, false, true><<<grid, FWD_THREADS, smem, st>>>(P.d, T, A, n_stages, stage_bytes, nullptr);
-  return 0;
+  return launch_reads_tc<3, true, false>(P.d, T, A, grid, st);
 }
 
 // Launches the tile planner, the weight packer (unless the images in `image_buf` are still valid) and the tensor-core
@@ -1489,7 +1446,8 @@ int pmt_launch_reads_tc(const Plan& P, const float* weights, const PmtBatch* bat
   int grid = est_tiles < n_sm ? (int)est_tiles : n_sm;
   if (grid < 1) grid = 1;
   pmt_profile_begin(st);
-  const int rc = mode == PMT_PRECISION_TF32 ? launch_tc<1>(P.d, T, A, grid, st) : launch_tc<3>(P.d, T, A, grid, st);
+  const int rc = mode == PMT_PRECISION_TF32 ? launch_reads_tc<1, false, false>(P.d, T, A, grid, st)
+                                         : launch_reads_tc<3, false, false>(P.d, T, A, grid, st);
   pmt_profile_end(st);
   return rc;
 }
@@ -1541,20 +1499,6 @@ size_t pmt_tc_long_bytes(const Plan& P, const PmtBatch* batch) {
   return long_layout(P, batch, &L) ? L.end + 1024 : 0;
 }
 
-template <int PASSES>
-static int launch_tc_long(const PmtModelDesc& D, const TcPlan& T, const TcArgs& A, int grid, cudaStream_t st) {
-  const int stage_bytes = PASSES == 3 ? T.slot_bytes : T.slot_bytes / 2;
-  const size_t fixed = 2 * XCH_ROWS * XCH_LD * sizeof(float) + 2 * SUMS_FLOATS * sizeof(float) + 2 * 2 * TILE * 2 * sizeof(float) +
-                       PMT_MAX_BLOCKS * BC_STRIDE * sizeof(float) + sizeof(HeadConstTc) + sizeof(Shared) + 1024 + 64;
-  int n_stages = (int)((227 * 1024 - fixed) / stage_bytes);
-  if (n_stages > NS_MAX) n_stages = NS_MAX;
-  PMT_CHECK(n_stages >= 2, "tensor-core forward: weight ring does not fit in shared memory");
-  const size_t smem = fixed + (size_t)n_stages * stage_bytes;
-  PMT_CUDA(cudaFuncSetAttribute(reads_forward_tc_kernel<PASSES, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  reads_forward_tc_kernel<PASSES, false, false, true><<<grid, FWD_THREADS, smem, st>>>(D, T, A, n_stages, stage_bytes, nullptr);
-  return 0;
-}
-
 // The sets plan_tiles_kernel left out, on the same tensor-core pipeline (the weight images in `image_buf` must be packed:
 // call after pmt_launch_reads_tc).  Every CTA of the grid has to be resident (a tile waits for the other tiles of its
 // set): one CTA per SM, grid = number of SMs.
@@ -1588,5 +1532,6 @@ int pmt_launch_reads_tc_long(const Plan& P, const float* weights, const PmtBatch
   A.lng.mf_part = reinterpret_cast<float*>(base + L.mf_part);
   A.lng.fin_part = reinterpret_cast<float*>(base + L.fin_part);
   const int grid = L.R / 2;
-  return mode == PMT_PRECISION_TF32 ? launch_tc_long<1>(P.d, T, A, grid, st) : launch_tc_long<3>(P.d, T, A, grid, st);
+  return mode == PMT_PRECISION_TF32 ? launch_reads_tc<1, false, true>(P.d, T, A, grid, st)
+                                     : launch_reads_tc<3, false, true>(P.d, T, A, grid, st);
 }

@@ -2,7 +2,7 @@
 // tile-sized read sets (misc_utils.py:125-127 calls loss.backward() through exactly these layers).
 //
 // Two kernels per range of tiles:
-//   reads_forward_tc_kernel<3, ., SAVE>  (pmt_tc.cu) recomputes the forward and leaves every layer's operand in global
+//   reads_forward_tc_kernel<3, SAVE>     (pmt_tc.cu) recomputes the forward and leaves every layer's operand in global
 //       memory as PANELS (pmt_tc.cuh): the layout an MN-major tf32 operand of tcgen05.mma must have
 //   reads_backward_tc_kernel             walks the layers in reverse.  Same organisation as the forward: one persistent
 //       CTA per SM, two tiles of 128 reads in flight, 16 epilogue warps (two threads per read), one MMA-issuer warp per
@@ -114,10 +114,9 @@ __device__ __forceinline__ void flush_dw(unsigned t_w, float* __restrict__ part,
   }
 }
 
-template <bool TRACE>
 __global__ void __launch_bounds__(THREADS, 1)
 reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_constant__ TcPlan TP, const __grid_constant__ TcBwdArgs A,
-                         int n_stages, int stage_bytes, long long* __restrict__ trace) {
+                         int n_stages, int stage_bytes) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   // carve: [operand buffers 2 slots][weight ring][xch 2 slots][3 per-variant tables x 2 slots][pair exchange][block scalars][HeadConst][SharedB]
   unsigned char* p = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -134,11 +133,6 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
   const int lane = tid & 31;
   const float* W = A.wflat;
-  int tr_n = 0;
-  const int tr_w = warp == 0 ? 0 : (warp == 8 ? 1 : (warp == MMA_WARP ? 2 : (warp == MMA_WARP + 1 ? 3 : -1)));
-  const bool tr_on = TRACE && trace != nullptr && blockIdx.x == 0 && lane == 0 && tr_w >= 0;
-  long long* tr = trace + (tr_w < 0 ? 0 : tr_w) * 2048;
-  auto TR = [&](int id) { if (TRACE && tr_on && tr_n < 1020) { tr[2 * tr_n] = id; tr[2 * tr_n + 1] = clock64(); ++tr_n; } };
   if (tid == 0) {
     for (int s = 0; s < 2; ++s) {
       mbar_init(smem_addr(&S->bar_a[s]), 8); mbar_init(smem_addr(&S->bar_d[s]), 1); mbar_init(smem_addr(&S->bar_w[s]), 1);
@@ -223,12 +217,10 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
       for (int step = n_steps - 1; step >= 0; --step) {
         const TcStep& o = TP.step[step];
         const int oN = o.N, oNd = o.Nd, oKSd = o.KSd;
-        TR(100 + step);
         if (step > 0) mbar_wait(smem_addr(&S->wfull[stage]), wparity);
         mbar_wait(bar_a, aparity);
         aparity ^= 1;
         tc_fence_after();
-        TR(200 + step);
         if (elect_one()) {
           if (step > 0) {   // data gradient: D[128 x Nd] = dY[128 x N] . W^T image
             const unsigned idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((unsigned)(oNd >> 3) << 17) | ((128u >> 4) << 24);
@@ -249,7 +241,6 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
         mbar_wait(act_full, fparity);
         fparity ^= 1;
         tc_fence_after();
-        TR(300 + step);
         if (elect_one()) {   // weight gradient: DW[m][n] = sum over the tile's rows of operand[r][m] * dY[r][n]
           const unsigned idesc = (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (1u << 16) | ((unsigned)(oN >> 3) << 17) | ((128u >> 4) << 24);
 #pragma unroll
@@ -259,7 +250,6 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
           mma_commit(act_free);
         }
         __syncwarp();
-        TR(350 + step);
       }
     }
   } else {
@@ -320,7 +310,6 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
       const int owner_row = my_ref_cnt > 0 ? (int)lds_u8(m_ref_start + mv) : (int)lds_u8(m_alt_start + mv);   // one row per variant
       const long long vg = (long long)v0 + mv;
 
-      TR(1);
       for (int step = n_steps - 1; step >= -1; --step) {
         // E(step): dL/d(output of `step`) from the data gradient of step + 1; step == -1 only drains the pipeline
         const int bepi = step >= 0 ? TP.step[step].bepi : -1;
@@ -328,13 +317,11 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
         float dy[32];
 #pragma unroll
         for (int i = 0; i < 32; ++i) dy[i] = 0.f;
-        TR(400 + step);
         if (!first) {
           mbar_wait(bar_d, dparity); dparity ^= 1;
           mbar_wait(act_full, fparity); fparity ^= 1;
           tc_fence_after();
         }
-        TR(500 + step);
         switch (bepi) {
           case BE_HEAD: {   // feature_clustering.py:82-135 and the set means (artifact_model.py:291-292) in reverse
             const bool live = is_alt && real;
@@ -625,7 +612,6 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
           } break;
           default: break;
         }
-        TR(600 + step);
         if (!first) {
           // the operand of step + 1 has been read; its weight gradient must have left shared memory and TMEM before
           // this step's dY and dW overwrite them
@@ -636,7 +622,6 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
           const TcStep& prev = TP.step[step + 1];
           flush_dw(t_w, part + prev.part_off, prev.N, prev.kw, quarter, half, lane);
         }
-        TR(700 + step);
         if (step < 0) break;
         switch (bepi) {
           case BE_HEAD: if (half == 0) store_dy<16>(t_dy, dy_s, row, 0, dy); break;
@@ -652,11 +637,9 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(bar_a);
-        TR(800 + step);
       }
     }
   }
-  if (TRACE && tr_on) tr[2046] = tr_n;
   tc_fence_before();
   __syncthreads();
   if (warp == MMA_WARP) {
@@ -965,9 +948,6 @@ size_t pmt_tc_bwd_workspace_bytes(const Plan& P, const PmtBatch* batch) {
   return bwd_layout(T, batch, kMaxGrid).total;
 }
 
-static long long* g_bwd_tc_trace = nullptr;
-void pmt_set_backward_tc_trace(long long* device_buffer) { g_bwd_tc_trace = device_buffer; }
-
 // Backward of the tile-sized read sets: writes d_info_seq for the variants of those sets and leaves the weight gradients
 // in the private buffers of the workspace; pmt_finish_reads_tc_backward adds them to d_weights.
 int pmt_launch_reads_tc_backward(const Plan& P, const float* weights, const PmtBatch* batch, const float* info_seq,
@@ -1014,8 +994,7 @@ int pmt_launch_reads_tc_backward(const Plan& P, const float* weights, const PmtB
   if (n_stages > NS_MAX) n_stages = NS_MAX;
   PMT_CHECK(n_stages >= 2, "tensor-core backward: weight ring does not fit in shared memory");
   const size_t smem = fixed + (size_t)n_stages * stage_bytes;
-  if (g_bwd_tc_trace) PMT_CUDA(cudaFuncSetAttribute(reads_backward_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  else PMT_CUDA(cudaFuncSetAttribute(reads_backward_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  PMT_CUDA(cudaFuncSetAttribute(reads_backward_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 
   PmtOutputs no_out;
   memset(&no_out, 0, sizeof(no_out));
@@ -1031,8 +1010,7 @@ int pmt_launch_reads_tc_backward(const Plan& P, const float* weights, const PmtB
     F.tile_limit = Bk.tile_limit = (c + 1) * L.chunk_tiles;
     if (saved) Bk.scratch = scratch + (size_t)Bk.tile_first * T.tile_bytes;   // the kernel indexes a pass's scratch from its first tile
     else if (pmt_launch_reads_tc_save(P, T, F, grid, st)) return 1;
-    if (g_bwd_tc_trace) reads_backward_tc_kernel<true><<<grid, THREADS, smem, st>>>(P.d, T, Bk, n_stages, stage_bytes, g_bwd_tc_trace);
-    else reads_backward_tc_kernel<false><<<grid, THREADS, smem, st>>>(P.d, T, Bk, n_stages, stage_bytes, nullptr);
+    reads_backward_tc_kernel<<<grid, THREADS, smem, st>>>(P.d, T, Bk, n_stages, stage_bytes);
   }
   pmt_profile_end(st);
   *grid_out = grid;

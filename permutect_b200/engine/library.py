@@ -92,7 +92,7 @@ class PmtLossGrads(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("g_supervised_b", "g_unsupervised_b", "g_alt_count_b", "g_source_b", "g_total_b")]
 
 
-EXPORTED_SYMBOLS = ["pmt_posterior_fit_step", "pmt_posterior_fit_workspace_size", "pmt_orthogonal_forward", "pmt_orthogonal_backward", "pmt_posterior_param_count", "pmt_posterior_log_posteriors", "pmt_dataset_read_indices", "pmt_pack_posterior", "pmt_adamw_step", "pmt_adamw_workspace_size", "pmt_losses_forward", "pmt_losses_backward", "pmt_losses_workspace_size", "pmt_set_cnn_trace", "pmt_set_reads_trace", "pmt_set_backward_trace", "pmt_last_error", "pmt_abi_version", "pmt_workspace_size", "pmt_forward", "pmt_forward_prepared", "pmt_backward",
+EXPORTED_SYMBOLS = ["pmt_posterior_fit_step", "pmt_posterior_fit_workspace_size", "pmt_orthogonal_forward", "pmt_orthogonal_backward", "pmt_posterior_param_count", "pmt_posterior_log_posteriors", "pmt_dataset_read_indices", "pmt_pack_posterior", "pmt_adamw_step", "pmt_adamw_workspace_size", "pmt_losses_forward", "pmt_losses_backward", "pmt_losses_workspace_size", "pmt_last_error", "pmt_abi_version", "pmt_workspace_size", "pmt_forward", "pmt_forward_prepared", "pmt_backward",
                     "pmt_decode_reads", "pmt_set_profile_events", "pmt_downsample_counts", "pmt_downsample_fill", "pmt_set_precision", "pmt_get_precision", "pmt_constraints_forward", "pmt_constraints_backward", "pmt_backward_kernels", "pmt_train_saved_bytes", "pmt_forward_train"]
 
 class PmtPosteriorDesc(C.Structure):
@@ -193,12 +193,6 @@ def load():
     lib.pmt_adamw_step.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_float,
                                    C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_size_t,
                                    C.c_void_p]
-    lib.pmt_set_reads_trace.restype = C.c_int
-    lib.pmt_set_reads_trace.argtypes = [C.c_void_p]
-    lib.pmt_set_cnn_trace.restype = C.c_int
-    lib.pmt_set_cnn_trace.argtypes = [C.c_void_p]
-    lib.pmt_set_backward_trace.restype = C.c_int
-    lib.pmt_set_backward_trace.argtypes = [C.c_void_p]
     lib.pmt_losses_forward.restype = C.c_int
     lib.pmt_losses_forward.argtypes = [C.POINTER(PmtLossDesc), C.c_void_p, C.POINTER(PmtLossBatch), C.POINTER(PmtLossOutputs),
                                        C.c_void_p]
