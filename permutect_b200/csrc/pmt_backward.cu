@@ -18,7 +18,7 @@
 #define PMT_NTHREADS 256
 #endif
 #include "pmt_cnn.cuh"
-#include "pmt_host.h"
+#include "pmt_call.h"
 #include "pmt_tile.cuh"
 
 namespace pmt {
@@ -1147,9 +1147,8 @@ static int pad_ld(int n) {   // smallest ld >= n + 12 with ld == 4 (mod 32)
   return ld;
 }
 
-int pmt_launch_cnn_backward(const Plan& P, const CnnGeom& G, const float* weights, const float* image,
-                            const PmtBatch* batch, const float* d_info_seq, float* partials, int n_partials,
-                            cudaStream_t st) {
+static int launch_cnn_backward(const Plan& P, const CnnGeom& G, const float* weights, const float* image, const PmtBatch* batch,
+                               const float* d_info_seq, float* partials, cudaStream_t st) {
   CnnBwdGeom Gb;
   const PmtModelDesc& d = P.d;
   const int ns = G.n_spatial;
@@ -1196,7 +1195,7 @@ int pmt_launch_cnn_backward(const Plan& P, const CnnGeom& G, const float* weight
   PMT_CHECK(vt >= 1, "haplotype CNN backward does not fit in shared memory");
   const int B = batch->n_variants;
   int grid = (B + vt - 1) / vt;
-  if (grid > n_partials) grid = n_partials;
+  if (grid > PMT_PARTIAL_CTAS) grid = PMT_PARTIAL_CTAS;
   PMT_CUDA(cudaFuncSetAttribute(hap_cnn_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   hap_cnn_backward_kernel<<<grid, NTHREADS, smem, st>>>(P, G, Gb, weights, image + P.img_total, batch->haplotypes,
                                                         batch->hap_kind, batch->hap_stride, B, d_info_seq, partials);
@@ -1214,8 +1213,6 @@ static int info_rows(const Plan& P) {
   for (int i = 0; i < P.d.n_info_ops; ++i) if (P.d.info_ops[i].out_dim > r) r = P.d.info_ops[i].out_dim;
   return r;
 }
-static const int kBwdGrid = 148;
-
 // Long-set kernel: every chunk of the longest set has its own recompute scratch + dL/dx + gate state (see the kernel).
 // The grid shrinks when the scratch of a full grid would pass kLongScratchBudget.
 static const size_t kLongScratchBudget = (size_t)16 << 30;
@@ -1228,106 +1225,103 @@ static int long_bwd_grid(const Plan& P, const PmtBatch* batch) {
   const size_t per_cta = long_bwd_floats_per_cta(P, batch) * sizeof(float);
   if (per_cta == 0) return 0;
   size_t grid = kLongScratchBudget / per_cta;
-  if (grid > (size_t)kBwdGrid) grid = kBwdGrid;
+  if (grid > (size_t)PMT_PARTIAL_CTAS) grid = PMT_PARTIAL_CTAS;
   if (grid > (size_t)batch->n_variants) grid = batch->n_variants;
   return grid < 1 ? 1 : (int)grid;
 }
-// The backward kernels of a call: the tensor-core read-path and haplotype-CNN kernels (pmt_tc_bwd.cu, pmt_cnn_bwd.cu)
-// unless the FP32 mode is selected or the model is outside their envelope, the FP32 SIMT kernels otherwise.
-static bool bwd_reads_tc(const Plan& P) { return pmt_precision_mode() != PMT_PRECISION_FP32 && pmt_tc_supported(P); }
-static bool bwd_cnn_tc(const Plan& P) { return pmt_precision_mode() != PMT_PRECISION_FP32 && pmt_cnn_bwd_mma_supported(P); }
 
-size_t pmt_backward_workspace_bytes(const Plan& P, const PmtBatch* batch) {
-  size_t bytes = 1024;
-  bytes += (size_t)kBwdGrid * P.d.n_params * sizeof(float);                                  // partials
-  const size_t scr = P.scratch_floats > P.info_scratch_floats ? P.scratch_floats : P.info_scratch_floats;
-  bytes += (size_t)kBwdGrid * scr * sizeof(float);                                           // activation scratch
-  if (batch) bytes += 2 * (size_t)batch->n_variants * (P.d.d_info + P.d.d_seq) * sizeof(float);   // info_seq, d_info_seq
-  bytes += (size_t)long_bwd_grid(P, batch) * long_bwd_floats_per_cta(P, batch) * sizeof(float) + 256;
-  if (pmt_tc_supported(P)) bytes += pmt_tc_bwd_workspace_bytes(P, batch) + 1024;
-  bytes += pmt_cnn_bwd_mma_workspace_bytes(P, batch) + 256;
-  return bytes;
+// Workspace layout of the backward:
+//   [256 B][SIMT images][partials][activation scratch][info_seq][d_info_seq] | [long-set scratch][tensor-core read-path
+//   backward][tensor-core CNN backward]
+struct BwdWsLayout {
+  size_t image, partials, scratch, info_seq, d_info_seq, long_scratch, tc, tc_bytes, cnn, cnn_bytes, end;
+  size_t scr_floats, long_floats;
+  int long_grid;
+};
+static BwdWsLayout backward_layout(const CallPlan& C, const PmtBatch* batch) {
+  const Plan& P = C.P;
+  const size_t w = batch ? (size_t)batch->n_variants * (P.d.d_info + P.d.d_seq) * sizeof(float) : 0;
+  BwdWsLayout L;
+  L.scr_floats = P.scratch_floats > P.info_scratch_floats ? P.scratch_floats : P.info_scratch_floats;
+  L.long_grid = long_bwd_grid(P, batch);
+  L.long_floats = long_bwd_floats_per_cta(P, batch);
+  size_t off = 256;
+  L.image = off; off += pmt_image_bytes(P, C.G); off = (off + 255) & ~(size_t)255;
+  L.partials = off; off += (size_t)PMT_PARTIAL_CTAS * P.d.n_params * sizeof(float);
+  L.scratch = off; off += (size_t)PMT_PARTIAL_CTAS * L.scr_floats * sizeof(float);
+  L.info_seq = off; off += w;
+  L.d_info_seq = off; off += w; off = (off + 255) & ~(size_t)255;
+  L.long_scratch = off; off += (size_t)L.long_grid * L.long_floats * sizeof(float); off = (off + 255) & ~(size_t)255;
+  L.tc_bytes = C.bwd_reads_tc ? C.tc_bwd.total + 1024 : 0;
+  L.tc = off; off += L.tc_bytes; off = (off + 255) & ~(size_t)255;
+  L.cnn_bytes = C.bwd_cnn_tc ? pmt_cnn_bwd_workspace_bytes(C, batch) : 0;
+  L.cnn = off; off += L.cnn_bytes;
+  L.end = off;
+  return L;
 }
+size_t pmt_backward_workspace_size(const CallPlan& C, const PmtBatch* batch) { return backward_layout(C, batch).end; }
 
 extern "C" int pmt_backward_kernels(const PmtModelDesc* desc, int32_t* reads_tc, int32_t* cnn_tc) {
-  Plan P;
-  if (pmt_build_plan(desc, &P)) return 1;
-  if (reads_tc) *reads_tc = bwd_reads_tc(P) ? 1 : 0;
-  if (cnn_tc) *cnn_tc = bwd_cnn_tc(P) ? 1 : 0;
+  CallPlan C;
+  if (pmt_call_plan(desc, nullptr, false, &C)) return 1;
+  if (reads_tc) *reads_tc = C.bwd_reads_tc ? 1 : 0;
+  if (cnn_tc) *cnn_tc = C.bwd_cnn_tc ? 1 : 0;
   return 0;
 }
 
 extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, const PmtBatch* batch, const PmtOutGrads* grads,
                             float* d_weights, void* workspace, size_t workspace_bytes, void* stream) {
-  Plan P;
-  CnnGeom G;
-  if (pmt_build_plan(desc, &P) || pmt_cnn_geometry(P, &G)) return 1;
+  CallPlan C;
+  if (pmt_call_plan(desc, batch, false, &C)) return 1;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const size_t need = pmt_workspace_size(desc, batch, 1);
-  PMT_CHECK(workspace && workspace_bytes >= need, "workspace too small: %zu < %zu", workspace_bytes, need);
+  const BwdWsLayout L = backward_layout(C, batch);
+  PMT_CHECK(workspace && workspace_bytes >= L.end, "workspace too small: %zu < %zu", workspace_bytes, L.end);
   PMT_CHECK(batch->n_variants > 0, "empty batch");
-  PMT_CHECK(NPART * desc->d_feat <= P.bwd_rows, "d_feat %d too wide for the backward kernel's head scratch", desc->d_feat);
-  const size_t smem = bwd_smem_bytes(P);
+  PMT_CHECK(NPART * desc->d_feat <= C.P.bwd_rows, "d_feat %d too wide for the backward kernel's head scratch", desc->d_feat);
+  const size_t smem = bwd_smem_bytes(C.P);
   PMT_CHECK(smem <= 227 * 1024, "model too wide for the backward kernel's shared-memory plan (%zu bytes)", smem);
 
   const int B = batch->n_variants, w = desc->d_info + desc->d_seq;
   char* ws = reinterpret_cast<char*>(workspace);
-  size_t off = 256;
-  float* image = reinterpret_cast<float*>(ws + off); off += pmt_image_bytes(P, G); off = (off + 255) & ~(size_t)255;
-  float* partials = reinterpret_cast<float*>(ws + off); off += (size_t)kBwdGrid * desc->n_params * sizeof(float);
-  const size_t scr_floats = P.scratch_floats > P.info_scratch_floats ? P.scratch_floats : P.info_scratch_floats;
-  float* scratch = reinterpret_cast<float*>(ws + off); off += (size_t)kBwdGrid * scr_floats * sizeof(float);
-  float* info_seq = reinterpret_cast<float*>(ws + off); off += (size_t)B * w * sizeof(float);
-  float* d_info_seq = reinterpret_cast<float*>(ws + off); off += (size_t)B * w * sizeof(float);
-  off = (off + 255) & ~(size_t)255;
-  const int lgrid = long_bwd_grid(P, batch);
-  const size_t long_floats = long_bwd_floats_per_cta(P, batch);
-  float* long_scratch = reinterpret_cast<float*>(ws + off); off += (size_t)lgrid * long_floats * sizeof(float);
-  const bool use_tc = bwd_reads_tc(P);   // tile-sized sets; longer sets always take the SIMT long-set kernel
-  off = (off + 255) & ~(size_t)255;
-  unsigned char* tc_ws = reinterpret_cast<unsigned char*>(ws + off);
-  const size_t tc_ws_bytes = use_tc ? pmt_tc_bwd_workspace_bytes(P, batch) + 1024 : 0;
-  off += tc_ws_bytes;
-  const bool cnn_mma = bwd_cnn_tc(P);
-  off = (off + 255) & ~(size_t)255;
-  unsigned char* cnn_ws = reinterpret_cast<unsigned char*>(ws + off);
-  const size_t cnn_ws_bytes = cnn_mma ? pmt_cnn_bwd_mma_workspace_bytes(P, batch) : 0;
-  off += cnn_ws_bytes;
-  PMT_CHECK(off <= workspace_bytes, "workspace layout overflow");
+  float* image = reinterpret_cast<float*>(ws + L.image);
+  float* partials = reinterpret_cast<float*>(ws + L.partials);
+  float* scratch = reinterpret_cast<float*>(ws + L.scratch);
+  float* info_seq = reinterpret_cast<float*>(ws + L.info_seq);
+  float* d_info_seq = reinterpret_cast<float*>(ws + L.d_info_seq);
+  float* long_scratch = reinterpret_cast<float*>(ws + L.long_scratch);
+  unsigned char* tc_ws = reinterpret_cast<unsigned char*>(ws + L.tc);
+  unsigned char* cnn_ws = reinterpret_cast<unsigned char*>(ws + L.cnn);
 
-  // what pmt_forward_train saved for this batch (PmtOutGrads.saved): [read path][haplotype CNN], as train_saved_split lays it out
+  // what pmt_forward_train saved for this batch (PmtOutGrads.saved), laid out by pmt_saved_layout
   const unsigned char* saved_tc = nullptr;
   const float* saved_cnn = nullptr;
   if (grads && grads->saved) {
-    PMT_CHECK(use_tc && cnn_mma && pmt_precision_mode() == PMT_PRECISION_TF32X3 && grads->info_seq_be,
+    PMT_CHECK(C.bwd_reads_tc && C.bwd_cnn_tc && C.mode == PMT_PRECISION_TF32X3 && grads->info_seq_be,
               "PmtOutGrads.saved needs the tf32x3 mode, the forward's info_seq_be, and the precision mode of the forward call");
-    const size_t tc = pmt_tc_train_saved_bytes(P, batch);
-    PMT_CHECK(tc > 0 && pmt_cnn_train_saved_bytes(P, batch) > 0, "PmtOutGrads.saved: no saved-forward path for this batch");
+    PMT_CHECK(C.saved.total > 0, "PmtOutGrads.saved: no saved-forward path for this batch");
     saved_tc = reinterpret_cast<const unsigned char*>(grads->saved);
-    saved_cnn = reinterpret_cast<const float*>(saved_tc + ((tc + 1023) & ~(size_t)1023));
+    saved_cnn = reinterpret_cast<const float*>(saved_tc + C.saved.cnn);
   }
-  PMT_CUDA(cudaMemsetAsync(partials, 0, (size_t)kBwdGrid * desc->n_params * sizeof(float), st));
+  PMT_CUDA(cudaMemsetAsync(partials, 0, (size_t)PMT_PARTIAL_CTAS * desc->n_params * sizeof(float), st));
   // conv images: only the SIMT haplotype-CNN kernels read them (the recompute below when the forward's embeddings are not
   // passed in, and the SIMT backward)
-  pmt_launch_prepare(P, G, weights, image, st, true, !cnn_mma || !(grads && grads->info_seq_be));
+  pmt_launch_prepare(C, weights, image, st, true, !C.bwd_cnn_tc || !(grads && grads->info_seq_be));
   if (grads && grads->info_seq_be) {
     cudaMemcpyAsync(info_seq, grads->info_seq_be, (size_t)B * w * sizeof(float), cudaMemcpyDeviceToDevice, st);
-  } else if (pmt_launch_variant_kernels(P, G, weights, image, batch, info_seq, PMT_PRECISION_FP32, nullptr, false, st)) {
+  } else if (pmt_launch_info_mlp(C, weights, image, batch, info_seq, st) || pmt_launch_hap_cnn_simt(C, weights, image, batch, info_seq, st)) {
     return 1;
   }
 
-  int dev = 0, n_sm = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
+  const int n_sm = C.n_sm;
   // Claims go to CTAs round-robin (fixed summation order), so their number is a multiple of the grid; every claim ends
   // with a partly filled tile, so a claim should hold >= 16 tiles (n_rows is an upper bound for a downsampled batch:
   // claims of ~4 tiles left a fifth of the rows of every tile empty).
-  const double rows_total = (double)(batch->n_rows > 0 ? batch->n_rows : 16LL * B);
-  int per_cta = (int)(rows_total / ((double)n_sm * 16.0 * TILE));
+  int per_cta = (int)((double)pmt_row_hint(batch) / ((double)n_sm * 16.0 * TILE));
   if (per_cta < 1) per_cta = 1;
   if (per_cta > 8) per_cta = 8;
   int claim = (int)((B + (long long)n_sm * per_cta - 1) / ((long long)n_sm * per_cta));
   if (claim < 1) claim = 1;
+  Plan P = C.P;
   P.claim_variants = claim;
 
   BwdArgs A;
@@ -1335,15 +1329,15 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
   A.d_logits_bk = grads ? grads->d_logits_bk : nullptr;
   A.d_alt_means = grads ? grads->d_alt_means_be : nullptr;
   A.d_ref_means = grads ? grads->d_ref_means_be : nullptr;
-  A.d_info_seq = d_info_seq; A.scratch = scratch; A.scratch_stride = (long long)scr_floats; A.partials = partials;
-  A.long_scratch = long_scratch; A.long_scratch_stride = (long long)long_floats;
+  A.d_info_seq = d_info_seq; A.scratch = scratch; A.scratch_stride = (long long)L.scr_floats; A.partials = partials;
+  A.long_scratch = long_scratch; A.long_scratch_stride = (long long)L.long_floats;
   A.n_claims = (B + claim - 1) / claim;
-  int grid = A.n_claims < kBwdGrid ? A.n_claims : kBwdGrid;
+  int grid = A.n_claims < PMT_PARTIAL_CTAS ? A.n_claims : PMT_PARTIAL_CTAS;
   if (grid > n_sm) grid = n_sm;
   int tc_grid = 0;
-  if (use_tc) {
-    if (pmt_launch_reads_tc_backward(P, weights, batch, info_seq, A.d_logits_bk, A.d_alt_means, A.d_ref_means, d_info_seq, tc_ws,
-                                     tc_ws_bytes, n_sm, &tc_grid, st, saved_tc))
+  if (C.bwd_reads_tc) {   // tile-sized sets; longer sets always take the SIMT long-set kernel
+    if (pmt_launch_reads_tc_backward(C, weights, batch, info_seq, A.d_logits_bk, A.d_alt_means, A.d_ref_means, d_info_seq, tc_ws,
+                                     L.tc_bytes, &tc_grid, st, saved_tc))
       return 1;
   } else {
     PMT_CUDA(cudaFuncSetAttribute(reads_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1351,29 +1345,28 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
     reads_backward_kernel<<<grid, NTHREADS, smem, st>>>(P, A);
     pmt_profile_end(st);
   }
-  if (lgrid > 0) {   // sets longer than a tile; same CTA-private gradient buffers, after the tile kernel: fixed order
+  if (L.long_grid > 0) {   // sets longer than a tile; same CTA-private gradient buffers, after the tile kernel: fixed order
     PMT_CUDA(cudaFuncSetAttribute(reads_backward_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    reads_backward_long_kernel<<<lgrid, NTHREADS, smem, st>>>(P, A);
+    reads_backward_long_kernel<<<L.long_grid, NTHREADS, smem, st>>>(P, A);
   }
   {
     const int rows = info_rows(P);
     const size_t ismem = (size_t)(4 * rows * LD + 2 * P.info_stage_floats) * sizeof(float);
     PMT_CHECK(ismem <= 227 * 1024, "info MLP too wide for the backward kernel (%zu bytes of shared memory)", ismem);
     const int n_tiles = (B + TILE - 1) / TILE;
-    const int igrid = n_tiles < kBwdGrid ? n_tiles : kBwdGrid;
+    const int igrid = n_tiles < PMT_PARTIAL_CTAS ? n_tiles : PMT_PARTIAL_CTAS;
     PMT_CUDA(cudaFuncSetAttribute(info_mlp_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ismem));
     info_mlp_backward_kernel<<<igrid, NTHREADS, ismem, st>>>(P, weights, image, batch->info, batch->info_kind,
                                                              batch->info_stride, B, d_info_seq, scratch,
-                                                             (long long)scr_floats, partials, rows);
+                                                             (long long)L.scr_floats, partials, rows);
   }
-  if (cnn_mma) {
-    if (pmt_launch_cnn_backward_mma(P, weights, batch, info_seq, d_info_seq, partials, kBwdGrid, cnn_ws, cnn_ws_bytes, n_sm, st, saved_cnn))
-      return 1;
-  } else if (pmt_launch_cnn_backward(P, G, weights, image, batch, d_info_seq, partials, kBwdGrid, st)) {
+  if (C.bwd_cnn_tc) {
+    if (pmt_launch_cnn_backward_mma(C, weights, batch, info_seq, d_info_seq, partials, cnn_ws, L.cnn_bytes, st, saved_cnn)) return 1;
+  } else if (launch_cnn_backward(P, C.G, weights, image, batch, d_info_seq, partials, st)) {
     return 1;
   }
-  reduce_partials_kernel<<<(desc->n_params + 255) / 256, 256, 0, st>>>(partials, kBwdGrid, desc->n_params, d_weights);
-  if (use_tc && pmt_finish_reads_tc_backward(P, weights, batch, d_weights, tc_ws, tc_grid, st)) return 1;
+  reduce_partials_kernel<<<(desc->n_params + 255) / 256, 256, 0, st>>>(partials, PMT_PARTIAL_CTAS, desc->n_params, d_weights);
+  if (C.bwd_reads_tc && pmt_finish_reads_tc_backward(C, weights, d_weights, tc_ws, tc_grid, st)) return 1;
   if (P.n_skipfix > 0) skip_fix_kernel<<<P.n_skipfix, 256, 0, st>>>(P, weights, d_weights);
   cudaError_t e = cudaGetLastError();
   PMT_CHECK(e == cudaSuccess, "pmt_backward launch failed: %s", cudaGetErrorString(e));

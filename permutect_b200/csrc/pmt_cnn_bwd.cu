@@ -19,41 +19,10 @@
 // tensor-core backward (pmt_tc_bwd.cu; tests/test_backward_tc_gpu.py).  Every sum has a fixed order: bitwise reproducible.
 #include <cstring>
 
-#include "pmt_cnn_tc.cuh"
+#include "pmt_call.h"
 
 namespace pmt {
 namespace cnnbwd {
-
-constexpr int THREADS = 512, WARPS = THREADS / 32;
-constexpr int MAXL = cnntc::MAX_LAYERS;
-constexpr int NT = 4;            // n-tiles of 8 columns per weight-gradient unit
-constexpr int SLOTS = 3;         // weight-gradient units per warp
-constexpr int MAX_UNITS = SLOTS * WARPS;
-constexpr int MAX_NPV = 4;       // data gradient: n-tiles of 8 input positions per variant
-
-struct BLayer {
-  int Cin, Cout, ks, L_in, L_out, L_pool;
-  int dup, pool2, selu, first, to_global, is_linear, flat_len;
-  int w_off, b_off, op_in_ch;
-  int Cin8, Cout8, Mt_w, Mt_d, kpv, npv;
-  int lm, lpg, ldy;        // dY_l: left margin (ks - 1), per-variant stride, row stride (floats)
-  int ld_a, a_smem;        // INPUT plane a_{l-1} in shared memory: row stride, float offset (l > 0)
-  int ld_g;                // row stride of g_{l-1}, the data gradient this layer produces (l > 0)
-  int img_off;             // float offset of the data-gradient image inside the image buffer
-  int save_in, save_bits;  // float offsets inside a group's save block: a_{l-1}; this layer's window bits (-1: none)
-  int bits_smem;           // byte offset of this layer's window bits in shared memory
-  int inv_vt_pad_;
-  float s_in;              // SELU scale of the previous layer (folded into the forward's weight images): a_{l-1} = s_in * saved
-};
-struct Unit { int layer, m, nt0, cnt; };
-struct BPlan {
-  int n_layers, VT, G, n_units, group_floats;
-  int img_total, a_total, dy_floats, g_floats, bits_bytes, codes_stride, L0;
-  int inv_vt;              // ceil(65536 / VT): pair / VT == (pair * inv_vt) >> 16 for pair < 1024
-  int smem_bytes;
-  BLayer layer[MAXL];
-  Unit unit[MAX_UNITS];
-};
 
 __device__ __forceinline__ float rna(float v) {
   unsigned r;
@@ -413,7 +382,7 @@ static int pad_mod(int n, int r, int m) {   // smallest ld >= n with ld == r (mo
 }
 
 // Layer program of the backward from the forward's; false: outside this kernel's envelope (the FP32 SIMT kernel runs).
-static bool build_bwd_plan(const pmt::Plan& P, const cnntc::Plan& T, BPlan* out) {
+bool pmt_build_cnn_bwd_plan(const pmt::Plan& P, const cnntc::Plan& T, BPlan* out) {
   BPlan& B = *out;
   memset(&B, 0, sizeof(B));
   cnntc::SaveLayout SL;
@@ -493,47 +462,30 @@ static bool build_bwd_plan(const pmt::Plan& P, const cnntc::Plan& T, BPlan* out)
 
 static const int kCnnBwdChunk = 65536;   // variants per recompute + backward pair: bounds the saved activations (5.3 KB per variant)
 
-bool pmt_cnn_bwd_mma_supported(const pmt::Plan& P) {
-  cnntc::Plan T;
-  BPlan B;
-  return pmt_build_cnn_tc_plan(P, &T) && build_bwd_plan(P, T, &B);
-}
-
-size_t pmt_cnn_bwd_mma_workspace_bytes(const pmt::Plan& P, const PmtBatch* batch) {
-  cnntc::Plan T;
-  BPlan B;
-  if (!pmt_build_cnn_tc_plan(P, &T) || !build_bwd_plan(P, T, &B)) return 0;
+// [forward weight images (the recompute)][data-gradient images][saved activations of one chunk]
+size_t pmt_cnn_bwd_workspace_bytes(const CallPlan& C, const PmtBatch* batch) {
+  if (!C.cnn_bwd_ok) return 0;
   const int n = batch ? (batch->n_variants < kCnnBwdChunk ? batch->n_variants : kCnnBwdChunk) : kCnnBwdChunk;
-  const size_t groups = ((size_t)n + T.G - 1) / T.G;
-  return pmt_cnn_tc_image_bytes(P) + 256 + (size_t)B.img_total * sizeof(float) + 256 + groups * B.group_floats * sizeof(float) + 1024;
+  const size_t groups = ((size_t)n + C.C.G - 1) / C.C.G;
+  return pmt_cnn_tc_image_bytes(C) + 256 + (size_t)C.CB.img_total * sizeof(float) + 256 + groups * C.CB.group_floats * sizeof(float) + 1024;
 }
 
-// ---- training without recompute: the training forward runs the SAVE variant over the whole batch (pmt_forward_train) ----
-size_t pmt_cnn_train_saved_bytes(const pmt::Plan& P, const PmtBatch* batch) {
-  cnntc::Plan T;
-  BPlan B;
-  if (!batch || batch->n_variants <= 0 || !pmt_build_cnn_tc_plan(P, &T) || !build_bwd_plan(P, T, &B)) return 0;
-  const size_t groups = ((size_t)batch->n_variants + T.G - 1) / T.G;
-  return groups * B.group_floats * sizeof(float) + 256;
+// the training forward runs the SAVE variant over the whole batch (pmt_forward_train); `save`: the CNN part of the saved
+// buffer (pmt_saved_layout)
+int pmt_cnn_forward_train(const CallPlan& C, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
+                          float* save, cudaStream_t st) {
+  if (pmt_pack_cnn_tc_images(C.P, C.C, weights, image, st)) return 1;
+  return pmt_launch_cnn_tc_save(C.P, C.C, weights, batch, 0, batch->n_variants, info_seq, image, save, C.n_sm, st);
 }
 
-int pmt_cnn_forward_train(const pmt::Plan& P, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
-                          float* save, int n_sm, cudaStream_t st) {
-  cnntc::Plan T;
-  PMT_CHECK(pmt_build_cnn_tc_plan(P, &T), "haplotype CNN outside the tensor-core envelope");
-  if (pmt_pack_cnn_tc_images(P, T, weights, image, st)) return 1;
-  return pmt_launch_cnn_tc_save(P, T, weights, batch, 0, batch->n_variants, info_seq, image, save, n_sm, st);
-}
-
-int pmt_launch_cnn_backward_mma(const pmt::Plan& P, const float* weights, const PmtBatch* batch, float* info_seq, const float* d_info_seq,
-                                float* partials, int n_partials, unsigned char* ws, size_t ws_bytes, int n_sm, cudaStream_t st,
-                                const float* saved) {
-  cnntc::Plan T;
-  BPlan B;
-  PMT_CHECK(pmt_build_cnn_tc_plan(P, &T) && build_bwd_plan(P, T, &B), "haplotype CNN outside the tensor-core backward's envelope");
-  PMT_CHECK(ws_bytes >= pmt_cnn_bwd_mma_workspace_bytes(P, batch), "CNN backward workspace too small");
+int pmt_launch_cnn_backward_mma(const CallPlan& C, const float* weights, const PmtBatch* batch, float* info_seq, const float* d_info_seq,
+                                float* partials, unsigned char* ws, size_t ws_bytes, cudaStream_t st, const float* saved) {
+  const pmt::Plan& P = C.P;
+  const cnntc::Plan& T = C.C;
+  const BPlan& B = C.CB;
+  PMT_CHECK(ws_bytes >= pmt_cnn_bwd_workspace_bytes(C, batch), "CNN backward workspace too small");
   unsigned char* p = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~uintptr_t(255));
-  unsigned char* fwd_image = p; p += (pmt_cnn_tc_image_bytes(P) + 255) & ~size_t(255);
+  unsigned char* fwd_image = p; p += (pmt_cnn_tc_image_bytes(C) + 255) & ~size_t(255);
   float* bwd_image = reinterpret_cast<float*>(p); p += ((size_t)B.img_total * sizeof(float) + 255) & ~size_t(255);
   float* save = reinterpret_cast<float*>(p);
   // weight images: the forward's (split precision; only for the recompute) and the data gradient's
@@ -546,10 +498,10 @@ int pmt_launch_cnn_backward_mma(const pmt::Plan& P, const float* weights, const 
   for (int v_first = 0; v_first < batch->n_variants; v_first += chunk) {
     const int n = batch->n_variants - v_first < chunk ? batch->n_variants - v_first : chunk;
     if (saved) save = const_cast<float*>(saved);
-    else if (pmt_launch_cnn_tc_save(P, T, weights, batch, v_first, n, info_seq, fwd_image, save, n_sm, st)) return 1;
+    else if (pmt_launch_cnn_tc_save(P, T, weights, batch, v_first, n, info_seq, fwd_image, save, C.n_sm, st)) return 1;
     const int n_groups = (n + B.VT - 1) / B.VT;
-    int grid = n_groups < n_sm ? n_groups : n_sm;
-    if (grid > n_partials) grid = n_partials;
+    int grid = n_groups < C.n_sm ? n_groups : C.n_sm;
+    if (grid > PMT_PARTIAL_CTAS) grid = PMT_PARTIAL_CTAS;
     const void* haps = reinterpret_cast<const unsigned char*>(batch->haplotypes) + (size_t)v_first * batch->hap_stride * esz;
     cnn_backward_mma_kernel<<<grid, THREADS, B.smem_bytes, st>>>(B, bwd_image, haps, batch->hap_kind, batch->hap_stride, n, save,
                                                                  info_seq + (size_t)v_first * out_w, d_info_seq + (size_t)v_first * out_w, out_w,

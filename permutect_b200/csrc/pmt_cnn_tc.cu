@@ -19,7 +19,7 @@
 // the whole remaining length.  SELU scales are folded into the consuming weights.  Precision modes as pmt_tc.cu.
 #include <cstring>
 
-#include "pmt_cnn_tc.cuh"
+#include "pmt_call.h"
 
 namespace pmt {
 namespace cnntc {
@@ -523,23 +523,14 @@ bool pmt_build_cnn_tc_plan(const pmt::Plan& P, cnntc::Plan* out) {
   return true;
 }
 
-bool pmt_cnn_tc_supported(const pmt::Plan& P) {
-  cnntc::Plan T;
-  return pmt_build_cnn_tc_plan(P, &T);
-}
-
-size_t pmt_cnn_tc_image_bytes(const pmt::Plan& P) {
-  cnntc::Plan T;
-  if (!pmt_build_cnn_tc_plan(P, &T)) return 0;
-  return (size_t)T.image_bytes + 256;
-}
+size_t pmt_cnn_tc_image_bytes(const CallPlan& C) { return C.cnn_tc_ok ? (size_t)C.C.image_bytes + 256 : 0; }
 
 template <int PASSES, bool SAVE>
 static int launch_cnn_tc(const cnntc::Plan& T, const unsigned char* image, const float* weights, const PmtModelDesc& D, const void* haps,
                          const PmtBatch* batch, int n, float* info_seq, const SaveLayout& SL, float* save, int grid, cudaStream_t st) {
   const size_t smem = 2 * BUF_BYTES + T.image_bytes + MAX_LAYERS * 32 * sizeof(float) + sizeof(Bars) + 1024 + 64;
   PMT_CUDA(cudaFuncSetAttribute(hap_cnn_tc_kernel<PASSES, SAVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  hap_cnn_tc_kernel<PASSES, SAVE><<<grid, THREADS, smem, st>>>(T, image, weights, D, haps, batch->hap_kind, batch->hap_stride, n, info_seq,
+  hap_cnn_tc_kernel<PASSES, SAVE><<<grid, cnntc::THREADS, smem, st>>>(T, image, weights, D, haps, batch->hap_kind, batch->hap_stride, n, info_seq,
                                                                SL, save);
   return 0;
 }
@@ -578,17 +569,16 @@ int pmt_pack_cnn_tc_images(const pmt::Plan& P, const cnntc::Plan& T, const float
   return 0;
 }
 
-// `image` is a 16-byte aligned device buffer of pmt_cnn_tc_image_bytes(P) bytes.
-int pmt_launch_cnn_tc(const pmt::Plan& P, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
-                      bool reuse_image, int n_sm, int mode, cudaStream_t st) {
-  cnntc::Plan T;
-  PMT_CHECK(pmt_build_cnn_tc_plan(P, &T), "haplotype CNN outside the tensor-core envelope");
-  if (!reuse_image) pack_cnn_tc_kernel<<<dim3(T.n_layers, 16), 256, 0, st>>>(P.d, T, weights, image);
+// `image` is a 16-byte aligned device buffer of pmt_cnn_tc_image_bytes(C) bytes.
+int pmt_launch_cnn_tc(const CallPlan& C, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
+                      bool reuse_image, cudaStream_t st) {
+  const cnntc::Plan& T = C.C;
+  if (!reuse_image) pack_cnn_tc_kernel<<<dim3(T.n_layers, 16), 256, 0, st>>>(C.P.d, T, weights, image);
   const int n_groups = (batch->n_variants + T.G - 1) / T.G;
-  const int grid = n_groups < n_sm ? n_groups : n_sm;
+  const int grid = n_groups < C.n_sm ? n_groups : C.n_sm;
   SaveLayout SL;
   memset(&SL, 0, sizeof(SL));
-  return mode == PMT_PRECISION_TF32
-             ? launch_cnn_tc<1, false>(T, image, weights, P.d, batch->haplotypes, batch, batch->n_variants, info_seq, SL, nullptr, grid, st)
-             : launch_cnn_tc<3, false>(T, image, weights, P.d, batch->haplotypes, batch, batch->n_variants, info_seq, SL, nullptr, grid, st);
+  return C.mode == PMT_PRECISION_TF32
+             ? launch_cnn_tc<1, false>(T, image, weights, C.P.d, batch->haplotypes, batch, batch->n_variants, info_seq, SL, nullptr, grid, st)
+             : launch_cnn_tc<3, false>(T, image, weights, C.P.d, batch->haplotypes, batch, batch->n_variants, info_seq, SL, nullptr, grid, st);
 }

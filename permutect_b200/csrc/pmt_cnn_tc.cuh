@@ -61,6 +61,42 @@ struct SaveLayout {
 };
 
 }  // namespace cnntc
+
+// the tensor-core CNN backward's plan (pmt_cnn_bwd.cu)
+namespace cnnbwd {
+
+constexpr int THREADS = 512, WARPS = THREADS / 32;
+constexpr int MAXL = cnntc::MAX_LAYERS;
+constexpr int NT = 4;            // n-tiles of 8 columns per weight-gradient unit
+constexpr int SLOTS = 3;         // weight-gradient units per warp
+constexpr int MAX_UNITS = SLOTS * WARPS;
+constexpr int MAX_NPV = 4;       // data gradient: n-tiles of 8 input positions per variant
+
+struct BLayer {
+  int Cin, Cout, ks, L_in, L_out, L_pool;
+  int dup, pool2, selu, first, to_global, is_linear, flat_len;
+  int w_off, b_off, op_in_ch;
+  int Cin8, Cout8, Mt_w, Mt_d, kpv, npv;
+  int lm, lpg, ldy;        // dY_l: left margin (ks - 1), per-variant stride, row stride (floats)
+  int ld_a, a_smem;        // INPUT plane a_{l-1} in shared memory: row stride, float offset (l > 0)
+  int ld_g;                // row stride of g_{l-1}, the data gradient this layer produces (l > 0)
+  int img_off;             // float offset of the data-gradient image inside the image buffer
+  int save_in, save_bits;  // float offsets inside a group's save block: a_{l-1}; this layer's window bits (-1: none)
+  int bits_smem;           // byte offset of this layer's window bits in shared memory
+  int inv_vt_pad_;
+  float s_in;              // SELU scale of the previous layer (folded into the forward's weight images): a_{l-1} = s_in * saved
+};
+struct Unit { int layer, m, nt0, cnt; };
+struct BPlan {
+  int n_layers, VT, G, n_units, group_floats;
+  int img_total, a_total, dy_floats, g_floats, bits_bytes, codes_stride, L0;
+  int inv_vt;              // ceil(65536 / VT): pair / VT == (pair * inv_vt) >> 16 for pair < 1024
+  int smem_bytes;
+  BLayer layer[MAXL];
+  Unit unit[MAX_UNITS];
+};
+
+}  // namespace cnnbwd
 }  // namespace pmt
 
 // host (pmt_cnn_tc.cu)

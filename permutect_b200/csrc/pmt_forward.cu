@@ -8,7 +8,7 @@
 #include <cstdio>
 #include <cstring>
 
-#include "pmt_host.h"
+#include "pmt_call.h"
 #include "pmt_tile.cuh"
 #include "pmt_cnn.cuh"
 
@@ -763,66 +763,102 @@ size_t pmt_image_bytes(const Plan& P, const CnnGeom& G) {
   return (size_t)(P.img_total + G.img_total + G.imgT_total + 64) * sizeof(float);
 }
 
-static size_t long_scratch_floats_per_cta(const Plan& P, const PmtBatch* batch);
-
-// Workspace layout of the forward: the packed weight images sit at FIXED offsets from the base (they depend on the model
-// only), the batch-dependent regions follow:
-//   [256 B counters][SIMT images][tcgen05 read-kernel images][tcgen05 CNN images] | [info_seq][long-set scratch][tile list]
-struct FwdLayout {
-  size_t image, tc_image, cnn_tc_image, info_seq, long_scratch, tiles, long_tc, long_tc_bytes, end;
-};
-static FwdLayout forward_layout(const Plan& P, const CnnGeom& G, const PmtModelDesc* desc, const PmtBatch* batch) {
-  FwdLayout L;
-  size_t off = 256;
-  L.image = off; off += pmt_image_bytes(P, G); off = (off + 1023) & ~(size_t)1023;
-  L.tc_image = off; off += pmt_tc_image_bytes(P); off = (off + 255) & ~(size_t)255;
-  L.cnn_tc_image = off; off += pmt_cnn_tc_image_bytes(P); off = (off + 255) & ~(size_t)255;
-  L.info_seq = off; off += (size_t)batch->n_variants * (desc->d_info + desc->d_seq) * sizeof(float); off = (off + 255) & ~(size_t)255;
-  L.long_scratch = off; off += long_scratch_floats_per_cta(P, batch) * sizeof(float) * 148; off = (off + 255) & ~(size_t)255;
-  L.tiles = off; off += pmt_tc_tiles_bytes(batch); off = (off + 255) & ~(size_t)255;
-  L.long_tc_bytes = pmt_tc_long_bytes(P, batch);
-  L.long_tc = off; off += L.long_tc_bytes;
-  L.end = off;
-  return L;
+int pmt_sm_count() {
+  int dev = 0, n_sm = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n_sm < 1)
+    return 148;   // no device: a B200's
+  return n_sm;
 }
 
-extern "C" size_t pmt_workspace_size(const PmtModelDesc* desc, const PmtBatch* batch, int for_backward) {
-  Plan P;
-  CnnGeom G;
-  if (pmt_build_plan(desc, &P) || pmt_cnn_geometry(P, &G)) return 0;
-  PmtBatch none;
-  memset(&none, 0, sizeof(none));
-  size_t bytes = forward_layout(P, G, desc, batch ? batch : &none).end + 1024;
-  if (for_backward) bytes += pmt_backward_workspace_bytes(P, batch);
-  return bytes;
+int pmt_call_plan(const PmtModelDesc* desc, const PmtBatch* batch, bool train, CallPlan* out) {
+  CallPlan& C = *out;
+  memset(&C, 0, sizeof(C));
+  if (pmt_build_plan(desc, &C.P) || pmt_cnn_geometry(C.P, &C.G)) return 1;
+  const Plan& P = C.P;
+  C.mode = pmt_precision_mode();
+  C.n_sm = pmt_sm_count();
+  C.reads_tc_ok = pmt_tc_supported(P);
+  pmt_tc_plan(P, &C.T);
+  C.cnn_tc_ok = pmt_build_cnn_tc_plan(P, &C.C);
+  C.cnn_bwd_ok = C.cnn_tc_ok && pmt_build_cnn_bwd_plan(P, C.C, &C.CB);
+  const bool fp32 = C.mode == PMT_PRECISION_FP32;
+  C.saved = pmt_saved_layout(C, batch);
+  train = train && C.saved.total > 0;
+  const int B = batch ? batch->n_variants : 0;
+  C.info_w4 = info_rows_w4(P.d);
+  C.info = C.info_w4 == 0 ? InfoKernel::TILE : B <= 4096 ? InfoKernel::WARP : InfoKernel::ROWS;   // small batch: latency, not throughput
+  C.cnn = train ? CnnKernel::TC_SAVE : !fp32 && C.cnn_tc_ok ? CnnKernel::TC : CnnKernel::SIMT;
+  C.reads = fp32 ? ReadsKernel::SIMT : train ? ReadsKernel::TC_SAVE : ReadsKernel::TC;
+  C.lng = !batch || !pmt_has_long_sets(batch)                            ? LongKernel::NONE
+          : !fp32 && pmt_tc_long_layout(P, batch, C.n_sm, &C.long_tc) ? LongKernel::TC
+                                                                       : LongKernel::SIMT;
+  // who reads the SIMT images in a tensor-core mode: the tile-GEMM info MLP (widths outside info_mlp_rows_kernel), the SIMT
+  // haplotype CNN (shapes outside the tensor-core envelope) -- and, depending on the batch, the FP32 long-set kernel
+  C.simt_gemm = fp32 || C.info == InfoKernel::TILE;
+  C.simt_conv = C.cnn == CnnKernel::SIMT;
+  // the backward: the tensor-core read-path and haplotype-CNN kernels (pmt_tc_bwd.cu, pmt_cnn_bwd.cu) unless the FP32 mode
+  // is selected or the model is outside their envelope, the FP32 SIMT kernels otherwise
+  C.bwd_reads_tc = !fp32 && C.reads_tc_ok;
+  C.bwd_cnn_tc = !fp32 && C.cnn_bwd_ok;
+  C.tc_bwd = pmt_tc_bwd_layout(C.T, batch);
+  return 0;
 }
 
-static size_t reads_kernel_smem(const Plan& P) { return tile_ctx_bytes(P, P.stage_floats); }
-
-// long-set scratch: per CTA, one (x, z) image pair per chunk of the longest variant
-static int long_grid(const PmtBatch* batch, int n_sm) { return batch->n_variants < n_sm ? batch->n_variants : n_sm; }
+// long-set scratch of the FP32 kernel: per CTA, one (x, z) image pair per chunk of the longest variant
 static size_t long_scratch_floats_per_cta(const Plan& P, const PmtBatch* batch) {
-  if (!batch || !pmt_has_long_sets(batch)) return 0;
   const size_t chunks = (size_t)((batch->max_rows_per_variant + 3 + TILE - 1) / TILE) + 1;
   return chunks * (size_t)(P.d.d_model + P.d.d_ffn) * LD;
 }
 
-// Weight images of the FP32 SIMT kernels.  need_gemm: the tile GEMMs (read path, info MLP, their backward); need_conv: the
-// SIMT haplotype CNN and its backward.  The tensor-core modes skip what none of their kernels reads.
-int pmt_launch_prepare(const Plan& P, const CnnGeom& G, const float* weights, float* image, cudaStream_t st, bool need_gemm,
-                       bool need_conv) {
-  if (need_gemm) pack_weights_kernel<<<dim3(P.n_gemm, 4), 256, 0, st>>>(P, weights, image);
-  if (need_conv && G.n_spatial > 0) pack_conv_kernel<<<G.n_spatial, 256, 0, st>>>(P, G, weights, image + P.img_total);
-  if (need_conv && G.n_spatial > 0) pack_convT_kernel<<<G.n_spatial, 256, 0, st>>>(P, G, weights, image + P.img_total);
+// Workspace layout of the forward: the packed weight images sit at FIXED offsets from the base (they depend on the model
+// only: pmt_forward_prepared finds them there), the batch-dependent regions follow:
+//   [256 B counters][SIMT images][tcgen05 read-kernel images][tcgen05 CNN images] | [info_seq][long-set scratch]
+//   [tile list, or the training forward's planner scratch][long-set tensor-core region]
+struct FwdLayout {
+  size_t image, tc_image, cnn_tc_image, info_seq, long_scratch, tiles, long_tc, end;
+};
+static FwdLayout forward_layout(const CallPlan& C, const PmtBatch* batch) {
+  const int B = batch ? batch->n_variants : 0;
+  FwdLayout L;
+  size_t off = 256;
+  L.image = off; off += pmt_image_bytes(C.P, C.G); off = (off + 1023) & ~(size_t)1023;
+  L.tc_image = off; off += (size_t)C.T.image_bytes + 2048; off = (off + 255) & ~(size_t)255;
+  L.cnn_tc_image = off; off += pmt_cnn_tc_image_bytes(C); off = (off + 255) & ~(size_t)255;
+  L.info_seq = off; off += (size_t)B * (C.P.d.d_info + C.P.d.d_seq) * sizeof(float); off = (off + 255) & ~(size_t)255;
+  L.long_scratch = off;
+  if (C.lng == LongKernel::SIMT) off += long_scratch_floats_per_cta(C.P, batch) * sizeof(float) * PMT_PARTIAL_CTAS;
+  off = (off + 255) & ~(size_t)255;
+  size_t tiles = pmt_tc_tiles_bytes(B);
+  const size_t claims = C.saved.total > 0 ? pmt_plan_claim_bytes(B, PMT_PARTIAL_CTAS) : 0;   // the training forward's planner
+  if (claims > tiles) tiles = claims;
+  L.tiles = off; off += tiles; off = (off + 255) & ~(size_t)255;
+  L.long_tc = off; off += C.lng == LongKernel::TC ? C.long_tc.end : 0;
+  L.end = off + 1024;
+  return L;
+}
+
+extern "C" size_t pmt_workspace_size(const PmtModelDesc* desc, const PmtBatch* batch, int for_backward) {
+  CallPlan C;
+  if (pmt_call_plan(desc, batch, false, &C)) return 0;
+  return for_backward ? pmt_backward_workspace_size(C, batch) : forward_layout(C, batch).end;
+}
+
+static size_t reads_kernel_smem(const Plan& P) { return tile_ctx_bytes(P, P.stage_floats); }
+
+int pmt_launch_prepare(const CallPlan& C, const float* weights, float* image, cudaStream_t st, bool gemm, bool conv) {
+  const Plan& P = C.P;
+  const CnnGeom& G = C.G;
+  if (gemm) pack_weights_kernel<<<dim3(P.n_gemm, 4), 256, 0, st>>>(P, weights, image);
+  if (conv && G.n_spatial > 0) pack_conv_kernel<<<G.n_spatial, 256, 0, st>>>(P, G, weights, image + P.img_total);
+  if (conv && G.n_spatial > 0) pack_convT_kernel<<<G.n_spatial, 256, 0, st>>>(P, G, weights, image + P.img_total);
   return 0;
 }
 
-int pmt_launch_variant_kernels(const Plan& P, const CnnGeom& G, const float* weights, const float* image,
-                               const PmtBatch* batch, float* info_seq, int mode, unsigned char* cnn_tc_image, bool reuse_images,
-                               cudaStream_t st, bool skip_cnn) {
+int pmt_launch_info_mlp(const CallPlan& C, const float* weights, const float* image, const PmtBatch* batch, float* info_seq,
+                        cudaStream_t st) {
+  const Plan& P = C.P;
   const int B = batch->n_variants;
-  const int w4 = info_rows_w4(P.d);
-  if (w4 > 0 && B <= 4096) {   // small batch: latency, not throughput (info_mlp_warp_kernel)
+  if (C.info == InfoKernel::WARP) {
     size_t floats = 0;
     for (int i = 0; i < P.d.n_info_ops; ++i) floats += (size_t)(P.d.info_ops[i].in_dim + 1) * 32;
     const size_t smem = floats * sizeof(float) + 16;
@@ -831,19 +867,17 @@ int pmt_launch_variant_kernels(const Plan& P, const CnnGeom& G, const float* wei
     const int blocks = (B + INFO_WARPS - 1) / INFO_WARPS;
     info_mlp_warp_kernel<<<blocks < 148 * 4 ? blocks : 148 * 4, 32 * INFO_WARPS, smem, st>>>(P.d, weights, batch->info, batch->info_kind,
                                                                                                batch->info_stride, B, info_seq);
-  } else if (w4 > 0) {
-    int rc = 1;
-    switch (w4) {
-      case 1: rc = launch_info_rows<1>(P.d, weights, batch, info_seq, st); break;
-      case 2: rc = launch_info_rows<2>(P.d, weights, batch, info_seq, st); break;
-      case 3: rc = launch_info_rows<3>(P.d, weights, batch, info_seq, st); break;
-      case 4: rc = launch_info_rows<4>(P.d, weights, batch, info_seq, st); break;
-      case 5: rc = launch_info_rows<5>(P.d, weights, batch, info_seq, st); break;
-      case 6: rc = launch_info_rows<6>(P.d, weights, batch, info_seq, st); break;
-      case 7: rc = launch_info_rows<7>(P.d, weights, batch, info_seq, st); break;
-      default: rc = launch_info_rows<8>(P.d, weights, batch, info_seq, st); break;
+  } else if (C.info == InfoKernel::ROWS) {
+    switch (C.info_w4) {
+      case 1: return launch_info_rows<1>(P.d, weights, batch, info_seq, st);
+      case 2: return launch_info_rows<2>(P.d, weights, batch, info_seq, st);
+      case 3: return launch_info_rows<3>(P.d, weights, batch, info_seq, st);
+      case 4: return launch_info_rows<4>(P.d, weights, batch, info_seq, st);
+      case 5: return launch_info_rows<5>(P.d, weights, batch, info_seq, st);
+      case 6: return launch_info_rows<6>(P.d, weights, batch, info_seq, st);
+      case 7: return launch_info_rows<7>(P.d, weights, batch, info_seq, st);
+      default: return launch_info_rows<8>(P.d, weights, batch, info_seq, st);
     }
-    if (rc) return 1;
   } else {
     const int in_rows = P.d.n_info_features > PMT_MAX_DIM ? PMT_MAX_INFO_DIM : PMT_MAX_DIM;
     const size_t smem = (size_t)((in_rows + 2 * PMT_MAX_DIM) * LD + 2 * P.info_stage_floats) * sizeof(float);
@@ -851,21 +885,19 @@ int pmt_launch_variant_kernels(const Plan& P, const CnnGeom& G, const float* wei
     info_mlp_kernel<<<(B + TILE - 1) / TILE, NTHREADS, smem, st>>>(P, weights, image, batch->info, batch->info_kind,
                                                                    batch->info_stride, B, info_seq);
   }
-  if (skip_cnn) return 0;   // the caller runs the haplotype CNN itself (training forward: its SAVE variant)
-  if (mode != PMT_PRECISION_FP32 && cnn_tc_image && pmt_cnn_tc_supported(P)) {
-    // tensor-core haplotype CNN (pmt_cnn_tc.cu); shapes outside its envelope run the FP32 SIMT kernel below
-    int dev = 0, n_sm = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-    if (pmt_launch_cnn_tc(P, weights, batch, info_seq, cnn_tc_image, reuse_images, n_sm, mode, st)) return 1;
-  } else {
-    const size_t smem = (size_t)(2 * G.buf_floats + G.img_total + 2 * G.vt * 256) * sizeof(float);
-    PMT_CUDA(cudaFuncSetAttribute(hap_cnn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int grid = (B + G.vt - 1) / G.vt;
-    if (grid > 148 * 4) grid = 148 * 4;
-    hap_cnn_kernel<<<grid, NTHREADS, smem, st>>>(P, G, weights, image + P.img_total, batch->haplotypes, batch->hap_kind,
-                                                 batch->hap_stride, B, info_seq);
-  }
+  return 0;
+}
+
+int pmt_launch_hap_cnn_simt(const CallPlan& C, const float* weights, const float* image, const PmtBatch* batch, float* info_seq,
+                            cudaStream_t st) {
+  const CnnGeom& G = C.G;
+  const int B = batch->n_variants;
+  const size_t smem = (size_t)(2 * G.buf_floats + G.img_total + 2 * G.vt * 256) * sizeof(float);
+  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int grid = (B + G.vt - 1) / G.vt;
+  if (grid > 148 * 4) grid = 148 * 4;
+  hap_cnn_kernel<<<grid, NTHREADS, smem, st>>>(C.P, G, weights, image + C.P.img_total, batch->haplotypes, batch->hap_kind,
+                                               batch->hap_stride, B, info_seq);
   return 0;
 }
 
@@ -880,104 +912,85 @@ static int choose_claim(const PmtBatch* batch, int n_sm) {
   return claim;
 }
 
-static size_t train_saved_split(const Plan& P, const PmtBatch* batch, size_t* cnn_off) {
-  // [read path: tile list + operand panels][haplotype CNN activations]; 0 when there is no such path for this call
-  if (pmt_precision_mode() != PMT_PRECISION_TF32X3 || !batch || !pmt_tc_supported(P) || !pmt_cnn_tc_supported(P) ||
-      !pmt_cnn_bwd_mma_supported(P))
-    return 0;
-  const size_t tc = pmt_tc_train_saved_bytes(P, batch), cnn = pmt_cnn_train_saved_bytes(P, batch);
-  if (tc == 0 || cnn == 0) return 0;
-  const size_t off = (tc + 1023) & ~(size_t)1023;
-  if (cnn_off) *cnn_off = off;
-  return off + cnn + 1024;
-}
-
 extern "C" size_t pmt_train_saved_bytes(const PmtModelDesc* desc, const PmtBatch* batch) {
-  Plan P;
-  if (pmt_build_plan(desc, &P)) return 0;
-  const size_t bytes = train_saved_split(P, batch, nullptr);
-  return bytes <= ((size_t)16 << 30) ? bytes : 0;
+  CallPlan C;
+  if (pmt_call_plan(desc, batch, true, &C)) return 0;
+  return C.saved.total;
 }
 
 static int forward_impl(const PmtModelDesc* desc, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
                         void* workspace, size_t workspace_bytes, void* stream, bool reuse_images, unsigned char* saved = nullptr,
                         size_t saved_bytes = 0) {
-  Plan P;
-  CnnGeom G;
-  if (pmt_build_plan(desc, &P) || pmt_cnn_geometry(P, &G)) return 1;
+  CallPlan C;
+  if (pmt_call_plan(desc, batch, saved != nullptr, &C)) return 1;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const size_t need = pmt_workspace_size(desc, batch, 0);
-  PMT_CHECK(workspace && workspace_bytes >= need, "workspace too small: %zu < %zu", workspace_bytes, need);
+  const FwdLayout L = forward_layout(C, batch);
+  PMT_CHECK(workspace && workspace_bytes >= L.end, "workspace too small: %zu < %zu", workspace_bytes, L.end);
   PMT_CHECK(batch->n_variants > 0, "empty batch");
-  const FwdLayout L = forward_layout(P, G, desc, batch);
-  PMT_CHECK(L.end <= workspace_bytes, "workspace layout overflow");
   char* ws = reinterpret_cast<char*>(workspace);
   int* counter = reinterpret_cast<int*>(ws);
   float* image = reinterpret_cast<float*>(ws + L.image);
   float* info_seq = out->info_seq_be;
   if (!info_seq) info_seq = reinterpret_cast<float*>(ws + L.info_seq);
   PMT_CUDA(cudaMemsetAsync(counter, 0, 256, st));
-  const int mode = pmt_precision_mode();
   {
-    // who still reads the SIMT images in a tensor-core mode: the tile-GEMM info MLP (widths outside info_mlp_rows_kernel),
-    // the SIMT haplotype CNN (shapes outside the tensor-core envelope), the FP32 long-set kernel
-    const bool simt_long = pmt_has_long_sets(batch) && !(mode != PMT_PRECISION_FP32 && L.long_tc_bytes > 0);
-    const bool need_gemm = mode == PMT_PRECISION_FP32 || info_rows_w4(P.d) == 0;
-    const bool need_conv = mode == PMT_PRECISION_FP32 || !pmt_cnn_tc_supported(P);
-    if (!reuse_images) pmt_launch_prepare(P, G, weights, image, st, need_gemm || simt_long, need_conv);
-    else if (simt_long && !need_gemm) pmt_launch_prepare(P, G, weights, image, st, true, false);   // depends on the batch: not covered by a prepared call
+    // a prepared call finds the images of the model; the FP32 long-set kernel's depend on the batch
+    const bool simt_long = C.lng == LongKernel::SIMT;
+    if (!reuse_images) pmt_launch_prepare(C, weights, image, st, C.simt_gemm || simt_long, C.simt_conv);
+    else if (simt_long && !C.simt_gemm) pmt_launch_prepare(C, weights, image, st, true, false);
   }
   unsigned char* tc_image = reinterpret_cast<unsigned char*>(ws + L.tc_image);
   unsigned char* cnn_tc_image = reinterpret_cast<unsigned char*>(ws + L.cnn_tc_image);
-  int dev = 0, n_sm = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-  size_t saved_cnn_off = 0;
   if (saved) {
-    const size_t need_saved = train_saved_split(P, batch, &saved_cnn_off);
-    PMT_CHECK(need_saved > 0 && saved_bytes >= need_saved, "pmt_forward_train: no saved-forward path for this call or buffer too small (%zu < %zu)",
-              saved_bytes, need_saved);
+    PMT_CHECK(C.saved.total > 0 && saved_bytes >= C.saved.total,
+              "pmt_forward_train: no saved-forward path for this call or buffer too small (%zu < %zu)", saved_bytes, C.saved.total);
     PMT_CHECK((reinterpret_cast<uintptr_t>(saved) & 255) == 0, "pmt_forward_train: the saved buffer must be 256-byte aligned");
-    // per-variant embeddings: the info MLP as always, the haplotype CNN in its SAVE variant (same results, activations kept)
-    if (pmt_launch_variant_kernels(P, G, weights, image, batch, info_seq, mode, nullptr, reuse_images, st, /*skip_cnn=*/true)) return 1;
-    if (pmt_cnn_forward_train(P, weights, batch, info_seq, cnn_tc_image, reinterpret_cast<float*>(saved + saved_cnn_off), n_sm, st)) return 1;
-  } else if (pmt_launch_variant_kernels(P, G, weights, image, batch, info_seq, mode, cnn_tc_image, reuse_images, st)) {
-    return 1;
+  }
+  // per-variant embeddings: the info MLP, then the haplotype CNN (in training its SAVE variant: same results, activations kept)
+  if (pmt_launch_info_mlp(C, weights, image, batch, info_seq, st)) return 1;
+  switch (C.cnn) {
+    case CnnKernel::TC:
+      if (pmt_launch_cnn_tc(C, weights, batch, info_seq, cnn_tc_image, reuse_images, st)) return 1;
+      break;
+    case CnnKernel::TC_SAVE:
+      if (pmt_cnn_forward_train(C, weights, batch, info_seq, cnn_tc_image, reinterpret_cast<float*>(saved + C.saved.cnn), st)) return 1;
+      break;
+    case CnnKernel::SIMT:
+      if (pmt_launch_hap_cnn_simt(C, weights, image, batch, info_seq, st)) return 1;
+      break;
   }
 
-  P.claim_variants = choose_claim(batch, n_sm);
+  Plan P = C.P;
+  P.claim_variants = choose_claim(batch, C.n_sm);
   ReadKernelArgs A;
   A.wflat = weights; A.image = image; A.batch = *batch; A.out = *out; A.out.info_seq_be = info_seq; A.claim_counter = counter;
   A.scratch = nullptr; A.scratch_stride = 0;
   const size_t smem = reads_kernel_smem(P);
   PMT_CUDA(cudaFuncSetAttribute(reads_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int n_claims = (batch->n_variants + P.claim_variants - 1) / P.claim_variants;
-  const int grid = n_claims < n_sm ? n_claims : n_sm;
-  if (mode != PMT_PRECISION_FP32) {
-    PMT_CHECK(pmt_tc_supported(P), "this model shape is outside the tensor-core kernel's envelope; use PMT_PRECISION_FP32");
-    PmtOutputs o2 = *out;
-    o2.info_seq_be = info_seq;
-    if (saved) {   // training forward: deterministic tile list + the SAVE variant of the read kernel, operands kept for the backward
-      if (pmt_tc_forward_train(P, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.tiles), saved, n_sm, st)) return 1;
-    } else if (pmt_launch_reads_tc(P, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.tiles), reuse_images, n_sm, mode, st)) {
+  PmtOutputs o2 = *out;
+  o2.info_seq_be = info_seq;
+  if (C.reads == ReadsKernel::SIMT) {
+    const int n_claims = (batch->n_variants + P.claim_variants - 1) / P.claim_variants;
+    pmt_profile_begin(st);
+    reads_forward_kernel<<<n_claims < C.n_sm ? n_claims : C.n_sm, NTHREADS, smem, st>>>(P, A);
+    pmt_profile_end(st);
+  } else {
+    PMT_CHECK(C.reads_tc_ok, "this model shape is outside the tensor-core kernel's envelope; use PMT_PRECISION_FP32");
+    if (C.reads == ReadsKernel::TC_SAVE) {   // deterministic tile list + the SAVE variant of the read kernel, operands kept for the backward
+      if (pmt_tc_forward_train(C, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.tiles), saved, st)) return 1;
+    } else if (pmt_launch_reads_tc(C, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.tiles), reuse_images, st)) {
       return 1;
     }
-  } else {
-    pmt_profile_begin(st);
-    reads_forward_kernel<<<grid, NTHREADS, smem, st>>>(P, A);
-    pmt_profile_end(st);
   }
-  if (pmt_has_long_sets(batch) && mode != PMT_PRECISION_FP32 && L.long_tc_bytes > 0) {
+  if (C.lng == LongKernel::TC) {
     // sets longer than a tile, cut into single-side tiles on the same tensor-core pipeline (pmt_tc.cuh: LongTile)
-    PmtOutputs o2 = *out;
-    o2.info_seq_be = info_seq;
-    if (pmt_launch_reads_tc_long(P, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.long_tc), mode, st)) return 1;
-  } else if (pmt_has_long_sets(batch)) {
+    if (pmt_launch_reads_tc_long(C, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.long_tc), st)) return 1;
+  } else if (C.lng == LongKernel::SIMT) {
     A.scratch = reinterpret_cast<float*>(ws + L.long_scratch);
     A.scratch_stride = (long long)long_scratch_floats_per_cta(P, batch);
-    const int lgrid = long_grid(batch, n_sm < 148 ? n_sm : 148);
+    const int n_sm = C.n_sm < PMT_PARTIAL_CTAS ? C.n_sm : PMT_PARTIAL_CTAS;
     PMT_CUDA(cudaFuncSetAttribute(reads_forward_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    reads_forward_long_kernel<<<lgrid, NTHREADS, smem, st>>>(P, A);
+    reads_forward_long_kernel<<<batch->n_variants < n_sm ? batch->n_variants : n_sm, NTHREADS, smem, st>>>(P, A);
   }
   cudaError_t e = cudaGetLastError();
   PMT_CHECK(e == cudaSuccess, "pmt_forward launch failed: %s", cudaGetErrorString(e));

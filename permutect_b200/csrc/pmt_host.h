@@ -31,49 +31,6 @@ inline bool pmt_has_long_sets(const PmtBatch* batch) { return batch->max_rows_pe
 int pmt_build_plan(const PmtModelDesc* d, pmt::Plan* out);
 int pmt_cnn_geometry(const pmt::Plan& P, pmt::CnnGeom* out);
 size_t pmt_image_bytes(const pmt::Plan& P, const pmt::CnnGeom& G);
-int pmt_launch_prepare(const pmt::Plan& P, const pmt::CnnGeom& G, const float* weights, float* image, cudaStream_t st,
-                       bool need_gemm = true, bool need_conv = true);
-int pmt_launch_variant_kernels(const pmt::Plan& P, const pmt::CnnGeom& G, const float* weights, const float* image,
-                               const PmtBatch* batch, float* info_seq, int mode, unsigned char* cnn_tc_image, bool reuse_images,
-                               cudaStream_t st, bool skip_cnn = false);
-size_t pmt_backward_workspace_bytes(const pmt::Plan& P, const PmtBatch* batch);
 void pmt_profile_begin(cudaStream_t st);
 void pmt_profile_end(cudaStream_t st);
-int pmt_launch_cnn_backward(const pmt::Plan& P, const pmt::CnnGeom& G, const float* weights, const float* image,
-                            const PmtBatch* batch, const float* d_info_seq, float* partials, int n_partials, cudaStream_t st);
 int pmt_precision_mode();
-bool pmt_tc_supported(const pmt::Plan& P);
-size_t pmt_tc_image_bytes(const pmt::Plan& P);
-size_t pmt_tc_tiles_bytes(const PmtBatch* batch);
-// host: sets longer than a tile on the tensor-core forward.  pmt_tc_long_bytes() == 0: not available for this batch (no long
-// sets, unknown row count, or a set longer than one round of tiles) -- the FP32 long-set kernel takes them.
-size_t pmt_tc_long_bytes(const pmt::Plan& P, const PmtBatch* batch);
-int pmt_launch_reads_tc_long(const pmt::Plan& P, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
-                             unsigned char* image_buf, unsigned char* long_buf, int mode, cudaStream_t st);
-int pmt_launch_reads_tc(const pmt::Plan& P, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
-                        unsigned char* image_buf, unsigned char* tiles_buf, bool reuse_images, int n_sm, int mode, cudaStream_t st);
-size_t pmt_tc_bwd_workspace_bytes(const pmt::Plan& P, const PmtBatch* batch);
-int pmt_launch_reads_tc_backward(const pmt::Plan& P, const float* weights, const PmtBatch* batch, const float* info_seq,
-                                 const float* d_logits_bk, const float* d_alt_means, const float* d_ref_means, float* d_info_seq,
-                                 unsigned char* ws, size_t ws_bytes, int n_sm, int* grid_out, cudaStream_t st,
-                                 const unsigned char* saved = nullptr);
-// training without recompute (pmt_tc_bwd.cu, pmt_cnn_bwd.cu): the training forward saves what the backward would recompute
-size_t pmt_tc_train_saved_bytes(const pmt::Plan& P, const PmtBatch* batch);
-int pmt_tc_forward_train(const pmt::Plan& P, const float* weights, const PmtBatch* batch, const PmtOutputs* out, unsigned char* image_buf,
-                         unsigned char* claim_buf, unsigned char* saved, int n_sm, cudaStream_t st);
-size_t pmt_plan_claim_bytes(int n_variants, int n_sm);
-size_t pmt_cnn_train_saved_bytes(const pmt::Plan& P, const PmtBatch* batch);
-int pmt_cnn_forward_train(const pmt::Plan& P, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
-                          float* save, int n_sm, cudaStream_t st);
-int pmt_finish_reads_tc_backward(const pmt::Plan& P, const float* weights, const PmtBatch* batch, float* d_weights, unsigned char* ws,
-                                 int grid, cudaStream_t st);
-bool pmt_cnn_tc_supported(const pmt::Plan& P);
-size_t pmt_cnn_tc_image_bytes(const pmt::Plan& P);
-int pmt_launch_cnn_tc(const pmt::Plan& P, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
-                      bool reuse_image, int n_sm, int mode, cudaStream_t st);
-// host (pmt_cnn_bwd.cu): tensor-core (mma.sync TF32) backward of the haplotype CNN
-bool pmt_cnn_bwd_mma_supported(const pmt::Plan& P);
-size_t pmt_cnn_bwd_mma_workspace_bytes(const pmt::Plan& P, const PmtBatch* batch);
-int pmt_launch_cnn_backward_mma(const pmt::Plan& P, const float* weights, const PmtBatch* batch, float* info_seq, const float* d_info_seq,
-                                float* partials, int n_partials, unsigned char* ws, size_t ws_bytes, int n_sm, cudaStream_t st,
-                                const float* saved = nullptr);

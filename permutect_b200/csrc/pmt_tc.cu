@@ -26,7 +26,7 @@
 #include <cstdlib>
 #include <cstring>
 
-#include "pmt_tc.cuh"
+#include "pmt_call.h"
 
 namespace pmt {
 namespace tc {
@@ -1335,23 +1335,15 @@ void pmt_tc_plan(const Plan& P, TcPlan* out) {
   T.part_floats = pad_to(part + 8 * SCAL_W, 64);
 }
 
-static size_t tiles_bytes(int n_variants) { return ((size_t)(2 + 2 * (size_t)n_variants) * sizeof(int) + 255) & ~(size_t)255; }
 static size_t perm_bytes(int n_variants) { return ((size_t)n_variants * sizeof(int) + 255) & ~(size_t)255; }
 // Batches below this size keep the sequential planner: packing saves ~5.5 % of the read kernel (1.13 ns per read), the packed
 // planner costs ~0.1 ms more than the sequential one (one lane per claim places 512 sets), so it pays from ~2 M reads.
 static const long long kPackedPlannerMinRows = 2000000;
 
-size_t pmt_tc_image_bytes(const Plan& P) {
-  TcPlan T;
-  pmt_tc_plan(P, &T);
-  return (size_t)T.image_bytes + 2048;
-}
-size_t pmt_tc_tiles_bytes(const PmtBatch* batch) {
-  const int B = batch ? batch->n_variants : 0;
-  return tiles_bytes(B) + perm_bytes(B) + 256;
-}
+// the inference tile list and the packed planner's variant order
+size_t pmt_tc_tiles_bytes(int n_variants) { return pmt_tile_list_bytes(n_variants) + perm_bytes(n_variants) + 256; }
 
-static int plan_claim_variants(int n_variants, int n_sm) {
+int pmt_plan_claim_variants(int n_variants, int n_sm) {
   // planner claims: large enough that the partial last tile of a claim is a small loss, small enough that a small
   // batch is planned by many warps (each claim is walked sequentially)
   int claim_variants = n_variants / (2 * n_sm);
@@ -1360,7 +1352,7 @@ static int plan_claim_variants(int n_variants, int n_sm) {
   return claim_variants;
 }
 size_t pmt_plan_claim_bytes(int n_variants, int n_sm) {
-  const int cv = plan_claim_variants(n_variants, n_sm);
+  const int cv = pmt_plan_claim_variants(n_variants, n_sm);
   const size_t n_claims = ((size_t)n_variants + cv - 1) / cv;
   return (n_claims * (1 + 2 * (size_t)cv) * sizeof(int) + 255) & ~(size_t)255;
 }
@@ -1368,7 +1360,7 @@ size_t pmt_plan_claim_bytes(int n_variants, int n_sm) {
 // fixed (claim order); claim_buf: pmt_plan_claim_bytes() bytes.
 int pmt_plan_tiles(const PmtBatch* batch, int max_variants, bool deterministic, int n_sm, int* tiles, int* claim_buf, int* n_claims_out,
                    cudaStream_t st) {
-  const int claim_variants = plan_claim_variants(batch->n_variants, n_sm);
+  const int claim_variants = pmt_plan_claim_variants(batch->n_variants, n_sm);
   const int n_claims = (batch->n_variants + claim_variants - 1) / claim_variants;
   if (n_claims_out) *n_claims_out = n_claims;
   const long long* ro = reinterpret_cast<const long long*>(batch->ref_off);
@@ -1412,64 +1404,46 @@ int pmt_launch_reads_tc_save(const Plan& P, const TcPlan& T, const TcArgs& A, in
 }
 
 // Launches the tile planner, the weight packer (unless the images in `image_buf` are still valid) and the tensor-core
-// read kernel.  `image_buf`: pmt_tc_image_bytes(P) bytes; `tiles_buf`: pmt_tc_tiles_bytes(batch) bytes.
-int pmt_launch_reads_tc(const Plan& P, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
-                        unsigned char* image_buf, unsigned char* tiles_buf, bool reuse_images, int n_sm, int mode, cudaStream_t st) {
-  TcPlan T;
-  pmt_tc_plan(P, &T);
+// read kernel.  `image_buf`: the forward layout's tc_image region; `tiles_buf`: pmt_tc_tiles_bytes(B) bytes.
+int pmt_launch_reads_tc(const CallPlan& C, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
+                        unsigned char* image_buf, unsigned char* tiles_buf, bool reuse_images, cudaStream_t st) {
+  const TcPlan& T = C.T;
   unsigned char* image = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(image_buf) + 1023) & ~uintptr_t(1023));
   int* tiles = reinterpret_cast<int*>((reinterpret_cast<uintptr_t>(tiles_buf) + 255) & ~uintptr_t(255));
   int n_claims = 0;
   int* perm = nullptr;
   const char* pk = getenv("PMT_TC_PACKED");   // measurement: 0 = the sequential planner for every batch
-  const long long plan_rows = batch->n_rows > 0 ? batch->n_rows : 16LL * batch->n_variants;
-  if (plan_rows >= kPackedPlannerMinRows && !(pk && atoi(pk) == 0)) {
-    perm = reinterpret_cast<int*>(reinterpret_cast<unsigned char*>(tiles) + tiles_bytes(batch->n_variants));
+  if (pmt_row_hint(batch) >= kPackedPlannerMinRows && !(pk && atoi(pk) == 0)) {
+    perm = reinterpret_cast<int*>(reinterpret_cast<unsigned char*>(tiles) + pmt_tile_list_bytes(batch->n_variants));
     n_claims = (batch->n_variants + PLAN_CLAIM - 1) / PLAN_CLAIM;
     PMT_CUDA(cudaMemsetAsync(tiles, 0, 2 * sizeof(int), st));
     plan_tiles_packed_kernel<<<(n_claims + 3) / 4, 128, 0, st>>>(reinterpret_cast<const long long*>(batch->ref_off),
                                                                 reinterpret_cast<const long long*>(batch->alt_off), batch->n_variants,
                                                                 PLAN_CLAIM, tiles, perm);
-  } else if (pmt_plan_tiles(batch, TILE, false, n_sm, tiles, nullptr, &n_claims, st)) {
+  } else if (pmt_plan_tiles(batch, TILE, false, C.n_sm, tiles, nullptr, &n_claims, st)) {
     return 1;
   }
-  if (!reuse_images) pack_tc_kernel<<<dim3(T.n_steps, 8), 256, 0, st>>>(P.d, T, weights, image);
+  if (!reuse_images) pack_tc_kernel<<<dim3(T.n_steps, 8), 256, 0, st>>>(C.P.d, T, weights, image);
   TcArgs A;
   A.wflat = weights; A.image = image; A.tiles = tiles; A.perm = perm; A.batch = *batch; A.out = *out;
   A.scratch = nullptr; A.tile_first = 0; A.tile_limit = 0x7fffffff;
   { const char* e = getenv("PMT_TC_SCHED"); A.sched = (e && atoi(e) == 1) ? 1 : 0; }   // measurement: one slot only
-  // the tile count is only known on the device: size the grid from the row-count hint (a tile holds ~110 rows of
-  // whole variants); one CTA per tile until every SM has one, the second slot of each CTA after that
-  const long long rows = batch->n_rows > 0 ? batch->n_rows : 16LL * batch->n_variants;
-  long long est_tiles = rows / 100 + n_claims;   // n_claims from pmt_plan_tiles
-  if (est_tiles > batch->n_variants) est_tiles = batch->n_variants;
-  int grid = est_tiles < n_sm ? (int)est_tiles : n_sm;
-  if (grid < 1) grid = 1;
+  // the second slot of each CTA takes a second tile once every SM has one
+  const int grid = pmt_tile_grid(batch, n_claims, C.n_sm);
   pmt_profile_begin(st);
-  const int rc = mode == PMT_PRECISION_TF32 ? launch_reads_tc<1, false, false>(P.d, T, A, grid, st)
-                                         : launch_reads_tc<3, false, false>(P.d, T, A, grid, st);
+  const int rc = C.mode == PMT_PRECISION_TF32 ? launch_reads_tc<1, false, false>(C.P.d, T, A, grid, st)
+                                           : launch_reads_tc<3, false, false>(C.P.d, T, A, grid, st);
   pmt_profile_end(st);
   return rc;
 }
 
 // ---- sets longer than a tile (pmt_tc.cuh: LongTile) ----
-static int long_grid_sms() {
-  static int n_sm = 0;
-  if (n_sm == 0) {
-    int dev = 0, v = 148;
-    if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) v = 148;
-    n_sm = v;
-  }
-  return n_sm;
-}
-struct LongLayout {
-  int cap, max_tiles, R;
-  size_t list, n_tiles, tiles, counters, counters_bytes, mf_part, fin_part, end;
-};
-static bool long_layout(const Plan& P, const PmtBatch* batch, LongLayout* L) {
+// false: the long-set tensor-core path is not available for this batch (no long sets, unknown row count, a set longer than
+// one round of tiles, or PMT_LONG_SIMT=1) -- the FP32 long-set kernel takes them.
+bool pmt_tc_long_layout(const Plan& P, const PmtBatch* batch, int n_sm, LongLayout* L) {
   if (!batch || !pmt_has_long_sets(batch) || batch->n_rows <= 0 || !pmt_tc_supported(P)) return false;
   if (getenv("PMT_LONG_SIMT") && atoi(getenv("PMT_LONG_SIMT")) == 1) return false;   // measurement: the FP32 long-set kernel
-  const int R = 2 * long_grid_sms();
+  const int R = 2 * n_sm;
   const long long t_max = (batch->max_rows_per_variant + TILE - 1) / TILE + 1;        // ceil per side
   if (t_max > R) return false;
   long long cap = batch->n_rows / (TILE - 2);
@@ -1485,29 +1459,21 @@ static bool long_layout(const Plan& P, const PmtBatch* batch, LongLayout* L) {
   L->list = take((size_t)(1 + cap) * sizeof(int));
   L->n_tiles = take(256);
   L->tiles = take((size_t)max_tiles * sizeof(LongTile));
-  L->counters = off;
-  take((size_t)max_tiles * P.d.n_blocks * sizeof(int));
-  take((size_t)max_tiles * sizeof(int));
+  L->counters = take((size_t)max_tiles * P.d.n_blocks * sizeof(int));
+  L->fin_cnt = take((size_t)max_tiles * sizeof(int));
   L->counters_bytes = off - L->counters;
   L->mf_part = take((size_t)max_tiles * P.d.n_blocks * MAXH * sizeof(float));
   L->fin_part = take((size_t)max_tiles * LONG_FIN_W * sizeof(float));
-  L->end = off;
+  L->end = off + 1024;
   return true;
-}
-size_t pmt_tc_long_bytes(const Plan& P, const PmtBatch* batch) {
-  LongLayout L;
-  return long_layout(P, batch, &L) ? L.end + 1024 : 0;
 }
 
 // The sets plan_tiles_kernel left out, on the same tensor-core pipeline (the weight images in `image_buf` must be packed:
 // call after pmt_launch_reads_tc).  Every CTA of the grid has to be resident (a tile waits for the other tiles of its
 // set): one CTA per SM, grid = number of SMs.
-int pmt_launch_reads_tc_long(const Plan& P, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
-                             unsigned char* image_buf, unsigned char* long_buf, int mode, cudaStream_t st) {
-  LongLayout L;
-  PMT_CHECK(long_layout(P, batch, &L), "long-set tensor-core path not available for this batch");
-  TcPlan T;
-  pmt_tc_plan(P, &T);
+int pmt_launch_reads_tc_long(const CallPlan& C, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
+                             unsigned char* image_buf, unsigned char* long_buf, cudaStream_t st) {
+  const LongLayout& L = C.long_tc;
   unsigned char* image = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(image_buf) + 1023) & ~uintptr_t(1023));
   unsigned char* base = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(long_buf) + 255) & ~uintptr_t(255));
   int* list = reinterpret_cast<int*>(base + L.list);
@@ -1519,7 +1485,7 @@ int pmt_launch_reads_tc_long(const Plan& P, const float* weights, const PmtBatch
   PMT_CUDA(cudaMemsetAsync(tiles, 0xFF, (size_t)L.max_tiles * sizeof(LongTile), st));
   PMT_CUDA(cudaMemsetAsync(base + L.counters, 0, L.counters_bytes, st));
   int blocks = (batch->n_variants + 255) / 256;
-  if (blocks > 4 * long_grid_sms()) blocks = 4 * long_grid_sms();
+  if (blocks > 4 * C.n_sm) blocks = 4 * C.n_sm;
   long_list_kernel<<<blocks, 256, 0, st>>>(ro, ao, batch->n_variants, L.cap, list);
   long_layout_kernel<<<1, 1024, 0, st>>>(ro, ao, list, L.cap, L.R, L.max_tiles, tiles, n_tiles);
   TcArgs A;
@@ -1528,10 +1494,10 @@ int pmt_launch_reads_tc_long(const Plan& P, const float* weights, const PmtBatch
   A.scratch = nullptr; A.tile_first = 0; A.tile_limit = 0x7fffffff; A.sched = 0;
   A.lng.tiles = tiles; A.lng.n_tiles = n_tiles;
   A.lng.mf_cnt = reinterpret_cast<int*>(base + L.counters);
-  A.lng.fin_cnt = A.lng.mf_cnt + (size_t)(((size_t)L.max_tiles * P.d.n_blocks * sizeof(int) + 255) & ~(size_t)255) / sizeof(int);
+  A.lng.fin_cnt = reinterpret_cast<int*>(base + L.fin_cnt);
   A.lng.mf_part = reinterpret_cast<float*>(base + L.mf_part);
   A.lng.fin_part = reinterpret_cast<float*>(base + L.fin_part);
   const int grid = L.R / 2;
-  return mode == PMT_PRECISION_TF32 ? launch_reads_tc<1, false, true>(P.d, T, A, grid, st)
-                                     : launch_reads_tc<3, false, true>(P.d, T, A, grid, st);
+  return C.mode == PMT_PRECISION_TF32 ? launch_reads_tc<1, false, true>(C.P.d, C.T, A, grid, st)
+                                      : launch_reads_tc<3, false, true>(C.P.d, C.T, A, grid, st);
 }

@@ -323,14 +323,6 @@ __host__ __device__ __forceinline__ int proj1_bwd_col(int nb, int H) {
 
 // host: the step program of the forward (pmt_tc.cu)
 void pmt_tc_plan(const pmt::Plan& P, pmt::tc::TcPlan* out);
-// host: tensor-core backward of the tile-sized sets (pmt_tc_bwd.cu)
-size_t pmt_tc_bwd_workspace_bytes(const pmt::Plan& P, const PmtBatch* batch);
-int pmt_launch_reads_tc_backward(const pmt::Plan& P, const float* weights, const PmtBatch* batch, const float* info_seq,
-                                 const float* d_logits_bk, const float* d_alt_means, const float* d_ref_means, float* d_info_seq,
-                                 unsigned char* ws, size_t ws_bytes, int n_sm, int* grid_out, cudaStream_t st,
-                                 const unsigned char* saved);   // default argument: pmt_host.h
-int pmt_finish_reads_tc_backward(const pmt::Plan& P, const float* weights, const PmtBatch* batch, float* d_weights, unsigned char* ws,
-                                 int grid, cudaStream_t st);
 int pmt_launch_pack_tc(const pmt::Plan& P, const pmt::tc::TcPlan& T, const float* weights, unsigned char* image, cudaStream_t st);
 // training recompute: the forward over tiles [tile_first, tile_limit) of a planned tile list, operands saved to `scratch`
 int pmt_launch_reads_tc_save(const pmt::Plan& P, const pmt::tc::TcPlan& T, const pmt::tc::TcArgs& A, int grid, cudaStream_t st);

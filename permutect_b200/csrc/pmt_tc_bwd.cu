@@ -26,7 +26,7 @@
 #include <cstdlib>
 #include <cstring>
 
-#include "pmt_tc.cuh"
+#include "pmt_call.h"
 
 namespace pmt {
 namespace tc {
@@ -822,16 +822,22 @@ __global__ void unfold_kernel(const __grid_constant__ PmtModelDesc D, const __gr
 using namespace pmt;
 using namespace pmt::tc;
 
-size_t pmt_plan_claim_bytes(int n_variants, int n_sm);
-
-static const int kMaxGrid = 148;
 // Tiles per recompute / backward pass: bounds the operand scratch (0.7 MB per tile: 5.9 GB).  The scratch is streamed through
 // HBM either way (it never was L2-sized), so fewer, longer passes only save launches -- the tile bound is an upper bound and most
 // passes beyond the first found nothing to do -- and the partly filled last round of every pass.
 static const int kChunkTiles = 8192;
+// measured: 9 GB (65 536 variants) wins 14 %, 27 GB (200 000) loses to the recompute
+static const size_t kTrainSavedBudget = (size_t)16 << 30;
+static const unsigned kTrainSavedMagic = 0x544d5031u;
+
+// claims of the training tile list (planned with PMT_PARTIAL_CTAS for the SM count, whatever the device)
+static int train_claims(int n_variants) {
+  const int cv = pmt_plan_claim_variants(n_variants, PMT_PARTIAL_CTAS);
+  return n_variants > 0 ? (n_variants + cv - 1) / cv : 0;
+}
 
 static long long tile_bound(const PmtBatch* batch, int n_claims) {
-  const long long rows = batch->n_rows > 0 ? batch->n_rows : 16LL * batch->n_variants;
+  const long long rows = pmt_row_hint(batch);
   // a tile is closed when the next set does not fit or it holds BWD_MAXV sets; the last tile of a claim may be short
   long long bound = 2 * rows / TILE + batch->n_variants / BWD_MAXV + n_claims + 8;
   if (batch->max_rows_per_variant > 0) {
@@ -844,27 +850,19 @@ static long long tile_bound(const PmtBatch* batch, int n_claims) {
   return bound < 1 ? 1 : bound;
 }
 
-struct BwdLayout {
-  size_t image_f, image_t, tiles, claims, partials, reduced, scratch, total;
-  int chunk_tiles, n_chunks, n_claims;
-};
-
-static BwdLayout bwd_layout(const TcPlan& T, const PmtBatch* batch, int n_sm) {
+BwdLayout pmt_tc_bwd_layout(const TcPlan& T, const PmtBatch* batch) {
   BwdLayout L;
   memset(&L, 0, sizeof(L));
   const int B = batch ? batch->n_variants : 0;
   size_t off = 1024;
   L.image_f = off; off += (size_t)T.image_bytes + 2048;
   L.image_t = off; off += (size_t)T.t_image_bytes + 2048;
-  L.tiles = off; off += ((size_t)(2 + 2 * (size_t)B) * sizeof(int) + 511) & ~(size_t)255;
-  L.claims = off; off += pmt_plan_claim_bytes(B, n_sm) + 256;
-  L.partials = off; off += (size_t)2 * kMaxGrid * T.part_floats * sizeof(float);
+  L.tiles = off; off += pmt_tile_list_bytes(B) + 256;
+  L.claims = off; off += pmt_plan_claim_bytes(B, PMT_PARTIAL_CTAS) + 256;
+  L.partials = off; off += (size_t)2 * PMT_PARTIAL_CTAS * T.part_floats * sizeof(float);
   L.reduced = off; off += (size_t)T.part_floats * sizeof(float) + 256;
   off = (off + 1023) & ~(size_t)1023;
-  int cv = B / (2 * n_sm);
-  if (cv < 64) cv = 64;
-  if (cv > PLAN_CLAIM) cv = PLAN_CLAIM;
-  L.n_claims = B > 0 ? (B + cv - 1) / cv : 0;
+  L.n_claims = train_claims(B);
   const long long bound = batch ? tile_bound(batch, L.n_claims) : 1;
   int chunk_cap = kChunkTiles;
   if (const char* e = getenv("PMT_BWD_CHUNK_TILES")) { const int v = atoi(e); if (v >= 1) chunk_cap = v; }   // tests: several passes on a small batch
@@ -875,29 +873,18 @@ static BwdLayout bwd_layout(const TcPlan& T, const PmtBatch* batch, int n_sm) {
   return L;
 }
 
-// ---- training without recompute: what the training forward leaves for the backward (pmt_forward_train) ----
-// [256-byte header][tile list][operand scratch of EVERY tile of the (deterministic) list].  The tile count is only known
-// on the device, so the scratch is sized for the bound; over the budget the caller keeps the recompute.
-static const size_t kTrainSavedBudget = (size_t)16 << 30;   // measured: 9 GB (65 536 variants) wins 14 %, 27 GB (200 000) loses to the recompute
-static const unsigned kTrainSavedMagic = 0x544d5031u;
-struct TrainSavedLayout { size_t tiles, scratch, total; long long bound; };
-static TrainSavedLayout train_saved_layout(const TcPlan& T, const PmtBatch* batch) {
-  TrainSavedLayout S;
-  const BwdLayout L = bwd_layout(T, batch, kMaxGrid);
-  S.bound = tile_bound(batch, L.n_claims);
+SavedLayout pmt_saved_layout(const CallPlan& C, const PmtBatch* batch) {
+  SavedLayout S;
+  memset(&S, 0, sizeof(S));
+  if (C.mode != PMT_PRECISION_TF32X3 || !batch || batch->n_variants <= 0 || !C.reads_tc_ok || !C.cnn_bwd_ok) return S;
+  const int B = batch->n_variants;
+  S.bound = tile_bound(batch, train_claims(B));
   S.tiles = 256;
-  size_t off = S.tiles + (((size_t)(2 + 2 * (size_t)batch->n_variants) * sizeof(int) + 511) & ~(size_t)255);
-  off = (off + 1023) & ~(size_t)1023;
-  S.scratch = off;
-  S.total = off + (size_t)S.bound * T.tile_bytes + 1024;
+  S.scratch = (S.tiles + pmt_tile_list_bytes(B) + 256 + 1023) & ~(size_t)1023;
+  S.cnn = (S.scratch + (size_t)S.bound * C.T.tile_bytes + 1024 + 1023) & ~(size_t)1023;
+  const size_t total = S.cnn + ((size_t)B + C.C.G - 1) / C.C.G * C.CB.group_floats * sizeof(float) + 256 + 1024;
+  if (total <= kTrainSavedBudget) S.total = total;
   return S;
-}
-size_t pmt_tc_train_saved_bytes(const Plan& P, const PmtBatch* batch) {
-  if (!batch || batch->n_variants <= 0 || !pmt_tc_supported(P)) return 0;
-  TcPlan T;
-  pmt_tc_plan(P, &T);
-  const TrainSavedLayout S = train_saved_layout(T, batch);
-  return S.total <= kTrainSavedBudget ? S.total : 0;
 }
 
 // The operand scratch is sized from an upper bound of the tile count (tile_bound): should the planner ever produce more
@@ -910,54 +897,41 @@ __global__ void check_tile_bound_kernel(const int* __restrict__ tiles, int bound
 }
 
 // The training forward of the tile-sized sets: deterministic tile list, then the SAVE variant of the read kernel over ALL
-// tiles with the outputs switched on.  `image_buf`: pmt_tc_image_bytes(P) bytes (forward weight images, packed here);
-// `claim_buf`: pmt_plan_claim_bytes(B, 148) + 256 bytes of scratch for the planner.
-int pmt_tc_forward_train(const Plan& P, const float* weights, const PmtBatch* batch, const PmtOutputs* out, unsigned char* image_buf,
-                         unsigned char* claim_buf, unsigned char* saved, int n_sm, cudaStream_t st) {
-  TcPlan T;
-  pmt_tc_plan(P, &T);
-  if (n_sm > kMaxGrid) n_sm = kMaxGrid;
-  const TrainSavedLayout S = train_saved_layout(T, batch);
+// tiles with the outputs switched on.  `image_buf`: the forward layout's tc_image region (weight images, packed here);
+// `claim_buf`: the forward layout's planner scratch.
+int pmt_tc_forward_train(const CallPlan& C, const float* weights, const PmtBatch* batch, const PmtOutputs* out, unsigned char* image_buf,
+                         unsigned char* claim_buf, unsigned char* saved, cudaStream_t st) {
+  const TcPlan& T = C.T;
+  const SavedLayout& S = C.saved;
   unsigned char* image = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(image_buf) + 1023) & ~uintptr_t(1023));
   int* tiles = reinterpret_cast<int*>(saved + S.tiles);
   int* claims = reinterpret_cast<int*>((reinterpret_cast<uintptr_t>(claim_buf) + 255) & ~uintptr_t(255));
   int n_claims = 0;
-  if (pmt_plan_tiles(batch, BWD_MAXV, true, kMaxGrid, tiles, claims, &n_claims, st)) return 1;
+  if (pmt_plan_tiles(batch, BWD_MAXV, true, PMT_PARTIAL_CTAS, tiles, claims, &n_claims, st)) return 1;
   check_tile_bound_kernel<<<1, 1, 0, st>>>(tiles, (int)S.bound);
-  if (pmt_launch_pack_tc(P, T, weights, image, st)) return 1;
+  if (pmt_launch_pack_tc(C.P, T, weights, image, st)) return 1;
   const unsigned header[4] = {kTrainSavedMagic, (unsigned)batch->n_variants, (unsigned)S.bound, 0u};
   PMT_CUDA(cudaMemcpyAsync(saved, header, sizeof(header), cudaMemcpyHostToDevice, st));
-  const long long rows = batch->n_rows > 0 ? batch->n_rows : 16LL * batch->n_variants;
-  long long est_tiles = rows / 100 + n_claims;
-  if (est_tiles > batch->n_variants) est_tiles = batch->n_variants;
-  int grid = est_tiles < n_sm ? (int)est_tiles : n_sm;
-  if (grid < 1) grid = 1;
+  const int grid = pmt_tile_grid(batch, n_claims, C.n_sm < PMT_PARTIAL_CTAS ? C.n_sm : PMT_PARTIAL_CTAS);
   TcArgs F;
   memset(&F, 0, sizeof(F));
   F.wflat = weights; F.image = image; F.tiles = tiles; F.perm = nullptr; F.batch = *batch; F.out = *out;
   F.scratch = saved + S.scratch; F.sched = 0; F.tile_first = 0; F.tile_limit = (int)S.bound;
   pmt_profile_begin(st);
-  const int rc = pmt_launch_reads_tc_save(P, T, F, grid, st);
+  const int rc = pmt_launch_reads_tc_save(C.P, T, F, grid, st);
   pmt_profile_end(st);
   return rc;
 }
 
-size_t pmt_tc_bwd_workspace_bytes(const Plan& P, const PmtBatch* batch) {
-  TcPlan T;
-  pmt_tc_plan(P, &T);
-  return bwd_layout(T, batch, kMaxGrid).total;
-}
-
 // Backward of the tile-sized read sets: writes d_info_seq for the variants of those sets and leaves the weight gradients
-// in the private buffers of the workspace; pmt_finish_reads_tc_backward adds them to d_weights.
-int pmt_launch_reads_tc_backward(const Plan& P, const float* weights, const PmtBatch* batch, const float* info_seq,
+// in the private buffers of the workspace; pmt_finish_reads_tc_backward adds them to d_weights.  `ws`: the backward
+// layout's tensor-core region (C.tc_bwd.total + 1024 bytes).
+int pmt_launch_reads_tc_backward(const CallPlan& C, const float* weights, const PmtBatch* batch, const float* info_seq,
                                  const float* d_logits_bk, const float* d_alt_means, const float* d_ref_means, float* d_info_seq,
-                                 unsigned char* ws, size_t ws_bytes, int n_sm, int* grid_out, cudaStream_t st, const unsigned char* saved) {
-  TcPlan T;
-  pmt_tc_plan(P, &T);
-  if (n_sm > kMaxGrid) n_sm = kMaxGrid;
+                                 unsigned char* ws, size_t ws_bytes, int* grid_out, cudaStream_t st, const unsigned char* saved) {
+  const TcPlan& T = C.T;
+  const BwdLayout& L = C.tc_bwd;
   unsigned char* base = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 1023) & ~uintptr_t(1023));
-  const BwdLayout L = bwd_layout(T, batch, kMaxGrid);
   PMT_CHECK((size_t)(base - ws) + L.total <= ws_bytes + 1024, "tensor-core backward: workspace too small (%zu < %zu)", ws_bytes, L.total);
   unsigned char* image_f = base + L.image_f;
   unsigned char* image_t = base + L.image_t;
@@ -967,26 +941,18 @@ int pmt_launch_reads_tc_backward(const Plan& P, const float* weights, const PmtB
   unsigned char* scratch = base + L.scratch;
 
   int n_claims = 0;
-  TrainSavedLayout SV;
-  memset(&SV, 0, sizeof(SV));
   if (saved) {   // the training forward left the tile list and every tile's operands (pmt_tc_forward_train): no recompute
-    SV = train_saved_layout(T, batch);
-    tiles = const_cast<int*>(reinterpret_cast<const int*>(saved + SV.tiles));
-    scratch = const_cast<unsigned char*>(saved + SV.scratch);
+    tiles = const_cast<int*>(reinterpret_cast<const int*>(saved + C.saved.tiles));
+    scratch = const_cast<unsigned char*>(saved + C.saved.scratch);
     n_claims = L.n_claims;
   } else {
-    if (pmt_plan_tiles(batch, BWD_MAXV, true, kMaxGrid, tiles, claims, &n_claims, st)) return 1;
-    if (pmt_launch_pack_tc(P, T, weights, image_f, st)) return 1;
+    if (pmt_plan_tiles(batch, BWD_MAXV, true, PMT_PARTIAL_CTAS, tiles, claims, &n_claims, st)) return 1;
+    if (pmt_launch_pack_tc(C.P, T, weights, image_f, st)) return 1;
   }
-  pack_tc_bwd_kernel<<<dim3(T.n_steps, 8), 256, 0, st>>>(P.d, T, weights, image_t);
+  pack_tc_bwd_kernel<<<dim3(T.n_steps, 8), 256, 0, st>>>(C.P.d, T, weights, image_t);
 
-  const long long rows = batch->n_rows > 0 ? batch->n_rows : 16LL * batch->n_variants;
-  long long est_tiles = rows / 100 + n_claims;
-  if (est_tiles > batch->n_variants) est_tiles = batch->n_variants;
-  int grid = est_tiles < n_sm ? (int)est_tiles : n_sm;
-  if (grid < 1) grid = 1;
+  const int grid = pmt_tile_grid(batch, n_claims, C.n_sm < PMT_PARTIAL_CTAS ? C.n_sm : PMT_PARTIAL_CTAS);
   PMT_CUDA(cudaMemsetAsync(partials, 0, (size_t)2 * grid * T.part_floats * sizeof(float), st));
-
   const int stage_bytes = (T.t_stage_bytes + 1023) & ~1023;
   const size_t fixed = 2 * OPBUF_BYTES + 2 * BXCH_ROWS * XCH_LD * sizeof(float) + 2 * 3 * BW_TAB * sizeof(float) + 2 * 2 * TILE * 4 * sizeof(float) +
                        PMT_MAX_BLOCKS * BC_STRIDE * sizeof(float) + sizeof(HeadConst) + sizeof(SharedB) + 1024 + 64;
@@ -1009,8 +975,8 @@ int pmt_launch_reads_tc_backward(const Plan& P, const float* weights, const PmtB
     F.tile_first = Bk.tile_first = c * L.chunk_tiles;
     F.tile_limit = Bk.tile_limit = (c + 1) * L.chunk_tiles;
     if (saved) Bk.scratch = scratch + (size_t)Bk.tile_first * T.tile_bytes;   // the kernel indexes a pass's scratch from its first tile
-    else if (pmt_launch_reads_tc_save(P, T, F, grid, st)) return 1;
-    reads_backward_tc_kernel<<<grid, THREADS, smem, st>>>(P.d, T, Bk, n_stages, stage_bytes);
+    else if (pmt_launch_reads_tc_save(C.P, T, F, grid, st)) return 1;
+    reads_backward_tc_kernel<<<grid, THREADS, smem, st>>>(C.P.d, T, Bk, n_stages, stage_bytes);
   }
   pmt_profile_end(st);
   *grid_out = grid;
@@ -1021,16 +987,13 @@ int pmt_launch_reads_tc_backward(const Plan& P, const float* weights, const PmtB
 
 // d_weights += the tile-sized sets' gradient (call after the other kernels' sums have been WRITTEN to d_weights and before
 // skip_fix_kernel: the last layer of a DenseSkipBlock is handed over un-scaled, as the SIMT kernels do).
-int pmt_finish_reads_tc_backward(const Plan& P, const float* weights, const PmtBatch* batch, float* d_weights, unsigned char* ws, int grid,
-                                 cudaStream_t st) {
-  TcPlan T;
-  pmt_tc_plan(P, &T);
+int pmt_finish_reads_tc_backward(const CallPlan& C, const float* weights, float* d_weights, unsigned char* ws, int grid, cudaStream_t st) {
+  const TcPlan& T = C.T;
   unsigned char* base = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 1023) & ~uintptr_t(1023));
-  const BwdLayout L = bwd_layout(T, batch, kMaxGrid);
-  const float* partials = reinterpret_cast<const float*>(base + L.partials);
-  float* reduced = reinterpret_cast<float*>(base + L.reduced);
+  const float* partials = reinterpret_cast<const float*>(base + C.tc_bwd.partials);
+  float* reduced = reinterpret_cast<float*>(base + C.tc_bwd.reduced);
   reduce_private_kernel<<<(T.part_floats + 255) / 256, 256, 0, st>>>(partials, 2 * grid, T.part_floats, reduced);
-  unfold_kernel<<<T.n_steps + P.d.n_blocks + 1, 256, 0, st>>>(P.d, T, weights, reduced, d_weights);
+  unfold_kernel<<<T.n_steps + C.P.d.n_blocks + 1, 256, 0, st>>>(C.P.d, T, weights, reduced, d_weights);
   cudaError_t e = cudaGetLastError();
   PMT_CHECK(e == cudaSuccess, "tensor-core backward (unfold) launch failed: %s", cudaGetErrorString(e));
   return 0;
