@@ -53,16 +53,16 @@ def decode_reads(reads_u8: np.ndarray) -> np.ndarray:
     return np.hstack((bits, wrapped.astype(np.float32) / 32.0))
 
 
-def one_hot_haplotypes(haplotypes: Tensor) -> Tensor:
+def one_hot_haplotypes(haplotypes: Tensor, dtype=torch.float32) -> Tensor:
     """batch.py:115-130.  [B,2L] codes -> [B,10,L]; channel 2c is 'ref has code c', 2c+1 'alt has code c'."""
     B, two_l = haplotypes.shape
     L = two_l // 2
-    out = torch.zeros(B, 10, L, dtype=torch.float32)
+    out = torch.zeros(B, 10, L, dtype=dtype)
     codes = haplotypes.long()
     for half in range(2):                       # 0 = ref haplotype, 1 = alt haplotype
         h = codes[:, half * L:(half + 1) * L]   # [B,L]
         for c in range(5):
-            out[:, 2 * c + half, :] = (h == c).float()
+            out[:, 2 * c + half, :] = (h == c).to(dtype)
     return out
 
 
@@ -265,19 +265,27 @@ def gather_reads(raw: dict) -> Tensor:
     return reads
 
 
-def forward(sd: Dict[str, Tensor], hp: dict, raw: dict) -> dict:
+def cast_state_dict(sd: Dict[str, Tensor], dtype) -> Dict[str, Tensor]:
+    """The floating-point tensors of ``sd`` in ``dtype`` (a no-op, graph included, when they already are)."""
+    return {k: (v.to(dtype) if v.dtype.is_floating_point else v) for k, v in sd.items()}
+
+
+def forward(sd: Dict[str, Tensor], hp: dict, raw: dict, dtype=torch.float32) -> dict:
     """artifact_model.py:239-297.  Returns every BatchOutput field plus the intermediates the
-    tests compare (per-read final features, info/seq embedding)."""
+    tests compare (per-read final features, info/seq embedding).  ``dtype=torch.float64`` casts the
+    state dict and every input on entry, so the whole restatement runs in double precision: the
+    high-precision reference the kernels are measured against."""
+    sd = cast_state_dict(sd, dtype)
     ref_counts = torch.as_tensor(np.asarray(raw["ref_counts"])).long()
     alt_counts = torch.as_tensor(np.asarray(raw["alt_counts"])).long()
     total_ref = int(ref_counts.sum())
-    reads = gather_reads(raw)
-    info = torch.as_tensor(np.asarray(raw["info"], dtype=np.float32))
+    reads = gather_reads(raw).to(dtype)
+    info = torch.as_tensor(np.asarray(raw["info"], dtype=np.float32)).to(dtype)
     haps = torch.as_tensor(np.asarray(raw["haplotypes"]))
 
     read_emb = mlp(sd, "read_embedding", [reads.shape[1]] + list(hp["read_layers"]), reads)
     info_emb = mlp(sd, "info_embedding", [info.shape[1]] + list(hp["info_layers"]), info)
-    seq_emb = haplotype_cnn(sd, "haplotypes_cnn", hp["ref_seq_layer_strings"], one_hot_haplotypes(haps))
+    seq_emb = haplotype_cnn(sd, "haplotypes_cnn", hp["ref_seq_layer_strings"], one_hot_haplotypes(haps, dtype))
     info_seq = torch.hstack((info_emb, seq_emb))
     per_read = torch.vstack((info_seq[segment_ids(ref_counts)], info_seq[segment_ids(alt_counts)]))
     x = torch.hstack((read_emb, per_read))
@@ -309,43 +317,46 @@ def source_predictor_sizes(num_sources: int, feat: int) -> List[int]:
 
 def losses(sd, hp: dict, raw: dict, out: dict, weights: Optional[Tensor] = None,
            source_weights: Optional[Tensor] = None, num_sources: int = 1,
-           source_adversarial_strength: float = 0.01) -> dict:
-    """artifact_model.py:299-325 with :267-279."""
+           source_adversarial_strength: float = 0.01, dtype=torch.float32) -> dict:
+    """artifact_model.py:299-325 with :267-279.  ``dtype``: as in ``forward`` (labels, weights and the
+    loss constants are cast too)."""
+    sd = cast_state_dict(sd, dtype)
     labels_int = torch.as_tensor(np.asarray(raw["labels"])).long()
     alt_counts = torch.as_tensor(np.asarray(raw["alt_counts"])).long()
-    labels = 1.0 * (labels_int == LABEL_ARTIFACT) + 0.5 * (labels_int == LABEL_UNLABELED)   # batch.py:100-102
-    is_labeled = (labels_int != LABEL_UNLABELED).float()
+    labels = (1.0 * (labels_int == LABEL_ARTIFACT) + 0.5 * (labels_int == LABEL_UNLABELED)).to(dtype)   # batch.py:100-102
+    is_labeled = (labels_int != LABEL_UNLABELED).to(dtype)
     B = len(labels_int)
-    weights = torch.ones(B) if weights is None else weights
-    source_weights = weights if source_weights is None else source_weights
+    weights = torch.ones(B, dtype=dtype) if weights is None else weights.to(dtype)
+    source_weights = weights if source_weights is None else source_weights.to(dtype)
     bce = lambda logit, target: F.binary_cross_entropy_with_logits(logit, target, reduction="none")
     supervised = is_labeled * bce(out["logits_b"], labels)
     clipped = out["outlier_binary_logits"].clamp(max=MAX_OUTLIER_LOGIT)
-    unsupervised = (1 - is_labeled) * bce(clipped, torch.zeros(B))
+    unsupervised = (1 - is_labeled) * bce(clipped, torch.zeros(B, dtype=dtype))
     feats = out["features_be"]
     E = feats.shape[1]
     pred = torch.sigmoid(mlp(sd, "alt_count_predictor.wrapped_module", [E, 30, -1, -1, -1, 1],
                              reverse_gradient(feats, 0.01)).view(-1))                   # artifact_model.py:180-182,276-279
-    alt_count = torch.square(pred - alt_counts.float() / MAX_ALT_COUNT)
+    alt_count = torch.square(pred - alt_counts.to(dtype) / MAX_ALT_COUNT)
     if num_sources > 1:                                                                # artifact_model.py:267-274
         src_logits = mlp(sd, "source_predictor.wrapped_module", source_predictor_sizes(num_sources, E),
                          reverse_gradient(feats, source_adversarial_strength))
-        onehot = F.one_hot(torch.as_tensor(np.asarray(raw["sources"])).long(), num_sources)
+        onehot = F.one_hot(torch.as_tensor(np.asarray(raw["sources"])).long(), num_sources).to(dtype)
         source = torch.sum(torch.square(torch.softmax(src_logits, dim=-1) - onehot), dim=-1)
     else:
-        source = torch.zeros(B)
+        source = torch.zeros(B, dtype=dtype)
     total_b = weights * (supervised + unsupervised + alt_count) + source_weights * source
     return dict(supervised_losses_b=supervised, unsupervised_losses_b=unsupervised, alt_count_losses_b=alt_count,
                 source_prediction_losses_b=source, total_losses_b=total_b, total_loss=total_b.sum())
 
 
-def loss_and_grads(sd: Dict[str, Tensor], hp: dict, raw: dict, trainable: Sequence[str], **loss_kw):
+def loss_and_grads(sd: Dict[str, Tensor], hp: dict, raw: dict, trainable: Sequence[str], dtype=torch.float32, **loss_kw):
     """Autograd through the restatement: gradient of total_loss w.r.t. the named state-dict tensors
-    (what ``loss.backward()`` leaves in ``param.grad``, misc_utils.py:125-127, before clipping)."""
-    leaf = {k: (v.detach().clone().requires_grad_(k in trainable) if v.dtype.is_floating_point else v)
+    (what ``loss.backward()`` leaves in ``param.grad``, misc_utils.py:125-127, before clipping).
+    With ``dtype=torch.float64`` the leaves, and so autograd, are double precision throughout."""
+    leaf = {k: (v.detach().to(dtype).clone().requires_grad_(k in trainable) if v.dtype.is_floating_point else v)
             for k, v in sd.items()}
-    out = forward(leaf, hp, raw)
-    ls = losses(leaf, hp, raw, out, **loss_kw)
+    out = forward(leaf, hp, raw, dtype=dtype)
+    ls = losses(leaf, hp, raw, out, dtype=dtype, **loss_kw)
     names = [k for k in trainable if leaf[k].requires_grad]
     grads = torch.autograd.grad(ls["total_loss"], [leaf[k] for k in names], allow_unused=True)
     return out, ls, {k: (g if g is not None else torch.zeros_like(leaf[k])) for k, g in zip(names, grads)}

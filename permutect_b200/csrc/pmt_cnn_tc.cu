@@ -472,6 +472,10 @@ bool pmt_build_cnn_tc_plan(const pmt::Plan& P, cnntc::Plan* out) {
   T.image_bytes = bytes;
   // variants per group: every layer's rows must fit MAX_CHUNKS chunks and the planes; pick the G with the fewest MMA
   // cycles per variant
+  // Every layer's weight image stays resident in shared memory next to the two activation buffers: that is the kernel's
+  // capacity limit.  v0.4.0's layer strings on haplotypes of 21 bases fit with 4.4 KB to spare; on 25 bases they leave
+  // 2 positions to the flatten, whose 2-tap Linear image (16 KB instead of 8 KB) is 3.6 KB too many, and that shape runs
+  // on the FP32 SIMT kernel (hap_cnn_kernel).
   const int fixed = 2 * BUF_BYTES + bytes + MAX_LAYERS * 32 * 4 + (int)sizeof(Bars) + 1024 + 64;
   if (fixed > 227 * 1024) return false;
   double best = 1e30;

@@ -655,6 +655,10 @@ int pmt_build_plan(const PmtModelDesc* d, Plan* out) {
   PMT_CHECK(d->n_info_features <= PMT_MAX_INFO_DIM, "n_info_features %d > %d", d->n_info_features, PMT_MAX_INFO_DIM);
   PMT_CHECK(d->d_model <= PMT_MAX_DIM && d->d_model == d->d_read + d->d_info + d->d_seq, "d_model %d unsupported", d->d_model);
   PMT_CHECK(d->d_ffn <= PMT_MAX_DIM && d->d_ffn % 2 == 0, "d_ffn %d unsupported", d->d_ffn);
+  // d_ffn 2: the spatial gating unit's LayerNorm sees one feature and outputs its bias whatever the input, so the ref reads
+  // never reach the loss and the gradients through that LayerNorm are rounding noise scaled by 1 / sqrt(eps)
+  PMT_CHECK(d->d_ffn >= 4, "d_ffn %d: self_attention_hidden_dimension must be at least 4 (a one-feature spatial gating unit "
+            "is constant)", d->d_ffn);
   PMT_CHECK(d->d_feat <= PMT_MAX_FEAT && d->n_clusters <= PMT_MAX_CLUSTERS && d->n_clusters >= 1, "d_feat/n_clusters unsupported");
   PMT_CHECK(d->n_blocks <= PMT_MAX_BLOCKS, "too many gated blocks");
   PMT_CHECK(d->n_read_ops <= PMT_MAX_MLP_OPS && d->n_info_ops <= PMT_MAX_MLP_OPS && d->n_red_ops <= PMT_MAX_MLP_OPS &&
@@ -782,6 +786,10 @@ int pmt_call_plan(const PmtModelDesc* desc, const PmtBatch* batch, bool train, C
   C.cnn_tc_ok = pmt_build_cnn_tc_plan(P, &C.C);
   C.cnn_bwd_ok = C.cnn_tc_ok && pmt_build_cnn_bwd_plan(P, C.C, &C.CB);
   const bool fp32 = C.mode == PMT_PRECISION_FP32;
+  // the backward: the tensor-core read-path and haplotype-CNN kernels (pmt_tc_bwd.cu, pmt_cnn_bwd.cu) unless the FP32 mode
+  // is selected or the model is outside their envelope, the FP32 SIMT kernels otherwise
+  C.bwd_reads_tc = !fp32 && C.reads_tc_ok;
+  C.bwd_cnn_tc = !fp32 && C.cnn_bwd_ok;
   C.saved = pmt_saved_layout(C, batch);
   train = train && C.saved.total > 0;
   const int B = batch ? batch->n_variants : 0;
@@ -796,10 +804,6 @@ int pmt_call_plan(const PmtModelDesc* desc, const PmtBatch* batch, bool train, C
   // haplotype CNN (shapes outside the tensor-core envelope) -- and, depending on the batch, the FP32 long-set kernel
   C.simt_gemm = fp32 || C.info == InfoKernel::TILE;
   C.simt_conv = C.cnn == CnnKernel::SIMT;
-  // the backward: the tensor-core read-path and haplotype-CNN kernels (pmt_tc_bwd.cu, pmt_cnn_bwd.cu) unless the FP32 mode
-  // is selected or the model is outside their envelope, the FP32 SIMT kernels otherwise
-  C.bwd_reads_tc = !fp32 && C.reads_tc_ok;
-  C.bwd_cnn_tc = !fp32 && C.cnn_bwd_ok;
   C.tc_bwd = pmt_tc_bwd_layout(C.T, batch);
   return 0;
 }

@@ -876,7 +876,7 @@ BwdLayout pmt_tc_bwd_layout(const TcPlan& T, const PmtBatch* batch) {
 SavedLayout pmt_saved_layout(const CallPlan& C, const PmtBatch* batch) {
   SavedLayout S;
   memset(&S, 0, sizeof(S));
-  if (C.mode != PMT_PRECISION_TF32X3 || !batch || batch->n_variants <= 0 || !C.reads_tc_ok || !C.cnn_bwd_ok) return S;
+  if (C.mode != PMT_PRECISION_TF32X3 || !batch || batch->n_variants <= 0 || !C.bwd_reads_tc || !C.bwd_cnn_tc) return S;
   const int B = batch->n_variants;
   S.bound = tile_bound(batch, train_claims(B));
   S.tiles = 256;

@@ -50,3 +50,24 @@ def test_gradients_match_reference(case):
         got = grads[k].numpy()
         scale = max(1.0, float(np.abs(want).max()))
         np.testing.assert_allclose(got, want, rtol=1e-3, atol=2e-5 * scale, err_msg=k)
+
+
+@pytest.mark.parametrize("case", CASES)
+def test_float64_oracle_computes_the_same_function(case):
+    """The double-precision oracle (the reference the kernel tests measure against) agrees with the float32 one, which the
+    fixtures pin, to float32 rounding: forward values, losses and every parameter gradient.  The absolute 1e-4 is the
+    float32 rounding accumulated over ~45 layers (measured up to 3.3e-5 on a logit), a tenth of the kernels' contract."""
+    g = load(case)
+    trainable = list(g.grad.keys())
+    kw = dict(num_sources=g.hp["num_sources"], source_adversarial_strength=g.hp["source_adversarial_strength"])
+    out32, ls32, gr32 = orc.loss_and_grads(g.sd, g.hp, g.raw(), trainable, **kw)
+    out64, ls64, gr64 = orc.loss_and_grads(g.sd, g.hp, g.raw(), trainable, dtype=torch.float64, **kw)
+    assert all(v.dtype == torch.float64 for v in out64.values()) and all(v.dtype == torch.float64 for v in gr64.values())
+    for k in g.out:
+        np.testing.assert_allclose(out32[k].detach().numpy(), out64[k].detach().numpy(), rtol=2e-5, atol=1e-4, err_msg=k)
+    for k in g.loss:
+        np.testing.assert_allclose(ls32[k].detach().numpy(), ls64[k].detach().numpy(), rtol=2e-5, atol=1e-4, err_msg=k)
+    for k in trainable:
+        want = gr64[k].numpy()
+        scale = max(1.0, float(np.abs(want).max()))
+        np.testing.assert_allclose(gr32[k].numpy(), want, rtol=1e-3, atol=2e-5 * scale, err_msg=k)
