@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define PMT_ABI_VERSION 2
+#define PMT_ABI_VERSION 3
 #define PMT_MAX_MLP_OPS 16
 #define PMT_MAX_BLOCKS 12
 #define PMT_MAX_CNN_OPS 16
@@ -179,6 +179,18 @@ int pmt_forward_prepared(const PmtModelDesc* desc, const float* weights, const P
  * tile (PMT_TILE_ROWS rows) are walked in chunks, like the forward.  Bitwise reproducible from run to run. */
 int pmt_backward(const PmtModelDesc* desc, const float* weights, const PmtBatch* batch, const PmtOutGrads* grads,
                  float* d_weights, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Backward of the clustering head alone: the gradient of pmt_forward's outputs w.r.t. the rotation, the translation and
+ * the feature-clustering parameters (translation, rotation, sigma_e, unit_ke, tau_k, mu_k, emg_sigma_k, lambda_k, logw_k),
+ * for steps in which nothing upstream of the rotation trains (calibration epochs, model_training.py:145-147).  It reads
+ * only final_re [n_rows][E], the per-read final features PmtOutputs.final_re of a pmt_forward of the same batch and
+ * weights, and grads->d_logits_bk / d_alt_means_be / d_ref_means_be (info_seq_be and saved are not read).  WRITES
+ * d_weights[n_params]: the head's slots, exact zeros everywhere else.  Takes every shape pmt_forward takes (none of the
+ * trunk backward's limits apply), reads all sizes from the device offsets (no host synchronisation) and is bitwise
+ * reproducible from run to run. */
+size_t pmt_head_backward_workspace_size(const PmtModelDesc* desc);
+int pmt_head_backward(const PmtModelDesc* desc, const float* weights, const PmtBatch* batch, const float* final_re,
+                      const PmtOutGrads* grads, float* d_weights, void* workspace, size_t workspace_bytes, void* stream);
 
 /* Arithmetic mode of the dense layers of the read path (process-wide; default PMT_PRECISION_FP32).
  *   FP32    FP32 FMA pipe (SIMT); forward and backward.

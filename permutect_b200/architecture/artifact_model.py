@@ -3,7 +3,8 @@
 Same constructor, attributes, methods, state-dict keys and ``.pt`` format as the reference, so its
 callers (model_training.py:151-165, filter_variants.py:292-320, prune_dataset.py) run unchanged.
 ``compute_batch_output`` is one call into the fused sm_100a kernels (pmt_forward); in training mode
-it is recorded as a single autograd node whose backward is pmt_backward.
+it is recorded as a single autograd node whose backward is pmt_backward, or pmt_head_backward when no tensor upstream
+of the rotation trains (calibration epochs).
 """
 from typing import Optional, Tuple
 
@@ -91,6 +92,7 @@ class ArtifactModel(nn.Module):
         self._loss_desc = None
         self._flat_cache = None
         self._param_list = None
+        self._trunk_params = None
         self._materialization_cache = None
         self._flat_optimizer = None
 
@@ -104,6 +106,7 @@ class ArtifactModel(nn.Module):
         self._loss_desc = None
         self._flat_cache = None
         self._param_list = None
+        self._trunk_params = None
         self._materialization_cache = None
 
     def ref_alt_seq_embedding_dimension(self) -> int:
@@ -142,6 +145,20 @@ class ArtifactModel(nn.Module):
         if self._param_list is None:
             self._param_list = list(self.parameters())
         return self._param_list
+
+    def _trunk_parameters(self):
+        """Cached parameters of everything upstream of the rotation: read_embedding, info_embedding, haplotypes_cnn,
+        ref_alt_reads_encoder and reducer (cleared with the parameter list)."""
+        if self._trunk_params is None:
+            self._trunk_params = [p for m in (self.read_embedding, self.info_embedding, self.haplotypes_cnn,
+                                              self.ref_alt_reads_encoder, self.reducer) for p in m.parameters()]
+        return self._trunk_params
+
+    def trunk_frozen(self) -> bool:
+        """True when no trunk parameter requires grad: the step trains the rotation, translation, clustering head or
+        adversarial heads only (a calibration epoch), and its backward needs nothing but the forward's per-read final
+        features (pmt_head_backward) instead of the whole model's backward."""
+        return not any(p.requires_grad for p in self._trunk_parameters())
 
     def flat_weights(self) -> Tensor:
         """Materialised weights as one flat fp32 tensor.  With grad enabled this is a fresh autograd
@@ -183,7 +200,8 @@ class ArtifactModel(nn.Module):
         desc = self.descriptor()
         flat = self.flat_weights()
         if flat.requires_grad:
-            logits_bk, alt_means, ref_means, logits_b, outlier = engine.FusedArtifactFunction.apply(flat, desc, batch)
+            logits_bk, alt_means, ref_means, logits_b, outlier = engine.FusedArtifactFunction.apply(flat, desc, batch,
+                                                                                                    self.trunk_frozen())
         else:
             key = self._flat_cache[0] if (self._flat_cache is not None and self._flat_cache[1] is flat) else None
             out = engine.forward_call(desc, flat, batch, weights_key=key)

@@ -135,16 +135,46 @@ def backward_call(desc: L.PmtModelDesc, flat: torch.Tensor, batch, d_logits_bk: 
     return d_flat
 
 
+def head_backward_call(desc: L.PmtModelDesc, flat: torch.Tensor, batch, final_re: torch.Tensor,
+                       d_logits_bk: Optional[torch.Tensor], d_alt_means: Optional[torch.Tensor],
+                       d_ref_means: Optional[torch.Tensor]) -> torch.Tensor:
+    """pmt_head_backward: gradient w.r.t. the flat materialised weights of the rotation, translation and clustering
+    head only (zeros elsewhere), from the per-read final features ``final_re`` of the forward of the same batch."""
+    lib = L.load()
+    _require_cuda(flat)
+    dev = flat.device
+    pb = batch.pmt_batch()
+    keep = [None if t is None else t.contiguous() for t in (d_logits_bk, d_alt_means, d_ref_means)]
+    pg = L.PmtOutGrads(*[None if t is None else t.data_ptr() for t in keep], None, None)
+    d_flat = torch.empty_like(flat)
+    need = lib.pmt_head_backward_workspace_size(C.byref(desc))
+    if need == 0:
+        raise RuntimeError("libpermutect_b200: " + lib.pmt_last_error().decode())
+    ws = _workspace(dev, need)
+    _PREPARED[dev] = None          # the partial sums go to the start of the shared workspace
+    L.check(lib.pmt_head_backward(C.byref(desc), flat.contiguous().data_ptr(), C.byref(pb), final_re.data_ptr(), C.byref(pg),
+                                  d_flat.data_ptr(), ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream))
+    return d_flat
+
+
 class FusedArtifactFunction(torch.autograd.Function):
-    """(flat weights, batch) -> (logits_bk, alt_means, ref_means, logits_b, outlier_logits)."""
+    """(flat weights, batch) -> (logits_bk, alt_means, ref_means, logits_b, outlier_logits).
+
+    ``head_only``: nothing upstream of the rotation trains, so the backward is pmt_head_backward over the per-read final
+    features this forward keeps, instead of pmt_backward over the whole model."""
 
     @staticmethod
-    def forward(ctx, flat, desc, batch):
-        # keep the forward's operands only when a backward can follow (not under no_grad, not for frozen weights)
-        out = forward_call(desc, flat, batch, for_training=bool(ctx.needs_input_grad[0]))
-        ctx.desc, ctx.batch = desc, batch
+    def forward(ctx, flat, desc, batch, head_only=False):
+        if head_only:
+            # sized from the batch's host row bound: the device offsets are not read back
+            out = forward_call(desc, flat, batch, want_final=True, n_rows=int(batch.pmt_batch().n_rows))
+        else:
+            # keep the forward's operands only when a backward can follow (not under no_grad, not for frozen weights)
+            out = forward_call(desc, flat, batch, for_training=bool(ctx.needs_input_grad[0]))
+        ctx.desc, ctx.batch, ctx.head_only = desc, batch, head_only
         ctx.save_for_backward(flat, out["logits_bk"], out["logits_b"])
         ctx.info_seq = out["info_seq"]
+        ctx.final_re = out.get("final_re")
         ctx.saved = out.get("saved")            # operand panels / CNN activations of the forward (None: the backward recomputes)
         ctx.saved_mode = L.get_precision()
         return out["logits_bk"], out["alt_means"], out["ref_means"], out["logits_b"], out["outlier_logits"]
@@ -165,10 +195,12 @@ class FusedArtifactFunction(torch.autograd.Function):
             g[:, 1] += g_out
             g[:, 0] -= g_out * sm[:, 0]
             g[:, 2:] -= g_out[:, None] * sm[:, 1:]
+        if ctx.head_only:
+            return head_backward_call(ctx.desc, flat, ctx.batch, ctx.final_re, g, g_alt, g_ref), None, None, None
         saved = ctx.saved if (ctx.saved is not None and L.get_precision() == ctx.saved_mode) else None
         d_flat = backward_call(ctx.desc, flat, ctx.batch, g, g_alt, g_ref, ctx.info_seq, saved)
         ctx.saved = None                        # a second backward through the same node recomputes
-        return d_flat, None, None
+        return d_flat, None, None, None
 
 
 def _loss_batch(batch, logits_b, outlier, features, weights, source_weights) -> L.PmtLossBatch:

@@ -138,7 +138,8 @@ class GraphedTrainStep:
         lib, desc = L.load(), self.model.descriptor()
         pb = self.static.pmt_batch()
         need = max(lib.pmt_workspace_size(engine.C.byref(desc), engine.C.byref(pb), 0),
-                   lib.pmt_workspace_size(engine.C.byref(desc), engine.C.byref(pb), 1))
+                   lib.pmt_workspace_size(engine.C.byref(desc), engine.C.byref(pb), 1),
+                   lib.pmt_head_backward_workspace_size(engine.C.byref(desc)))
         if self.workspace is None or self.workspace.numel() < need:
             self.workspace = torch.empty(int(need) + 4096, dtype=torch.uint8, device=self.device)
         # the optimiser state must not move during the warm-up replays of the capture

@@ -7,7 +7,7 @@ missing the compute entry points raise -- there is no fallback implementation.
 import ctypes as C
 import os
 
-PMT_ABI_VERSION = 2
+PMT_ABI_VERSION = 3
 MAX_MLP_OPS, MAX_BLOCKS, MAX_CNN_OPS = 16, 12, 16
 MAX_DIM, MAX_INFO_DIM, MAX_FEAT, MAX_CLUSTERS, TILE_ROWS = 64, 128, 32, 14, 128
 
@@ -93,7 +93,8 @@ class PmtLossGrads(C.Structure):
 
 
 EXPORTED_SYMBOLS = ["pmt_posterior_fit_step", "pmt_posterior_fit_workspace_size", "pmt_orthogonal_forward", "pmt_orthogonal_backward", "pmt_posterior_param_count", "pmt_posterior_log_posteriors", "pmt_dataset_read_indices", "pmt_pack_posterior", "pmt_adamw_step", "pmt_adamw_workspace_size", "pmt_losses_forward", "pmt_losses_backward", "pmt_losses_workspace_size", "pmt_last_error", "pmt_abi_version", "pmt_workspace_size", "pmt_forward", "pmt_forward_prepared", "pmt_backward",
-                    "pmt_decode_reads", "pmt_set_profile_events", "pmt_downsample_counts", "pmt_downsample_fill", "pmt_set_precision", "pmt_get_precision", "pmt_constraints_forward", "pmt_constraints_backward", "pmt_backward_kernels", "pmt_train_saved_bytes", "pmt_forward_train"]
+                    "pmt_decode_reads", "pmt_set_profile_events", "pmt_downsample_counts", "pmt_downsample_fill", "pmt_set_precision", "pmt_get_precision", "pmt_constraints_forward", "pmt_constraints_backward", "pmt_backward_kernels", "pmt_train_saved_bytes", "pmt_forward_train",
+                    "pmt_head_backward_workspace_size", "pmt_head_backward"]
 
 class PmtPosteriorDesc(C.Structure):
     _fields_ = [("n_components", C.c_int32), ("hap_start", C.c_int32), ("hap_len", C.c_int32), ("no_germline_mode", C.c_int32),
@@ -148,6 +149,11 @@ def load():
     lib.pmt_backward.restype = C.c_int
     lib.pmt_backward.argtypes = [C.POINTER(PmtModelDesc), C.c_void_p, C.POINTER(PmtBatch), C.POINTER(PmtOutGrads),
                                  C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
+    lib.pmt_head_backward_workspace_size.restype = C.c_size_t
+    lib.pmt_head_backward_workspace_size.argtypes = [C.POINTER(PmtModelDesc)]
+    lib.pmt_head_backward.restype = C.c_int
+    lib.pmt_head_backward.argtypes = [C.POINTER(PmtModelDesc), C.c_void_p, C.POINTER(PmtBatch), C.c_void_p,
+                                      C.POINTER(PmtOutGrads), C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
     lib.pmt_decode_reads.restype = C.c_int
     lib.pmt_decode_reads.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p]
     lib.pmt_downsample_counts.restype = C.c_int
