@@ -56,16 +56,21 @@ __global__ void __launch_bounds__(FWD_THREADS, 1)
 reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_constant__ TcPlan TP, const __grid_constant__ TcArgs A,
                         int n_stages, int stage_bytes) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
-  // carve: [weight ring: n_stages x stage_bytes][xch 2 slots][sums 2 slots][pair exchange][block scalars][HeadConst][Shared]
-  unsigned char* p = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const unsigned ring = smem_addr(p); p += (size_t)n_stages * stage_bytes;
-  const unsigned xch_all = smem_addr(p); p += 2 * XCH_ROWS * XCH_LD * sizeof(float);
-  const unsigned sums_all = smem_addr(p); p += 2 * SUMS_FLOATS * sizeof(float);
-  const unsigned pairx_all = smem_addr(p); p += 2 * 2 * TILE * 2 * sizeof(float);
-  float* blkc = reinterpret_cast<float*>(p); p += PMT_MAX_BLOCKS * BC_STRIDE * sizeof(float);
-  HeadConstTc* HCT = reinterpret_cast<HeadConstTc*>(p); p += sizeof(HeadConstTc);
+  // carve (pmt_tc.cuh): [Shared][xch 2 slots][sums 2 slots][pair exchange][block scalars][HeadConstTc][step table] at
+  // constant offsets from `sb`, then the weight ring (n_stages x stage_bytes) at sb + FWD_RING, 1024-aligned
+  const unsigned raw = smem_addr(smem_raw);
+  const unsigned sb = ((raw + FWD_RING + 1023u) & ~1023u) - FWD_RING;
+  const unsigned ring = sb + FWD_RING;
+  unsigned char* const p = smem_raw + (sb - raw);
+  Shared* S = reinterpret_cast<Shared*>(p);
+  float* blkc = reinterpret_cast<float*>(p + FWD_BLKC);
+  HeadConstTc* HCT = reinterpret_cast<HeadConstTc*>(p + FWD_HEAD);
   HeadConst* HC = &HCT->h;
-  Shared* S = reinterpret_cast<Shared*>((reinterpret_cast<uintptr_t>(p) + 15) & ~uintptr_t(15));
+  constexpr unsigned SH_TB = offsetof(Shared, tb), TB_BYTES = sizeof(TileBuf);
+  constexpr unsigned TB_IDX = offsetof(TileBuf, idx), TB_SRC = offsetof(TileBuf, src), TB_WORDS = offsetof(TileBuf, words),
+                     TB_VAR = offsetof(TileBuf, var), TB_V0 = offsetof(TileBuf, v0), TB_NV = offsetof(TileBuf, nv),
+                     TB_REF_PAD = offsetof(TileBuf, ref_pad), TB_LT = offsetof(TileBuf, lt), TB_M = offsetof(TileBuf, m);
+  constexpr unsigned HC_H = FWD_HEAD + offsetof(HeadConstTc, h);
 
   const int tid = threadIdx.x;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
@@ -79,6 +84,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     head_constants(D, W, HC);
     for (int e = 0; e < MAXE; ++e) HCT->inv_sigma[e] = e < D.d_feat ? 1.f / HC->sigma[e] : 0.f;
+    for (int s = 0; s < TP.n_steps; ++s) p[FWD_STEPS + s] = (unsigned char)(TP.step[s].epi | TP.step[s].blk << 4);
     for (int k = 0; k < MAXK; ++k) {
       const bool on = k < D.n_clusters;
       HCT->inv_two_tau2[k] = on ? 1.f / HC->two_tau2[k] : 0.f;
@@ -328,10 +334,11 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
     const int row = quarter * 32 + lane;
     const int srow = half * TILE + row;              // 0..255 inside the slot
     const int slot_bar = 1 + slot, pair_bar = 3 + slot * 4 + quarter;
-    const unsigned xch = xch_all + slot * XCH_ROWS * XCH_LD * 4;    // [XCH_ROWS][XCH_LD] floats
-    const unsigned sums = sums_all + slot * SUMS_FLOATS * 4;        // [segment = 2 * variant + side][MAXH]
-    const unsigned px_mine = pairx_all + ((slot * 2 + half) * TILE + row) * 8, px_other = pairx_all + ((slot * 2 + (half ^ 1)) * TILE + row) * 8;
-    const unsigned bar_a = smem_addr(&S->bar_a[slot]), bar_d = smem_addr(&S->bar_d[slot]);
+    const unsigned xch = sb + FWD_XCH + slot * XCH_ROWS * XCH_LD * 4;    // [XCH_ROWS][XCH_LD] floats
+    const unsigned sums = sb + FWD_SUMS + slot * SUMS_FLOATS * 4;        // [segment = 2 * variant + side][MAXH]
+    const unsigned px_mine = sb + FWD_PAIRX + ((slot * 2 + half) * TILE + row) * 8, px_other = sb + FWD_PAIRX + ((slot * 2 + (half ^ 1)) * TILE + row) * 8;
+    const unsigned bar_a = sb + offsetof(Shared, bar_a) + slot * 8, bar_d = sb + offsetof(Shared, bar_d) + slot * 8;
+    const unsigned steps = sb + FWD_STEPS;
     const unsigned trow = tmem_base + slot * SLOT_COLS + ((unsigned)(quarter * 32) << 16);
     const unsigned t_x = trow + COL_X, t_z = trow + COL_Z, t_hi = trow + COL_AHI, t_lo = trow + COL_ALO;
     const int E = D.d_feat, K = D.n_clusters, Dm = D.d_model, H = D.d_ffn / 2, DR = D.d_read, F = D.n_read_features;
@@ -345,21 +352,25 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
     for (int round = 0; round < rounds; ++round) {
       const int t = (int)blockIdx.x + slot * (int)gridDim.x + round * n_slots;
       // ---------------- tile meta: prepared by the meta warp while the previous tile was computed ----------------
-      TileBuf* const TB = &S->tb[slot][round & 1];
-      const unsigned m_rowvar = smem_addr(TB->m.rowvar), m_ref_start = smem_addr(TB->m.ref_start), m_ref_cnt = smem_addr(TB->m.ref_cnt),
-                     m_alt_start = smem_addr(TB->m.alt_start), m_alt_cnt = smem_addr(TB->m.alt_cnt);
-      mbar_wait(smem_addr(&S->meta_full[slot][round & 1]), (round >> 1) & 1);
-      const int v0 = TB->v0, nv = TB->nv, ref_pad = TB->ref_pad;
-      const int lt_first = LONG ? TB->lt[0] : 0, lt_k = LONG ? TB->lt[1] : 0, lt_tref = LONG ? TB->lt[2] : 0, lt_talt = LONG ? TB->lt[3] : 0,
-                lt_side = LONG ? TB->lt[4] : 0, lt_rows = LONG ? TB->lt[5] : 0, set_ref = LONG ? TB->lt[6] : 0, set_alt = LONG ? TB->lt[7] : 0;
-      const long long my_idx = TB->idx[row], my_src = TB->src[row];
+      const unsigned tb = sb + SH_TB + (slot * 2 + (round & 1)) * TB_BYTES;   // this round's TileBuf
+      const unsigned m_rowvar = tb + TB_M + offsetof(SlotMeta, rowvar), m_ref_start = tb + TB_M + offsetof(SlotMeta, ref_start),
+                     m_ref_cnt = tb + TB_M + offsetof(SlotMeta, ref_cnt), m_alt_start = tb + TB_M + offsetof(SlotMeta, alt_start),
+                     m_alt_cnt = tb + TB_M + offsetof(SlotMeta, alt_cnt), tb_var = tb + TB_VAR;
+      mbar_wait(sb + offsetof(Shared, meta_full) + (slot * 2 + (round & 1)) * 8, (round >> 1) & 1);
+      const int v0 = lds_s32(tb + TB_V0), nv = lds_s32(tb + TB_NV), ref_pad = lds_s32(tb + TB_REF_PAD);
+      const int lt_first = LONG ? lds_s32(tb + TB_LT) : 0, lt_k = LONG ? lds_s32(tb + TB_LT + 4) : 0, lt_tref = LONG ? lds_s32(tb + TB_LT + 8) : 0,
+                lt_talt = LONG ? lds_s32(tb + TB_LT + 12) : 0, lt_side = LONG ? lds_s32(tb + TB_LT + 16) : 0, lt_rows = LONG ? lds_s32(tb + TB_LT + 20) : 0,
+                set_ref = LONG ? lds_s32(tb + TB_LT + 24) : 0, set_alt = LONG ? lds_s32(tb + TB_LT + 28) : 0;
+      const long long my_idx = lds_s64(tb + TB_IDX + row * 8), my_src = lds_s64(tb + TB_SRC + row * 8);
       unsigned char* const scr = (SAVE && t < n_tiles) ? A.scratch + (size_t)t * TP.tile_bytes : nullptr;
       const int rv = (int)lds_u8(m_rowvar + row);
       const int my_var = rv == 255 ? -1 : rv;
       const bool is_alt = row >= ref_pad;
 
+      // step kind and gated block (epi | blk << 4): the next step's entry is read before the accumulator wait
+      unsigned code = lds_u8(steps);
       for (int step = 0; step < n_steps; ++step) {
-        const int epi = TP.step[step].epi;
+        const int epi = (int)(code & 15u), blk = (int)(code >> 4);
         unsigned char* const scr_op = (SAVE && scr) ? scr + TP.step[step].scr_off : nullptr;
         switch (epi) {
           case EPI_DECODE: {   // batch.py:51-56, plain_text_data.py:510-511 (quirk Q2: the uint8 de-quantisation wraps)
@@ -374,11 +385,11 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
                 unsigned bytes[8];   // this half's 8 source bytes: packed bytes 0..3, or packed bytes 4..6 + quantised 7..
                 if (rb == 12) {      // the meta warp fetched the row
                   if (half == 0) {
-                    const unsigned w0 = TB->words[row * 3];
+                    const unsigned w0 = (unsigned)lds_s32(tb + TB_WORDS + row * 12);
 #pragma unroll
                     for (int b = 0; b < 4; ++b) bytes[b] = (w0 >> (8 * b)) & 255u;
                   } else {
-                    const unsigned w1 = TB->words[row * 3 + 1], w2 = TB->words[row * 3 + 2];
+                    const unsigned w1 = (unsigned)lds_s32(tb + TB_WORDS + row * 12 + 4), w2 = (unsigned)lds_s32(tb + TB_WORDS + row * 12 + 8);
 #pragma unroll
                     for (int b = 0; b < 4; ++b) { bytes[b] = (w1 >> (8 * b)) & 255u; bytes[4 + b] = (w2 >> (8 * b)) & 255u; }
                   }
@@ -426,16 +437,19 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
             float v[16];
             load_cols<16>(t_z + half * 16, v);
             unsigned r[16];
+            selu_u_n<16>(v);
 #pragma unroll
-            for (int i = 0; i < 16; ++i) { v[i] = SELU_SCALE * selu_u(v[i]); r[i] = __float_as_uint(v[i]); }
+            for (int i = 0; i < 16; i += 2) {
+              up2(mul2(pk2(v[i], v[i + 1]), pk2(SELU_SCALE, SELU_SCALE)), v[i], v[i + 1]);
+              r[i] = __float_as_uint(v[i]); r[i + 1] = __float_as_uint(v[i + 1]);
+            }
             tmem_st16(t_x + half * 16, r);
             if (SAVE && scr) {
               float* x0 = reinterpret_cast<float*>(scr + TP.x0_off) + (half * 16) * TILE + row;
 #pragma unroll
               for (int i = 0; i < 16; ++i) x0[i * TILE] = v[i];
             }
-#pragma unroll
-            for (int i = 0; i < 16; ++i) v[i] = selu_u(v[i]);
+            selu_u_n<16>(v);
             if (half == 1) v[15] = 1.f;   // operand column 31: bias
             if (SAVE && scr_op) save_operand<16>(scr_op, row, half * 16, v);
             store_operand<16, PASSES>(t_hi + half * 16, t_lo + half * 16, v, true);
@@ -444,8 +458,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
           case EPI_ACT_X32: {
             float v[16];
             load_cols<16>((epi == EPI_ACT_Z32 ? t_z : t_x) + half * 16, v);
-#pragma unroll
-            for (int i = 0; i < 16; ++i) v[i] = selu_u(v[i]);
+            selu_u_n<16>(v);
             if (half == 1) v[15] = 1.f;
             if (SAVE && scr_op) save_operand<16>(scr_op, row, half * 16, v);
             store_operand<16, PASSES>(t_hi + half * 16, t_lo + half * 16, v, true);
@@ -454,7 +467,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
           case EPI_LN: {   // gated_mlp.py:185 (LayerNorm affine folded into proj1); artifact_model.py:246-251 concat
             float v[32];
             if (epi == EPI_LN_FIRST && half == 1) {
-              const float* src = my_var >= 0 ? A.out.info_seq_be + (long long)TB->var[my_var] * DIS : nullptr;
+              const float* src = my_var >= 0 ? A.out.info_seq_be + (long long)lds_s32(tb_var + my_var * 4) * DIS : nullptr;
               unsigned r[32];
 #pragma unroll
               for (int i = 0; i < 32; ++i) { v[i] = (src && i < DIS) ? __ldg(src + i) : 0.f; r[i] = __float_as_uint(v[i]); }
@@ -475,18 +488,20 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
             const float var = (q_h + oth.y + dm * dm * nh * no / (float)Dm) / (float)Dm;
             const float rstd = rsqrtf(fmaxf(var, 0.f) + LN_EPS);
             const float shift = -mean * rstd;
+            {
+              const f32x2 rs2 = pk2(rstd, rstd), sh2 = pk2(shift, shift);
 #pragma unroll
-            for (int i = 0; i < 32; ++i) v[i] = fmaf(v[i], rstd, shift);
+              for (int i = 0; i < 32; i += 2) up2(fma2(pk2(v[i], v[i + 1]), rs2, sh2), v[i], v[i + 1]);
+            }
             if (half == 0) v[31] = 1.f;   // operand column 31: bias
             if (SAVE && scr_op) {
               save_operand<32>(scr_op, row, half * 32, v);
-              if (half == 0) reinterpret_cast<float*>(scr + TP.rstd_off)[TP.step[step].blk * TILE + row] = rstd;
+              if (half == 0) reinterpret_cast<float*>(scr + TP.rstd_off)[blk * TILE + row] = rstd;
             }
             store_operand<32, PASSES>(t_hi + half * 32, t_lo + half * 32, v, true);
           } break;
           case EPI_GATE: {   // gated_mlp.py:186-190, 228-251; this thread gates hidden units [k0, k0 + 6)
-            const float* bc = blkc + TP.step[step].blk * BC_STRIDE;
-            const unsigned bcs = smem_addr(bc);
+            const unsigned bcs = sb + FWD_BLKC + blk * BC_STRIDE * 4;
             // proj1 output: [ref set | alt set], one set = [z1 at 0..H) | z2 at 12..12+H)]
             float z1s[16], z2s[16];
             {
@@ -517,8 +532,13 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
             // z1s[j] = z1[k0 + j] (j < 6), z2s[k] = z2[k] (k < 12; columns >= H are zero)
             const int k0 = half * 6;
             float z2[12];
+            selu_u_n<12>(z2s);
 #pragma unroll
-            for (int k = 0; k < 12; ++k) z2[k] = k < H ? SELU_SCALE * selu_u(z2s[k]) : 0.f;
+            for (int k = 0; k < 12; k += 2) {
+              float s0, s1;
+              up2(mul2(pk2(z2s[k], z2s[k + 1]), pk2(SELU_SCALE, SELU_SCALE)), s0, s1);
+              z2[k] = k < H ? s0 : 0.f; z2[k + 1] = k + 1 < H ? s1 : 0.f;
+            }
             const float mean = sum_n<12>(z2) / (float)H;
             float var;
             {
@@ -539,7 +559,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
               z2n[j] = (zz - mean) * rstd * lds_f32(bcs + (BC_LN2W + k0 + j) * 4) + lds_f32(bcs + (BC_LN2B + k0 + j) * 4);
               if (k0 + j < H) sts_f32(xch + ((k0 + j) * XCH_LD + row) * 4, z2n[j]);
               if (SAVE && scr) {   // what the backward of the gate needs: xhat2, selu'(z2), (z1 below), 1 / std
-                float* gi = reinterpret_cast<float*>(scr + TP.gate_off) + ((TP.step[step].blk * GATE_ITEMS) * 2 + half) * TILE + row;
+                float* gi = reinterpret_cast<float*>(scr + TP.gate_off) + ((blk * GATE_ITEMS) * 2 + half) * TILE + row;
                 gi[(6 + j) * 2 * TILE] = (zz - mean) * rstd;
                 gi[(12 + j) * 2 * TILE] = zz > 0.f ? SELU_SCALE : zz + SELU_SCALE * SELU_ALPHA;
                 if (j == 0) gi[18 * 2 * TILE] = rstd;
@@ -547,12 +567,13 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
             }
             // the z1 activations do not depend on the other rows: computed while the slower warps reach the barrier
             float z1a[6];
+            selu_u_n<6>(z1s);
 #pragma unroll
-            for (int j = 0; j < 6; ++j) z1a[j] = SELU_SCALE * selu_u(z1s[j]);
+            for (int j = 0; j < 6; j += 2) up2(mul2(pk2(z1s[j], z1s[j + 1]), pk2(SELU_SCALE, SELU_SCALE)), z1a[j], z1a[j + 1]);
             named_barrier(slot_bar, 256);
             if (LONG) {   // mean fields of a set spread over many tiles (pmt_tc.cuh: LongTile)
               const float regw = lds_f32(bcs + BC_REGW * 4);
-              const int blk = TP.step[step].blk, nb = D.n_blocks;
+              const int nb = D.n_blocks;
               // (a) column sums of this tile's rows -> the tile's slot in global memory; a lane pair per hidden unit
               if (srow < 32) {
                 const int f = lane >> 1, part = lane & 1;
@@ -625,7 +646,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
                   const float den = (float)cnt + (s == 0 ? regw : 1e-4f);
                   const float m = __fdividef(num, den);
                   sts_f32(sums + (seg * MAXH + f) * 4, m);
-                  if (SAVE && scr) reinterpret_cast<float*>(scr + TP.means_off)[(TP.step[step].blk * 2 * BWD_MAXV + seg) * MAXH + f] = m;
+                  if (SAVE && scr) reinterpret_cast<float*>(scr + TP.means_off)[(blk * 2 * BWD_MAXV + seg) * MAXH + f] = m;
                 }
               }
             }
@@ -653,7 +674,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
                   const float z1 = z1a[j];
                   tk[j] = z1 * gate;
                   if (SAVE && scr)
-                    reinterpret_cast<float*>(scr + TP.gate_off)[((TP.step[step].blk * GATE_ITEMS + j) * 2 + half) * TILE + row] = z1;
+                    reinterpret_cast<float*>(scr + TP.gate_off)[((blk * GATE_ITEMS + j) * 2 + half) * TILE + row] = z1;
                 }
               }
               if (half == 0) {
@@ -674,10 +695,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
           case EPI_COPY_X64: {
             float v[32];
             load_cols<32>((epi == EPI_ACT_Z64 ? t_z : t_x) + half * 32, v);
-            if (epi != EPI_COPY_X64) {
-#pragma unroll
-              for (int i = 0; i < 32; ++i) v[i] = selu_u(v[i]);
-            }
+            if (epi != EPI_COPY_X64) selu_u_n<32>(v);
             if (half == 0) v[31] = 1.f;
             if (SAVE && scr_op) save_operand<32>(scr_op, row, half * 32, v);
             store_operand<32, PASSES>(t_hi + half * 32, t_lo + half * 32, v, true);
@@ -688,6 +706,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(bar_a);
+        code = lds_u8(steps + (step + 1 < n_steps ? step + 1 : 0));
         mbar_wait(bar_d, dparity);
         dparity ^= 1;
         tc_fence_after();
@@ -715,21 +734,24 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
         {   // (f / (2 sigma))^2 == (f / sigma)^2 / 4 exactly: one sum serves the non-artifact and the outlier Gaussians
           float q = 0.f;
 #pragma unroll
-          for (int e = 0; e < MAXE; ++e) { const float a = f[e] * HCT->inv_sigma[e]; q = fmaf(a, a, q); }
-          sts_f32(xch + ((MAXE + half) * XCH_LD + row) * 4, half ? HC->c_out - q * 0.125f : HC->c_non - q * 0.5f);
+          for (int e = 0; e < MAXE; ++e) { const float a = f[e] * lds_f32(sb + FWD_HEAD + offsetof(HeadConstTc, inv_sigma) + e * 4); q = fmaf(a, a, q); }
+          const float c_ = lds_f32(sb + HC_H + (half ? offsetof(HeadConst, c_out) : offsetof(HeadConst, c_non)));
+          sts_f32(xch + ((MAXE + half) * XCH_LD + row) * 4, half ? c_ - q * 0.125f : c_ - q * 0.5f);
         }
         for (int k = half; k < K; k += 2) {
-          const float* u = HCT->unit[k];
+          const unsigned u = sb + FWD_HEAD + offsetof(HeadConstTc, unit) + k * MAXE * 4, hk = sb + HC_H + k * 4;
           float pr = 0.f;
 #pragma unroll
-          for (int e = 0; e < MAXE; ++e) pr = fmaf(f[e], u[e], pr);
+          for (int e = 0; e < MAXE; ++e) pr = fmaf(f[e], lds_f32(u + e * 4), pr);
           float o2 = 0.f;
 #pragma unroll
-          for (int e = 0; e < MAXE; ++e) { const float dd = fmaf(-pr, u[e], f[e]); o2 = fmaf(dd, dd, o2); }
+          for (int e = 0; e < MAXE; ++e) { const float dd = fmaf(-pr, lds_f32(u + e * 4), f[e]); o2 = fmaf(dd, dd, o2); }
           const float dist = sqrtf(o2);
-          const float ll_orth = HC->c_orth[k] - (dist * dist) * HCT->inv_two_tau2[k];
-          const float ll_par = HC->log_half_lambda[k] + logerfc((HC->shift[k] - pr) * HCT->inv_sqrt2_sigma[k]) +
-                               HC->half_lambda[k] * (HC->two_mu_plus[k] - 2.f * pr);
+          const float ll_orth = lds_f32(hk + offsetof(HeadConst, c_orth)) -
+                                (dist * dist) * lds_f32(sb + FWD_HEAD + offsetof(HeadConstTc, inv_two_tau2) + k * 4);
+          const float ll_par = lds_f32(hk + offsetof(HeadConst, log_half_lambda)) +
+                               logerfc((lds_f32(hk + offsetof(HeadConst, shift)) - pr) * lds_f32(sb + FWD_HEAD + offsetof(HeadConstTc, inv_sqrt2_sigma) + k * 4)) +
+                               lds_f32(hk + offsetof(HeadConst, half_lambda)) * (lds_f32(hk + offsetof(HeadConst, two_mu_plus)) - 2.f * pr);
           sts_f32(xch + ((MAXE + 2 + k) * XCH_LD + row) * 4, ll_orth + ll_par);
         }
       }
@@ -785,7 +807,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
             float acc = 0.f;
             if (term) {
               for (int tt = 0; tt < lt_talt; ++tt) acc += __ldcg(base + (size_t)(lt_tref + tt) * LONG_FIN_W + MAXE + k);
-              if (k >= 2) acc += HC->logw[k - 2];
+              if (k >= 2) acc += lds_f32(sb + HC_H + offsetof(HeadConst, logw) + (k - 2) * 4);
             }
             const bool art_term = term && k >= 2;
             float art_max = art_term ? acc : -INFINITY;
@@ -820,7 +842,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
           a3 += i + 3 < cnt ? x3 : 0.f;
         }
         float* dst = s ? A.out.alt_means_be : A.out.ref_means_be;
-        if (dst) dst[(long long)TB->var[j] * E + e] = __fdividef((a0 + a1) + (a2 + a3), (float)cnt + 1e-4f);
+        if (dst) dst[(long long)lds_s32(tb_var + j * 4) * E + e] = __fdividef((a0 + a1) + (a2 + a3), (float)cnt + 1e-4f);
       }
       // log-likelihood sums: one (variant, term) per thread in groups of eight lanes, HIGH threads first (the two gathers
       // run side by side on different warps); the terms of a variant meet through shuffles
@@ -843,7 +865,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
               a3 += i + 3 < ac ? x3 : 0.f;
             }
             acc = (a0 + a1) + (a2 + a3);
-            if (k >= 2) acc += HC->logw[k - 2];
+            if (k >= 2) acc += lds_f32(sb + HC_H + offsetof(HeadConst, logw) + (k - 2) * 4);
           }
           const bool art_term = term && k >= 2;
           float art_max = art_term ? acc : -INFINITY;
@@ -856,7 +878,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
           const int lane_k0 = (lane | 7);
           const float ll0 = __shfl_sync(0xffffffffu, acc, lane_k0), ll1 = __shfl_sync(0xffffffffu, acc, lane_k0 - 1);
           if (term) {
-            const long long v = TB->var[j];
+            const long long v = lds_s32(tb_var + j * 4);
             const float art = art_max + logf(sacc);
             if (A.out.logits_bk) A.out.logits_bk[v * (K + 2) + k] = acc;
             if (k == 0 && A.out.logits_b) A.out.logits_b[v] = 20.f * tanhf((art - ll0) / 20.f);
@@ -866,7 +888,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
       }
       }   // !LONG
       __syncwarp();
-      if (lane == 0) mbar_arrive(smem_addr(&S->meta_free[slot][round & 1]));   // the tile's tables may be refilled
+      if (lane == 0) mbar_arrive(sb + offsetof(Shared, meta_free) + (slot * 2 + (round & 1)) * 8);   // the tile's tables may be refilled
     }
   }
   tc_fence_before();
@@ -1382,8 +1404,7 @@ int pmt_plan_tiles(const PmtBatch* batch, int max_variants, bool deterministic, 
 template <int PASSES, bool SAVE, bool LONG>
 static int launch_reads_tc(const PmtModelDesc& D, const TcPlan& T, const TcArgs& A, int grid, cudaStream_t st) {
   const int stage_bytes = PASSES == 3 ? T.slot_bytes : T.slot_bytes / 2;
-  const size_t fixed = 2 * XCH_ROWS * XCH_LD * sizeof(float) + 2 * SUMS_FLOATS * sizeof(float) + 2 * 2 * TILE * 2 * sizeof(float) +
-                       PMT_MAX_BLOCKS * BC_STRIDE * sizeof(float) + sizeof(HeadConstTc) + sizeof(Shared) + 1024 + 64;
+  const size_t fixed = FWD_FIXED_BYTES;
   int n_stages = (int)((227 * 1024 - fixed) / stage_bytes);
   if (n_stages > NS_MAX) n_stages = NS_MAX;
   PMT_CHECK(n_stages >= 2, "tensor-core forward: weight ring does not fit in shared memory");

@@ -1,5 +1,6 @@
 // Declarations shared by the tensor-core read-path kernels: the forward (pmt_tc.cu) and the backward (pmt_tc_bwd.cu).
 #pragma once
+#include <cstddef>
 #include <cstring>
 
 #include "pmt_host.h"
@@ -170,6 +171,21 @@ struct HeadConstTc {
 constexpr int BC_LN2W = 0, BC_LN2B = 12, BC_REG = 24, BC_AREF = 36, BC_AALT = 37, BC_BREF = 38, BC_BALT = 39, BC_GAMMA = 40,
               BC_REGW = 41, BC_STRIDE = 48;
 
+// Dynamic shared memory of the forward: the regions below at fixed byte offsets from one 8-aligned base, then the weight
+// ring (the only runtime-sized region) at FWD_RING, 1024-aligned.  Every epilogue address is the base plus a constant.
+constexpr unsigned FWD_XCH = (sizeof(Shared) + 7) & ~7u;                            // [2 slots][XCH_ROWS][XCH_LD] floats
+constexpr unsigned FWD_SUMS = FWD_XCH + 2 * XCH_ROWS * XCH_LD * 4;                  // [2 slots][SUMS_FLOATS]
+constexpr unsigned FWD_PAIRX = FWD_SUMS + 2 * SUMS_FLOATS * 4;                      // [2 slots][2 halves][TILE] float2
+constexpr unsigned FWD_BLKC = FWD_PAIRX + 2 * 2 * TILE * 2 * 4;                     // [PMT_MAX_BLOCKS][BC_STRIDE] floats
+constexpr unsigned FWD_HEAD = FWD_BLKC + PMT_MAX_BLOCKS * BC_STRIDE * 4;            // HeadConstTc
+constexpr unsigned FWD_STEPS = FWD_HEAD + sizeof(HeadConstTc);                      // [MAX_STEPS] bytes: epi | blk << 4
+constexpr unsigned FWD_RING = (FWD_STEPS + MAX_STEPS + 7) & ~7u;
+// what the launch reserves next to the ring (the base is found by rounding the ring's start up to 1024)
+constexpr size_t FWD_FIXED_BYTES = 2 * XCH_ROWS * XCH_LD * sizeof(float) + 2 * SUMS_FLOATS * sizeof(float) + 2 * 2 * TILE * 2 * sizeof(float) +
+                                   PMT_MAX_BLOCKS * BC_STRIDE * sizeof(float) + sizeof(HeadConstTc) + sizeof(Shared) + 1024 + 64;
+static_assert(FWD_RING + 1023 <= FWD_FIXED_BYTES, "forward shared-memory carve exceeds the launch's reservation");
+static_assert(EPI_COPY_X64 < 16 && PMT_MAX_BLOCKS <= 16, "step table packs epi and blk into 4 bits each");
+
 template <int NC>
 __device__ __forceinline__ void tmem_st_n(unsigned taddr, const unsigned* r) {
   static_assert(NC == 4 || NC == 8 || NC == 12 || NC == 16 || NC == 32, "unsupported operand width");
@@ -190,7 +206,11 @@ __device__ __forceinline__ void store_operand(unsigned t_hi, unsigned t_lo, cons
   tmem_st_n<NC>(t_hi, r);
   if (PASSES == 3 && lo_pass) {
 #pragma unroll
-    for (int i = 0; i < NC; ++i) r[i] = __float_as_uint(v[i] - __uint_as_float(r[i] & 0xFFFFE000u));
+    for (int i = 0; i < NC; i += 2) {   // remainder v - trunc(v): paired subtractions
+      float a, b;
+      up2(sub2(pk2(v[i], v[i + 1]), pk2(__uint_as_float(r[i] & 0xFFFFE000u), __uint_as_float(r[i + 1] & 0xFFFFE000u))), a, b);
+      r[i] = __float_as_uint(a); r[i + 1] = __float_as_uint(b);
+    }
     tmem_st_n<NC>(t_lo, r);
   }
 }
@@ -221,22 +241,28 @@ __device__ __forceinline__ void issue_chain(unsigned d, unsigned a_hi, unsigned 
   }
 }
 
-// 4-way partial sums: short dependency chains for the two warps that share an SM sub-partition
+// 4-way partial sums: short dependency chains for the two warps that share an SM sub-partition.  Partial sums (a0, a1)
+// and (a2, a3) are independent, so each pair is one paired instruction per step.
 template <int N>
 __device__ __forceinline__ float sum_n(const float* v) {
-  float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
+  f32x2 a01 = pk2(0.f, 0.f), a23 = pk2(0.f, 0.f);
 #pragma unroll
-  for (int i = 0; i < N; i += 4) { a0 += v[i]; a1 += v[i + 1]; a2 += v[i + 2]; a3 += v[i + 3]; }
+  for (int i = 0; i < N; i += 4) { a01 = add2(a01, pk2(v[i], v[i + 1])); a23 = add2(a23, pk2(v[i + 2], v[i + 3])); }
+  float a0, a1, a2, a3;
+  up2(a01, a0, a1); up2(a23, a2, a3);
   return (a0 + a1) + (a2 + a3);
 }
 template <int N>
 __device__ __forceinline__ float sumsq_centered_n(const float* v, float m) {
-  float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
+  const f32x2 mm = pk2(m, m);
+  f32x2 a01 = pk2(0.f, 0.f), a23 = pk2(0.f, 0.f);
 #pragma unroll
   for (int i = 0; i < N; i += 4) {
-    const float d0 = v[i] - m, d1 = v[i + 1] - m, d2 = v[i + 2] - m, d3 = v[i + 3] - m;
-    a0 = fmaf(d0, d0, a0); a1 = fmaf(d1, d1, a1); a2 = fmaf(d2, d2, a2); a3 = fmaf(d3, d3, a3);
+    const f32x2 d01 = sub2(pk2(v[i], v[i + 1]), mm), d23 = sub2(pk2(v[i + 2], v[i + 3]), mm);
+    a01 = fma2(d01, d01, a01); a23 = fma2(d23, d23, a23);
   }
+  float a0, a1, a2, a3;
+  up2(a01, a0, a1); up2(a23, a2, a3);
   return (a0 + a1) + (a2 + a3);
 }
 

@@ -98,6 +98,16 @@ __device__ __forceinline__ void tmem_st32(unsigned taddr, const unsigned* r) {
       : "memory");
 }
 
+// Paired FP32 (FFMA2 / FADD2 / FMUL2): two independent lanes, each rounded exactly as the scalar instruction would round it
+// (round-to-nearest, no flush to zero), so pairing changes no value.  nvcc does not pair scalar code on its own.
+typedef unsigned long long f32x2;
+__device__ __forceinline__ f32x2 pk2(float a, float b) { f32x2 r; asm("mov.b64 %0, {%1,%2};" : "=l"(r) : "f"(a), "f"(b)); return r; }
+__device__ __forceinline__ void up2(f32x2 r, float& a, float& b) { asm("mov.b64 {%0,%1}, %2;" : "=f"(a), "=f"(b) : "l"(r)); }
+__device__ __forceinline__ f32x2 fma2(f32x2 a, f32x2 b, f32x2 c) { f32x2 d; asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c)); return d; }
+__device__ __forceinline__ f32x2 add2(f32x2 a, f32x2 b) { f32x2 d; asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
+__device__ __forceinline__ f32x2 sub2(f32x2 a, f32x2 b) { f32x2 d; asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
+__device__ __forceinline__ f32x2 mul2(f32x2 a, f32x2 b) { f32x2 d; asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b)); return d; }
+
 // u(x) = x > 0 ? x : alpha (e^x - 1); selu(x) = scale * u(x).  The scale is folded into the consuming weights
 // wherever a SELU output feeds a Linear layer.
 __device__ __forceinline__ float selu_u(float x) {
@@ -106,11 +116,29 @@ __device__ __forceinline__ float selu_u(float x) {
   const float neg = fmaf(SELU_ALPHA, e, -SELU_ALPHA);
   return x > 0.f ? x : neg;
 }
+// selu_u of v[0..N), bitwise equal to N selu_u calls: the exponent arguments are paired multiplies.  The alpha FMA stays
+// scalar: it is predicated on x <= 0, which a paired FMA would turn into an FMA plus a select.
+template <int N>
+__device__ __forceinline__ void selu_u_n(float* v) {
+  static_assert(N % 2 == 0, "pairs");
+  const f32x2 l2e = pk2(1.4426950408889634f, 1.4426950408889634f);
+#pragma unroll
+  for (int i = 0; i < N; i += 2) {
+    float t0, t1, e0, e1;
+    up2(mul2(pk2(v[i], v[i + 1]), l2e), t0, t1);
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e0) : "f"(t0));
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e1) : "f"(t1));
+    v[i] = v[i] > 0.f ? v[i] : fmaf(SELU_ALPHA, e0, -SELU_ALPHA);
+    v[i + 1] = v[i + 1] > 0.f ? v[i + 1] : fmaf(SELU_ALPHA, e1, -SELU_ALPHA);
+  }
+}
 
 __device__ __forceinline__ float lds_f32(unsigned a) { float v; asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a)); return v; }
 __device__ __forceinline__ void sts_f32(unsigned a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
 __device__ __forceinline__ float2 lds_f32x2(unsigned a) { float2 v; asm volatile("ld.shared.v2.f32 {%0,%1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(a)); return v; }
 __device__ __forceinline__ void sts_f32x2(unsigned a, float x, float y) { asm volatile("st.shared.v2.f32 [%0], {%1,%2};" ::"r"(a), "f"(x), "f"(y) : "memory"); }
+__device__ __forceinline__ int lds_s32(unsigned a) { int v; asm volatile("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
+__device__ __forceinline__ long long lds_s64(unsigned a) { long long v; asm volatile("ld.shared.s64 %0, [%1];" : "=l"(v) : "r"(a)); return v; }
 __device__ __forceinline__ unsigned lds_u8(unsigned a) { unsigned v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
 __device__ __forceinline__ void named_barrier(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 

@@ -1,12 +1,14 @@
 """SASS opcode histogram of every cubin in libpermutect_b200.so (evidence for which kernels run on the tensor pipe):
     python profiles/sass_histogram.py > profiles/r2/sass_histogram.md
-UTCHMMA = tcgen05.mma, HMMA = warp-level mma.sync, LDTM / STTM = tcgen05.ld / st, UBLKCP = cp.async.bulk, UTCBAR = tcgen05.commit, SYNCS = mbarrier."""
+UTCHMMA = tcgen05.mma, HMMA = warp-level mma.sync, LDTM / STTM = tcgen05.ld / st, UBLKCP = cp.async.bulk, UTCBAR = tcgen05.commit, SYNCS = mbarrier,
+FFMA2 / FADD2 / FMUL2 = paired FP32, LD = generic-address load."""
 import collections, os, re, subprocess, sys
 
 R = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 so = os.path.join(R, "permutect_b200", "csrc", "libpermutect_b200.so")
 objdir = os.path.join(R, "permutect_b200", "csrc", "build")
-KEY = ["UTCHMMA", "HMMA", "LDTM", "STTM", "UBLKCP", "UTCBAR", "SYNCS", "FFMA", "MUFU", "LDL", "STL", "RED", "ATOMG", "SHFL", "LDS", "STS", "LDG", "STG"]
+KEY = ["UTCHMMA", "HMMA", "LDTM", "STTM", "UBLKCP", "UTCBAR", "SYNCS", "FFMA", "FFMA2", "FADD", "FADD2", "FMUL", "FMUL2", "MUFU", "LDL",
+       "STL", "RED", "ATOMG", "SHFL", "LD", "LDS", "STS", "LDG", "STG"]
 print("| object | kernel | " + " | ".join(KEY) + " | all |\n|---|---|" + "---|" * (len(KEY) + 1))
 for obj in sorted(os.listdir(objdir)):
     if not obj.endswith(".o"):

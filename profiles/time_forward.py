@@ -1,6 +1,7 @@
 """Times ArtifactModel.compute_batch_output on a resident WGS-shaped shard (CUDA events) and the read kernel inside it:
-python profiles/time_forward.py [n_variants] [steps] [precision]        (PMT_TC_PACKED=0: the sequential tile planner)"""
-import os, sys
+python profiles/time_forward.py [n_variants] [steps] [precision]        (PMT_TC_PACKED=0: the sequential tile planner)
+The last line holds a SHA-256 of every BatchOutput field, so two builds of the library compare in one line."""
+import hashlib, os, sys
 R = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [R, os.path.join(R, "tests")]
 import torch
@@ -33,3 +34,6 @@ with torch.inference_mode():
 ms = e0.elapsed_time(e1) / steps
 print(f"packed={os.environ.get('PMT_TC_PACKED', '1')} n={n} step_ms={ms:.3f} read_kernel_ms={prof.mean_ms():.3f} "
       f"variants_per_s={n / ms * 1e3:.4g} checksum={float(out.logits_b.double().sum()):.6f}")
+digest = {k: hashlib.sha256(v.detach().float().contiguous().cpu().numpy().tobytes()).hexdigest()[:16]
+          for k, v in sorted(vars(out).items()) if isinstance(v, torch.Tensor)}
+print("sha256 " + " ".join(f"{k}={h}" for k, h in digest.items()))

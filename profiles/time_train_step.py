@@ -1,6 +1,7 @@
 """Times the training step and the backward kernel (CUDA events; the numbers of profiles/r1_backward_session4.md):
-python profiles/time_train_step.py [n_variants] [steps]     (NOFLAT=1: per-parameter autograd path)"""
-import os, sys
+python profiles/time_train_step.py [n_variants] [steps]     (NOFLAT=1: per-parameter autograd path)
+Prints a SHA-256 of the flat gradient of the first step, so two builds of the library compare in one line."""
+import hashlib, os, sys
 R = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [R, os.path.join(R, "tests")]
 import torch
@@ -32,7 +33,11 @@ def step(i, profile=False):
     if profile: prof.disarm()
     return losses
 traj = []
-for i in range(3): traj.append(float(step(i).total_loss.detach())/n)
+for i in range(3):
+    traj.append(float(step(i).total_loss.detach())/n)
+    if i == 0:   # the gradients of the first step, before the optimiser has changed any weight they depend on
+        g = opt.flat_grad if hasattr(opt, "flat_grad") else torch.cat([p.grad.reshape(-1) for p in model.parameters() if p.grad is not None])
+        print("grad_sha256", hashlib.sha256(g.detach().float().cpu().numpy().tobytes()).hexdigest()[:16])
 torch.cuda.synchronize()
 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
 e0.record()
