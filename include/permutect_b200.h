@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define PMT_ABI_VERSION 3
+#define PMT_ABI_VERSION 4
 #define PMT_MAX_MLP_OPS 16
 #define PMT_MAX_BLOCKS 12
 #define PMT_MAX_CNN_OPS 16
@@ -378,6 +378,27 @@ size_t pmt_posterior_fit_workspace_size(int32_t n_variants, int32_t n_components
 int pmt_posterior_fit_step(const PmtPosteriorDesc* desc, const float* params, const int16_t* int_array,
                            int64_t int_stride, const void* float_array, int32_t float_kind, int64_t float_stride,
                            int32_t n_variants, float* loss_out, float* grads_out, float* posterior_totals_tc,
+                           float* somatic_snv_totals_rrra, float* snv_context_totals_rrra, void* workspace,
+                           size_t workspace_bytes, void* stream);
+
+/* One pass of PosteriorModel.learn_priors_and_spectra's batch loop (posterior_model.py:128-151) in one launch: the
+ * records [n_records] are taken in order in batches of batch_size (the last may be shorter), and every batch gets the E
+ * step of pmt_posterior_fit_step and then one step of torch.optim.Adam (betas 0.9 / 0.999, eps 1e-8, no weight decay,
+ * bias corrections from the step count) on the RAW spectra entries, the constrained values of the next batch being
+ * re-materialised through the parametrisations (cf_k, mean_multiplier_v: BoundedNumber(0, 1); log_weights_k: LogWeights;
+ * artifact and normal-artifact alpha_dv / beta_dv, concentration_v: PositiveNumber).  `params`: as for
+ * pmt_posterior_log_posteriors, the constrained values of raw_params at the start of the pass; its priors and background
+ * entries stay fixed for the pass.  raw_params, adam_m, adam_v [2K + 70] (in / out) in the order of
+ * pmt_posterior_fit_step's grads_out; adam_step[1] (in / out) += the number of batches.  batch_losses_out[number of
+ * batches] = every batch's loss.  posterior_totals_tc, somatic_snv_totals_rrra, snv_context_totals_rrra += the pass's
+ * E-step totals, as pmt_posterior_fit_step adds them (any may be NULL).  Every sum has a fixed order and no atomics:
+ * the pass is bitwise reproducible.  One CTA walks the batches; workspace: pmt_posterior_fit_pass_workspace_size(K)
+ * bytes (0 for a K outside 1..PMT_POSTERIOR_MAX_COMPONENTS). */
+size_t pmt_posterior_fit_pass_workspace_size(int32_t n_components);
+int pmt_posterior_fit_pass(const PmtPosteriorDesc* desc, const float* params, float* raw_params, float* adam_m, float* adam_v,
+                           int64_t* adam_step, double learning_rate, const int16_t* int_array, int64_t int_stride,
+                           const void* float_array, int32_t float_kind, int64_t float_stride, int64_t n_records,
+                           int32_t batch_size, float* batch_losses_out, float* posterior_totals_tc,
                            float* somatic_snv_totals_rrra, float* snv_context_totals_rrra, void* workspace,
                            size_t workspace_bytes, void* stream);
 

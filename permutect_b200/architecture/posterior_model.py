@@ -5,7 +5,9 @@ posterior model fitted by the reference loads here and ``log_posterior_and_ingre
 ``posterior_probabilities_bc`` / ``error_probabilities_b`` are one kernel launch (pmt_posterior_log_posteriors).
 
 ``learn_priors_and_spectra`` (posterior_model.py:101-165) runs its E step -- negative log evidence, its gradient w.r.t.
-the spectra, the posterior totals -- as pmt_posterior_fit_step and the optimiser / M step on the host.  Context-dependent
+the spectra, the posterior totals -- as pmt_posterior_fit_step and the optimiser / M step on the host; with its records
+resident on the model's device (``PosteriorRecords``) every pass of the batch loop, E steps and Adam steps, is one
+launch of pmt_posterior_fit_pass and only the M step stays on the host.  Context-dependent
 SNV priors are switched on for the second half of the iterations as in the reference (:125-127); its M step for them, a
 PyMC ADVI fit (posterior_model_priors.py:157-203), is replaced by a deterministic fit of the same model and variational
 family (architecture/snv_context_priors.py; pymc is absent from the image, so that one step has no reference golden).
@@ -236,8 +238,10 @@ class PosteriorModel(nn.Module):
                                  learning_rate: float = 0.001):
         """posterior_model.py:101-165: Adam on the spectra against the negative log evidence (E step, one kernel per
         batch), then the priors' M step; context-dependent SNV priors from the second half of the iterations on.
-        ``posterior_loader`` yields batches of posterior records on the model's device.  Returns the mean loss of every
-        iteration."""
+        ``posterior_loader`` yields batches of posterior records on the model's device; a ``PosteriorRecords`` there has
+        every pass run as one kernel (``_learn_on_device``).  Returns the mean loss of every iteration."""
+        if isinstance(posterior_loader, PosteriorRecords) and _same_device(posterior_loader.device, self._device):
+            return self._learn_on_device(posterior_loader, num_iterations, ignored_to_non_ignored_ratio, summary_writer, learning_rate)
         optimizer = torch.optim.Adam(self.spectra.parameters(), lr=learning_rate)
         self.priors.disable_context_dependent_snv_priors()
         history = []
@@ -261,6 +265,69 @@ class PosteriorModel(nn.Module):
             if summary_writer is not None:
                 summary_writer.add_scalar("spectrum negative log evidence", history[-1], epoch)
         return history
+
+    def _raw_spectra_tensors(self):
+        """The raw (unconstrained) tensors behind ``_spectra_tensors``, in the same order."""
+        s, na = self.spectra.somatic_spectrum, self.spectra.normal_artifact_spectra
+        art, nart = self.spectra.artifact_spectra, na.normal_spectrum
+        return [s.parametrizations.cf_k.original, s.parametrizations.log_weights_k.original, art.parametrizations.alpha_dv.original,
+                art.parametrizations.beta_dv.original, nart.parametrizations.alpha_dv.original, nart.parametrizations.beta_dv.original,
+                na.parametrizations.mean_multiplier_v.original, na.parametrizations.concentration_v.original]
+
+    def _learn_on_device(self, records: "PosteriorRecords", num_iterations, ignored_to_non_ignored_ratio: float, summary_writer,
+                         learning_rate: float):
+        """learn_priors_and_spectra with one pmt_posterior_fit_pass per iteration: the batches of ``records`` in order,
+        each an E step and an Adam step of the raw spectra (the loop's fresh optimiser: zero moments, step 0, in flat
+        device buffers for the call), then the same M step.  The raw parameters go back into the module after every pass."""
+        dev = records.device
+        lib = L.load()
+        K = self.spectra.somatic_spectrum.K
+        raws = self._raw_spectra_tensors()
+        with torch.no_grad():
+            raw = torch.cat([t.detach().reshape(-1) for t in raws]).to(torch.float32).contiguous()
+        adam_m, adam_v = torch.zeros_like(raw), torch.zeros_like(raw)
+        adam_step = torch.zeros(1, dtype=torch.int64, device=dev)
+        ws = torch.empty(int(lib.pmt_posterior_fit_pass_workspace_size(K)), dtype=torch.uint8, device=dev)
+        it, ft = records.int_tensor, records.float_tensor
+        n_batches = len(records)
+        losses = torch.empty(n_batches, dtype=torch.float32, device=dev)
+        sizes = torch.full((n_batches,), float(records.batch_size), dtype=torch.float64, device=dev)
+        sizes[-1] = records.size() - (n_batches - 1) * records.batch_size
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        self.priors.disable_context_dependent_snv_priors()
+        history = []
+        for epoch in range(1, num_iterations + 1):
+            if epoch > (num_iterations / 2):
+                self.priors.enable_context_dependent_snv_priors()
+            totals_tc = torch.zeros((len(Variation), NUM_CALLS), device=dev)
+            somatic_snv_rrra = torch.zeros((5, 5, 5, 5), device=dev)
+            snv_context_rrra = torch.zeros((5, 5, 5, 5), device=dev)
+            _, _, desc, flat = self._inputs(records)
+            L.check(lib.pmt_posterior_fit_pass(C.byref(desc), flat.data_ptr(), raw.data_ptr(), adam_m.data_ptr(), adam_v.data_ptr(),
+                                               adam_step.data_ptr(), float(learning_rate), it.data_ptr(), it.stride(0), ft.data_ptr(),
+                                               L.F16 if ft.dtype == torch.float16 else L.F32, ft.stride(0), records.size(),
+                                               records.batch_size, losses.data_ptr(), totals_tc.data_ptr(), somatic_snv_rrra.data_ptr(),
+                                               snv_context_rrra.data_ptr(), ws.data_ptr(), ws.numel(), stream))
+            with torch.no_grad():
+                off = 0
+                for t in raws:
+                    t.copy_(raw[off:off + t.numel()].view_as(t))
+                    off += t.numel()
+            self.update_priors_m_step(totals_tc, ignored_to_non_ignored_ratio, somatic_snv_rrra, snv_context_rrra)
+            history.append(float((losses.double() * sizes).sum()) / records.size())
+            if summary_writer is not None:
+                summary_writer.add_scalar("spectrum negative log evidence", history[-1], epoch)
+        return history
+
+
+def _same_device(a, b) -> bool:
+    a, b = torch.device(a), torch.device(b)
+    if a.type != b.type:
+        return False
+    if a.type != "cuda":
+        return a == b
+    cur = torch.cuda.current_device()
+    return (cur if a.index is None else a.index) == (cur if b.index is None else b.index)
 
 
 def theoretical_roc_best_threshold(error_probs_b: Tensor, recall_weight: float = 1.0) -> Tuple[float, float, float]:
@@ -318,3 +385,43 @@ class PosteriorBatch:
 
     def size(self) -> int:
         return self.int_tensor.shape[0]
+
+
+class PosteriorRecords:
+    """Posterior records resident on one CUDA device -- int16 [n, columns] and fp16 / fp32 [n, columns] tensors, the arrays
+    of generate_posterior_arrays / posterior_arrays_on_device -- served as ``PosteriorBatch`` views of ``batch_size``
+    consecutive records in order (the last batch may be shorter), so it serves wherever a loader of posterior batches does.
+    ``PosteriorModel.learn_priors_and_spectra`` given one on the model's device runs each pass as one kernel."""
+
+    def __init__(self, int_array, float_array, batch_size: int = 64, device=None):
+        if int(batch_size) < 1:
+            raise ValueError(f"batch_size must be >= 1, got {batch_size}")
+        it, ft = torch.as_tensor(int_array), torch.as_tensor(float_array)
+        dev = torch.device(device) if device is not None else (it.device if it.is_cuda else torch.device("cuda"))
+        if dev.type != "cuda":
+            raise RuntimeError("PosteriorRecords live on a CUDA device (no CPU fallback)")
+        if it.ndim != 2 or ft.ndim != 2 or it.shape[0] != ft.shape[0] or it.shape[0] == 0:
+            raise ValueError(f"need int [n, columns] and float [n, columns] arrays of the same n > 0, got {tuple(it.shape)} and {tuple(ft.shape)}")
+        if ft.dtype not in (torch.float16, torch.float32):
+            ft = ft.to(torch.float32)
+        self.int_tensor = it.to(device=dev, dtype=torch.int16).contiguous()
+        self.float_tensor = ft.to(device=dev).contiguous()
+        self.batch_size = int(batch_size)
+        self.device = self.int_tensor.device
+
+    @classmethod
+    def from_batches(cls, pairs, batch_size: int = 64, device=None) -> "PosteriorRecords":
+        """Concatenates (int array, float array) pairs -- what generate_posterior_arrays yields, host or device."""
+        ints, floats = zip(*[(torch.as_tensor(i), torch.as_tensor(f)) for i, f in pairs])
+        dev = torch.device(device) if device is not None else (ints[0].device if ints[0].is_cuda else torch.device("cuda"))
+        return cls(torch.cat([i.to(dev) for i in ints]), torch.cat([f.to(dev) for f in floats]), batch_size, dev)
+
+    def size(self) -> int:
+        return self.int_tensor.shape[0]
+
+    def __len__(self) -> int:
+        return (self.size() + self.batch_size - 1) // self.batch_size
+
+    def __iter__(self):
+        for start in range(0, self.size(), self.batch_size):
+            yield PosteriorBatch(self.int_tensor[start:start + self.batch_size], self.float_tensor[start:start + self.batch_size])

@@ -7,7 +7,7 @@ missing the compute entry points raise -- there is no fallback implementation.
 import ctypes as C
 import os
 
-PMT_ABI_VERSION = 3
+PMT_ABI_VERSION = 4
 MAX_MLP_OPS, MAX_BLOCKS, MAX_CNN_OPS = 16, 12, 16
 MAX_DIM, MAX_INFO_DIM, MAX_FEAT, MAX_CLUSTERS, TILE_ROWS = 64, 128, 32, 14, 128
 
@@ -92,7 +92,8 @@ class PmtLossGrads(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("g_supervised_b", "g_unsupervised_b", "g_alt_count_b", "g_source_b", "g_total_b")]
 
 
-EXPORTED_SYMBOLS = ["pmt_posterior_fit_step", "pmt_posterior_fit_workspace_size", "pmt_orthogonal_forward", "pmt_orthogonal_backward", "pmt_posterior_param_count", "pmt_posterior_log_posteriors", "pmt_dataset_read_indices", "pmt_pack_posterior", "pmt_adamw_step", "pmt_adamw_workspace_size", "pmt_losses_forward", "pmt_losses_backward", "pmt_losses_workspace_size", "pmt_last_error", "pmt_abi_version", "pmt_workspace_size", "pmt_forward", "pmt_forward_prepared", "pmt_backward",
+EXPORTED_SYMBOLS = ["pmt_posterior_fit_step", "pmt_posterior_fit_workspace_size", "pmt_posterior_fit_pass",
+                    "pmt_posterior_fit_pass_workspace_size", "pmt_orthogonal_forward", "pmt_orthogonal_backward", "pmt_posterior_param_count", "pmt_posterior_log_posteriors", "pmt_dataset_read_indices", "pmt_pack_posterior", "pmt_adamw_step", "pmt_adamw_workspace_size", "pmt_losses_forward", "pmt_losses_backward", "pmt_losses_workspace_size", "pmt_last_error", "pmt_abi_version", "pmt_workspace_size", "pmt_forward", "pmt_forward_prepared", "pmt_backward",
                     "pmt_decode_reads", "pmt_set_profile_events", "pmt_downsample_counts", "pmt_downsample_fill", "pmt_set_precision", "pmt_get_precision", "pmt_constraints_forward", "pmt_constraints_backward", "pmt_backward_kernels", "pmt_train_saved_bytes", "pmt_forward_train",
                     "pmt_head_backward_workspace_size", "pmt_head_backward"]
 
@@ -189,6 +190,12 @@ def load():
     lib.pmt_posterior_fit_step.argtypes = [C.POINTER(PmtPosteriorDesc), C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_int64,
                                            C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
                                            C.c_void_p]
+    lib.pmt_posterior_fit_pass_workspace_size.restype = C.c_size_t
+    lib.pmt_posterior_fit_pass_workspace_size.argtypes = [C.c_int32]
+    lib.pmt_posterior_fit_pass.restype = C.c_int
+    lib.pmt_posterior_fit_pass.argtypes = [C.POINTER(PmtPosteriorDesc), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_double, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_int64, C.c_int64, C.c_int32,
+                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
     lib.pmt_posterior_param_count.restype = C.c_int
     lib.pmt_posterior_param_count.argtypes = [C.c_int32]
     lib.pmt_posterior_log_posteriors.restype = C.c_int
