@@ -341,7 +341,11 @@ static int info_rows_w4(const PmtModelDesc& d) {
 template <int W4>
 static int launch_info_rows(const PmtModelDesc& d, const float* weights, const PmtBatch* batch, float* info_seq, cudaStream_t st) {
   const int W = 4 * W4;
-  size_t floats = (size_t)d.n_info_features * (INFO_TPB + 1);
+  // the input tile: feature-major floats, or (raw16) a tile's fp16 rows as one span of up to 127 strides of I + 8 halves
+  // plus a last row, which is the larger of the two below 8 features
+  const size_t I = (size_t)d.n_info_features;
+  const size_t raw16_words = ((INFO_TPB - 1) * (I + 8) + I + 1) / 2;
+  size_t floats = I * (INFO_TPB + 1) > raw16_words ? I * (INFO_TPB + 1) : raw16_words;
   for (int i = 0; i < d.n_info_ops; ++i) floats += (size_t)(d.info_ops[i].in_dim + 1) * W;
   const size_t smem = floats * sizeof(float) + 16;
   PMT_CHECK(smem <= 200 * 1024, "info MLP does not fit in shared memory");

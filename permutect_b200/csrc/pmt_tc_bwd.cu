@@ -837,7 +837,9 @@ static int train_claims(int n_variants) {
 }
 
 static long long tile_bound(const PmtBatch* batch, int n_claims) {
-  const long long rows = pmt_row_hint(batch);
+  // without a row count (n_rows <= 0) nothing bounds the rows per variant: a training tile holds at least one whole set
+  if (batch->n_rows <= 0) return batch->n_variants < 1 ? 1 : batch->n_variants;
+  const long long rows = batch->n_rows;
   // a tile is closed when the next set does not fit or it holds BWD_MAXV sets; the last tile of a claim may be short
   long long bound = 2 * rows / TILE + batch->n_variants / BWD_MAXV + n_claims + 8;
   if (batch->max_rows_per_variant > 0) {

@@ -58,6 +58,18 @@ def _require_cuda(t: torch.Tensor):
         raise RuntimeError("permutect_b200 computes on CUDA devices only (no CPU fallback)")
 
 
+def _check_read_width(desc: L.PmtModelDesc, batch):
+    """The batch's read rows must have the model's width: the C-ABI carries no row width, so the kernels would read rows of
+    any other width at the model's stride."""
+    reads = batch.reads
+    if reads.dtype == torch.uint8:
+        want, unit = desc.read_row_bytes, "bytes (compressed)"
+    else:
+        want, unit = desc.n_read_features, "features (decoded)"
+    if reads.dim() != 2 or reads.shape[1] != want:
+        raise ValueError(f"read rows of shape {tuple(reads.shape)} do not match the model: it takes rows of {want} {unit}")
+
+
 def forward_call(desc: L.PmtModelDesc, flat: torch.Tensor, batch, want_final: bool = False,
                  n_rows: Optional[int] = None, weights_key=None, for_training: bool = False) -> Dict[str, torch.Tensor]:
     """pmt_forward: one fused pass over a batch.  Returns logits_bk, logits_b, outlier_logits, alt/ref means,
@@ -70,6 +82,7 @@ def forward_call(desc: L.PmtModelDesc, flat: torch.Tensor, batch, want_final: bo
     ``for_training``: when the library has a saved-forward path for this call (tf32x3 mode, shapes inside the tensor-core
     envelopes, buffer within its budget) the pass goes through pmt_forward_train and ``out["saved"]`` holds what the
     backward would otherwise recompute; hand it to ``backward_call``.  PERMUTECT_B200_TRAIN_SAVED=0 keeps the recompute."""
+    _check_read_width(desc, batch)
     lib = L.load()
     _require_cuda(flat)
     dev = flat.device
@@ -116,6 +129,7 @@ def backward_call(desc: L.PmtModelDesc, flat: torch.Tensor, batch, d_logits_bk: 
                   d_alt_means: Optional[torch.Tensor], d_ref_means: Optional[torch.Tensor],
                   info_seq: Optional[torch.Tensor] = None, saved: Optional[torch.Tensor] = None) -> torch.Tensor:
     """pmt_backward: gradient of the fused pass w.r.t. the flat materialised weights."""
+    _check_read_width(desc, batch)
     lib = L.load()
     _require_cuda(flat)
     dev = flat.device
@@ -140,6 +154,7 @@ def head_backward_call(desc: L.PmtModelDesc, flat: torch.Tensor, batch, final_re
                        d_ref_means: Optional[torch.Tensor]) -> torch.Tensor:
     """pmt_head_backward: gradient w.r.t. the flat materialised weights of the rotation, translation and clustering
     head only (zeros elsewhere), from the per-read final features ``final_re`` of the forward of the same batch."""
+    _check_read_width(desc, batch)
     lib = L.load()
     _require_cuda(flat)
     dev = flat.device

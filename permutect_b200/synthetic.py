@@ -1,6 +1,7 @@
 """Synthetic variants shaped like the reference's datasets (SURVEY.md §8d), generated in bulk with numpy.
 
-Record layout follows datum.py:51-89: int16[16 + 2L], float16[6 + I], uint8[reads][12].
+Record layout follows datum.py:51-89: int16[16 + 2L], float16[6 + I], uint8[reads][row_bytes] (12 in the reference's
+datasets: 7 bytes of 56 packed binary features, then one quantised float per byte).
 """
 import numpy as np
 
@@ -28,7 +29,7 @@ def panel_counts(n: int, rng) -> tuple:
     return ref, alt
 
 
-def make_arrays(ref: np.ndarray, alt: np.ndarray, rng, n_info: int = N_INFO, hap_len: int = HAP_LEN):
+def make_arrays(ref: np.ndarray, alt: np.ndarray, rng, n_info: int = N_INFO, hap_len: int = HAP_LEN, row_bytes: int = 12):
     n = len(ref)
     ia = np.zeros((n, 16 + 2 * hap_len), np.int16)
     fa = np.zeros((n, 6 + n_info), np.float16)
@@ -48,10 +49,10 @@ def make_arrays(ref: np.ndarray, alt: np.ndarray, rng, n_info: int = N_INFO, hap
     info[:, 1::2] = (rng.random((n, (n_info) // 2)) < 0.3)
     fa[:, 6:] = info.astype(np.float16)
     total = int(ref.sum() + alt.sum())
-    reads = np.empty((total, 12), np.uint8)
+    reads = np.empty((total, row_bytes), np.uint8)
     reads[:, :7] = rng.integers(0, 256, (total, 7), dtype=np.uint8)
     reads[:, 6] &= 0xF0                                                 # 4 pad bits of the last packed byte are zero
-    reads[:, 7:] = np.clip(np.rint(32 * rng.standard_normal((total, 5)) + 128), 0, 255).astype(np.uint8)
+    reads[:, 7:] = np.clip(np.rint(32 * rng.standard_normal((total, row_bytes - 7)) + 128), 0, 255).astype(np.uint8)
     return ia, fa, reads
 
 

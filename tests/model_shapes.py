@@ -22,6 +22,7 @@ class Shape:
     reads_tc: bool = True            # the tensor-core read kernels take this shape (tf32x3 / tf32)
     cnn_tc: bool = True              # the tensor-core haplotype CNN takes it
     n_info: int = 71
+    n_read_features: int = 61        # decoded width F; compressed rows of F - 49 bytes (7 packed + F - 56 quantised)
     hap_len: int = 21                # per haplotype; the model's haplotypes_length is twice this
     num_sources: int = 1
     seed: int = 0                    # build_model's seed: logits of both signs, mostly far from saturation
@@ -31,6 +32,10 @@ class Shape:
     @property
     def bwd_tc(self) -> bool:
         return self.reads_tc if self.bwd_reads_tc is None else self.bwd_reads_tc
+
+    @property
+    def row_bytes(self) -> int:
+        return self.n_read_features - 49
 
     @property
     def hp(self) -> dict:
@@ -89,7 +94,7 @@ def build_model(shape: Shape, device, seed=None):
     hp = shape.hp
     seed = shape.seed if seed is None else seed
     torch.manual_seed(seed)
-    model = ArtifactModel(params_from_hp(hp), 61, shape.n_info, 2 * shape.hap_len, device=torch.device("cpu"))
+    model = ArtifactModel(params_from_hp(hp), shape.n_read_features, shape.n_info, 2 * shape.hap_len, device=torch.device("cpu"))
     if shape.num_sources > 1:
         model.reset_source_predictor(shape.num_sources)
     model.source_predictor.set_adversarial_strength(0.3)
@@ -116,7 +121,7 @@ def make_raw(shape: Shape, n_variants: int, seed: int) -> dict:
     from permutect_b200.synthetic import make_arrays, wgs_counts
     rng = np.random.default_rng(seed)
     ref, alt = wgs_counts(n_variants, rng)
-    ia, fa, reads = make_arrays(ref, alt, rng, n_info=shape.n_info, hap_len=shape.hap_len)
+    ia, fa, reads = make_arrays(ref, alt, rng, n_info=shape.n_info, hap_len=shape.hap_len, row_bytes=shape.row_bytes)
     sources = rng.integers(0, shape.num_sources, n_variants) if shape.num_sources > 1 else np.zeros(n_variants, np.int64)
     return dict(reads_u8=reads, read_indices=None, ref_counts=ia[:, 0].astype(np.int64), alt_counts=ia[:, 1].astype(np.int64),
                 info=fa[:, 6:].astype(np.float32), haplotypes=ia[:, 16:], labels=ia[:, 2].astype(np.int64),
@@ -129,7 +134,7 @@ def long_set_raw(shape: Shape, sets, seed: int) -> dict:
     rng = np.random.default_rng(seed)
     ref = np.array([r for r, _ in sets], np.int64)
     alt = np.array([a for _, a in sets], np.int64)
-    ia, fa, reads = make_arrays(ref, alt, rng, n_info=shape.n_info, hap_len=shape.hap_len)
+    ia, fa, reads = make_arrays(ref, alt, rng, n_info=shape.n_info, hap_len=shape.hap_len, row_bytes=shape.row_bytes)
     B = len(sets)
     sources = rng.integers(0, shape.num_sources, B) if shape.num_sources > 1 else np.zeros(B, np.int64)
     return dict(reads_u8=reads, read_indices=None, ref_counts=ref, alt_counts=alt, info=fa[:, 6:].astype(np.float32),
