@@ -32,7 +32,9 @@ size_t pmt_plan_claim_bytes(int n_variants, int n_sm);
 namespace pmt {
 
 enum class InfoKernel { WARP, ROWS, TILE };     // info_mlp_warp_kernel (small batches), info_mlp_rows_kernel<W4>, info_mlp_kernel
-enum class CnnKernel { TC, TC_SAVE, SIMT };     // hap_cnn_tc_kernel, its SAVE variant (training forward), hap_cnn_kernel
+// hap_cnn_tc_kernel over every layer, the head + tail pair (hap_cnn_tc_kernel over the head layers, then
+// hap_cnn_tail_kernel), the SAVE variant of the first (training forward), hap_cnn_kernel
+enum class CnnKernel { TC, TC_TAIL, TC_SAVE, SIMT };
 enum class ReadsKernel { TC, TC_SAVE, SIMT };   // reads_forward_tc_kernel, its SAVE variant (training forward), reads_forward_kernel
 enum class LongKernel { NONE, TC, SIMT };       // sets longer than a tile: reads_forward_tc_kernel<.., LONG>, reads_forward_long_kernel
 
@@ -65,6 +67,9 @@ struct CallPlan {
   bool cnn_tc_ok, cnn_bwd_ok;  // ... of the tensor-core haplotype CNN forward, and of its backward
   tc::TcPlan T;                // step program of the read path (built for every model: its image is part of the layout)
   cnntc::Plan C;               // cnn_tc_ok
+  bool cnn_split;              // cnn_tc_ok and the CNN has a tail: CH + CT are planned
+  cnntc::Plan CH;              // cnn_split: the head layers
+  cnntc::TailPlan CT;          // cnn_split: the tail layers
   cnnbwd::BPlan CB;            // cnn_bwd_ok
   // forward
   InfoKernel info;
@@ -116,8 +121,10 @@ int pmt_finish_reads_tc_backward(const pmt::CallPlan& C, const float* weights, f
                                  cudaStream_t st);
 // pmt_cnn_tc.cu
 size_t pmt_cnn_tc_image_bytes(const pmt::CallPlan& C);
+size_t pmt_cnn_tail_buffer_bytes(const pmt::CallPlan& C, int n_variants);
+// C.cnn TC or TC_TAIL (`tail_buf`: pmt_cnn_tail_buffer_bytes, 16-byte aligned); the images of both are packed unless reuse_image
 int pmt_launch_cnn_tc(const pmt::CallPlan& C, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
-                      bool reuse_image, cudaStream_t st);
+                      bool reuse_image, float* tail_buf, cudaStream_t st);
 // pmt_cnn_bwd.cu
 bool pmt_build_cnn_bwd_plan(const pmt::Plan& P, const pmt::cnntc::Plan& T, pmt::cnnbwd::BPlan* out);
 size_t pmt_cnn_bwd_workspace_bytes(const pmt::CallPlan& C, const PmtBatch* batch);

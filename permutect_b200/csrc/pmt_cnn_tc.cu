@@ -17,6 +17,9 @@
 // a MaxPool(kernel 2, stride 1) that follows it is fused by computing the conv at p and p+1 side by side in N.
 // MaxPool(2, 2) elsewhere is a lane shuffle (row strides are even).  Flatten + Linear is a conv whose kernel covers
 // the whole remaining length.  SELU scales are folded into the consuming weights.  Precision modes as pmt_tc.cu.
+// Inference splits the layers: this kernel runs the head and hands its last activation to hap_cnn_tail_kernel through
+// global memory, so the short tail layers (few rows per group, a full MMA -> epilogue round trip each) run as dense layers
+// over 128 variants.  The training forward (SAVE) runs every layer here.
 #include <cstring>
 
 #include "pmt_call.h"
@@ -96,7 +99,7 @@ struct EpiItem {   // per-item epilogue constants (three 16-byte shared loads)
   int inv_L, L_in, L_pool, L_next;
   int row0, out_ch, save_a, save_bits;   // SAVE: float offsets inside a group's block of the save buffer (-1: none)
 };
-constexpr int F_DUP = 1, F_POOL2 = 2, F_GLOBAL = 4, F_SELU = 8;
+constexpr int F_DUP = 1, F_POOL2 = 2, F_GLOBAL = 4, F_SELU = 8, F_TAIL = 16;
 
 struct Bars {
   EpiItem epi[MAX_ITEMS];
@@ -112,7 +115,7 @@ __global__ void __launch_bounds__(THREADS, 1)
 hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restrict__ image, const float* __restrict__ wflat,
                   const __grid_constant__ PmtModelDesc D, const void* __restrict__ haps, int hap_kind, long long hap_stride,
                   int n_variants, float* __restrict__ info_seq,
-                  const __grid_constant__ SaveLayout SL, float* __restrict__ save) {
+                  const __grid_constant__ SaveLayout SL, float* __restrict__ save, float* __restrict__ tail_buf) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   unsigned char* p = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const unsigned act = smem_addr(p); p += 2 * BUF_BYTES;                 // hi buffer, then lo buffer (planes 8..15)
@@ -158,7 +161,8 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
     o.d = tmem_base + I.chunk * CHUNK_COLS;
     o.first = Ly.first; o.count = Ly.first ? Ly.ksteps : Ly.taps; o.N = Ly.N; o.need = I.need;
     EpiItem& e = S->epi[tid];
-    e.flags = (Ly.dup ? F_DUP : 0) | (Ly.pool2 ? F_POOL2 : 0) | (Ly.to_global ? F_GLOBAL : 0) | (Ly.act == PMT_ACT_SELU ? F_SELU : 0);
+    e.flags = (Ly.dup ? F_DUP : 0) | (Ly.pool2 ? F_POOL2 : 0) | (Ly.to_global ? F_GLOBAL : 0) | (Ly.act == PMT_ACT_SELU ? F_SELU : 0) |
+              (Ly.to_tail ? F_TAIL : 0);
     e.lo_col = Ly.N; e.tmem_col = I.chunk * CHUNK_COLS; e.bias_off = I.layer * 32 * (int)sizeof(float);
     e.inv_L = Ly.inv_L; e.L_in = Ly.L_in; e.L_pool = Ly.L_pool; e.L_next = Ly.L_next;
     e.row0 = I.chunk * 128; e.out_ch = Ly.out_ch;
@@ -329,7 +333,14 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
             }
             if (save_bits >= 0) reinterpret_cast<unsigned char*>(sg + save_bits)[cq * cols + col] = (unsigned char)win;
           }
-          if (valid) {
+          if (!SAVE && (flags & F_TAIL)) {   // the split forward: fp32 into the tail kernel's A layout (pmt_cnn_tc.cuh)
+            if (valid) {
+              const int gv = v0 + v;
+              float* dst = tail_buf + ((size_t)(gv >> 7) * (L_next * 8) + pp * 8 + 2 * cq) * (TAIL_PLANE / 4) + (gv & 127) * 4;
+              *reinterpret_cast<float4*>(dst) = make_float4(x[0], x[1], x[2], x[3]);
+              *reinterpret_cast<float4*>(dst + TAIL_PLANE / 4) = make_float4(x[4], x[5], x[6], x[7]);
+            }
+          } else if (valid) {
             const unsigned dst = act + (2 * cq) * PLANE_BYTES + (v * L_next + pp) * 16;
             sts128(dst, make_float4(x[0], x[1], x[2], x[3]));
             sts128(dst + PLANE_BYTES, make_float4(x[4], x[5], x[6], x[7]));
@@ -350,6 +361,249 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
   tc_fence_before();
   __syncthreads();
   if (warp == MMA_WARP) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
+}
+
+// ------------------------------------------------------------------------------------------------
+// The tail of the split forward (pmt_cnn_tc.cuh: TailPlan): persistent CTAs over tiles of 128 variants, M = 128.
+//   warps 0-7  epilogue: thread = variant (TMEM lane) x 16 output channels; they also derive each stage's A_lo rows from
+//              the A_hi rows the loader brought in (A_hi is the fp32 activation itself: the MMA reads its TF32 part).
+//   warp  8    MMA issuer: the first tail layer streams its K through TAIL_STAGES stages of 32 floats, the others read
+//              the previous tail layer's output from the `mid` buffer.
+//   warp  9    loader: one bulk copy per stage.
+// TMEM: the first layer's accumulator in columns [0, 2 N0), tail layer t >= 1 (N = 32) in [64 + 64 t, 128 + 64 t).
+// Every wait's phase follows from the stage-use counter u or the tile counter it.
+// ------------------------------------------------------------------------------------------------
+struct TailBars {
+  unsigned long long loaded[TAIL_STAGES];   // A_hi of the stage landed (expect_tx)
+  unsigned long long full[TAIL_STAGES];     // A_lo written (epilogue warps)
+  unsigned long long empty[TAIL_STAGES];    // the stage's MMAs completed (tcgen05.commit)
+  unsigned long long acc[MAX_TAIL];         // tail layer t's accumulator complete
+  unsigned long long mid;                   // the mid buffer holds the next tail layer's input (epilogue warps)
+  unsigned long long free0;                 // the first layer's accumulator has been read (epilogue warps)
+  unsigned tmem_base;
+  int pad_;
+};
+constexpr int TAIL_TMEM_COLS = 256;
+__host__ __device__ constexpr int tail_acc_col(int t) { return t == 0 ? 0 : 64 + 64 * t; }
+
+// 4 k-steps of one dense tail layer: A (128 rows) and B in the no-swizzle K-major layout, K chunks TAIL_PLANE apart in A
+template <int N, int PASSES>
+__device__ __forceinline__ void issue_dense(unsigned d, unsigned a_hi, unsigned a_lo, unsigned b, bool first) {
+  constexpr int R = 2 * N;
+#pragma unroll
+  for (int ks = 0; ks < 4; ++ks) {
+    const unsigned ao = (unsigned)(2 * ks * (TAIL_PLANE / 16)), bo = (unsigned)(2 * ks * R);
+    const unsigned acc = (first && ks == 0) ? 0u : 1u;
+    if (PASSES == 3) {
+      mma_ss<make_idesc(2 * N)>(d, a_hi + ao, b + bo, acc);
+      mma_ss<make_idesc(N)>(d, a_lo + ao, b + bo, 1u);
+    } else {
+      mma_ss<make_idesc(N)>(d, a_hi + ao, b + bo, acc);
+    }
+  }
+}
+template <int PASSES>
+__device__ __forceinline__ void issue_dense_n(int N, unsigned d, unsigned a_hi, unsigned a_lo, unsigned b, bool first) {
+  if (N == 64) issue_dense<64, PASSES>(d, a_hi, a_lo, b, first);
+  else issue_dense<32, PASSES>(d, a_hi, a_lo, b, first);
+}
+
+template <int PASSES>
+__global__ void __launch_bounds__(TAIL_THREADS, 1)
+hap_cnn_tail_kernel(const __grid_constant__ TailPlan TT, const unsigned char* __restrict__ image, const float* __restrict__ wflat,
+                    const __grid_constant__ PmtModelDesc D, const float* __restrict__ tail_buf, int n_variants,
+                    float* __restrict__ info_seq) {
+  extern __shared__ __align__(1024) unsigned char smem_raw[];
+  unsigned char* p = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  const unsigned stage_s = smem_addr(p); p += TAIL_STAGES * 2 * TAIL_STAGE_BYTES;   // stage s: A_hi, then A_lo
+  const unsigned mid_s = smem_addr(p); p += 2 * TAIL_STAGE_BYTES;                    // A_hi, A_lo of tail layers 1..
+  unsigned char* img_s = p; p += TT.image_bytes;
+  float* bias_s = reinterpret_cast<float*>(p); p += MAX_TAIL * 32 * sizeof(float);
+  TailBars* S = reinterpret_cast<TailBars*>((reinterpret_cast<uintptr_t>(p) + 15) & ~uintptr_t(15));
+
+  const int tid = threadIdx.x;
+  const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
+  const int lane = tid & 31;
+  const int nt = TT.n_layers, ns = TT.K0 / (4 * TAIL_STAGE_CHUNKS);   // stages per tile
+  const int n_tiles = (n_variants + 127) / 128;
+
+  if (tid == 0) {
+    for (int s = 0; s < TAIL_STAGES; ++s) {
+      mbar_init(smem_addr(&S->loaded[s]), 1);
+      mbar_init(smem_addr(&S->full[s]), TAIL_EPI_WARPS);
+      mbar_init(smem_addr(&S->empty[s]), 1);
+    }
+    for (int t = 0; t < MAX_TAIL; ++t) mbar_init(smem_addr(&S->acc[t]), 1);
+    mbar_init(smem_addr(&S->mid), TAIL_EPI_WARPS);
+    mbar_init(smem_addr(&S->free0), TAIL_EPI_WARPS);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  for (int i = tid; i < TT.image_bytes / 16; i += TAIL_THREADS)
+    reinterpret_cast<uint4*>(img_s)[i] = __ldg(reinterpret_cast<const uint4*>(image) + i);
+  for (int i = tid; i < nt * 32; i += TAIL_THREADS) {
+    const Layer& Ly = TT.layer[i / 32];
+    const int n = i % 32, b_off = D.cnn_ops[Ly.op].b_off;
+    bias_s[i] = (n < Ly.out_ch && b_off >= 0) ? __ldg(wflat + b_off + n) : 0.f;
+  }
+  if (warp == TAIL_EPI_WARPS) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_addr(&S->tmem_base)), "r"(TAIL_TMEM_COLS));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
+  }
+  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const unsigned tmem_base = __shfl_sync(0xffffffffu, S->tmem_base, 0);
+  const unsigned img_a = smem_addr(img_s);
+
+  if (warp == TAIL_EPI_WARPS + 1) {
+    // ===================================== loader =====================================
+    if (elect_one()) {
+      int u = 0;
+      for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        const float* src = tail_buf + (size_t)tile * (TT.K0 / 4) * (TAIL_PLANE / 4);
+        for (int k = 0; k < ns; ++k, ++u) {
+          const int s = u % TAIL_STAGES;
+          if (u >= TAIL_STAGES) mbar_wait(smem_addr(&S->empty[s]), (u / TAIL_STAGES - 1) & 1);
+          mbar_expect_tx(smem_addr(&S->loaded[s]), TAIL_STAGE_BYTES);
+          bulk_g2s(stage_s + s * 2 * TAIL_STAGE_BYTES, src + (size_t)k * (TAIL_STAGE_BYTES / 4), TAIL_STAGE_BYTES,
+                   smem_addr(&S->loaded[s]));
+        }
+      }
+    }
+    __syncwarp();
+  } else if (warp == TAIL_EPI_WARPS) {
+    // ===================================== MMA issuer =====================================
+    const Layer& L0y = TT.layer[0];
+    const int N0 = L0y.N;
+    int u = 0;
+    for (int tile = blockIdx.x, it = 0; tile < n_tiles; tile += gridDim.x, ++it) {
+      if (it > 0) mbar_wait(smem_addr(&S->free0), (it - 1) & 1);
+      for (int k = 0; k < ns; ++k, ++u) {
+        const int s = u % TAIL_STAGES;
+        mbar_wait(smem_addr(&S->full[s]), (u / TAIL_STAGES) & 1);
+        tc_fence_after();
+        if (elect_one()) {
+          const unsigned a = stage_s + s * 2 * TAIL_STAGE_BYTES;
+          const unsigned b = img_a + L0y.img_off + k * TAIL_STAGE_CHUNKS * (2 * N0 * 16);
+          issue_dense_n<PASSES>(N0, tmem_base, desc_lo(a, TAIL_PLANE), desc_lo(a + TAIL_STAGE_BYTES, TAIL_PLANE), desc_lo(b, 2 * N0 * 16),
+                                k == 0);
+          mma_commit(smem_addr(&S->empty[s]));
+          if (k == ns - 1) mma_commit(smem_addr(&S->acc[0]));
+        }
+        __syncwarp();
+      }
+      for (int t = 1; t < nt; ++t) {
+        const Layer& Ly = TT.layer[t];
+        mbar_wait(smem_addr(&S->mid), (it * (nt - 1) + t - 1) & 1);
+        tc_fence_after();
+        if (elect_one()) {
+          issue_dense_n<PASSES>(Ly.N, tmem_base + tail_acc_col(t), desc_lo(mid_s, TAIL_PLANE), desc_lo(mid_s + TAIL_STAGE_BYTES, TAIL_PLANE),
+                                desc_lo(img_a + Ly.img_off, 2 * Ly.N * 16), true);
+          mma_commit(smem_addr(&S->acc[t]));
+        }
+        __syncwarp();
+      }
+    }
+  } else {
+    // ===================================== epilogue warps =====================================
+    const int quarter = warp & 3, cq = warp >> 2;
+    const int row = quarter * 32 + lane;       // TMEM lane = variant inside the tile
+    const int c0 = cq * 16;                    // this thread's 16 output channels
+    const unsigned trow = tmem_base + ((unsigned)(quarter * 32) << 16) + c0;
+    int u = 0;
+    for (int tile = blockIdx.x, it = 0; tile < n_tiles; tile += gridDim.x, ++it) {
+      for (int k = 0; k < ns; ++k, ++u) {
+        const int s = u % TAIL_STAGES;
+        mbar_wait(smem_addr(&S->loaded[s]), (u / TAIL_STAGES) & 1);
+        if (PASSES == 3) {   // A_lo = A - its TF32 part, as the head layers' epilogue splits its activations
+          const unsigned hi = stage_s + s * 2 * TAIL_STAGE_BYTES;
+#pragma unroll
+          for (int i = 0; i < TAIL_STAGE_BYTES / 16 / (32 * TAIL_EPI_WARPS); ++i) {
+            const unsigned o = (unsigned)((i * 32 * TAIL_EPI_WARPS + tid) * 16);
+            float4 v = lds128(hi + o);
+            v.x -= __uint_as_float(__float_as_uint(v.x) & 0xFFFFE000u);
+            v.y -= __uint_as_float(__float_as_uint(v.y) & 0xFFFFE000u);
+            v.z -= __uint_as_float(__float_as_uint(v.z) & 0xFFFFE000u);
+            v.w -= __uint_as_float(__float_as_uint(v.w) & 0xFFFFE000u);
+            sts128(hi + TAIL_STAGE_BYTES + o, v);
+          }
+          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(smem_addr(&S->full[s]));
+      }
+      const int gv = tile * 128 + row;
+      const bool valid = gv < n_variants;
+      for (int t = 0; t < nt; ++t) {
+        const Layer& Ly = TT.layer[t];
+        const int N = Ly.N;
+        const unsigned tcol = trow + tail_acc_col(t);
+        const unsigned bias_a = smem_addr(bias_s) + (t * 32 + c0) * (int)sizeof(float);
+        mbar_wait(smem_addr(&S->acc[t]), it & 1);
+        tc_fence_after();
+        float x[16];
+        {
+          unsigned r[16], rl[16];
+          tmem_ld16(tcol, r);
+          if (PASSES == 3) tmem_ld16(tcol + N, rl);
+          if (Ly.pool2) {   // N = 64: the conv at the two positions of the pooling window, side by side
+            unsigned r2[16], rl2[16];
+            tmem_ld16(tcol + 32, r2);
+            if (PASSES == 3) tmem_ld16(tcol + N + 32, rl2);
+            tmem_wait_ld();
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+              const float u0 = PASSES == 3 ? __uint_as_float(r[i]) + __uint_as_float(rl[i]) : __uint_as_float(r[i]);
+              const float u1 = PASSES == 3 ? __uint_as_float(r2[i]) + __uint_as_float(rl2[i]) : __uint_as_float(r2[i]);
+              x[i] = fmaxf(u0, u1);
+            }
+          } else {
+            tmem_wait_ld();
+#pragma unroll
+            for (int i = 0; i < 16; ++i) x[i] = PASSES == 3 ? __uint_as_float(r[i]) + __uint_as_float(rl[i]) : __uint_as_float(r[i]);
+          }
+        }
+        tc_fence_before();   // the accumulator has been read
+        if (t == 0) {
+          __syncwarp();
+          if (lane == 0) mbar_arrive(smem_addr(&S->free0));
+        }
+#pragma unroll
+        for (int i = 0; i < 16; i += 4) {
+          const float4 b = lds128(bias_a + i * 4);
+          x[i] += b.x; x[i + 1] += b.y; x[i + 2] += b.z; x[i + 3] += b.w;
+        }
+        const bool selu = Ly.act == PMT_ACT_SELU;
+        if (Ly.to_global) {
+          if (valid) {
+            float* dst = info_seq + (long long)gv * (D.d_info + D.d_seq) + D.d_info + c0;
+#pragma unroll
+            for (int i = 0; i < 16; ++i)
+              if (c0 + i < Ly.out_ch) dst[i] = selu ? SELU_SCALE * selu_u(x[i]) : x[i];
+          }
+        } else {
+          if (selu) selu_u_n<16>(x);
+#pragma unroll
+          for (int i = 0; i < 16; i += 4) {
+            const unsigned dst = mid_s + ((c0 + i) / 4) * TAIL_PLANE + row * 16;
+            sts128(dst, make_float4(x[i], x[i + 1], x[i + 2], x[i + 3]));
+            if (PASSES == 3) {
+#pragma unroll
+              for (int j = i; j < i + 4; ++j) x[j] -= __uint_as_float(__float_as_uint(x[j]) & 0xFFFFE000u);
+              sts128(dst + TAIL_STAGE_BYTES, make_float4(x[i], x[i + 1], x[i + 2], x[i + 3]));
+            }
+          }
+          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          __syncwarp();
+          if (lane == 0) mbar_arrive(smem_addr(&S->mid));
+        }
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == TAIL_EPI_WARPS) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TAIL_TMEM_COLS));
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -385,6 +639,23 @@ __global__ void pack_cnn_tc_kernel(const __grid_constant__ PmtModelDesc D, const
   }
 }
 
+// tail images: a dense layer over the whole input window.  Row n = 32 pos + co (hi rows [0, N), remainders [N, 2N)) holds
+// output position pos; K column kk = 32 p + ci is input position p, channel ci: the conv's tap p - pos
+__global__ void pack_cnn_tail_kernel(const __grid_constant__ PmtModelDesc D, const __grid_constant__ TailPlan TT, const float* __restrict__ w,
+                                     unsigned char* __restrict__ image) {
+  const Layer& Ly = TT.layer[blockIdx.x];
+  const int N = Ly.N, R = 2 * N, chunks = Ly.L_in * 8;
+  for (int idx = blockIdx.y * blockDim.x + threadIdx.x; idx < chunks * R * 4; idx += gridDim.y * blockDim.x) {
+    const int e = idx & 3, r = (idx >> 2) % R, ch = (idx >> 2) / R;
+    const int kk = ch * 4 + e, n = r % N, tap = (kk >> 5) - (n >> 5);
+    const float v = tap >= 0 && tap < Ly.taps ? cnn_weight(D, Ly, w, tap, n & 31, kk & 31) : 0.f;
+    unsigned hb;
+    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(v));
+    const float hi = __uint_as_float(hb);
+    *reinterpret_cast<float*>(image + (size_t)Ly.img_off + (size_t)idx * 4) = r < N ? hi : v - hi;
+  }
+}
+
 }  // namespace cnntc
 }  // namespace pmt
 
@@ -393,6 +664,8 @@ __global__ void pack_cnn_tc_kernel(const __grid_constant__ PmtModelDesc D, const
 // ================================================================================================
 using namespace pmt;
 using namespace pmt::cnntc;
+
+static bool schedule_groups(cnntc::Plan& T, int hap_len);
 
 // Builds the layer program; returns false when the CNN is outside this kernel's envelope (the FP32 SIMT kernel
 // hap_cnn_kernel then runs instead).
@@ -470,6 +743,12 @@ bool pmt_build_cnn_tc_plan(const pmt::Plan& P, cnntc::Plan* out) {
     Ly.inv_L = 65536 / Ly.L_in + 1;
   }
   T.image_bytes = bytes;
+  return schedule_groups(T, d.hap_len);
+}
+
+// The group size G and the item list of hap_cnn_tc_kernel over T's layers.
+static bool schedule_groups(cnntc::Plan& T, int hap_len) {
+  const int bytes = T.image_bytes;
   // variants per group: every layer's rows must fit MAX_CHUNKS chunks and the planes; pick the G with the fewest MMA
   // cycles per variant
   // Every layer's weight image stays resident in shared memory next to the two activation buffers: that is the kernel's
@@ -481,7 +760,7 @@ bool pmt_build_cnn_tc_plan(const pmt::Plan& P, cnntc::Plan* out) {
   double best = 1e30;
   int best_g = 0;
   for (int G = 1; G <= 128; ++G) {
-    if (G * d.hap_len > PLANE_ROWS) break;
+    if (G * hap_len > PLANE_ROWS) break;
     double cost = 0;
     bool ok = true;
     for (int l = 0; l < T.n_layers; ++l) {
@@ -527,15 +806,64 @@ bool pmt_build_cnn_tc_plan(const pmt::Plan& P, cnntc::Plan* out) {
   return true;
 }
 
-size_t pmt_cnn_tc_image_bytes(const CallPlan& C) { return C.cnn_tc_ok ? (size_t)C.C.image_bytes + 256 : 0; }
+bool pmt_build_cnn_split_plan(const cnntc::Plan& T, int hap_len, cnntc::Plan* head, cnntc::TailPlan* tail) {
+  cnntc::Plan& H = *head;
+  cnntc::TailPlan& TT = *tail;
+  memset(&H, 0, sizeof(H));
+  memset(&TT, 0, sizeof(TT));
+  int s = -1;   // the first tail layer: the earliest from which every layer qualifies
+  for (int c = 1; c < T.n_layers && s < 0; ++c) {
+    bool ok = T.n_layers - c <= MAX_TAIL;
+    for (int l = c; ok && l < T.n_layers; ++l) {
+      const Layer& Ly = T.layer[l];
+      ok = Ly.L_pool == 1 && (Ly.L_out == 1 || (Ly.L_out == 2 && Ly.pool2)) && Ly.L_in * 32 <= (l == c ? TAIL_MAX_K : 32);
+    }
+    if (ok) s = c;
+  }
+  if (s < 0) return false;
+  TT.n_layers = T.n_layers - s;
+  TT.K0 = T.layer[s].L_in * 32;
+  TT.image_off = (T.image_bytes + 255) & ~255;
+  int bytes = 0;
+  for (int t = 0; t < TT.n_layers; ++t) {
+    Layer& Ly = TT.layer[t];
+    Ly = T.layer[s + t];
+    Ly.N = 32 * Ly.L_out;
+    Ly.img_off = bytes;
+    Ly.img_bytes = Ly.L_in * 8 * 2 * Ly.N * 16;
+    bytes += Ly.img_bytes;
+  }
+  TT.image_bytes = bytes;
+  TT.smem = 1024 + TAIL_STAGES * 2 * TAIL_STAGE_BYTES + 2 * TAIL_STAGE_BYTES + bytes + MAX_TAIL * 32 * 4 + (int)sizeof(TailBars) + 64;
+  if (TT.smem > 227 * 1024) return false;
+  // the head: the layers before s, their images where the single kernel has them
+  H.n_layers = s;
+  H.L0 = T.L0;
+  for (int l = 0; l < s; ++l) H.layer[l] = T.layer[l];
+  H.layer[s - 1].to_tail = 1;
+  H.image_bytes = T.layer[s].img_off;
+  return schedule_groups(H, hap_len);
+}
+
+size_t pmt_cnn_tc_image_bytes(const CallPlan& C) {
+  if (!C.cnn_tc_ok) return 0;
+  return (C.cnn_split ? (size_t)C.CT.image_off + C.CT.image_bytes : (size_t)C.C.image_bytes) + 256;
+}
+
+size_t pmt_cnn_tail_buffer_bytes(const CallPlan& C, int n_variants) {
+  // whenever the pair may run (PMT_CNN_SINGLE=0 selects it below its batch-size threshold)
+  const bool may_split = C.cnn_split && (C.cnn == CnnKernel::TC || C.cnn == CnnKernel::TC_TAIL);
+  return may_split ? (size_t)(n_variants + 127) / 128 * 128 * C.CT.K0 * sizeof(float) : 0;
+}
 
 template <int PASSES, bool SAVE>
 static int launch_cnn_tc(const cnntc::Plan& T, const unsigned char* image, const float* weights, const PmtModelDesc& D, const void* haps,
-                         const PmtBatch* batch, int n, float* info_seq, const SaveLayout& SL, float* save, int grid, cudaStream_t st) {
+                         const PmtBatch* batch, int n, float* info_seq, const SaveLayout& SL, float* save, int grid, cudaStream_t st,
+                         float* tail_buf = nullptr) {
   const size_t smem = 2 * BUF_BYTES + T.image_bytes + MAX_LAYERS * 32 * sizeof(float) + sizeof(Bars) + 1024 + 64;
   PMT_CUDA(cudaFuncSetAttribute(hap_cnn_tc_kernel<PASSES, SAVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   hap_cnn_tc_kernel<PASSES, SAVE><<<grid, cnntc::THREADS, smem, st>>>(T, image, weights, D, haps, batch->hap_kind, batch->hap_stride, n, info_seq,
-                                                               SL, save);
+                                                               SL, save, tail_buf);
   return 0;
 }
 
@@ -573,16 +901,34 @@ int pmt_pack_cnn_tc_images(const pmt::Plan& P, const cnntc::Plan& T, const float
   return 0;
 }
 
+template <int PASSES>
+static int launch_cnn_tail(const TailPlan& TT, const unsigned char* image, const float* weights, const PmtModelDesc& D, const float* tail_buf,
+                           int n, float* info_seq, int n_sm, cudaStream_t st) {
+  const int n_tiles = (n + 127) / 128;
+  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_tail_kernel<PASSES>, cudaFuncAttributeMaxDynamicSharedMemorySize, TT.smem));
+  hap_cnn_tail_kernel<PASSES><<<n_tiles < n_sm ? n_tiles : n_sm, TAIL_THREADS, TT.smem, st>>>(TT, image + TT.image_off, weights, D, tail_buf, n,
+                                                                                               info_seq);
+  return 0;
+}
+
 // `image` is a 16-byte aligned device buffer of pmt_cnn_tc_image_bytes(C) bytes.
 int pmt_launch_cnn_tc(const CallPlan& C, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
-                      bool reuse_image, cudaStream_t st) {
-  const cnntc::Plan& T = C.C;
-  if (!reuse_image) pack_cnn_tc_kernel<<<dim3(T.n_layers, 16), 256, 0, st>>>(C.P.d, T, weights, image);
-  const int n_groups = (batch->n_variants + T.G - 1) / T.G;
+                      bool reuse_image, float* tail_buf, cudaStream_t st) {
+  if (!reuse_image) {   // both forms' images, so that a prepared call finds whichever it runs
+    pack_cnn_tc_kernel<<<dim3(C.C.n_layers, 16), 256, 0, st>>>(C.P.d, C.C, weights, image);
+    if (C.cnn_split) pack_cnn_tail_kernel<<<dim3(C.CT.n_layers, 16), 256, 0, st>>>(C.P.d, C.CT, weights, image + C.CT.image_off);
+  }
+  const bool split = C.cnn == CnnKernel::TC_TAIL;
+  const cnntc::Plan& T = split ? C.CH : C.C;
+  const int n = batch->n_variants;
+  const int n_groups = (n + T.G - 1) / T.G;
   const int grid = n_groups < C.n_sm ? n_groups : C.n_sm;
   SaveLayout SL;
   memset(&SL, 0, sizeof(SL));
-  return C.mode == PMT_PRECISION_TF32
-             ? launch_cnn_tc<1, false>(T, image, weights, C.P.d, batch->haplotypes, batch, batch->n_variants, info_seq, SL, nullptr, grid, st)
-             : launch_cnn_tc<3, false>(T, image, weights, C.P.d, batch->haplotypes, batch, batch->n_variants, info_seq, SL, nullptr, grid, st);
+  if (C.mode == PMT_PRECISION_TF32) {
+    if (launch_cnn_tc<1, false>(T, image, weights, C.P.d, batch->haplotypes, batch, n, info_seq, SL, nullptr, grid, st, tail_buf)) return 1;
+    return split ? launch_cnn_tail<1>(C.CT, image, weights, C.P.d, tail_buf, n, info_seq, C.n_sm, st) : 0;
+  }
+  if (launch_cnn_tc<3, false>(T, image, weights, C.P.d, batch->haplotypes, batch, n, info_seq, SL, nullptr, grid, st, tail_buf)) return 1;
+  return split ? launch_cnn_tail<3>(C.CT, image, weights, C.P.d, tail_buf, n, info_seq, C.n_sm, st) : 0;
 }

@@ -31,6 +31,7 @@ struct Layer {
   int L_in, L_out, L_pool, L_next;
   int inv_L;      // ceil(65536 / L_in) + : row / L_in == (row * inv_L) >> 16 for rows < 512
   int act, to_global, out_ch;
+  int to_tail;    // the split forward's last head layer: writes its pooled activation to the tail buffer
   int img_off, img_bytes;
   // packing
   int op, in_ch, ksize, flat_len, scale_in, is_linear;
@@ -46,6 +47,31 @@ struct Plan {
   int n_chunks[MAX_LAYERS];
   Layer layer[MAX_LAYERS];
   Item item[MAX_ITEMS];
+};
+
+// ---- the split inference forward: hap_cnn_tc_kernel runs the head layers, hap_cnn_tail_kernel the short tail ----
+// The tail is the trailing layers that each produce one position (after pooling), the first of them reading at most
+// TAIL_MAX_K floats per variant and the others 32.  Every tail layer is a dense layer over its whole input window,
+// M = 128 variants per tile: a conv's output positions sit side by side in N (N = 32 L_out) and a MaxPool(2, 2) that
+// follows it is the max of the two column halves.  The head writes its last layer's pooled activation (selu_u applied)
+// as fp32 to the tail buffer, [tile of 128 variants][K / 4 chunks][128 rows][4 floats]: the tail kernel's A operand in
+// the no-swizzle K-major layout, so a K-stage of one tile is one contiguous bulk copy.
+constexpr int TAIL_MAX_K = 256;
+constexpr int MAX_TAIL = 3;
+constexpr int TAIL_STAGE_CHUNKS = 8;                          // 16-byte K chunks per pipeline stage: 32 floats, 4 k-steps
+constexpr int TAIL_PLANE = 128 * 16;                          // one K chunk of a 128-row tile
+constexpr int TAIL_STAGE_BYTES = TAIL_STAGE_CHUNKS * TAIL_PLANE;
+constexpr int TAIL_STAGES = 2;
+constexpr int TAIL_EPI_WARPS = 8;                             // warps 0-7 epilogue, 8 MMA issuer, 9 bulk loader
+constexpr int TAIL_THREADS = 32 * (TAIL_EPI_WARPS + 2);
+
+struct TailPlan {
+  int n_layers;
+  int K0;              // floats per variant in the tail buffer: the first tail layer's input, L_in * 32
+  int image_off;       // byte offset of the tail images inside the CNN image buffer (after the single kernel's)
+  int image_bytes;
+  int smem;            // dynamic shared memory of hap_cnn_tail_kernel
+  Layer layer[MAX_TAIL];   // N = 32 L_out; img_off inside the tail images; to_global on the last
 };
 
 // ---- training: what the SAVE variant of the forward leaves in global memory for the backward (pmt_cnn_bwd.cu) ----
@@ -101,6 +127,8 @@ struct BPlan {
 
 // host (pmt_cnn_tc.cu)
 bool pmt_build_cnn_tc_plan(const pmt::Plan& P, pmt::cnntc::Plan* out);
+// The head + tail pair of the inference forward from the single kernel's plan; false when the CNN has no tail.
+bool pmt_build_cnn_split_plan(const pmt::cnntc::Plan& T, int hap_len, pmt::cnntc::Plan* head, pmt::cnntc::TailPlan* tail);
 void pmt_cnn_save_layout(const pmt::cnntc::Plan& T, pmt::cnntc::SaveLayout* out);
 int pmt_pack_cnn_tc_images(const pmt::Plan& P, const pmt::cnntc::Plan& T, const float* weights, unsigned char* image, cudaStream_t st);
 // the forward over variants [v_first, v_first + n) of the batch with every layer's activations saved; `image` must hold

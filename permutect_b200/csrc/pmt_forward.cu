@@ -6,6 +6,7 @@
 //   reads_forward_kernel  decode -> read_embedding -> concat -> gated ref/alt blocks -> reducer ->
 //                         rotation -> clustering head -> per-variant sums (artifact_model.py:243-297)
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 
 #include "pmt_call.h"
@@ -789,6 +790,7 @@ int pmt_call_plan(const PmtModelDesc* desc, const PmtBatch* batch, bool train, C
   pmt_tc_plan(P, &C.T);
   C.cnn_tc_ok = pmt_build_cnn_tc_plan(P, &C.C);
   C.cnn_bwd_ok = C.cnn_tc_ok && pmt_build_cnn_bwd_plan(P, C.C, &C.CB);
+  C.cnn_split = C.cnn_tc_ok && pmt_build_cnn_split_plan(C.C, P.d.hap_len, &C.CH, &C.CT);
   const bool fp32 = C.mode == PMT_PRECISION_FP32;
   // the backward: the tensor-core read-path and haplotype-CNN kernels (pmt_tc_bwd.cu, pmt_cnn_bwd.cu) unless the FP32 mode
   // is selected or the model is outside their envelope, the FP32 SIMT kernels otherwise
@@ -799,7 +801,12 @@ int pmt_call_plan(const PmtModelDesc* desc, const PmtBatch* batch, bool train, C
   const int B = batch ? batch->n_variants : 0;
   C.info_w4 = info_rows_w4(P.d);
   C.info = C.info_w4 == 0 ? InfoKernel::TILE : B <= 4096 ? InfoKernel::WARP : InfoKernel::ROWS;   // small batch: latency, not throughput
-  C.cnn = train ? CnnKernel::TC_SAVE : !fp32 && C.cnn_tc_ok ? CnnKernel::TC : CnnKernel::SIMT;
+  // the head + tail pair once the head kernel has a group for every SM; below that a call is a chain of latencies, and the
+  // pair's second launch and global round trip cost more than the tail's MMA round trips it saves
+  C.cnn = train                                        ? CnnKernel::TC_SAVE
+          : fp32 || !C.cnn_tc_ok                        ? CnnKernel::SIMT
+          : C.cnn_split && B >= (long long)C.CH.G * C.n_sm ? CnnKernel::TC_TAIL
+                                                        : CnnKernel::TC;
   C.reads = fp32 ? ReadsKernel::SIMT : train ? ReadsKernel::TC_SAVE : ReadsKernel::TC;
   C.lng = !batch || !pmt_has_long_sets(batch)                            ? LongKernel::NONE
           : !fp32 && pmt_tc_long_layout(P, batch, C.n_sm, &C.long_tc) ? LongKernel::TC
@@ -821,9 +828,9 @@ static size_t long_scratch_floats_per_cta(const Plan& P, const PmtBatch* batch) 
 // Workspace layout of the forward: the packed weight images sit at FIXED offsets from the base (they depend on the model
 // only: pmt_forward_prepared finds them there), the batch-dependent regions follow:
 //   [256 B counters][SIMT images][tcgen05 read-kernel images][tcgen05 CNN images] | [info_seq][long-set scratch]
-//   [tile list, or the training forward's planner scratch][long-set tensor-core region]
+//   [tile list, or the training forward's planner scratch][long-set tensor-core region][CNN tail buffer]
 struct FwdLayout {
-  size_t image, tc_image, cnn_tc_image, info_seq, long_scratch, tiles, long_tc, end;
+  size_t image, tc_image, cnn_tc_image, info_seq, long_scratch, tiles, long_tc, cnn_tail, end;
 };
 static FwdLayout forward_layout(const CallPlan& C, const PmtBatch* batch) {
   const int B = batch ? batch->n_variants : 0;
@@ -840,7 +847,8 @@ static FwdLayout forward_layout(const CallPlan& C, const PmtBatch* batch) {
   const size_t claims = C.saved.total > 0 ? pmt_plan_claim_bytes(B, PMT_PARTIAL_CTAS) : 0;   // the training forward's planner
   if (claims > tiles) tiles = claims;
   L.tiles = off; off += tiles; off = (off + 255) & ~(size_t)255;
-  L.long_tc = off; off += C.lng == LongKernel::TC ? C.long_tc.end : 0;
+  L.long_tc = off; off += C.lng == LongKernel::TC ? C.long_tc.end : 0; off = (off + 255) & ~(size_t)255;
+  L.cnn_tail = off; off += pmt_cnn_tail_buffer_bytes(C, B);
   L.end = off + 1024;
   return L;
 }
@@ -934,6 +942,13 @@ static int forward_impl(const PmtModelDesc* desc, const float* weights, const Pm
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const FwdLayout L = forward_layout(C, batch);
   PMT_CHECK(workspace && workspace_bytes >= L.end, "workspace too small: %zu < %zu", workspace_bytes, L.end);
+  if (C.cnn == CnnKernel::TC || C.cnn == CnnKernel::TC_TAIL) {
+    // measurement and tests (profiles/time_cnn_forward.py, tests/test_cnn_tail_gpu.py): PMT_CNN_SINGLE=1 runs
+    // hap_cnn_tc_kernel over every layer, PMT_CNN_SINGLE=0 the head + tail pair at any batch size
+    const char* e = getenv("PMT_CNN_SINGLE");
+    if (e && atoi(e) == 1) C.cnn = CnnKernel::TC;
+    else if (e && atoi(e) == 0 && C.cnn_split) C.cnn = CnnKernel::TC_TAIL;
+  }
   PMT_CHECK(batch->n_variants > 0, "empty batch");
   char* ws = reinterpret_cast<char*>(workspace);
   int* counter = reinterpret_cast<int*>(ws);
@@ -958,7 +973,8 @@ static int forward_impl(const PmtModelDesc* desc, const float* weights, const Pm
   if (pmt_launch_info_mlp(C, weights, image, batch, info_seq, st)) return 1;
   switch (C.cnn) {
     case CnnKernel::TC:
-      if (pmt_launch_cnn_tc(C, weights, batch, info_seq, cnn_tc_image, reuse_images, st)) return 1;
+    case CnnKernel::TC_TAIL:
+      if (pmt_launch_cnn_tc(C, weights, batch, info_seq, cnn_tc_image, reuse_images, reinterpret_cast<float*>(ws + L.cnn_tail), st)) return 1;
       break;
     case CnnKernel::TC_SAVE:
       if (pmt_cnn_forward_train(C, weights, batch, info_seq, cnn_tc_image, reinterpret_cast<float*>(saved + C.saved.cnn), st)) return 1;
