@@ -167,7 +167,7 @@ class ArtifactModel(nn.Module):
         if torch.is_grad_enabled() and any(p.requires_grad for p in params):
             opt = getattr(self, "_flat_optimizer", None)
             if opt is not None and opt.backs(params):
-                return planner.materialize_flat(self, opt)          # one clone + 13 constrained slots (training/step.py)
+                return planner.materialize_flat(opt)          # constraint kernels on the optimiser's flat buffer
             return torch.cat([t.reshape(-1) for t in planner.materialized_tensors(self)])
         try:
             versions = tuple(p._version for p in params) + tuple(p.data_ptr() for p in params[:4])

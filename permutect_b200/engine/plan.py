@@ -134,201 +134,97 @@ def _constrained_value(module, attr):
     return t
 
 
-def constrained_parameter_indices(model) -> List[int]:
-    """Positions in named_parameters() order of the raw parameters of parametrised tensors."""
-    return [i for i, (_, module, _) in enumerate(_materialization_recipe(model)) if module is not None]
-
-
-class _FlatMaterialize(torch.autograd.Function):
-    """flat materialised weights = the optimiser's flat raw-parameter buffer with the slots of the parametrised tensors
-    replaced by their constrained values.  Backward: the whole gradient goes to the optimiser's flat gradient buffer in
-    one copy (the unparametrised parameters are NOT autograd inputs), the parametrised slots are returned to autograd,
-    which chains the constraint Jacobians as before."""
-
-    @staticmethod
-    def forward(ctx, opt, anchor, *constrained):
-        w = opt.flat.detach().clone()
-        if constrained:
-            w.index_copy_(0, opt._constrained_index, torch.cat([t.detach().reshape(-1) for t in constrained]))
-        ctx.opt = opt
-        ctx.shapes = [t.shape for t in constrained]
-        return w
-
-    @staticmethod
-    def backward(ctx, d_flat):
-        opt = ctx.opt
-        d_flat = d_flat.contiguous()
-        opt.receive_flat_gradient(d_flat)
-        grads = []
-        for i, shape in zip(opt._constrained, ctx.shapes):
-            grads.append(d_flat[opt._offsets[i]:opt._offsets[i + 1]].view(shape))
-        return (None, None, *grads)
-
-
 class _ConstraintPack:
-    """The parametrised tensors of a model grouped by constraint, as positions in the optimiser's flat buffer, so that
-    their values and Jacobians are a dozen batched tensor ops instead of 12 module-property evaluations and their autograd
-    chains (≈1.5 ms of host time per training step).  ``rotation``: the one tensor that stays on autograd (matrix
-    exponential).  ``ok`` is False when a parametrisation other than the reference's five is present."""
+    """The parametrised tensors of a model as positions in the flat buffer, built once when a FlatAdamW attaches: the
+    byte mask of the entries that belong to a constraint group and the group table of pmt_constraints_forward /
+    _backward, both resident on the device, and ``rotation`` = (raw parameter, owner module, attribute, offset, size) of
+    the orthogonal matrix, or None.  A parametrisation other than the reference's five is refused here."""
 
-    def __init__(self, model, opt):
-        recipe = _materialization_recipe(model)
-        dev = opt.flat.device
-        exp_idx, bnd_idx, bnd_size, bnd_min = [], [], [], []
-        self.units, self.logws, self.rotation, self.ok = [], [], None, True
-        for i in constrained_parameter_indices(model):
-            p, module, attr = recipe[i]
-            off, n = opt._offsets[i], opt._sizes[i]
+    def __init__(self, model, device):
+        import numpy as np
+        offsets, n_flat = flat_layout(model)
+        groups, self.rotation = [], None
+        for name, p in model.named_parameters():
+            if _PARAM_TAG not in name:
+                continue
+            module, attr = _owner_and_attr(model, name)
+            off, n = offsets[name], p.numel()
             plist = getattr(module.parametrizations, attr)
             kind = type(plist[0]).__name__ if len(plist) == 1 else "?"
             if kind == "PositiveNumber":
-                exp_idx.append(torch.arange(off, off + n))
+                groups.append((L.CONSTRAINT_EXP, off, 1, n, 0.0, 0.0))
             elif kind == "BoundedNumber":
-                bnd_idx.append(torch.arange(off, off + n))
-                bnd_size.append(torch.full((n,), float(plist[0].size)))
-                bnd_min.append(torch.full((n,), float(plist[0].min_val)))
+                groups.append((L.CONSTRAINT_BOUNDED, off, 1, n, float(plist[0].size), float(plist[0].min_val)))
             elif kind == "UnitVector" and p.dim() == 2:
-                self.units.append((off, p.shape[0], p.shape[1], attr == "artifact_directions_ke"))
+                twice = attr == "artifact_directions_ke"
+                groups.append((L.CONSTRAINT_UNIT_TWICE if twice else L.CONSTRAINT_UNIT, off, p.shape[0], p.shape[1], 0.0, 0.0))
             elif kind == "LogWeights" and p.dim() == 1:
-                self.logws.append((off, n))
-            elif kind == "_Orthogonal" and self.rotation is None:
-                self.rotation = (i, module, attr, off, n)
-            else:
-                self.ok = False
-        cat = lambda xs, dt=torch.long: torch.cat(xs).to(dev) if xs else torch.zeros(0, dtype=dt, device=dev)
-        self.exp_idx, self.bnd_idx = cat(exp_idx), cat(bnd_idx)
-        self.bnd_size, self.bnd_min = cat(bnd_size, torch.float32), cat(bnd_min, torch.float32)
-        # the same grouping for pmt_constraints_forward / _backward (one launch each on a CUDA device): a byte mask of the
-        # entries that belong to a group and the group table, both resident on the device
-        self.device_groups = None
-        if self.ok and dev.type == "cuda":
-            import numpy as np
-            groups = []
-            for idx in exp_idx:
-                groups.append((L.CONSTRAINT_EXP, int(idx[0]), 1, idx.numel(), 0.0, 0.0))
-            for idx, size, lo in zip(bnd_idx, bnd_size, bnd_min):
-                groups.append((L.CONSTRAINT_BOUNDED, int(idx[0]), 1, idx.numel(), float(size[0]), float(lo[0])))
-            for off, k, d, twice in self.units:
-                groups.append((L.CONSTRAINT_UNIT_TWICE if twice else L.CONSTRAINT_UNIT, off, k, d, 0.0, 0.0))
-            for off, n in self.logws:
                 groups.append((L.CONSTRAINT_LOGSOFTMAX, off, 1, n, 0.0, 0.0))
-            mask = np.zeros(opt.flat.numel(), np.uint8)
-            table = np.zeros(max(len(groups), 1), dtype=[("type", "<i4"), ("off", "<i4"), ("rows", "<i4"), ("cols", "<i4"),
-                                                         ("a", "<f4"), ("b", "<f4")])
-            for j, (t, off, rows, cols, a, b) in enumerate(groups):
-                table[j] = (t, off, rows, cols, a, b)
-                mask[off:off + rows * cols] = 1
-            self.device_groups = (torch.from_numpy(mask).to(dev), torch.from_numpy(table.view(np.uint8).copy()).to(dev), len(groups))
+            elif (kind == "_Orthogonal" and self.rotation is None and plist[0].orthogonal_map.name == "matrix_exp"
+                  and p.dim() == 2 and p.shape[0] == p.shape[1]):        # what _orthogonal_without_sync evaluates
+                self.rotation = (p, module, attr, off, n)
+            else:
+                raise NotImplementedError(f"{name}: no constraint kernel for this parametrisation")
+        mask = np.zeros(n_flat, np.uint8)
+        table = np.zeros(max(len(groups), 1), dtype=[("type", "<i4"), ("off", "<i4"), ("rows", "<i4"), ("cols", "<i4"),
+                                                     ("a", "<f4"), ("b", "<f4")])
+        for j, (t, off, rows, cols, a, b) in enumerate(groups):
+            table[j] = (t, off, rows, cols, a, b)
+            mask[off:off + rows * cols] = 1
+        self.mask = torch.from_numpy(mask).to(device)
+        self.table, self.n_groups = torch.from_numpy(table.view(np.uint8).copy()).to(device), len(groups)
+        self.anchor = torch.zeros((), device=device, requires_grad=True)      # keeps the node in the graph
 
 
 class _FastMaterialize(torch.autograd.Function):
-    """_FlatMaterialize with the constraint Jacobians of parameterizations.py written out (PositiveNumber: exp;
-    BoundedNumber: size * sigmoid + min; UnitVector: x / |x|, applied twice for the cluster directions, quirk Q5;
-    LogWeights: log_softmax); only the rotation matrix is an autograd input."""
+    """flat materialised weights = the optimiser's flat raw-parameter buffer with the slots of the parametrised tensors
+    replaced by their constrained values: parameterizations.py's maps in one kernel (PositiveNumber: exp; BoundedNumber:
+    size * sigmoid + min; UnitVector: x / |x|, applied twice for the cluster directions, quirk Q5; LogWeights:
+    log_softmax) and the rotation matrix as _orthogonal_without_sync evaluates it.  The raw parameters are not autograd
+    inputs: backward hands the whole vector-Jacobian product, the rotation's included, to the optimiser's flat gradient."""
 
     @staticmethod
-    def forward(ctx, opt, pack, anchor, rot_q):
+    def forward(ctx, opt, pack, anchor):
         raw = opt.flat.detach()
-        if pack.device_groups is not None:       # CUDA: the whole map is one kernel (pmt_constraints_forward)
-            mask, table, n_groups = pack.device_groups
-            w = torch.empty_like(raw)
-            L.check(L.load().pmt_constraints_forward(raw.data_ptr(), mask.data_ptr(), raw.numel(), table.data_ptr(), n_groups,
-                                                     w.data_ptr(), torch.cuda.current_stream(raw.device).cuda_stream))
-            if pack.rotation is not None:
-                _, _, _, off, n = pack.rotation
-                w[off:off + n] = rot_q.detach().reshape(-1)
-            ctx.opt, ctx.pack = opt, pack
-            ctx.save_for_backward(raw, w)
-            ctx.rot_shape = None if rot_q is None else rot_q.shape
-            return w
-        w = raw.clone()
-        e = torch.exp(raw[pack.exp_idx])
-        w[pack.exp_idx] = e
-        sg = torch.sigmoid(raw[pack.bnd_idx])
-        w[pack.bnd_idx] = pack.bnd_size * sg + pack.bnd_min
-        units = []
-        for off, k, d, twice in pack.units:
-            x = raw[off:off + k * d].view(k, d)
-            n1 = torch.norm(x, dim=-1, keepdim=True)
-            u = x / n1
-            if twice:
-                n2 = torch.norm(u, dim=-1, keepdim=True)
-                u2 = u / n2
-            else:
-                n2, u2 = None, u
-            w[off:off + k * d] = u2.reshape(-1)
-            units.append((n1, u, n2, u2))
-        lws = []
-        for off, n in pack.logws:
-            lw = torch.log_softmax(raw[off:off + n], dim=-1)
-            w[off:off + n] = lw
-            lws.append(lw)
+        w = torch.empty_like(raw)
+        L.check(L.load().pmt_constraints_forward(raw.data_ptr(), pack.mask.data_ptr(), raw.numel(), pack.table.data_ptr(),
+                                                 pack.n_groups, w.data_ptr(), torch.cuda.current_stream(raw.device).cuda_stream))
         if pack.rotation is not None:
-            _, _, _, off, n = pack.rotation
-            w[off:off + n] = rot_q.detach().reshape(-1)
-        ctx.opt, ctx.pack, ctx.saved_small = opt, pack, (e, sg, units, lws)
-        ctx.rot_shape = None if rot_q is None else rot_q.shape
+            _, module, attr, off, n = pack.rotation
+            w[off:off + n] = _orthogonal_without_sync(module, attr).reshape(-1)
+        ctx.opt, ctx.pack = opt, pack
+        ctx.save_for_backward(raw, w)
         return w
 
     @staticmethod
     def backward(ctx, d_flat):
         opt, pack = ctx.opt, ctx.pack
-        if pack.device_groups is not None:
-            mask, table, n_groups = pack.device_groups
-            raw, w = ctx.saved_tensors
-            d_flat = d_flat.contiguous()
-            g = torch.empty_like(d_flat)
-            L.check(L.load().pmt_constraints_backward(raw.data_ptr(), w.data_ptr(), d_flat.data_ptr(), mask.data_ptr(), d_flat.numel(),
-                                                      table.data_ptr(), n_groups, g.data_ptr(),
-                                                      torch.cuda.current_stream(d_flat.device).cuda_stream))
-            d_rot = None
-            if pack.rotation is not None:
-                _, _, _, off, n = pack.rotation
-                d_rot = d_flat[off:off + n].view(ctx.rot_shape)
-            opt.receive_flat_gradient(g)
-            return None, None, None, d_rot
-        e, sg, units, lws = ctx.saved_small
-        g = d_flat.clone()
-        g[pack.exp_idx] = d_flat[pack.exp_idx] * e
-        g[pack.bnd_idx] = d_flat[pack.bnd_idx] * pack.bnd_size * sg * (1 - sg)
-        for (off, k, d, twice), (n1, u, n2, u2) in zip(pack.units, units):
-            gu = d_flat[off:off + k * d].view(k, d)
-            if twice:
-                gu = (gu - u2 * (u2 * gu).sum(-1, keepdim=True)) / n2
-            gx = (gu - u * (u * gu).sum(-1, keepdim=True)) / n1
-            g[off:off + k * d] = gx.reshape(-1)
-        for (off, n), lw in zip(pack.logws, lws):
-            gl = d_flat[off:off + n]
-            g[off:off + n] = gl - torch.exp(lw) * gl.sum()
-        d_rot = None
-        if pack.rotation is not None:
-            _, _, _, off, n = pack.rotation
-            d_rot = d_flat[off:off + n].view(ctx.rot_shape)
+        raw, w = ctx.saved_tensors
+        lib, stream = L.load(), torch.cuda.current_stream(d_flat.device).cuda_stream
+        d_flat = d_flat.contiguous()
+        g = torch.empty_like(d_flat)
+        L.check(lib.pmt_constraints_backward(raw.data_ptr(), w.data_ptr(), d_flat.data_ptr(), pack.mask.data_ptr(), d_flat.numel(),
+                                             pack.table.data_ptr(), pack.n_groups, g.data_ptr(), stream))
+        if pack.rotation is not None and pack.rotation[0].requires_grad:
+            X, module, attr, off, n = pack.rotation
+            dQ = d_flat[off:off + n]
+            if X.shape[0] <= _ROTATION_KERNEL_MAX_N:          # _RotationFunction.backward, written into the slot
+                base = getattr(getattr(module.parametrizations, attr)[0], "base", None)
+                base = None if base is None else base.detach().contiguous()
+                L.check(lib.pmt_orthogonal_backward(raw[off:off + n].data_ptr(), None if base is None else base.data_ptr(),
+                                                    dQ.data_ptr(), X.shape[0], g[off:off + n].data_ptr(), stream))
+            else:
+                with torch.enable_grad():
+                    dX, = torch.autograd.grad(_orthogonal_without_sync(module, attr), X, dQ.view(X.shape))
+                g[off:off + n] = dX.reshape(-1)
         opt.receive_flat_gradient(g)
-        return None, None, None, d_rot
+        return None, None, None
 
 
-def materialize_flat(model, opt) -> torch.Tensor:
-    """The training-time fast path of ``ArtifactModel.flat_weights`` when a FlatAdamW backs the parameters."""
-    pack = getattr(opt, "_constraint_pack", None)
-    if pack is None:
-        pack = opt._constraint_pack = _ConstraintPack(model, opt)
-    anchor = getattr(opt, "_anchor", None)
-    if anchor is None:
-        anchor = opt._anchor = torch.zeros((), device=opt.flat.device, requires_grad=True)   # keeps the node in the graph
-    recipe = _materialization_recipe(model)
-    if pack.ok:
-        rot_q = None
-        if pack.rotation is not None:
-            rot_q = _constrained_value(pack.rotation[1], pack.rotation[2])
-        if getattr(pack, "installed", None) is not opt:      # from now on only the rotation's gradient arrives through autograd
-            opt._constrained = [] if pack.rotation is None else [pack.rotation[0]]
-            opt._constrained_index = None if pack.rotation is None else torch.arange(
-                pack.rotation[3], pack.rotation[3] + pack.rotation[4], device=opt.flat.device)
-            pack.installed = opt
-        return _FastMaterialize.apply(opt, pack, anchor, rot_q)
-    constrained = [_constrained_value(recipe[i][1], recipe[i][2]) for i in opt._constrained]
-    return _FlatMaterialize.apply(opt, anchor, *constrained)
+def materialize_flat(opt) -> torch.Tensor:
+    """The training-time path of ``ArtifactModel.flat_weights`` when a FlatAdamW backs the parameters."""
+    pack = opt._constraint_pack
+    return _FastMaterialize.apply(opt, pack, pack.anchor)
 
 
 def _mlp_ops(offsets: Dict[str, int], prefix: str, layer_sizes: List[int]):

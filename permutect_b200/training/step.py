@@ -14,6 +14,7 @@ import torch
 from torch import nn
 
 from permutect_b200.engine import library as L
+from permutect_b200.engine import plan as planner
 from permutect_b200.training import distributed as pdist
 
 
@@ -44,24 +45,16 @@ class FlatAdamW(torch.optim.Optimizer):
         self.flat_grad = torch.zeros_like(self.flat)
         self._grad_views = [v.view_as(p) for p, v in zip(self._params, self.flat_grad.split(self._sizes))]
         self._flat_grad_valid = False
-        self._constrained = []          # indices (into self._params) of the parametrised tensors' raw parameters
-        self._constrained_index = None  # flat positions of those slots
         self._mask_cache = (None, None)
 
     # ---- flat gradient path -------------------------------------------------------------------------------
-    def attach(self, model, constrained_indices):
+    def attach(self, model):
         """Called by make_optimizer: from now on ``model.flat_weights()`` builds the materialised weight buffer from
-        ``self.flat`` directly (engine/plan.py:materialize_flat) and its backward writes the whole gradient into
-        ``self.flat_grad`` instead of ~190 per-parameter accumulations; only the parametrised tensors (13 for the shipped
-        architecture) keep a constraint Jacobian, and engine/plan.py writes those out (only the rotation matrix stays an
-        autograd input, itself a kernel pair).  The host side of a training step drops from 5.7 to 1.8 ms."""
-        self._constrained = list(constrained_indices)
-        offsets = [0]
-        for n in self._sizes:
-            offsets.append(offsets[-1] + n)
-        self._offsets = offsets
-        idx = [torch.arange(offsets[i], offsets[i + 1]) for i in self._constrained]
-        self._constrained_index = torch.cat(idx).to(self.flat.device) if idx else None
+        ``self.flat`` directly (engine/plan.py:materialize_flat: the constraint maps of every parametrised tensor, the
+        rotation matrix included, in one autograd node) and its backward writes the whole gradient into
+        ``self.flat_grad`` instead of ~190 per-parameter accumulations.  The host side of a training step drops from 5.7
+        to 1.8 ms."""
+        self._constraint_pack = planner._ConstraintPack(model, self.flat.device)
         model._flat_optimizer = self
 
     def backs(self, params) -> bool:
@@ -71,16 +64,15 @@ class FlatAdamW(torch.optim.Optimizer):
 
     def receive_flat_gradient(self, d_flat: torch.Tensor):
         """Backward hook of materialize_flat: accumulate (torch semantics: gradients add up until zero_grad) and expose
-        the slices as ``.grad`` of the trainable, unparametrised parameters."""
+        the slices as ``.grad`` of the trainable parameters."""
         if self._flat_grad_valid:
             self.flat_grad.add_(d_flat)
         else:
             self.flat_grad.copy_(d_flat)
             self._flat_grad_valid = True
-        constrained = set(self._constrained)
-        for i, p in enumerate(self._params):
-            if i not in constrained and p.requires_grad and p.grad is None:
-                p.grad = self._grad_views[i]
+        for p, view in zip(self._params, self._grad_views):
+            if p.requires_grad and p.grad is None:
+                p.grad = view
 
     def zero_grad(self, set_to_none: bool = True):
         if set_to_none:
@@ -89,17 +81,9 @@ class FlatAdamW(torch.optim.Optimizer):
                 p.grad = None
         else:
             self.flat_grad.zero_()
-            for i in self._constrained:
-                if self._params[i].grad is not None:
-                    self._params[i].grad.zero_()
 
     def _flat_path_gradient(self):
-        """(flat gradient, mask or None) when the gradient arrived through receive_flat_gradient: the slots of the
-        parametrised tensors are replaced by the gradients autograd left on their raw parameters."""
-        if self._constrained:
-            pieces = [self._params[i].grad.reshape(-1) if self._params[i].grad is not None
-                      else torch.zeros(self._sizes[i], device=self.flat.device) for i in self._constrained]
-            self.flat_grad.index_copy_(0, self._constrained_index, torch.cat(pieces))
+        """(flat gradient, mask or None) when the gradient arrived through receive_flat_gradient."""
         flags = tuple(p.requires_grad and (p.grad is not None) for p in self._params)
         if all(flags):
             return self.flat_grad, None
@@ -164,8 +148,7 @@ def make_optimizer(model: nn.Module, learning_rate: float = 1e-3, weight_decay: 
     if len(params) > 0 and params[0].is_cuda:
         opt = FlatAdamW(params, lr=learning_rate, weight_decay=weight_decay)
         if hasattr(model, "flat_weights"):
-            from permutect_b200.engine import plan as planner
-            opt.attach(model, planner.constrained_parameter_indices(model))
+            opt.attach(model)
         return opt
     raise RuntimeError("make_optimizer needs the model's parameters on a CUDA device (FlatAdamW; there is no CPU optimiser path)")
 

@@ -213,46 +213,3 @@ def test_sync_free_rotation_equals_torch_orthogonal():
         g_got, = torch.autograd.grad((got * w).sum(), rot.parametrizations.weight.original)
         torch.testing.assert_close(g_got, g_want, rtol=1e-4, atol=1e-5)
 
-
-def test_fast_materialisation_matches_the_autograd_formulation():
-    """engine/plan.py:_FastMaterialize (constraint maps and their Jacobians written out, gradient delivered as ONE flat
-    tensor) against torch.cat of the parametrised tensors and autograd, on the CPU with a stand-in for the optimiser's
-    flat buffers."""
-    import torch
-    import bench
-    from permutect_b200.engine import plan as planner
-
-    torch.manual_seed(0)
-    model = bench.make_model(torch.device("cpu"))
-    with torch.no_grad():
-        for p in model.parameters():
-            p.add_(0.1 * torch.randn_like(p))
-    params = list(model.parameters())
-
-    class Stub:
-        pass
-
-    opt = Stub()
-    opt._params, opt._sizes = params, [p.numel() for p in params]
-    opt.flat = torch.cat([p.detach().reshape(-1) for p in params])
-    opt._offsets = [0]
-    for n in opt._sizes:
-        opt._offsets.append(opt._offsets[-1] + n)
-    opt._constrained = planner.constrained_parameter_indices(model)
-    received = {}
-    opt.receive_flat_gradient = lambda g: received.__setitem__("g", g)
-
-    w_fast = planner.materialize_flat(model, opt)
-    w_ref = torch.cat([t.reshape(-1) for t in planner.materialized_tensors(model)])
-    assert opt._constraint_pack.ok and len(opt._constrained) == 1          # only the rotation stays on autograd
-    torch.testing.assert_close(w_fast, w_ref, rtol=0, atol=0)
-    dw = torch.randn_like(w_ref)
-    w_ref.backward(dw)
-    want = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).reshape(-1) for p in params])
-    for p in params:
-        p.grad = None
-    w_fast.backward(dw)
-    got = received["g"].clone()
-    i, _, _, off, n = opt._constraint_pack.rotation
-    got[off:off + n] = params[i].grad.reshape(-1)
-    torch.testing.assert_close(got, want, rtol=1e-5, atol=1e-6)

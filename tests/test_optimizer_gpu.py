@@ -136,35 +136,19 @@ def test_rotation_kernels_match_the_torch_formulation():
             torch.testing.assert_close(X.grad.double(), Xl.grad.tril(), rtol=1e-4, atol=1e-5)
 
 
-def test_constraint_kernels_match_the_autograd_formulation():
-    """pmt_constraints_forward / _backward (engine/plan.py:_FastMaterialize on a CUDA device: one launch each) against
-    torch.cat of the parametrised tensors (utils/parameterizations.py) and autograd through them."""
-    import bench
+def _check_flat_materialisation(model):
+    """engine/plan.py:_FastMaterialize (pmt_constraints_forward / _backward and the rotation) against torch.cat of the
+    parametrised tensors (utils/parameterizations.py) and autograd through them; the rotation's slot of the gradient bit
+    for bit, since it is the same calls on the same dQ as autograd through _orthogonal_without_sync."""
     from permutect_b200.engine import plan as planner
 
-    dev = torch.device("cuda:0")
-    torch.manual_seed(0)
-    model = bench.make_model(dev)
-    with torch.no_grad():
-        for p in model.parameters():
-            p.add_(0.1 * torch.randn_like(p))
     params = list(model.parameters())
-
-    class Stub:
-        pass
-
-    opt = Stub()
-    opt._params, opt._sizes = params, [p.numel() for p in params]
-    opt.flat = torch.cat([p.detach().reshape(-1) for p in params])
-    opt._offsets = [0]
-    for n in opt._sizes:
-        opt._offsets.append(opt._offsets[-1] + n)
-    opt._constrained = planner.constrained_parameter_indices(model)
+    opt = FlatAdamW(params)
+    opt.attach(model)
     received = {}
     opt.receive_flat_gradient = lambda g: received.__setitem__("g", g)
 
-    w_fast = planner.materialize_flat(model, opt)
-    assert opt._constraint_pack.ok and opt._constraint_pack.device_groups is not None
+    w_fast = planner.materialize_flat(opt)
     w_ref = torch.cat([t.reshape(-1) for t in planner.materialized_tensors(model)])
     torch.testing.assert_close(w_fast, w_ref, rtol=2e-6, atol=1e-7)
     dw = torch.randn_like(w_ref)
@@ -173,7 +157,25 @@ def test_constraint_kernels_match_the_autograd_formulation():
     for p in params:
         p.grad = None
     w_fast.backward(dw)
-    got = received["g"].clone()
-    i, _, _, off, n = opt._constraint_pack.rotation
-    got[off:off + n] = params[i].grad.reshape(-1)
+    got = received["g"]
     torch.testing.assert_close(got, want, rtol=1e-5, atol=1e-6)
+    _, _, _, off, n = opt._constraint_pack.rotation
+    assert torch.equal(got[off:off + n], want[off:off + n])
+
+
+def test_flat_materialisation_matches_the_autograd_formulation():
+    """The v0.4.0 model: the rotation (10 x 10) through pmt_orthogonal_forward / _backward."""
+    import bench
+    torch.manual_seed(0)
+    model = bench.make_model(torch.device("cuda:0"))
+    with torch.no_grad():
+        for p in model.parameters():
+            p.add_(0.1 * torch.randn_like(p))
+    _check_flat_materialisation(model)
+
+
+def test_flat_materialisation_with_the_float64_rotation_matches_the_autograd_formulation():
+    """d_feat 17 (model_shapes.py's e_17): the rotation is past the kernel pair's n <= 16 and takes the float64
+    scaling-and-squaring inside the node."""
+    from model_shapes import BY_NAME, build_model
+    _check_flat_materialisation(build_model(BY_NAME["e_17"], torch.device("cuda:0")))
