@@ -195,9 +195,12 @@ int pmt_head_backward(const PmtModelDesc* desc, const float* weights, const PmtB
 /* Arithmetic mode of the dense layers of the read path (process-wide; default PMT_PRECISION_FP32).
  *   FP32    FP32 FMA pipe (SIMT); forward and backward.
  *   TF32X3  tcgen05 tensor cores, TF32 with a hi/lo split of both operands (3 MMAs, ~2^-21 relative error):
- *           the fp32-parity mode on tensor cores.  Forward (inference) only; backward stays FP32.
+ *           the fp32-parity mode on tensor cores.
  *   TF32    tcgen05 tensor cores, plain TF32 (10-bit mantissa); logits are NOT within 1e-3 of the reference,
- *           tolerance stated separately (DESIGN.md).  Forward only. */
+ *           tolerance stated separately (DESIGN.md).
+ * In both tensor-core modes the backward runs on the tensor cores too, for models inside their envelope
+ * (pmt_backward_kernels): it recomputes the forward in split precision and multiplies the gradients in TF32 with fp32
+ * accumulation, in either mode.  Models outside it take the FP32 backward. */
 #define PMT_PRECISION_FP32 0
 #define PMT_PRECISION_TF32X3 1
 #define PMT_PRECISION_TF32 2

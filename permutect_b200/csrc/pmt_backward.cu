@@ -9,6 +9,7 @@
 //   hap_cnn_backward_kernel   DNASequenceConvolution
 //   reduce_partials_kernel    sum of the CTA-private buffers in CTA order (bitwise reproducible)
 //   skip_fix_kernel           DenseSkipBlock.alpha gradients and the alpha scaling of its last layer
+#include <cstdio>
 #include <cstring>
 
 // The per-row phases are written for NPART = NTHREADS / TILE threads per tile row.  Measured on B200 (65 536 variants,
@@ -822,16 +823,9 @@ __global__ void skip_fix_kernel(const __grid_constant__ Plan P, const float* __r
 // haplotype CNN backward (dna_sequence_convolution.py:57-111).  VT variants per pass; every layer's
 // activation of the pass stays in shared memory, channel-major with a per-variant stride lp[i] (multiple of 4)
 // and a channel stride ld[i] == 4 (mod 32) so that 16-byte loads by lanes on consecutive channels are
-// conflict-free.  conv data gradient = the forward conv routine on the zero-padded output gradient with the
-// flipped/transposed image; conv weight gradient = register-tiled reduction over (variant, position).
+// conflict-free (CnnBwdGeom, pmt_call.h).  conv data gradient = the forward conv routine on the zero-padded output
+// gradient with the flipped/transposed image; conv weight gradient = register-tiled reduction over (variant, position).
 // ------------------------------------------------------------------------------------------------
-struct CnnBwdGeom {
-  int vt, n_spatial, n_linear, vs;
-  int ch[PMT_MAX_CNN_OPS + 1], len[PMT_MAX_CNN_OPS + 1], lp[PMT_MAX_CNN_OPS + 1], ld[PMT_MAX_CNN_OPS + 1];
-  int act_off[PMT_MAX_CNN_OPS + 1];   // activation entering spatial op i ([n_spatial] = last output)
-  int lpg[PMT_MAX_CNN_OPS], ldg[PMT_MAX_CNN_OPS];   // zero-padded layout of conv op i's output gradient
-  int act_total, gbuf_floats, stage_floats;
-};
 
 // Walks idx = tid, tid + NTHREADS, ... of a [C][V][L] index space keeping (c, v, p) without per-element integer
 // divisions (they were a quarter of this kernel's instructions).
@@ -1147,17 +1141,20 @@ static int pad_ld(int n) {   // smallest ld >= n + 12 with ld == 4 (mod 32)
   return ld;
 }
 
-static int launch_cnn_backward(const Plan& P, const CnnGeom& G, const float* weights, const float* image, const PmtBatch* batch,
-                               const float* d_info_seq, float* partials, cudaStream_t st) {
-  CnnBwdGeom Gb;
+// The largest pass of variants (at most 16) whose activations, gradients and weight stage fit in shared memory.
+static bool cnn_bwd_simt_geom(const Plan& P, const CnnGeom& G, CnnBwdGeom* out, size_t* smem_out, const char** why) {
+  CnnBwdGeom& Gb = *out;
   const PmtModelDesc& d = P.d;
   const int ns = G.n_spatial;
+  if (d.n_cnn_ops - ns < 1 || d.n_cnn_ops - ns > 4) {
+    *why = "haplotype CNN backward supports 1..4 linear layers after flatten";
+    return false;
+  }
   size_t smem = 0;
   int vt = 16;
   for (; vt >= 1; --vt) {
     memset(&Gb, 0, sizeof(Gb));
     Gb.vt = vt; Gb.n_spatial = ns; Gb.n_linear = d.n_cnn_ops - ns;
-    PMT_CHECK(Gb.n_linear >= 1 && Gb.n_linear <= 4, "haplotype CNN backward supports 1..4 linear layers after flatten");
     Gb.ch[0] = 10; Gb.len[0] = d.hap_len;
     for (int i = 0; i < ns; ++i) {
       const PmtCnnOp& op = d.cnn_ops[i];
@@ -1192,13 +1189,23 @@ static int launch_cnn_backward(const Plan& P, const CnnGeom& G, const float* wei
     smem = (size_t)(Gb.act_total + 2 * Gb.gbuf_floats + Gb.stage_floats + (Gb.n_linear + 3) * vt * Gb.vs + 16) * sizeof(float);
     if (smem <= 220 * 1024) break;
   }
-  PMT_CHECK(vt >= 1, "haplotype CNN backward does not fit in shared memory");
+  if (vt < 1) {
+    *why = "haplotype CNN backward does not fit in shared memory";
+    return false;
+  }
+  *smem_out = smem;
+  return true;
+}
+
+static int launch_cnn_backward(const CallPlan& C, const float* weights, const float* image, const PmtBatch* batch,
+                               const float* d_info_seq, float* partials, cudaStream_t st) {
+  const CnnBwdGeom& Gb = C.cnn_bwd;
   const int B = batch->n_variants;
-  int grid = (B + vt - 1) / vt;
+  int grid = (B + Gb.vt - 1) / Gb.vt;
   if (grid > PMT_PARTIAL_CTAS) grid = PMT_PARTIAL_CTAS;
-  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  hap_cnn_backward_kernel<<<grid, NTHREADS, smem, st>>>(P, G, Gb, weights, image + P.img_total, batch->haplotypes,
-                                                        batch->hap_kind, batch->hap_stride, B, d_info_seq, partials);
+  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C.cnn_bwd_smem));
+  hap_cnn_backward_kernel<<<grid, NTHREADS, C.cnn_bwd_smem, st>>>(C.P, C.G, Gb, weights, image + C.P.img_total, batch->haplotypes,
+                                                                  batch->hap_kind, batch->hap_stride, B, d_info_seq, partials);
   return 0;
 }
 
@@ -1212,6 +1219,41 @@ static int info_rows(const Plan& P) {
   int r = P.d.n_info_features;
   for (int i = 0; i < P.d.n_info_ops; ++i) if (P.d.info_ops[i].out_dim > r) r = P.d.info_ops[i].out_dim;
   return r;
+}
+// Claims go to CTAs round-robin (fixed summation order), so their number is a multiple of the grid; every claim ends with
+// a partly filled tile, so a claim should hold >= 16 tiles (n_rows is an upper bound for a downsampled batch: claims of
+// ~4 tiles left a fifth of the rows of every tile empty).
+static Claims backward_claims(const PmtBatch* batch, int n_sm) {
+  const int B = batch->n_variants;
+  int per_cta = (int)((double)pmt_row_hint(batch) / ((double)n_sm * 16.0 * TILE));
+  if (per_cta < 1) per_cta = 1;
+  if (per_cta > 8) per_cta = 8;
+  Claims K;
+  K.claim = (int)((B + (long long)n_sm * per_cta - 1) / ((long long)n_sm * per_cta));
+  if (K.claim < 1) K.claim = 1;
+  K.n_claims = (B + K.claim - 1) / K.claim;
+  K.grid = K.n_claims < PMT_PARTIAL_CTAS ? K.n_claims : PMT_PARTIAL_CTAS;
+  if (K.grid > n_sm) K.grid = n_sm;
+  return K;
+}
+
+void pmt_plan_backward(CallPlan& C, const PmtBatch* batch) {
+  const Plan& P = C.P;
+  C.bwd_smem = bwd_smem_bytes(P);
+  C.info_bwd_smem = (size_t)(4 * info_rows(P) * LD + 2 * P.info_stage_floats) * sizeof(float);
+  if (batch) C.bwd_claims = backward_claims(batch, C.n_sm);
+  const char* cnn_why = nullptr;
+  const bool cnn_ok = C.bwd_cnn_tc || cnn_bwd_simt_geom(P, C.G, &C.cnn_bwd, &C.cnn_bwd_smem, &cnn_why);
+  char* why = C.bwd_refusal;
+  const size_t n = sizeof(C.bwd_refusal);
+  if (NPART * P.d.d_feat > P.bwd_rows)
+    snprintf(why, n, "d_feat %d too wide for the backward kernel's head scratch", P.d.d_feat);
+  else if (C.bwd_smem > 227 * 1024)
+    snprintf(why, n, "model too wide for the backward kernel's shared-memory plan (%zu bytes)", C.bwd_smem);
+  else if (C.info_bwd_smem > 227 * 1024)
+    snprintf(why, n, "info MLP too wide for the backward kernel (%zu bytes of shared memory)", C.info_bwd_smem);
+  else if (!cnn_ok)
+    snprintf(why, n, "%s", cnn_why);
 }
 // Long-set kernel: every chunk of the longest set has its own recompute scratch + dL/dx + gate state (see the kernel).
 // The grid shrinks when the scratch of a full grid would pass kLongScratchBudget.
@@ -1277,9 +1319,7 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
   const BwdWsLayout L = backward_layout(C, batch);
   PMT_CHECK(workspace && workspace_bytes >= L.end, "workspace too small: %zu < %zu", workspace_bytes, L.end);
   PMT_CHECK(batch->n_variants > 0, "empty batch");
-  PMT_CHECK(NPART * desc->d_feat <= C.P.bwd_rows, "d_feat %d too wide for the backward kernel's head scratch", desc->d_feat);
-  const size_t smem = bwd_smem_bytes(C.P);
-  PMT_CHECK(smem <= 227 * 1024, "model too wide for the backward kernel's shared-memory plan (%zu bytes)", smem);
+  PMT_CHECK(!C.bwd_refusal[0], "%s", C.bwd_refusal);
 
   const int B = batch->n_variants, w = desc->d_info + desc->d_seq;
   char* ws = reinterpret_cast<char*>(workspace);
@@ -1312,17 +1352,9 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
     return 1;
   }
 
-  const int n_sm = C.n_sm;
-  // Claims go to CTAs round-robin (fixed summation order), so their number is a multiple of the grid; every claim ends
-  // with a partly filled tile, so a claim should hold >= 16 tiles (n_rows is an upper bound for a downsampled batch:
-  // claims of ~4 tiles left a fifth of the rows of every tile empty).
-  int per_cta = (int)((double)pmt_row_hint(batch) / ((double)n_sm * 16.0 * TILE));
-  if (per_cta < 1) per_cta = 1;
-  if (per_cta > 8) per_cta = 8;
-  int claim = (int)((B + (long long)n_sm * per_cta - 1) / ((long long)n_sm * per_cta));
-  if (claim < 1) claim = 1;
   Plan P = C.P;
-  P.claim_variants = claim;
+  P.claim_variants = C.bwd_claims.claim;
+  const size_t smem = C.bwd_smem;
 
   BwdArgs A;
   A.wflat = weights; A.image = image; A.batch = *batch; A.info_seq = info_seq;
@@ -1331,9 +1363,7 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
   A.d_ref_means = grads ? grads->d_ref_means_be : nullptr;
   A.d_info_seq = d_info_seq; A.scratch = scratch; A.scratch_stride = (long long)L.scr_floats; A.partials = partials;
   A.long_scratch = long_scratch; A.long_scratch_stride = (long long)L.long_floats;
-  A.n_claims = (B + claim - 1) / claim;
-  int grid = A.n_claims < PMT_PARTIAL_CTAS ? A.n_claims : PMT_PARTIAL_CTAS;
-  if (grid > n_sm) grid = n_sm;
+  A.n_claims = C.bwd_claims.n_claims;
   int tc_grid = 0;
   if (C.bwd_reads_tc) {   // tile-sized sets; longer sets always take the SIMT long-set kernel
     if (pmt_launch_reads_tc_backward(C, weights, batch, info_seq, A.d_logits_bk, A.d_alt_means, A.d_ref_means, d_info_seq, tc_ws,
@@ -1342,7 +1372,7 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
   } else {
     PMT_CUDA(cudaFuncSetAttribute(reads_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     pmt_profile_begin(st);
-    reads_backward_kernel<<<grid, NTHREADS, smem, st>>>(P, A);
+    reads_backward_kernel<<<C.bwd_claims.grid, NTHREADS, smem, st>>>(P, A);
     pmt_profile_end(st);
   }
   if (L.long_grid > 0) {   // sets longer than a tile; same CTA-private gradient buffers, after the tile kernel: fixed order
@@ -1350,19 +1380,17 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
     reads_backward_long_kernel<<<L.long_grid, NTHREADS, smem, st>>>(P, A);
   }
   {
-    const int rows = info_rows(P);
-    const size_t ismem = (size_t)(4 * rows * LD + 2 * P.info_stage_floats) * sizeof(float);
-    PMT_CHECK(ismem <= 227 * 1024, "info MLP too wide for the backward kernel (%zu bytes of shared memory)", ismem);
+    const size_t ismem = C.info_bwd_smem;
     const int n_tiles = (B + TILE - 1) / TILE;
     const int igrid = n_tiles < PMT_PARTIAL_CTAS ? n_tiles : PMT_PARTIAL_CTAS;
     PMT_CUDA(cudaFuncSetAttribute(info_mlp_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ismem));
     info_mlp_backward_kernel<<<igrid, NTHREADS, ismem, st>>>(P, weights, image, batch->info, batch->info_kind,
                                                              batch->info_stride, B, d_info_seq, scratch,
-                                                             (long long)L.scr_floats, partials, rows);
+                                                             (long long)L.scr_floats, partials, info_rows(P));
   }
   if (C.bwd_cnn_tc) {
     if (pmt_launch_cnn_backward_mma(C, weights, batch, info_seq, d_info_seq, partials, cnn_ws, L.cnn_bytes, st, saved_cnn)) return 1;
-  } else if (launch_cnn_backward(P, C.G, weights, image, batch, d_info_seq, partials, st)) {
+  } else if (launch_cnn_backward(C, weights, image, batch, d_info_seq, partials, st)) {
     return 1;
   }
   reduce_partials_kernel<<<(desc->n_params + 255) / 256, 256, 0, st>>>(partials, PMT_PARTIAL_CTAS, desc->n_params, d_weights);

@@ -1,6 +1,10 @@
 // The call plan: which kernels one C-ABI call of the model (pmt_workspace_size, pmt_train_saved_bytes,
-// pmt_backward_kernels, pmt_forward, pmt_forward_prepared, pmt_forward_train, pmt_backward) runs and where their buffers
-// live.  pmt_call_plan decides all of it once per call from the model, the batch, the precision mode and the device; the
+// pmt_backward_kernels, pmt_forward, pmt_forward_prepared, pmt_forward_train, pmt_backward) runs, with what launch geometry,
+// and where their buffers live.  pmt_call_plan decides all of it once per call from the model, the batch, the precision
+// mode, the device and the test and measurement overrides (read_overrides in pmt_forward.cu, its only reader): the kernels,
+// the tile planner, the pass count, the claim sizes and grids of the SIMT kernels, every kernel's dynamic shared memory and
+// weight-ring stages.  It also decides whether the forward or the backward would be refused (fwd_refusal, bwd_refusal);
+// the entry points check that before their first CUDA call, so a refused call leaves the caller's buffers untouched.  The
 // launchers take their plans, grids and regions from it and decide nothing again.
 #pragma once
 #include "pmt_cnn_tc.cuh"
@@ -58,11 +62,37 @@ struct SavedLayout {
   long long bound;
 };
 
+// A tensor-core kernel's weight ring: n_stages stages of stage_bytes next to its fixed carve, `smem` dynamic bytes in all.
+// n_stages < 2: the ring does not fit.
+struct Ring {
+  int stage_bytes, n_stages;
+  size_t smem;
+};
+
+// The SIMT haplotype-CNN backward (hap_cnn_backward_kernel, pmt_backward.cu): vt variants per pass; every layer's
+// activation of the pass stays in shared memory, channel-major with a per-variant stride lp[i] (multiple of 4) and a
+// channel stride ld[i] == 4 (mod 32).
+struct CnnBwdGeom {
+  int vt, n_spatial, n_linear, vs;
+  int ch[PMT_MAX_CNN_OPS + 1], len[PMT_MAX_CNN_OPS + 1], lp[PMT_MAX_CNN_OPS + 1], ld[PMT_MAX_CNN_OPS + 1];
+  int act_off[PMT_MAX_CNN_OPS + 1];   // activation entering spatial op i ([n_spatial] = last output)
+  int lpg[PMT_MAX_CNN_OPS], ldg[PMT_MAX_CNN_OPS];   // zero-padded layout of conv op i's output gradient
+  int act_total, gbuf_floats, stage_floats;
+};
+
+// A SIMT kernel that claims variants from a counter: `claim` variants per claim, `grid` CTAs.
+struct Claims {
+  int claim, n_claims, grid;
+};
+
 struct CallPlan {
   Plan P;
   CnnGeom G;
   int mode;                    // PMT_PRECISION_*
+  int passes;                  // MMA passes of the tensor-core inference kernels: 1 in PMT_PRECISION_TF32, 3 (split TF32) else
   int n_sm;
+  // why pmt_forward / pmt_forward_prepared / pmt_forward_train, and why pmt_backward, would be refused ("": they run)
+  char fwd_refusal[160], bwd_refusal[160];
   bool reads_tc_ok;            // the model is inside the envelope of the tensor-core read kernels
   bool cnn_tc_ok, cnn_bwd_ok;  // ... of the tensor-core haplotype CNN forward, and of its backward
   tc::TcPlan T;                // step program of the read path (built for every model: its image is part of the layout)
@@ -74,8 +104,16 @@ struct CallPlan {
   // forward
   InfoKernel info;
   int info_w4;                 // InfoKernel::ROWS: the template width
+  size_t info_smem;            // ... and the dynamic shared memory of the info MLP kernel `info`
   CnnKernel cnn;
+  size_t cnn_simt_smem;        // hap_cnn_kernel (the CNN forward of CnnKernel::SIMT and of the backward's recompute)
   ReadsKernel reads;
+  bool packed_planner;         // ReadsKernel::TC: plan_tiles_packed_kernel; else the sequential planner (pmt_plan_tiles)
+  Ring ring;                   // reads_forward_tc_kernel<passes, false, *> (inference, and the long-set tiles)
+  Ring ring_save;              // reads_forward_tc_kernel<3, true, false> (training forward, the backward's recompute)
+  size_t reads_smem;           // reads_forward_kernel and reads_forward_long_kernel
+  Claims fwd_claims;           // reads_forward_kernel (batch given)
+  int fwd_long_grid;           // reads_forward_long_kernel (batch given)
   LongKernel lng;
   bool simt_gemm, simt_conv;   // SIMT weight images of the tile GEMMs / the convolutions that the batch-independent kernels read
   LongLayout long_tc;          // lng == LongKernel::TC
@@ -83,6 +121,12 @@ struct CallPlan {
   // backward
   bool bwd_reads_tc, bwd_cnn_tc;
   BwdLayout tc_bwd;            // reads_tc_ok
+  Ring ring_bwd;               // reads_backward_tc_kernel
+  size_t bwd_smem;             // reads_backward_kernel and reads_backward_long_kernel
+  size_t info_bwd_smem;        // info_mlp_backward_kernel
+  Claims bwd_claims;           // reads_backward_kernel (batch given)
+  CnnBwdGeom cnn_bwd;          // !bwd_cnn_tc: hap_cnn_backward_kernel's geometry ...
+  size_t cnn_bwd_smem;         // ... and dynamic shared memory
 };
 
 }  // namespace pmt
@@ -101,16 +145,23 @@ int pmt_launch_hap_cnn_simt(const pmt::CallPlan& C, const float* weights, const 
                             cudaStream_t st);
 // pmt_backward.cu
 size_t pmt_backward_workspace_size(const pmt::CallPlan& C, const PmtBatch* batch);
+// the SIMT backward's shared memory, claims and CNN geometry, and bwd_refusal for them (pmt_call_plan, once
+// bwd_reads_tc and bwd_cnn_tc are decided)
+void pmt_plan_backward(pmt::CallPlan& C, const PmtBatch* batch);
 // pmt_tc.cu
 bool pmt_tc_supported(const pmt::Plan& P);
 bool pmt_tc_long_layout(const pmt::Plan& P, const PmtBatch* batch, int n_sm, pmt::LongLayout* L);
 size_t pmt_tc_tiles_bytes(int n_variants);
+pmt::Ring pmt_tc_ring(const pmt::tc::TcPlan& T, int passes);
 int pmt_launch_reads_tc(const pmt::CallPlan& C, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
                         unsigned char* image_buf, unsigned char* tiles_buf, bool reuse_images, cudaStream_t st);
 int pmt_launch_reads_tc_long(const pmt::CallPlan& C, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
                              unsigned char* image_buf, unsigned char* long_buf, cudaStream_t st);
 // pmt_tc_bwd.cu
-pmt::BwdLayout pmt_tc_bwd_layout(const pmt::tc::TcPlan& T, const PmtBatch* batch);
+// `max_chunk_tiles` >= 1: at most that many tiles per recompute + backward pass (else the default)
+pmt::BwdLayout pmt_tc_bwd_layout(const pmt::tc::TcPlan& T, const PmtBatch* batch, int max_chunk_tiles);
+pmt::Ring pmt_tc_bwd_ring(const pmt::tc::TcPlan& T);
+int pmt_launch_reads_tc_save(const pmt::CallPlan& C, const pmt::tc::TcArgs& A, int grid, cudaStream_t st);
 pmt::SavedLayout pmt_saved_layout(const pmt::CallPlan& C, const PmtBatch* batch);
 int pmt_tc_forward_train(const pmt::CallPlan& C, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
                          unsigned char* image_buf, unsigned char* claim_buf, unsigned char* saved, cudaStream_t st);

@@ -757,6 +757,7 @@ static bool schedule_groups(cnntc::Plan& T, int hap_len) {
   // on the FP32 SIMT kernel (hap_cnn_kernel).
   const int fixed = 2 * BUF_BYTES + bytes + MAX_LAYERS * 32 * 4 + (int)sizeof(Bars) + 1024 + 64;
   if (fixed > 227 * 1024) return false;
+  T.smem = fixed;
   double best = 1e30;
   int best_g = 0;
   for (int G = 1; G <= 128; ++G) {
@@ -851,18 +852,19 @@ size_t pmt_cnn_tc_image_bytes(const CallPlan& C) {
 }
 
 size_t pmt_cnn_tail_buffer_bytes(const CallPlan& C, int n_variants) {
-  // whenever the pair may run (PMT_CNN_SINGLE=0 selects it below its batch-size threshold)
-  const bool may_split = C.cnn_split && (C.cnn == CnnKernel::TC || C.cnn == CnnKernel::TC_TAIL);
-  return may_split ? (size_t)(n_variants + 127) / 128 * 128 * C.CT.K0 * sizeof(float) : 0;
+  // Sized whenever the CNN has a tail and inference runs a tensor-core CNN, even where the plan chose the single kernel:
+  // sizing for C.cnn == TC_TAIL alone would shrink pmt_workspace_size below the pair's batch-size threshold, and the
+  // sizes the library reports stay as they were.
+  const bool tc = C.cnn == CnnKernel::TC || C.cnn == CnnKernel::TC_TAIL;
+  return C.cnn_split && tc ? (size_t)(n_variants + 127) / 128 * 128 * C.CT.K0 * sizeof(float) : 0;
 }
 
 template <int PASSES, bool SAVE>
 static int launch_cnn_tc(const cnntc::Plan& T, const unsigned char* image, const float* weights, const PmtModelDesc& D, const void* haps,
                          const PmtBatch* batch, int n, float* info_seq, const SaveLayout& SL, float* save, int grid, cudaStream_t st,
                          float* tail_buf = nullptr) {
-  const size_t smem = 2 * BUF_BYTES + T.image_bytes + MAX_LAYERS * 32 * sizeof(float) + sizeof(Bars) + 1024 + 64;
-  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_tc_kernel<PASSES, SAVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  hap_cnn_tc_kernel<PASSES, SAVE><<<grid, cnntc::THREADS, smem, st>>>(T, image, weights, D, haps, batch->hap_kind, batch->hap_stride, n, info_seq,
+  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_tc_kernel<PASSES, SAVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, T.smem));
+  hap_cnn_tc_kernel<PASSES, SAVE><<<grid, cnntc::THREADS, T.smem, st>>>(T, image, weights, D, haps, batch->hap_kind, batch->hap_stride, n, info_seq,
                                                                SL, save, tail_buf);
   return 0;
 }
@@ -925,7 +927,7 @@ int pmt_launch_cnn_tc(const CallPlan& C, const float* weights, const PmtBatch* b
   const int grid = n_groups < C.n_sm ? n_groups : C.n_sm;
   SaveLayout SL;
   memset(&SL, 0, sizeof(SL));
-  if (C.mode == PMT_PRECISION_TF32) {
+  if (C.passes == 1) {
     if (launch_cnn_tc<1, false>(T, image, weights, C.P.d, batch->haplotypes, batch, n, info_seq, SL, nullptr, grid, st, tail_buf)) return 1;
     return split ? launch_cnn_tail<1>(C.CT, image, weights, C.P.d, tail_buf, n, info_seq, C.n_sm, st) : 0;
   }

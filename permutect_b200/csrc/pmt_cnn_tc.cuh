@@ -44,6 +44,7 @@ struct Item {
 
 struct Plan {
   int n_layers, n_items, G, L0, image_bytes;
+  int smem;       // dynamic shared memory of hap_cnn_tc_kernel over these layers
   int n_chunks[MAX_LAYERS];
   Layer layer[MAX_LAYERS];
   Item item[MAX_ITEMS];

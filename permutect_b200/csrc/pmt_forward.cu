@@ -340,16 +340,8 @@ static int info_rows_w4(const PmtModelDesc& d) {
 }
 
 template <int W4>
-static int launch_info_rows(const PmtModelDesc& d, const float* weights, const PmtBatch* batch, float* info_seq, cudaStream_t st) {
-  const int W = 4 * W4;
-  // the input tile: feature-major floats, or (raw16) a tile's fp16 rows as one span of up to 127 strides of I + 8 halves
-  // plus a last row, which is the larger of the two below 8 features
-  const size_t I = (size_t)d.n_info_features;
-  const size_t raw16_words = ((INFO_TPB - 1) * (I + 8) + I + 1) / 2;
-  size_t floats = I * (INFO_TPB + 1) > raw16_words ? I * (INFO_TPB + 1) : raw16_words;
-  for (int i = 0; i < d.n_info_ops; ++i) floats += (size_t)(d.info_ops[i].in_dim + 1) * W;
-  const size_t smem = floats * sizeof(float) + 16;
-  PMT_CHECK(smem <= 200 * 1024, "info MLP does not fit in shared memory");
+static int launch_info_rows(const PmtModelDesc& d, const float* weights, const PmtBatch* batch, float* info_seq, size_t smem,
+                            cudaStream_t st) {
   PMT_CUDA(cudaFuncSetAttribute(info_mlp_rows_kernel<W4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int n_tiles = (batch->n_variants + INFO_TPB - 1) / INFO_TPB;
   int per_sm = (int)((220 * 1024) / smem);
@@ -779,12 +771,65 @@ int pmt_sm_count() {
   return n_sm;
 }
 
+// Test and measurement overrides of the call plan's choices, unset in normal use.  read_overrides is their only reader and
+// pmt_call_plan its only caller, so every C-ABI call of the model, the size queries included, sees the same choices.
+//   PMT_CNN_SINGLE=1       inference runs hap_cnn_tc_kernel over every layer; =0: the head + tail pair at any batch size
+//   PMT_TC_PACKED=0        the sequential tile planner for every batch
+//   PMT_LONG_SIMT=1        sets longer than a tile take the FP32 long-set kernel
+//   PMT_BWD_CHUNK_TILES=n  the tensor-core backward recomputes and differentiates at most n >= 1 tiles per pass
+struct Overrides {
+  int cnn_single, tc_packed, long_simt, bwd_chunk_tiles;
+};
+static Overrides read_overrides() {
+  auto get = [](const char* name) { const char* e = getenv(name); return e ? atoi(e) : -1; };
+  return {get("PMT_CNN_SINGLE"), get("PMT_TC_PACKED"), get("PMT_LONG_SIMT"), get("PMT_BWD_CHUNK_TILES")};
+}
+
+// Batches below this size keep the sequential planner: packing saves ~5.5 % of the read kernel (1.13 ns per read), the packed
+// planner costs ~0.1 ms more than the sequential one (one lane per claim places 512 sets), so it pays from ~2 M reads.
+static const long long kPackedPlannerMinRows = 2000000;
+
+static size_t info_kernel_smem(const Plan& P, InfoKernel k, int w4) {
+  const PmtModelDesc& d = P.d;
+  if (k == InfoKernel::TILE) {
+    const int in_rows = d.n_info_features > PMT_MAX_DIM ? PMT_MAX_INFO_DIM : PMT_MAX_DIM;
+    return (size_t)((in_rows + 2 * PMT_MAX_DIM) * LD + 2 * P.info_stage_floats) * sizeof(float);
+  }
+  size_t floats = 0;
+  const int W = k == InfoKernel::WARP ? 32 : 4 * w4;
+  if (k == InfoKernel::ROWS) {
+    // the input tile: feature-major floats, or (raw16) a tile's fp16 rows as one span of up to 127 strides of I + 8 halves
+    // plus a last row, which is the larger of the two below 8 features
+    const size_t I = (size_t)d.n_info_features;
+    const size_t raw16_words = ((INFO_TPB - 1) * (I + 8) + I + 1) / 2;
+    floats = I * (INFO_TPB + 1) > raw16_words ? I * (INFO_TPB + 1) : raw16_words;
+  }
+  for (int i = 0; i < d.n_info_ops; ++i) floats += (size_t)(d.info_ops[i].in_dim + 1) * W;
+  return floats * sizeof(float) + 16;
+}
+
+// reads_forward_kernel: aim for ~8 tiles per claim, but keep at least ~2 claims per SM when the batch is small
+static Claims forward_claims(const PmtBatch* batch, int n_sm) {
+  const double avg = (batch->n_variants > 0 && batch->n_rows > 0) ? (double)batch->n_rows / batch->n_variants : 16.0;
+  Claims K;
+  K.claim = (int)(8.0 * TILE / (avg + 1.0));
+  const int by_parallelism = batch->n_variants / (2 * n_sm);
+  if (K.claim > by_parallelism) K.claim = by_parallelism;
+  if (K.claim > 512) K.claim = 512;
+  if (K.claim < 1) K.claim = 1;
+  K.n_claims = (batch->n_variants + K.claim - 1) / K.claim;
+  K.grid = K.n_claims < n_sm ? K.n_claims : n_sm;
+  return K;
+}
+
 int pmt_call_plan(const PmtModelDesc* desc, const PmtBatch* batch, bool train, CallPlan* out) {
   CallPlan& C = *out;
   memset(&C, 0, sizeof(C));
   if (pmt_build_plan(desc, &C.P) || pmt_cnn_geometry(C.P, &C.G)) return 1;
   const Plan& P = C.P;
+  const Overrides ov = read_overrides();
   C.mode = pmt_precision_mode();
+  C.passes = C.mode == PMT_PRECISION_TF32 ? 1 : 3;
   C.n_sm = pmt_sm_count();
   C.reads_tc_ok = pmt_tc_supported(P);
   pmt_tc_plan(P, &C.T);
@@ -801,21 +846,57 @@ int pmt_call_plan(const PmtModelDesc* desc, const PmtBatch* batch, bool train, C
   const int B = batch ? batch->n_variants : 0;
   C.info_w4 = info_rows_w4(P.d);
   C.info = C.info_w4 == 0 ? InfoKernel::TILE : B <= 4096 ? InfoKernel::WARP : InfoKernel::ROWS;   // small batch: latency, not throughput
+  C.info_smem = info_kernel_smem(P, C.info, C.info_w4);
   // the head + tail pair once the head kernel has a group for every SM; below that a call is a chain of latencies, and the
   // pair's second launch and global round trip cost more than the tail's MMA round trips it saves
   C.cnn = train                                        ? CnnKernel::TC_SAVE
           : fp32 || !C.cnn_tc_ok                        ? CnnKernel::SIMT
           : C.cnn_split && B >= (long long)C.CH.G * C.n_sm ? CnnKernel::TC_TAIL
                                                         : CnnKernel::TC;
+  if (C.cnn == CnnKernel::TC || C.cnn == CnnKernel::TC_TAIL) {
+    if (ov.cnn_single == 1) C.cnn = CnnKernel::TC;
+    else if (ov.cnn_single == 0 && C.cnn_split) C.cnn = CnnKernel::TC_TAIL;
+  }
+  C.cnn_simt_smem = (size_t)(2 * C.G.buf_floats + C.G.img_total + 2 * C.G.vt * 256) * sizeof(float);
   C.reads = fp32 ? ReadsKernel::SIMT : train ? ReadsKernel::TC_SAVE : ReadsKernel::TC;
-  C.lng = !batch || !pmt_has_long_sets(batch)                            ? LongKernel::NONE
-          : !fp32 && pmt_tc_long_layout(P, batch, C.n_sm, &C.long_tc) ? LongKernel::TC
-                                                                       : LongKernel::SIMT;
+  C.packed_planner = C.reads == ReadsKernel::TC && batch && pmt_row_hint(batch) >= kPackedPlannerMinRows && ov.tc_packed != 0;
+  C.ring = pmt_tc_ring(C.T, C.passes);
+  C.ring_save = pmt_tc_ring(C.T, 3);
+  C.reads_smem = tile_ctx_bytes(P, P.stage_floats);
+  C.lng = !batch || !pmt_has_long_sets(batch)                                               ? LongKernel::NONE
+          : !fp32 && ov.long_simt != 1 && pmt_tc_long_layout(P, batch, C.n_sm, &C.long_tc) ? LongKernel::TC
+                                                                                          : LongKernel::SIMT;
+  if (batch) {
+    C.fwd_claims = forward_claims(batch, C.n_sm);
+    const int n_sm = C.n_sm < PMT_PARTIAL_CTAS ? C.n_sm : PMT_PARTIAL_CTAS;
+    C.fwd_long_grid = batch->n_variants < n_sm ? batch->n_variants : n_sm;
+  }
   // who reads the SIMT images in a tensor-core mode: the tile-GEMM info MLP (widths outside info_mlp_rows_kernel), the SIMT
   // haplotype CNN (shapes outside the tensor-core envelope) -- and, depending on the batch, the FP32 long-set kernel
   C.simt_gemm = fp32 || C.info == InfoKernel::TILE;
   C.simt_conv = C.cnn == CnnKernel::SIMT;
-  C.tc_bwd = pmt_tc_bwd_layout(C.T, batch);
+  C.tc_bwd = pmt_tc_bwd_layout(C.T, batch, ov.bwd_chunk_tiles);
+  C.ring_bwd = pmt_tc_bwd_ring(C.T);
+
+  // refusals, in the order the kernels would run
+  const bool info_fits = C.info == InfoKernel::TILE || C.info_smem <= 200 * 1024;
+  const bool ring_fits = (C.reads != ReadsKernel::TC_SAVE || C.ring_save.n_stages >= 2) &&
+                         ((C.reads != ReadsKernel::TC && C.lng != LongKernel::TC) || C.ring.n_stages >= 2);
+  const char* fwd_why = !info_fits                                       ? "info MLP does not fit in shared memory"
+                        : C.reads != ReadsKernel::SIMT && !C.reads_tc_ok ? "this model shape is outside the tensor-core kernel's envelope; use PMT_PRECISION_FP32"
+                        : !ring_fits                                     ? "tensor-core forward: weight ring does not fit in shared memory"
+                                                                         : "";
+  snprintf(C.fwd_refusal, sizeof(C.fwd_refusal), "%s", fwd_why);
+  // the backward recomputes the info MLP when the forward's embeddings are not passed in, and the read path's forward
+  // operands when they were not saved
+  pmt_plan_backward(C, batch);
+  if (!C.bwd_refusal[0]) {
+    const char* bwd_why = !info_fits                                          ? "info MLP does not fit in shared memory"
+                          : C.bwd_reads_tc && C.ring_save.n_stages < 2        ? "tensor-core forward: weight ring does not fit in shared memory"
+                          : C.bwd_reads_tc && C.ring_bwd.n_stages < 2         ? "tensor-core backward: weight ring does not fit in shared memory"
+                                                                              : "";
+    snprintf(C.bwd_refusal, sizeof(C.bwd_refusal), "%s", bwd_why);
+  }
   return 0;
 }
 
@@ -859,8 +940,6 @@ extern "C" size_t pmt_workspace_size(const PmtModelDesc* desc, const PmtBatch* b
   return for_backward ? pmt_backward_workspace_size(C, batch) : forward_layout(C, batch).end;
 }
 
-static size_t reads_kernel_smem(const Plan& P) { return tile_ctx_bytes(P, P.stage_floats); }
-
 int pmt_launch_prepare(const CallPlan& C, const float* weights, float* image, cudaStream_t st, bool gemm, bool conv) {
   const Plan& P = C.P;
   const CnnGeom& G = C.G;
@@ -874,29 +953,24 @@ int pmt_launch_info_mlp(const CallPlan& C, const float* weights, const float* im
                         cudaStream_t st) {
   const Plan& P = C.P;
   const int B = batch->n_variants;
+  const size_t smem = C.info_smem;
   if (C.info == InfoKernel::WARP) {
-    size_t floats = 0;
-    for (int i = 0; i < P.d.n_info_ops; ++i) floats += (size_t)(P.d.info_ops[i].in_dim + 1) * 32;
-    const size_t smem = floats * sizeof(float) + 16;
-    PMT_CHECK(smem <= 200 * 1024, "info MLP does not fit in shared memory");
     PMT_CUDA(cudaFuncSetAttribute(info_mlp_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int blocks = (B + INFO_WARPS - 1) / INFO_WARPS;
     info_mlp_warp_kernel<<<blocks < 148 * 4 ? blocks : 148 * 4, 32 * INFO_WARPS, smem, st>>>(P.d, weights, batch->info, batch->info_kind,
                                                                                                batch->info_stride, B, info_seq);
   } else if (C.info == InfoKernel::ROWS) {
     switch (C.info_w4) {
-      case 1: return launch_info_rows<1>(P.d, weights, batch, info_seq, st);
-      case 2: return launch_info_rows<2>(P.d, weights, batch, info_seq, st);
-      case 3: return launch_info_rows<3>(P.d, weights, batch, info_seq, st);
-      case 4: return launch_info_rows<4>(P.d, weights, batch, info_seq, st);
-      case 5: return launch_info_rows<5>(P.d, weights, batch, info_seq, st);
-      case 6: return launch_info_rows<6>(P.d, weights, batch, info_seq, st);
-      case 7: return launch_info_rows<7>(P.d, weights, batch, info_seq, st);
-      default: return launch_info_rows<8>(P.d, weights, batch, info_seq, st);
+      case 1: return launch_info_rows<1>(P.d, weights, batch, info_seq, smem, st);
+      case 2: return launch_info_rows<2>(P.d, weights, batch, info_seq, smem, st);
+      case 3: return launch_info_rows<3>(P.d, weights, batch, info_seq, smem, st);
+      case 4: return launch_info_rows<4>(P.d, weights, batch, info_seq, smem, st);
+      case 5: return launch_info_rows<5>(P.d, weights, batch, info_seq, smem, st);
+      case 6: return launch_info_rows<6>(P.d, weights, batch, info_seq, smem, st);
+      case 7: return launch_info_rows<7>(P.d, weights, batch, info_seq, smem, st);
+      default: return launch_info_rows<8>(P.d, weights, batch, info_seq, smem, st);
     }
   } else {
-    const int in_rows = P.d.n_info_features > PMT_MAX_DIM ? PMT_MAX_INFO_DIM : PMT_MAX_DIM;
-    const size_t smem = (size_t)((in_rows + 2 * PMT_MAX_DIM) * LD + 2 * P.info_stage_floats) * sizeof(float);
     PMT_CUDA(cudaFuncSetAttribute(info_mlp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     info_mlp_kernel<<<(B + TILE - 1) / TILE, NTHREADS, smem, st>>>(P, weights, image, batch->info, batch->info_kind,
                                                                    batch->info_stride, B, info_seq);
@@ -908,24 +982,12 @@ int pmt_launch_hap_cnn_simt(const CallPlan& C, const float* weights, const float
                             cudaStream_t st) {
   const CnnGeom& G = C.G;
   const int B = batch->n_variants;
-  const size_t smem = (size_t)(2 * G.buf_floats + G.img_total + 2 * G.vt * 256) * sizeof(float);
-  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  PMT_CUDA(cudaFuncSetAttribute(hap_cnn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C.cnn_simt_smem));
   int grid = (B + G.vt - 1) / G.vt;
   if (grid > 148 * 4) grid = 148 * 4;
-  hap_cnn_kernel<<<grid, NTHREADS, smem, st>>>(C.P, G, weights, image + C.P.img_total, batch->haplotypes, batch->hap_kind,
+  hap_cnn_kernel<<<grid, NTHREADS, C.cnn_simt_smem, st>>>(C.P, G, weights, image + C.P.img_total, batch->haplotypes, batch->hap_kind,
                                                batch->hap_stride, B, info_seq);
   return 0;
-}
-
-static int choose_claim(const PmtBatch* batch, int n_sm) {
-  // aim for ~8 tiles per claim, but keep at least ~2 claims per SM when the batch is small
-  const double avg = (batch->n_variants > 0 && batch->n_rows > 0) ? (double)batch->n_rows / batch->n_variants : 16.0;
-  int claim = (int)(8.0 * TILE / (avg + 1.0));
-  const int by_parallelism = batch->n_variants / (2 * n_sm);
-  if (claim > by_parallelism) claim = by_parallelism;
-  if (claim > 512) claim = 512;
-  if (claim < 1) claim = 1;
-  return claim;
 }
 
 extern "C" size_t pmt_train_saved_bytes(const PmtModelDesc* desc, const PmtBatch* batch) {
@@ -942,14 +1004,13 @@ static int forward_impl(const PmtModelDesc* desc, const float* weights, const Pm
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const FwdLayout L = forward_layout(C, batch);
   PMT_CHECK(workspace && workspace_bytes >= L.end, "workspace too small: %zu < %zu", workspace_bytes, L.end);
-  if (C.cnn == CnnKernel::TC || C.cnn == CnnKernel::TC_TAIL) {
-    // measurement and tests (profiles/time_cnn_forward.py, tests/test_cnn_tail_gpu.py): PMT_CNN_SINGLE=1 runs
-    // hap_cnn_tc_kernel over every layer, PMT_CNN_SINGLE=0 the head + tail pair at any batch size
-    const char* e = getenv("PMT_CNN_SINGLE");
-    if (e && atoi(e) == 1) C.cnn = CnnKernel::TC;
-    else if (e && atoi(e) == 0 && C.cnn_split) C.cnn = CnnKernel::TC_TAIL;
-  }
   PMT_CHECK(batch->n_variants > 0, "empty batch");
+  PMT_CHECK(!C.fwd_refusal[0], "%s", C.fwd_refusal);
+  if (saved) {
+    PMT_CHECK(C.saved.total > 0 && saved_bytes >= C.saved.total,
+              "pmt_forward_train: no saved-forward path for this call or buffer too small (%zu < %zu)", saved_bytes, C.saved.total);
+    PMT_CHECK((reinterpret_cast<uintptr_t>(saved) & 255) == 0, "pmt_forward_train: the saved buffer must be 256-byte aligned");
+  }
   char* ws = reinterpret_cast<char*>(workspace);
   int* counter = reinterpret_cast<int*>(ws);
   float* image = reinterpret_cast<float*>(ws + L.image);
@@ -964,11 +1025,6 @@ static int forward_impl(const PmtModelDesc* desc, const float* weights, const Pm
   }
   unsigned char* tc_image = reinterpret_cast<unsigned char*>(ws + L.tc_image);
   unsigned char* cnn_tc_image = reinterpret_cast<unsigned char*>(ws + L.cnn_tc_image);
-  if (saved) {
-    PMT_CHECK(C.saved.total > 0 && saved_bytes >= C.saved.total,
-              "pmt_forward_train: no saved-forward path for this call or buffer too small (%zu < %zu)", saved_bytes, C.saved.total);
-    PMT_CHECK((reinterpret_cast<uintptr_t>(saved) & 255) == 0, "pmt_forward_train: the saved buffer must be 256-byte aligned");
-  }
   // per-variant embeddings: the info MLP, then the haplotype CNN (in training its SAVE variant: same results, activations kept)
   if (pmt_launch_info_mlp(C, weights, image, batch, info_seq, st)) return 1;
   switch (C.cnn) {
@@ -985,21 +1041,19 @@ static int forward_impl(const PmtModelDesc* desc, const float* weights, const Pm
   }
 
   Plan P = C.P;
-  P.claim_variants = choose_claim(batch, C.n_sm);
+  P.claim_variants = C.fwd_claims.claim;
   ReadKernelArgs A;
   A.wflat = weights; A.image = image; A.batch = *batch; A.out = *out; A.out.info_seq_be = info_seq; A.claim_counter = counter;
   A.scratch = nullptr; A.scratch_stride = 0;
-  const size_t smem = reads_kernel_smem(P);
+  const size_t smem = C.reads_smem;
   PMT_CUDA(cudaFuncSetAttribute(reads_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   PmtOutputs o2 = *out;
   o2.info_seq_be = info_seq;
   if (C.reads == ReadsKernel::SIMT) {
-    const int n_claims = (batch->n_variants + P.claim_variants - 1) / P.claim_variants;
     pmt_profile_begin(st);
-    reads_forward_kernel<<<n_claims < C.n_sm ? n_claims : C.n_sm, NTHREADS, smem, st>>>(P, A);
+    reads_forward_kernel<<<C.fwd_claims.grid, NTHREADS, smem, st>>>(P, A);
     pmt_profile_end(st);
   } else {
-    PMT_CHECK(C.reads_tc_ok, "this model shape is outside the tensor-core kernel's envelope; use PMT_PRECISION_FP32");
     if (C.reads == ReadsKernel::TC_SAVE) {   // deterministic tile list + the SAVE variant of the read kernel, operands kept for the backward
       if (pmt_tc_forward_train(C, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.tiles), saved, st)) return 1;
     } else if (pmt_launch_reads_tc(C, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.tiles), reuse_images, st)) {
@@ -1012,9 +1066,8 @@ static int forward_impl(const PmtModelDesc* desc, const float* weights, const Pm
   } else if (C.lng == LongKernel::SIMT) {
     A.scratch = reinterpret_cast<float*>(ws + L.long_scratch);
     A.scratch_stride = (long long)long_scratch_floats_per_cta(P, batch);
-    const int n_sm = C.n_sm < PMT_PARTIAL_CTAS ? C.n_sm : PMT_PARTIAL_CTAS;
     PMT_CUDA(cudaFuncSetAttribute(reads_forward_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    reads_forward_long_kernel<<<batch->n_variants < n_sm ? batch->n_variants : n_sm, NTHREADS, smem, st>>>(P, A);
+    reads_forward_long_kernel<<<C.fwd_long_grid, NTHREADS, smem, st>>>(P, A);
   }
   cudaError_t e = cudaGetLastError();
   PMT_CHECK(e == cudaSuccess, "pmt_forward launch failed: %s", cudaGetErrorString(e));

@@ -80,7 +80,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
       mbar_init(smem_addr(&S->bar_a[s]), 8); mbar_init(smem_addr(&S->bar_d[s]), 1);
       for (int b = 0; b < 2; ++b) { mbar_init(smem_addr(&S->meta_full[s][b]), 1); mbar_init(smem_addr(&S->meta_free[s][b]), 8); }
     }
-    for (int i = 0; i < n_stages; ++i) { mbar_init(smem_addr(&S->wfull[i]), 1); mbar_init(smem_addr(&S->wfree[i]), A.sched == 1 ? 1 : 2); }
+    for (int i = 0; i < n_stages; ++i) { mbar_init(smem_addr(&S->wfull[i]), 1); mbar_init(smem_addr(&S->wfree[i]), 2); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     head_constants(D, W, HC);
     for (int e = 0; e < MAXE; ++e) HCT->inv_sigma[e] = e < D.d_feat ? 1.f / HC->sigma[e] : 0.f;
@@ -119,8 +119,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
   static_assert(!(LONG && SAVE), "the long-set tiles are forward only");
   const int tile_first = SAVE ? A.tile_first : 0;
   const int n_tiles = LONG ? __ldg(A.lng.n_tiles) : (SAVE ? min(__ldg(A.tiles), A.tile_limit) - tile_first : __ldg(A.tiles));
-  const int sched = A.sched;
-  const int n_slots = (sched == 1 ? 1 : 2) * gridDim.x;
+  const int n_slots = 2 * gridDim.x;
   // every slot of the CTA runs the same number of rounds (an idle slot processes an empty tile)
   // tile t of round r: slot 0 of every CTA first, then slot 1 (a small batch spreads over the SMs before it doubles up)
   const int rounds = n_tiles > (int)blockIdx.x ? (n_tiles - (int)blockIdx.x + n_slots - 1) / n_slots : 0;   // rounds of slot 0 >= slot 1
@@ -140,7 +139,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
     for (int round = 0; round < rounds; ++round) {
       const int b = round & 1;
       const unsigned fparity = ((round >> 1) & 1) ^ 1;   // the first use of each buffer finds it free
-      for (int slot = 0; slot < (sched == 1 ? 1 : 2); ++slot) {
+      for (int slot = 0; slot < 2; ++slot) {
         TileBuf* TB = &S->tb[slot][b];
         mbar_wait(smem_addr(&S->meta_free[slot][b]), fparity);
         const int t = (int)blockIdx.x + slot * (int)gridDim.x + round * n_slots;
@@ -289,8 +288,6 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
       }
     }
     __syncwarp();
-  } else if (sched == 1 && (warp == MMA_WARP + 1 || (warp >= 8 && warp < 16))) {
-    // measurement mode: slot 1 stays idle
   } else if (warp >= MMA_WARP) {
     // ===================================== MMA issuers: one warp per slot =====================================
     // Each warp blocks only on ITS slot's operand barrier, so the two slots drift apart freely and one slot's
@@ -1358,9 +1355,6 @@ void pmt_tc_plan(const Plan& P, TcPlan* out) {
 }
 
 static size_t perm_bytes(int n_variants) { return ((size_t)n_variants * sizeof(int) + 255) & ~(size_t)255; }
-// Batches below this size keep the sequential planner: packing saves ~5.5 % of the read kernel (1.13 ns per read), the packed
-// planner costs ~0.1 ms more than the sequential one (one lane per claim places 512 sets), so it pays from ~2 M reads.
-static const long long kPackedPlannerMinRows = 2000000;
 
 // the inference tile list and the packed planner's variant order
 size_t pmt_tc_tiles_bytes(int n_variants) { return pmt_tile_list_bytes(n_variants) + perm_bytes(n_variants) + 256; }
@@ -1399,18 +1393,20 @@ int pmt_plan_tiles(const PmtBatch* batch, int max_variants, bool deterministic, 
   return 0;
 }
 
-// Sizes the weight ring (as many stages as fit next to the fixed carve, at most NS_MAX) and launches one instantiation
-// of the read kernel.
+// The read kernel's weight ring: as many stages as fit next to the fixed carve, at most NS_MAX.
+Ring pmt_tc_ring(const TcPlan& T, int passes) {
+  Ring R;
+  R.stage_bytes = passes == 3 ? T.slot_bytes : T.slot_bytes / 2;
+  R.n_stages = (int)((227 * 1024 - FWD_FIXED_BYTES) / R.stage_bytes);
+  if (R.n_stages > NS_MAX) R.n_stages = NS_MAX;
+  R.smem = FWD_FIXED_BYTES + (size_t)R.n_stages * R.stage_bytes;
+  return R;
+}
+
 template <int PASSES, bool SAVE, bool LONG>
-static int launch_reads_tc(const PmtModelDesc& D, const TcPlan& T, const TcArgs& A, int grid, cudaStream_t st) {
-  const int stage_bytes = PASSES == 3 ? T.slot_bytes : T.slot_bytes / 2;
-  const size_t fixed = FWD_FIXED_BYTES;
-  int n_stages = (int)((227 * 1024 - fixed) / stage_bytes);
-  if (n_stages > NS_MAX) n_stages = NS_MAX;
-  PMT_CHECK(n_stages >= 2, "tensor-core forward: weight ring does not fit in shared memory");
-  const size_t smem = fixed + (size_t)n_stages * stage_bytes;
-  PMT_CUDA(cudaFuncSetAttribute(reads_forward_tc_kernel<PASSES, SAVE, LONG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  reads_forward_tc_kernel<PASSES, SAVE, LONG><<<grid, FWD_THREADS, smem, st>>>(D, T, A, n_stages, stage_bytes);
+static int launch_reads_tc(const PmtModelDesc& D, const TcPlan& T, const TcArgs& A, int grid, const Ring& R, cudaStream_t st) {
+  PMT_CUDA(cudaFuncSetAttribute(reads_forward_tc_kernel<PASSES, SAVE, LONG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)R.smem));
+  reads_forward_tc_kernel<PASSES, SAVE, LONG><<<grid, FWD_THREADS, R.smem, st>>>(D, T, A, R.n_stages, R.stage_bytes);
   return 0;
 }
 
@@ -1419,9 +1415,10 @@ int pmt_launch_pack_tc(const Plan& P, const TcPlan& T, const float* weights, uns
   return 0;
 }
 
-// Training recompute (always the split-precision mode: the saved activations are the fp32-parity ones).
-int pmt_launch_reads_tc_save(const Plan& P, const TcPlan& T, const TcArgs& A, int grid, cudaStream_t st) {
-  return launch_reads_tc<3, true, false>(P.d, T, A, grid, st);
+// Training recompute: the forward over tiles [tile_first, tile_limit) of a planned tile list, operands saved to `scratch`
+// (always the split-precision mode: the saved activations are the fp32-parity ones).
+int pmt_launch_reads_tc_save(const CallPlan& C, const TcArgs& A, int grid, cudaStream_t st) {
+  return launch_reads_tc<3, true, false>(C.P.d, C.T, A, grid, C.ring_save, st);
 }
 
 // Launches the tile planner, the weight packer (unless the images in `image_buf` are still valid) and the tensor-core
@@ -1433,8 +1430,7 @@ int pmt_launch_reads_tc(const CallPlan& C, const float* weights, const PmtBatch*
   int* tiles = reinterpret_cast<int*>((reinterpret_cast<uintptr_t>(tiles_buf) + 255) & ~uintptr_t(255));
   int n_claims = 0;
   int* perm = nullptr;
-  const char* pk = getenv("PMT_TC_PACKED");   // measurement: 0 = the sequential planner for every batch
-  if (pmt_row_hint(batch) >= kPackedPlannerMinRows && !(pk && atoi(pk) == 0)) {
+  if (C.packed_planner) {
     perm = reinterpret_cast<int*>(reinterpret_cast<unsigned char*>(tiles) + pmt_tile_list_bytes(batch->n_variants));
     n_claims = (batch->n_variants + PLAN_CLAIM - 1) / PLAN_CLAIM;
     PMT_CUDA(cudaMemsetAsync(tiles, 0, 2 * sizeof(int), st));
@@ -1448,22 +1444,20 @@ int pmt_launch_reads_tc(const CallPlan& C, const float* weights, const PmtBatch*
   TcArgs A;
   A.wflat = weights; A.image = image; A.tiles = tiles; A.perm = perm; A.batch = *batch; A.out = *out;
   A.scratch = nullptr; A.tile_first = 0; A.tile_limit = 0x7fffffff;
-  { const char* e = getenv("PMT_TC_SCHED"); A.sched = (e && atoi(e) == 1) ? 1 : 0; }   // measurement: one slot only
   // the second slot of each CTA takes a second tile once every SM has one
   const int grid = pmt_tile_grid(batch, n_claims, C.n_sm);
   pmt_profile_begin(st);
-  const int rc = C.mode == PMT_PRECISION_TF32 ? launch_reads_tc<1, false, false>(C.P.d, T, A, grid, st)
-                                           : launch_reads_tc<3, false, false>(C.P.d, T, A, grid, st);
+  const int rc = C.passes == 1 ? launch_reads_tc<1, false, false>(C.P.d, T, A, grid, C.ring, st)
+                               : launch_reads_tc<3, false, false>(C.P.d, T, A, grid, C.ring, st);
   pmt_profile_end(st);
   return rc;
 }
 
 // ---- sets longer than a tile (pmt_tc.cuh: LongTile) ----
-// false: the long-set tensor-core path is not available for this batch (no long sets, unknown row count, a set longer than
-// one round of tiles, or PMT_LONG_SIMT=1) -- the FP32 long-set kernel takes them.
+// false: the long-set tensor-core path is not available for this batch (no long sets, unknown row count, or a set longer
+// than one round of tiles) -- the FP32 long-set kernel takes them.
 bool pmt_tc_long_layout(const Plan& P, const PmtBatch* batch, int n_sm, LongLayout* L) {
   if (!batch || !pmt_has_long_sets(batch) || batch->n_rows <= 0 || !pmt_tc_supported(P)) return false;
-  if (getenv("PMT_LONG_SIMT") && atoi(getenv("PMT_LONG_SIMT")) == 1) return false;   // measurement: the FP32 long-set kernel
   const int R = 2 * n_sm;
   const long long t_max = (batch->max_rows_per_variant + TILE - 1) / TILE + 1;        // ceil per side
   if (t_max > R) return false;
@@ -1512,13 +1506,13 @@ int pmt_launch_reads_tc_long(const CallPlan& C, const float* weights, const PmtB
   TcArgs A;
   memset(&A, 0, sizeof(A));
   A.wflat = weights; A.image = image; A.tiles = nullptr; A.batch = *batch; A.out = *out;
-  A.scratch = nullptr; A.tile_first = 0; A.tile_limit = 0x7fffffff; A.sched = 0;
+  A.scratch = nullptr; A.tile_first = 0; A.tile_limit = 0x7fffffff;
   A.lng.tiles = tiles; A.lng.n_tiles = n_tiles;
   A.lng.mf_cnt = reinterpret_cast<int*>(base + L.counters);
   A.lng.fin_cnt = reinterpret_cast<int*>(base + L.fin_cnt);
   A.lng.mf_part = reinterpret_cast<float*>(base + L.mf_part);
   A.lng.fin_part = reinterpret_cast<float*>(base + L.fin_part);
   const int grid = L.R / 2;
-  return C.mode == PMT_PRECISION_TF32 ? launch_reads_tc<1, false, true>(C.P.d, C.T, A, grid, st)
-                                      : launch_reads_tc<3, false, true>(C.P.d, C.T, A, grid, st);
+  return C.passes == 1 ? launch_reads_tc<1, false, true>(C.P.d, C.T, A, grid, C.ring, st)
+                       : launch_reads_tc<3, false, true>(C.P.d, C.T, A, grid, C.ring, st);
 }

@@ -117,7 +117,6 @@ struct TcArgs {
   // scratch + (t - tile_first) * TcPlan.tile_bytes
   unsigned char* scratch;
   int tile_first, tile_limit;
-  int sched;              // 0 = both slots; 1 = one slot only (measurement: what a tile costs without its neighbour)
   LongArgs lng;           // LONG kernels only
 };
 
@@ -350,7 +349,5 @@ __host__ __device__ __forceinline__ int proj1_bwd_col(int nb, int H) {
 // host: the step program of the forward (pmt_tc.cu)
 void pmt_tc_plan(const pmt::Plan& P, pmt::tc::TcPlan* out);
 int pmt_launch_pack_tc(const pmt::Plan& P, const pmt::tc::TcPlan& T, const float* weights, unsigned char* image, cudaStream_t st);
-// training recompute: the forward over tiles [tile_first, tile_limit) of a planned tile list, operands saved to `scratch`
-int pmt_launch_reads_tc_save(const pmt::Plan& P, const pmt::tc::TcPlan& T, const pmt::tc::TcArgs& A, int grid, cudaStream_t st);
 int pmt_plan_tiles(const PmtBatch* batch, int max_variants, bool deterministic, int n_sm, int* tiles, int* claim_buf, int* n_claims_out,
                    cudaStream_t st);

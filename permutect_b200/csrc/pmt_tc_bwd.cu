@@ -852,7 +852,7 @@ static long long tile_bound(const PmtBatch* batch, int n_claims) {
   return bound < 1 ? 1 : bound;
 }
 
-BwdLayout pmt_tc_bwd_layout(const TcPlan& T, const PmtBatch* batch) {
+BwdLayout pmt_tc_bwd_layout(const TcPlan& T, const PmtBatch* batch, int max_chunk_tiles) {
   BwdLayout L;
   memset(&L, 0, sizeof(L));
   const int B = batch ? batch->n_variants : 0;
@@ -866,8 +866,7 @@ BwdLayout pmt_tc_bwd_layout(const TcPlan& T, const PmtBatch* batch) {
   off = (off + 1023) & ~(size_t)1023;
   L.n_claims = train_claims(B);
   const long long bound = batch ? tile_bound(batch, L.n_claims) : 1;
-  int chunk_cap = kChunkTiles;
-  if (const char* e = getenv("PMT_BWD_CHUNK_TILES")) { const int v = atoi(e); if (v >= 1) chunk_cap = v; }   // tests: several passes on a small batch
+  const int chunk_cap = max_chunk_tiles >= 1 ? max_chunk_tiles : kChunkTiles;
   L.chunk_tiles = (int)(bound < chunk_cap ? bound : chunk_cap);
   L.n_chunks = (int)((bound + L.chunk_tiles - 1) / L.chunk_tiles);
   L.scratch = off; off += (size_t)L.chunk_tiles * T.tile_bytes;
@@ -898,6 +897,18 @@ __global__ void check_tile_bound_kernel(const int* __restrict__ tiles, int bound
   }
 }
 
+// The backward kernel's weight ring: as many stages as fit next to the fixed carve, at most NS_MAX.
+Ring pmt_tc_bwd_ring(const TcPlan& T) {
+  const size_t fixed = 2 * OPBUF_BYTES + 2 * BXCH_ROWS * XCH_LD * sizeof(float) + 2 * 3 * BW_TAB * sizeof(float) + 2 * 2 * TILE * 4 * sizeof(float) +
+                       PMT_MAX_BLOCKS * BC_STRIDE * sizeof(float) + sizeof(HeadConst) + sizeof(SharedB) + 1024 + 64;
+  Ring R;
+  R.stage_bytes = (T.t_stage_bytes + 1023) & ~1023;
+  R.n_stages = (int)((227 * 1024 - fixed) / R.stage_bytes);
+  if (R.n_stages > NS_MAX) R.n_stages = NS_MAX;
+  R.smem = fixed + (size_t)R.n_stages * R.stage_bytes;
+  return R;
+}
+
 // The training forward of the tile-sized sets: deterministic tile list, then the SAVE variant of the read kernel over ALL
 // tiles with the outputs switched on.  `image_buf`: the forward layout's tc_image region (weight images, packed here);
 // `claim_buf`: the forward layout's planner scratch.
@@ -918,9 +929,9 @@ int pmt_tc_forward_train(const CallPlan& C, const float* weights, const PmtBatch
   TcArgs F;
   memset(&F, 0, sizeof(F));
   F.wflat = weights; F.image = image; F.tiles = tiles; F.perm = nullptr; F.batch = *batch; F.out = *out;
-  F.scratch = saved + S.scratch; F.sched = 0; F.tile_first = 0; F.tile_limit = (int)S.bound;
+  F.scratch = saved + S.scratch; F.tile_first = 0; F.tile_limit = (int)S.bound;
   pmt_profile_begin(st);
-  const int rc = pmt_launch_reads_tc_save(C.P, T, F, grid, st);
+  const int rc = pmt_launch_reads_tc_save(C, F, grid, st);
   pmt_profile_end(st);
   return rc;
 }
@@ -955,20 +966,14 @@ int pmt_launch_reads_tc_backward(const CallPlan& C, const float* weights, const 
 
   const int grid = pmt_tile_grid(batch, n_claims, C.n_sm < PMT_PARTIAL_CTAS ? C.n_sm : PMT_PARTIAL_CTAS);
   PMT_CUDA(cudaMemsetAsync(partials, 0, (size_t)2 * grid * T.part_floats * sizeof(float), st));
-  const int stage_bytes = (T.t_stage_bytes + 1023) & ~1023;
-  const size_t fixed = 2 * OPBUF_BYTES + 2 * BXCH_ROWS * XCH_LD * sizeof(float) + 2 * 3 * BW_TAB * sizeof(float) + 2 * 2 * TILE * 4 * sizeof(float) +
-                       PMT_MAX_BLOCKS * BC_STRIDE * sizeof(float) + sizeof(HeadConst) + sizeof(SharedB) + 1024 + 64;
-  int n_stages = (int)((227 * 1024 - fixed) / stage_bytes);
-  if (n_stages > NS_MAX) n_stages = NS_MAX;
-  PMT_CHECK(n_stages >= 2, "tensor-core backward: weight ring does not fit in shared memory");
-  const size_t smem = fixed + (size_t)n_stages * stage_bytes;
-  PMT_CUDA(cudaFuncSetAttribute(reads_backward_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const Ring& R = C.ring_bwd;
+  PMT_CUDA(cudaFuncSetAttribute(reads_backward_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)R.smem));
 
   PmtOutputs no_out;
   memset(&no_out, 0, sizeof(no_out));
   no_out.info_seq_be = const_cast<float*>(info_seq);   // read by the first gated block's concat
   TcArgs F;
-  F.wflat = weights; F.image = image_f; F.tiles = tiles; F.perm = nullptr; F.batch = *batch; F.out = no_out; F.scratch = scratch; F.sched = 0;
+  F.wflat = weights; F.image = image_f; F.tiles = tiles; F.perm = nullptr; F.batch = *batch; F.out = no_out; F.scratch = scratch;
   TcBwdArgs Bk;
   Bk.wflat = weights; Bk.image_t = image_t; Bk.tiles = tiles; Bk.batch = *batch; Bk.d_logits_bk = d_logits_bk;
   Bk.d_alt_means = d_alt_means; Bk.d_ref_means = d_ref_means; Bk.d_info_seq = d_info_seq; Bk.scratch = scratch; Bk.partials = partials;
@@ -977,8 +982,8 @@ int pmt_launch_reads_tc_backward(const CallPlan& C, const float* weights, const 
     F.tile_first = Bk.tile_first = c * L.chunk_tiles;
     F.tile_limit = Bk.tile_limit = (c + 1) * L.chunk_tiles;
     if (saved) Bk.scratch = scratch + (size_t)Bk.tile_first * T.tile_bytes;   // the kernel indexes a pass's scratch from its first tile
-    else if (pmt_launch_reads_tc_save(C.P, T, F, grid, st)) return 1;
-    reads_backward_tc_kernel<<<grid, THREADS, smem, st>>>(C.P.d, T, Bk, n_stages, stage_bytes);
+    else if (pmt_launch_reads_tc_save(C, F, grid, st)) return 1;
+    reads_backward_tc_kernel<<<grid, THREADS, R.smem, st>>>(C.P.d, T, Bk, R.n_stages, R.stage_bytes);
   }
   pmt_profile_end(st);
   *grid_out = grid;

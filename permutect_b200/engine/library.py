@@ -227,8 +227,9 @@ def check(rc: int):
 
 def set_precision(mode: str) -> None:
     """Arithmetic of the read path's dense layers: "fp32" (FP32 FMA pipe, forward + backward), "tf32x3" (tcgen05
-    tensor cores with split-precision TF32: the fp32-parity mode on tensor cores, forward only) or "tf32"
-    (plain TF32 on tensor cores; tolerance stated separately, forward only)."""
+    tensor cores with split-precision TF32: the fp32-parity mode on tensor cores) or "tf32" (plain TF32 on tensor
+    cores; tolerance stated separately).  In both tensor-core modes the backward runs on the tensor cores too where the
+    model allows it (backward_kernels)."""
     check(load().pmt_set_precision(PRECISION_MODES[mode]))
 
 
