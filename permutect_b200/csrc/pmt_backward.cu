@@ -1255,54 +1255,6 @@ void pmt_plan_backward(CallPlan& C, const PmtBatch* batch) {
   else if (!cnn_ok)
     snprintf(why, n, "%s", cnn_why);
 }
-// Long-set kernel: every chunk of the longest set has its own recompute scratch + dL/dx + gate state (see the kernel).
-// The grid shrinks when the scratch of a full grid would pass kLongScratchBudget.
-static const size_t kLongScratchBudget = (size_t)16 << 30;
-static size_t long_bwd_floats_per_cta(const Plan& P, const PmtBatch* batch) {
-  if (!batch || !pmt_has_long_sets(batch)) return 0;
-  const size_t chunks = (size_t)((batch->max_rows_per_variant + 3 + TILE - 1) / TILE);
-  return chunks * ((size_t)P.scratch_floats + (size_t)(P.d.d_model + 3 * P.d.d_ffn) * LD);
-}
-static int long_bwd_grid(const Plan& P, const PmtBatch* batch) {
-  const size_t per_cta = long_bwd_floats_per_cta(P, batch) * sizeof(float);
-  if (per_cta == 0) return 0;
-  size_t grid = kLongScratchBudget / per_cta;
-  if (grid > (size_t)PMT_PARTIAL_CTAS) grid = PMT_PARTIAL_CTAS;
-  if (grid > (size_t)batch->n_variants) grid = batch->n_variants;
-  return grid < 1 ? 1 : (int)grid;
-}
-
-// Workspace layout of the backward:
-//   [256 B][SIMT images][partials][activation scratch][info_seq][d_info_seq] | [long-set scratch][tensor-core read-path
-//   backward][tensor-core CNN backward]
-struct BwdWsLayout {
-  size_t image, partials, scratch, info_seq, d_info_seq, long_scratch, tc, tc_bytes, cnn, cnn_bytes, end;
-  size_t scr_floats, long_floats;
-  int long_grid;
-};
-static BwdWsLayout backward_layout(const CallPlan& C, const PmtBatch* batch) {
-  const Plan& P = C.P;
-  const size_t w = batch ? (size_t)batch->n_variants * (P.d.d_info + P.d.d_seq) * sizeof(float) : 0;
-  BwdWsLayout L;
-  L.scr_floats = P.scratch_floats > P.info_scratch_floats ? P.scratch_floats : P.info_scratch_floats;
-  L.long_grid = long_bwd_grid(P, batch);
-  L.long_floats = long_bwd_floats_per_cta(P, batch);
-  size_t off = 256;
-  L.image = off; off += pmt_image_bytes(P, C.G); off = (off + 255) & ~(size_t)255;
-  L.partials = off; off += (size_t)PMT_PARTIAL_CTAS * P.d.n_params * sizeof(float);
-  L.scratch = off; off += (size_t)PMT_PARTIAL_CTAS * L.scr_floats * sizeof(float);
-  L.info_seq = off; off += w;
-  L.d_info_seq = off; off += w; off = (off + 255) & ~(size_t)255;
-  L.long_scratch = off; off += (size_t)L.long_grid * L.long_floats * sizeof(float); off = (off + 255) & ~(size_t)255;
-  L.tc_bytes = C.bwd_reads_tc ? C.tc_bwd.total + 1024 : 0;
-  L.tc = off; off += L.tc_bytes; off = (off + 255) & ~(size_t)255;
-  L.cnn_bytes = C.bwd_cnn_tc ? pmt_cnn_bwd_workspace_bytes(C, batch) : 0;
-  L.cnn = off; off += L.cnn_bytes;
-  L.end = off;
-  return L;
-}
-size_t pmt_backward_workspace_size(const CallPlan& C, const PmtBatch* batch) { return backward_layout(C, batch).end; }
-
 extern "C" int pmt_backward_kernels(const PmtModelDesc* desc, int32_t* reads_tc, int32_t* cnn_tc) {
   CallPlan C;
   if (pmt_call_plan(desc, nullptr, false, &C)) return 1;
@@ -1316,33 +1268,27 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
   CallPlan C;
   if (pmt_call_plan(desc, batch, false, &C)) return 1;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const BwdWsLayout L = backward_layout(C, batch);
-  PMT_CHECK(workspace && workspace_bytes >= L.end, "workspace too small: %zu < %zu", workspace_bytes, L.end);
+  BwdBuffers W;
+  if (pmt_backward_buffers(C, workspace, workspace_bytes, &W)) return 1;
   PMT_CHECK(batch->n_variants > 0, "empty batch");
   PMT_CHECK(!C.bwd_refusal[0], "%s", C.bwd_refusal);
 
   const int B = batch->n_variants, w = desc->d_info + desc->d_seq;
-  char* ws = reinterpret_cast<char*>(workspace);
-  float* image = reinterpret_cast<float*>(ws + L.image);
-  float* partials = reinterpret_cast<float*>(ws + L.partials);
-  float* scratch = reinterpret_cast<float*>(ws + L.scratch);
-  float* info_seq = reinterpret_cast<float*>(ws + L.info_seq);
-  float* d_info_seq = reinterpret_cast<float*>(ws + L.d_info_seq);
-  float* long_scratch = reinterpret_cast<float*>(ws + L.long_scratch);
-  unsigned char* tc_ws = reinterpret_cast<unsigned char*>(ws + L.tc);
-  unsigned char* cnn_ws = reinterpret_cast<unsigned char*>(ws + L.cnn);
+  float* image = W.image;
+  float* partials = W.partials;
+  float* info_seq = W.info_seq;
+  float* d_info_seq = W.d_info_seq;
 
-  // what pmt_forward_train saved for this batch (PmtOutGrads.saved), laid out by pmt_saved_layout
-  const unsigned char* saved_tc = nullptr;
-  const float* saved_cnn = nullptr;
-  if (grads && grads->saved) {
+  // what pmt_forward_train saved for this batch (PmtOutGrads.saved); the caller passes the buffer without its size
+  SavedBuffers S;
+  const bool saved = grads && grads->saved;
+  if (saved) {
     PMT_CHECK(C.bwd_reads_tc && C.bwd_cnn_tc && C.mode == PMT_PRECISION_TF32X3 && grads->info_seq_be,
               "PmtOutGrads.saved needs the tf32x3 mode, the forward's info_seq_be, and the precision mode of the forward call");
     PMT_CHECK(C.saved.total > 0, "PmtOutGrads.saved: no saved-forward path for this batch");
-    saved_tc = reinterpret_cast<const unsigned char*>(grads->saved);
-    saved_cnn = reinterpret_cast<const float*>(saved_tc + C.saved.cnn);
+    if (pmt_saved_buffers(C, grads->saved, C.saved.total, &S)) return 1;
   }
-  PMT_CUDA(cudaMemsetAsync(partials, 0, (size_t)PMT_PARTIAL_CTAS * desc->n_params * sizeof(float), st));
+  PMT_CUDA(cudaMemsetAsync(partials, 0, C.bwd.partials.bytes, st));
   // conv images: only the SIMT haplotype-CNN kernels read them (the recompute below when the forward's embeddings are not
   // passed in, and the SIMT backward)
   pmt_launch_prepare(C, weights, image, st, true, !C.bwd_cnn_tc || !(grads && grads->info_seq_be));
@@ -1361,13 +1307,13 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
   A.d_logits_bk = grads ? grads->d_logits_bk : nullptr;
   A.d_alt_means = grads ? grads->d_alt_means_be : nullptr;
   A.d_ref_means = grads ? grads->d_ref_means_be : nullptr;
-  A.d_info_seq = d_info_seq; A.scratch = scratch; A.scratch_stride = (long long)L.scr_floats; A.partials = partials;
-  A.long_scratch = long_scratch; A.long_scratch_stride = (long long)L.long_floats;
+  A.d_info_seq = d_info_seq; A.scratch = W.scratch; A.scratch_stride = (long long)C.bwd.scr_floats; A.partials = partials;
+  A.long_scratch = W.long_scratch; A.long_scratch_stride = (long long)C.bwd.long_floats;
   A.n_claims = C.bwd_claims.n_claims;
   int tc_grid = 0;
   if (C.bwd_reads_tc) {   // tile-sized sets; longer sets always take the SIMT long-set kernel
-    if (pmt_launch_reads_tc_backward(C, weights, batch, info_seq, A.d_logits_bk, A.d_alt_means, A.d_ref_means, d_info_seq, tc_ws,
-                                     L.tc_bytes, &tc_grid, st, saved_tc))
+    if (pmt_launch_reads_tc_backward(C, weights, batch, info_seq, A.d_logits_bk, A.d_alt_means, A.d_ref_means, d_info_seq, W.tc,
+                                     &tc_grid, st, saved ? &S : nullptr))
       return 1;
   } else {
     PMT_CUDA(cudaFuncSetAttribute(reads_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1375,9 +1321,9 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
     reads_backward_kernel<<<C.bwd_claims.grid, NTHREADS, smem, st>>>(P, A);
     pmt_profile_end(st);
   }
-  if (L.long_grid > 0) {   // sets longer than a tile; same CTA-private gradient buffers, after the tile kernel: fixed order
+  if (C.bwd.long_grid > 0) {   // sets longer than a tile; same CTA-private gradient buffers, after the tile kernel: fixed order
     PMT_CUDA(cudaFuncSetAttribute(reads_backward_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    reads_backward_long_kernel<<<L.long_grid, NTHREADS, smem, st>>>(P, A);
+    reads_backward_long_kernel<<<C.bwd.long_grid, NTHREADS, smem, st>>>(P, A);
   }
   {
     const size_t ismem = C.info_bwd_smem;
@@ -1385,16 +1331,16 @@ extern "C" int pmt_backward(const PmtModelDesc* desc, const float* weights, cons
     const int igrid = n_tiles < PMT_PARTIAL_CTAS ? n_tiles : PMT_PARTIAL_CTAS;
     PMT_CUDA(cudaFuncSetAttribute(info_mlp_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ismem));
     info_mlp_backward_kernel<<<igrid, NTHREADS, ismem, st>>>(P, weights, image, batch->info, batch->info_kind,
-                                                             batch->info_stride, B, d_info_seq, scratch,
-                                                             (long long)L.scr_floats, partials, info_rows(P));
+                                                             batch->info_stride, B, d_info_seq, W.scratch,
+                                                             (long long)C.bwd.scr_floats, partials, info_rows(P));
   }
   if (C.bwd_cnn_tc) {
-    if (pmt_launch_cnn_backward_mma(C, weights, batch, info_seq, d_info_seq, partials, cnn_ws, L.cnn_bytes, st, saved_cnn)) return 1;
+    if (pmt_launch_cnn_backward_mma(C, weights, batch, info_seq, d_info_seq, partials, W.cnn, st, saved ? S.cnn : nullptr)) return 1;
   } else if (launch_cnn_backward(C, weights, image, batch, d_info_seq, partials, st)) {
     return 1;
   }
   reduce_partials_kernel<<<(desc->n_params + 255) / 256, 256, 0, st>>>(partials, PMT_PARTIAL_CTAS, desc->n_params, d_weights);
-  if (C.bwd_reads_tc && pmt_finish_reads_tc_backward(C, weights, d_weights, tc_ws, tc_grid, st)) return 1;
+  if (C.bwd_reads_tc && pmt_finish_reads_tc_backward(C, weights, d_weights, W.tc, tc_grid, st)) return 1;
   if (P.n_skipfix > 0) skip_fix_kernel<<<P.n_skipfix, 256, 0, st>>>(P, weights, d_weights);
   cudaError_t e = cudaGetLastError();
   PMT_CHECK(e == cudaSuccess, "pmt_backward launch failed: %s", cudaGetErrorString(e));

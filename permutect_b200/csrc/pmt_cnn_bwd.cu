@@ -460,18 +460,8 @@ bool pmt_build_cnn_bwd_plan(const pmt::Plan& P, const cnntc::Plan& T, BPlan* out
   return false;
 }
 
-static const int kCnnBwdChunk = 65536;   // variants per recompute + backward pair: bounds the saved activations (5.3 KB per variant)
-
-// [forward weight images (the recompute)][data-gradient images][saved activations of one chunk]
-size_t pmt_cnn_bwd_workspace_bytes(const CallPlan& C, const PmtBatch* batch) {
-  if (!C.cnn_bwd_ok) return 0;
-  const int n = batch ? (batch->n_variants < kCnnBwdChunk ? batch->n_variants : kCnnBwdChunk) : kCnnBwdChunk;
-  const size_t groups = ((size_t)n + C.C.G - 1) / C.C.G;
-  return pmt_cnn_tc_image_bytes(C) + 256 + (size_t)C.CB.img_total * sizeof(float) + 256 + groups * C.CB.group_floats * sizeof(float) + 1024;
-}
-
 // the training forward runs the SAVE variant over the whole batch (pmt_forward_train); `save`: the CNN part of the saved
-// buffer (pmt_saved_layout)
+// buffer
 int pmt_cnn_forward_train(const CallPlan& C, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
                           float* save, cudaStream_t st) {
   if (pmt_pack_cnn_tc_images(C.P, C.C, weights, image, st)) return 1;
@@ -479,31 +469,27 @@ int pmt_cnn_forward_train(const CallPlan& C, const float* weights, const PmtBatc
 }
 
 int pmt_launch_cnn_backward_mma(const CallPlan& C, const float* weights, const PmtBatch* batch, float* info_seq, const float* d_info_seq,
-                                float* partials, unsigned char* ws, size_t ws_bytes, cudaStream_t st, const float* saved) {
+                                float* partials, const CnnBwdBuffers& W, cudaStream_t st, const float* saved) {
   const pmt::Plan& P = C.P;
   const cnntc::Plan& T = C.C;
   const BPlan& B = C.CB;
-  PMT_CHECK(ws_bytes >= pmt_cnn_bwd_workspace_bytes(C, batch), "CNN backward workspace too small");
-  unsigned char* p = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~uintptr_t(255));
-  unsigned char* fwd_image = p; p += (pmt_cnn_tc_image_bytes(C) + 255) & ~size_t(255);
-  float* bwd_image = reinterpret_cast<float*>(p); p += ((size_t)B.img_total * sizeof(float) + 255) & ~size_t(255);
-  float* save = reinterpret_cast<float*>(p);
+  float* save = W.save;
   // weight images: the forward's (split precision; only for the recompute) and the data gradient's
-  if (!saved && pmt_pack_cnn_tc_images(P, T, weights, fwd_image, st)) return 1;
-  pack_cnn_bwd_kernel<<<dim3(B.n_layers, 8), 256, 0, st>>>(B, weights, bwd_image);
+  if (!saved && pmt_pack_cnn_tc_images(P, T, weights, W.fwd_image, st)) return 1;
+  pack_cnn_bwd_kernel<<<dim3(B.n_layers, 8), 256, 0, st>>>(B, weights, W.bwd_image);
   PMT_CUDA(cudaFuncSetAttribute(cnn_backward_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, B.smem_bytes));
   const int out_w = P.d.d_info + P.d.d_seq;
   const size_t esz = batch->hap_kind == PMT_I64 ? 8 : 2;
-  const int chunk = saved ? batch->n_variants : kCnnBwdChunk;   // saved by the training forward: the whole batch at once
+  const int chunk = saved ? batch->n_variants : PMT_CNN_BWD_CHUNK;   // saved by the training forward: the whole batch at once
   for (int v_first = 0; v_first < batch->n_variants; v_first += chunk) {
     const int n = batch->n_variants - v_first < chunk ? batch->n_variants - v_first : chunk;
     if (saved) save = const_cast<float*>(saved);
-    else if (pmt_launch_cnn_tc_save(P, T, weights, batch, v_first, n, info_seq, fwd_image, save, C.n_sm, st)) return 1;
+    else if (pmt_launch_cnn_tc_save(P, T, weights, batch, v_first, n, info_seq, W.fwd_image, save, C.n_sm, st)) return 1;
     const int n_groups = (n + B.VT - 1) / B.VT;
     int grid = n_groups < C.n_sm ? n_groups : C.n_sm;
     if (grid > PMT_PARTIAL_CTAS) grid = PMT_PARTIAL_CTAS;
     const void* haps = reinterpret_cast<const unsigned char*>(batch->haplotypes) + (size_t)v_first * batch->hap_stride * esz;
-    cnn_backward_mma_kernel<<<grid, THREADS, B.smem_bytes, st>>>(B, bwd_image, haps, batch->hap_kind, batch->hap_stride, n, save,
+    cnn_backward_mma_kernel<<<grid, THREADS, B.smem_bytes, st>>>(B, W.bwd_image, haps, batch->hap_kind, batch->hap_stride, n, save,
                                                                  info_seq + (size_t)v_first * out_w, d_info_seq + (size_t)v_first * out_w, out_w,
                                                                  P.d.d_info, partials, P.d.n_params);
   }

@@ -851,14 +851,6 @@ size_t pmt_cnn_tc_image_bytes(const CallPlan& C) {
   return (C.cnn_split ? (size_t)C.CT.image_off + C.CT.image_bytes : (size_t)C.C.image_bytes) + 256;
 }
 
-size_t pmt_cnn_tail_buffer_bytes(const CallPlan& C, int n_variants) {
-  // Sized whenever the CNN has a tail and inference runs a tensor-core CNN, even where the plan chose the single kernel:
-  // sizing for C.cnn == TC_TAIL alone would shrink pmt_workspace_size below the pair's batch-size threshold, and the
-  // sizes the library reports stay as they were.
-  const bool tc = C.cnn == CnnKernel::TC || C.cnn == CnnKernel::TC_TAIL;
-  return C.cnn_split && tc ? (size_t)(n_variants + 127) / 128 * 128 * C.CT.K0 * sizeof(float) : 0;
-}
-
 template <int PASSES, bool SAVE>
 static int launch_cnn_tc(const cnntc::Plan& T, const unsigned char* image, const float* weights, const PmtModelDesc& D, const void* haps,
                          const PmtBatch* batch, int n, float* info_seq, const SaveLayout& SL, float* save, int grid, cudaStream_t st,
@@ -913,9 +905,11 @@ static int launch_cnn_tail(const TailPlan& TT, const unsigned char* image, const
   return 0;
 }
 
-// `image` is a 16-byte aligned device buffer of pmt_cnn_tc_image_bytes(C) bytes.
-int pmt_launch_cnn_tc(const CallPlan& C, const float* weights, const PmtBatch* batch, float* info_seq, unsigned char* image,
-                      bool reuse_image, float* tail_buf, cudaStream_t st) {
+// W.cnn_tc_image: the weight images (16-byte aligned); W.cnn_tail: the head kernel's output to the tail kernel
+int pmt_launch_cnn_tc(const CallPlan& C, const float* weights, const PmtBatch* batch, float* info_seq, const FwdBuffers& W,
+                      bool reuse_image, cudaStream_t st) {
+  unsigned char* image = W.cnn_tc_image;
+  float* tail_buf = W.cnn_tail;
   if (!reuse_image) {   // both forms' images, so that a prepared call finds whichever it runs
     pack_cnn_tc_kernel<<<dim3(C.C.n_layers, 16), 256, 0, st>>>(C.P.d, C.C, weights, image);
     if (C.cnn_split) pack_cnn_tail_kernel<<<dim3(C.CT.n_layers, 16), 256, 0, st>>>(C.P.d, C.CT, weights, image + C.CT.image_off);

@@ -897,47 +897,8 @@ int pmt_call_plan(const PmtModelDesc* desc, const PmtBatch* batch, bool train, C
                                                                               : "";
     snprintf(C.bwd_refusal, sizeof(C.bwd_refusal), "%s", bwd_why);
   }
+  pmt_plan_workspaces(C, batch);
   return 0;
-}
-
-// long-set scratch of the FP32 kernel: per CTA, one (x, z) image pair per chunk of the longest variant
-static size_t long_scratch_floats_per_cta(const Plan& P, const PmtBatch* batch) {
-  const size_t chunks = (size_t)((batch->max_rows_per_variant + 3 + TILE - 1) / TILE) + 1;
-  return chunks * (size_t)(P.d.d_model + P.d.d_ffn) * LD;
-}
-
-// Workspace layout of the forward: the packed weight images sit at FIXED offsets from the base (they depend on the model
-// only: pmt_forward_prepared finds them there), the batch-dependent regions follow:
-//   [256 B counters][SIMT images][tcgen05 read-kernel images][tcgen05 CNN images] | [info_seq][long-set scratch]
-//   [tile list, or the training forward's planner scratch][long-set tensor-core region][CNN tail buffer]
-struct FwdLayout {
-  size_t image, tc_image, cnn_tc_image, info_seq, long_scratch, tiles, long_tc, cnn_tail, end;
-};
-static FwdLayout forward_layout(const CallPlan& C, const PmtBatch* batch) {
-  const int B = batch ? batch->n_variants : 0;
-  FwdLayout L;
-  size_t off = 256;
-  L.image = off; off += pmt_image_bytes(C.P, C.G); off = (off + 1023) & ~(size_t)1023;
-  L.tc_image = off; off += (size_t)C.T.image_bytes + 2048; off = (off + 255) & ~(size_t)255;
-  L.cnn_tc_image = off; off += pmt_cnn_tc_image_bytes(C); off = (off + 255) & ~(size_t)255;
-  L.info_seq = off; off += (size_t)B * (C.P.d.d_info + C.P.d.d_seq) * sizeof(float); off = (off + 255) & ~(size_t)255;
-  L.long_scratch = off;
-  if (C.lng == LongKernel::SIMT) off += long_scratch_floats_per_cta(C.P, batch) * sizeof(float) * PMT_PARTIAL_CTAS;
-  off = (off + 255) & ~(size_t)255;
-  size_t tiles = pmt_tc_tiles_bytes(B);
-  const size_t claims = C.saved.total > 0 ? pmt_plan_claim_bytes(B, PMT_PARTIAL_CTAS) : 0;   // the training forward's planner
-  if (claims > tiles) tiles = claims;
-  L.tiles = off; off += tiles; off = (off + 255) & ~(size_t)255;
-  L.long_tc = off; off += C.lng == LongKernel::TC ? C.long_tc.end : 0; off = (off + 255) & ~(size_t)255;
-  L.cnn_tail = off; off += pmt_cnn_tail_buffer_bytes(C, B);
-  L.end = off + 1024;
-  return L;
-}
-
-extern "C" size_t pmt_workspace_size(const PmtModelDesc* desc, const PmtBatch* batch, int for_backward) {
-  CallPlan C;
-  if (pmt_call_plan(desc, batch, false, &C)) return 0;
-  return for_backward ? pmt_backward_workspace_size(C, batch) : forward_layout(C, batch).end;
 }
 
 int pmt_launch_prepare(const CallPlan& C, const float* weights, float* image, cudaStream_t st, bool gemm, bool conv) {
@@ -990,50 +951,41 @@ int pmt_launch_hap_cnn_simt(const CallPlan& C, const float* weights, const float
   return 0;
 }
 
-extern "C" size_t pmt_train_saved_bytes(const PmtModelDesc* desc, const PmtBatch* batch) {
-  CallPlan C;
-  if (pmt_call_plan(desc, batch, true, &C)) return 0;
-  return C.saved.total;
-}
-
 static int forward_impl(const PmtModelDesc* desc, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
                         void* workspace, size_t workspace_bytes, void* stream, bool reuse_images, unsigned char* saved = nullptr,
                         size_t saved_bytes = 0) {
   CallPlan C;
   if (pmt_call_plan(desc, batch, saved != nullptr, &C)) return 1;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  const FwdLayout L = forward_layout(C, batch);
-  PMT_CHECK(workspace && workspace_bytes >= L.end, "workspace too small: %zu < %zu", workspace_bytes, L.end);
+  FwdBuffers W;
+  if (pmt_forward_buffers(C, workspace, workspace_bytes, &W)) return 1;
   PMT_CHECK(batch->n_variants > 0, "empty batch");
   PMT_CHECK(!C.fwd_refusal[0], "%s", C.fwd_refusal);
+  SavedBuffers S{};
   if (saved) {
     PMT_CHECK(C.saved.total > 0 && saved_bytes >= C.saved.total,
               "pmt_forward_train: no saved-forward path for this call or buffer too small (%zu < %zu)", saved_bytes, C.saved.total);
     PMT_CHECK((reinterpret_cast<uintptr_t>(saved) & 255) == 0, "pmt_forward_train: the saved buffer must be 256-byte aligned");
+    if (pmt_saved_buffers(C, saved, saved_bytes, &S)) return 1;
   }
-  char* ws = reinterpret_cast<char*>(workspace);
-  int* counter = reinterpret_cast<int*>(ws);
-  float* image = reinterpret_cast<float*>(ws + L.image);
-  float* info_seq = out->info_seq_be;
-  if (!info_seq) info_seq = reinterpret_cast<float*>(ws + L.info_seq);
-  PMT_CUDA(cudaMemsetAsync(counter, 0, 256, st));
+  float* image = W.image;
+  float* info_seq = out->info_seq_be ? out->info_seq_be : W.info_seq;
+  PMT_CUDA(cudaMemsetAsync(W.counters, 0, C.fwd.counters.bytes, st));
   {
     // a prepared call finds the images of the model; the FP32 long-set kernel's depend on the batch
     const bool simt_long = C.lng == LongKernel::SIMT;
     if (!reuse_images) pmt_launch_prepare(C, weights, image, st, C.simt_gemm || simt_long, C.simt_conv);
     else if (simt_long && !C.simt_gemm) pmt_launch_prepare(C, weights, image, st, true, false);
   }
-  unsigned char* tc_image = reinterpret_cast<unsigned char*>(ws + L.tc_image);
-  unsigned char* cnn_tc_image = reinterpret_cast<unsigned char*>(ws + L.cnn_tc_image);
   // per-variant embeddings: the info MLP, then the haplotype CNN (in training its SAVE variant: same results, activations kept)
   if (pmt_launch_info_mlp(C, weights, image, batch, info_seq, st)) return 1;
   switch (C.cnn) {
     case CnnKernel::TC:
     case CnnKernel::TC_TAIL:
-      if (pmt_launch_cnn_tc(C, weights, batch, info_seq, cnn_tc_image, reuse_images, reinterpret_cast<float*>(ws + L.cnn_tail), st)) return 1;
+      if (pmt_launch_cnn_tc(C, weights, batch, info_seq, W, reuse_images, st)) return 1;
       break;
     case CnnKernel::TC_SAVE:
-      if (pmt_cnn_forward_train(C, weights, batch, info_seq, cnn_tc_image, reinterpret_cast<float*>(saved + C.saved.cnn), st)) return 1;
+      if (pmt_cnn_forward_train(C, weights, batch, info_seq, W.cnn_tc_image, S.cnn, st)) return 1;
       break;
     case CnnKernel::SIMT:
       if (pmt_launch_hap_cnn_simt(C, weights, image, batch, info_seq, st)) return 1;
@@ -1043,7 +995,7 @@ static int forward_impl(const PmtModelDesc* desc, const float* weights, const Pm
   Plan P = C.P;
   P.claim_variants = C.fwd_claims.claim;
   ReadKernelArgs A;
-  A.wflat = weights; A.image = image; A.batch = *batch; A.out = *out; A.out.info_seq_be = info_seq; A.claim_counter = counter;
+  A.wflat = weights; A.image = image; A.batch = *batch; A.out = *out; A.out.info_seq_be = info_seq; A.claim_counter = W.counters;
   A.scratch = nullptr; A.scratch_stride = 0;
   const size_t smem = C.reads_smem;
   PMT_CUDA(cudaFuncSetAttribute(reads_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1055,17 +1007,17 @@ static int forward_impl(const PmtModelDesc* desc, const float* weights, const Pm
     pmt_profile_end(st);
   } else {
     if (C.reads == ReadsKernel::TC_SAVE) {   // deterministic tile list + the SAVE variant of the read kernel, operands kept for the backward
-      if (pmt_tc_forward_train(C, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.tiles), saved, st)) return 1;
-    } else if (pmt_launch_reads_tc(C, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.tiles), reuse_images, st)) {
+      if (pmt_tc_forward_train(C, weights, batch, &o2, W, S, st)) return 1;
+    } else if (pmt_launch_reads_tc(C, weights, batch, &o2, W, reuse_images, st)) {
       return 1;
     }
   }
   if (C.lng == LongKernel::TC) {
     // sets longer than a tile, cut into single-side tiles on the same tensor-core pipeline (pmt_tc.cuh: LongTile)
-    if (pmt_launch_reads_tc_long(C, weights, batch, &o2, tc_image, reinterpret_cast<unsigned char*>(ws + L.long_tc), st)) return 1;
+    if (pmt_launch_reads_tc_long(C, weights, batch, &o2, W, st)) return 1;
   } else if (C.lng == LongKernel::SIMT) {
-    A.scratch = reinterpret_cast<float*>(ws + L.long_scratch);
-    A.scratch_stride = (long long)long_scratch_floats_per_cta(P, batch);
+    A.scratch = W.long_scratch;
+    A.scratch_stride = (long long)C.fwd.long_scratch_floats;
     PMT_CUDA(cudaFuncSetAttribute(reads_forward_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     reads_forward_long_kernel<<<C.fwd_long_grid, NTHREADS, smem, st>>>(P, A);
   }

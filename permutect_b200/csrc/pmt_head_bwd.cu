@@ -228,7 +228,7 @@ extern "C" int pmt_head_backward(const PmtModelDesc* desc, const float* weights,
   if (grid > PMT_PARTIAL_CTAS) grid = PMT_PARTIAL_CTAS;
   const int per_cta = (B + grid - 1) / grid;
   grid = (B + per_cta - 1) / per_cta;
-  float* partials = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
+  float* partials = reinterpret_cast<float*>(pmt_align_up(workspace, 256));
   PMT_CUDA(cudaMemsetAsync(d_weights, 0, (size_t)desc->n_params * sizeof(float), st));
   headbwd::head_backward_kernel<<<grid, headbwd::THREADS, 0, st>>>(
       *desc, weights, batch->ref_off, batch->alt_off, B, final_re, grads ? grads->d_logits_bk : nullptr,

@@ -24,6 +24,12 @@ void pmt_set_error(const char* fmt, ...);
     }                                                                                         \
   } while (0)
 
+// The first address at or after `p` that is a multiple of `align` (a power of two): the C-ABI does not require aligned
+// buffers, so regions that a kernel needs aligned are realigned inside the caller's buffer.
+inline unsigned char* pmt_align_up(void* p, size_t align) {
+  return reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(p) + align - 1) & ~(uintptr_t)(align - 1));
+}
+
 // A set occupies pad4(ref rows) + alt rows of a tile, so a set of up to TILE - 3 rows always fits in one tile; anything
 // longer MAY be left to the long-set kernels by build_tile / plan_tiles_kernel (which then do nothing if it did fit).
 inline bool pmt_has_long_sets(const PmtBatch* batch) { return batch->max_rows_per_variant + 3 > PMT_TILE_ROWS; }

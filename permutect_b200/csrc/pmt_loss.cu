@@ -399,7 +399,7 @@ extern "C" int pmt_losses_backward(const PmtLossDesc* desc, const float* weights
   B.a.d = *desc; B.a.b = *batch; B.a.wflat = weights;
   B.g = *grads;
   B.d_logits_b = d_logits_b; B.d_outlier_logits_b = d_outlier_logits_b; B.d_features_be = d_features_be;
-  B.partials = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
+  B.partials = reinterpret_cast<float*>(pmt_align_up(workspace, 256));
   const int grid = loss_grid(batch->n_variants);
   const size_t smem = (size_t)(2 * (na + ns) + 8 + (2 * MAXW + 1) * NTP) * sizeof(float);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);

@@ -84,7 +84,7 @@ extern "C" int pmt_adamw_step(float* params, const float* grads, float* exp_avg,
   PMT_CHECK(params && grads && exp_avg && exp_avg_sq && step_count && n > 0, "pmt_adamw_step: bad arguments");
   PMT_CHECK(workspace && workspace_bytes >= pmt_adamw_workspace_size(), "pmt_adamw_step: workspace too small");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  float* partials = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
+  float* partials = reinterpret_cast<float*>(pmt_align_up(workspace, 256));
   grad_sqnorm_kernel<<<NORM_CTAS, NT, 0, st>>>(grads, mask, n, partials);
   AdamArgs A;
   A.param = params; A.grad = grads; A.exp_avg = exp_avg; A.exp_avg_sq = exp_avg_sq; A.mask = mask; A.partials = partials;

@@ -1354,11 +1354,6 @@ void pmt_tc_plan(const Plan& P, TcPlan* out) {
   T.part_floats = pad_to(part + 8 * SCAL_W, 64);
 }
 
-static size_t perm_bytes(int n_variants) { return ((size_t)n_variants * sizeof(int) + 255) & ~(size_t)255; }
-
-// the inference tile list and the packed planner's variant order
-size_t pmt_tc_tiles_bytes(int n_variants) { return pmt_tile_list_bytes(n_variants) + perm_bytes(n_variants) + 256; }
-
 int pmt_plan_claim_variants(int n_variants, int n_sm) {
   // planner claims: large enough that the partial last tile of a claim is a small loss, small enough that a small
   // batch is planned by many warps (each claim is walked sequentially)
@@ -1421,17 +1416,16 @@ int pmt_launch_reads_tc_save(const CallPlan& C, const TcArgs& A, int grid, cudaS
   return launch_reads_tc<3, true, false>(C.P.d, C.T, A, grid, C.ring_save, st);
 }
 
-// Launches the tile planner, the weight packer (unless the images in `image_buf` are still valid) and the tensor-core
-// read kernel.  `image_buf`: the forward layout's tc_image region; `tiles_buf`: pmt_tc_tiles_bytes(B) bytes.
+// Launches the tile planner, the weight packer (unless the images in W.tc_image are still valid) and the tensor-core
+// read kernel.
 int pmt_launch_reads_tc(const CallPlan& C, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
-                        unsigned char* image_buf, unsigned char* tiles_buf, bool reuse_images, cudaStream_t st) {
+                        const FwdBuffers& W, bool reuse_images, cudaStream_t st) {
   const TcPlan& T = C.T;
-  unsigned char* image = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(image_buf) + 1023) & ~uintptr_t(1023));
-  int* tiles = reinterpret_cast<int*>((reinterpret_cast<uintptr_t>(tiles_buf) + 255) & ~uintptr_t(255));
+  unsigned char* image = W.tc_image;
+  int* tiles = W.tiles;
+  int* perm = W.perm;
   int n_claims = 0;
-  int* perm = nullptr;
   if (C.packed_planner) {
-    perm = reinterpret_cast<int*>(reinterpret_cast<unsigned char*>(tiles) + pmt_tile_list_bytes(batch->n_variants));
     n_claims = (batch->n_variants + PLAN_CLAIM - 1) / PLAN_CLAIM;
     PMT_CUDA(cudaMemsetAsync(tiles, 0, 2 * sizeof(int), st));
     plan_tiles_packed_kernel<<<(n_claims + 3) / 4, 128, 0, st>>>(reinterpret_cast<const long long*>(batch->ref_off),
@@ -1454,64 +1448,31 @@ int pmt_launch_reads_tc(const CallPlan& C, const float* weights, const PmtBatch*
 }
 
 // ---- sets longer than a tile (pmt_tc.cuh: LongTile) ----
-// false: the long-set tensor-core path is not available for this batch (no long sets, unknown row count, or a set longer
-// than one round of tiles) -- the FP32 long-set kernel takes them.
-bool pmt_tc_long_layout(const Plan& P, const PmtBatch* batch, int n_sm, LongLayout* L) {
-  if (!batch || !pmt_has_long_sets(batch) || batch->n_rows <= 0 || !pmt_tc_supported(P)) return false;
-  const int R = 2 * n_sm;
-  const long long t_max = (batch->max_rows_per_variant + TILE - 1) / TILE + 1;        // ceil per side
-  if (t_max > R) return false;
-  long long cap = batch->n_rows / (TILE - 2);
-  if (cap > batch->n_variants) cap = batch->n_variants;
-  if (cap < 1) cap = 1;
-  const long long sum_t = batch->n_rows / TILE + 2 * cap;
-  const long long rounds = sum_t / (R - t_max + 1) + 1;
-  const long long max_tiles = sum_t + rounds * (t_max - 1) + R;
-  if (max_tiles > 0x3fffffff) return false;
-  L->cap = (int)cap; L->max_tiles = (int)max_tiles; L->R = R;
-  size_t off = 0;
-  auto take = [&](size_t bytes) { const size_t o = off; off += (bytes + 255) & ~(size_t)255; return o; };
-  L->list = take((size_t)(1 + cap) * sizeof(int));
-  L->n_tiles = take(256);
-  L->tiles = take((size_t)max_tiles * sizeof(LongTile));
-  L->counters = take((size_t)max_tiles * P.d.n_blocks * sizeof(int));
-  L->fin_cnt = take((size_t)max_tiles * sizeof(int));
-  L->counters_bytes = off - L->counters;
-  L->mf_part = take((size_t)max_tiles * P.d.n_blocks * MAXH * sizeof(float));
-  L->fin_part = take((size_t)max_tiles * LONG_FIN_W * sizeof(float));
-  L->end = off + 1024;
-  return true;
-}
-
-// The sets plan_tiles_kernel left out, on the same tensor-core pipeline (the weight images in `image_buf` must be packed:
+// The sets plan_tiles_kernel left out, on the same tensor-core pipeline (the weight images in W.tc_image must be packed:
 // call after pmt_launch_reads_tc).  Every CTA of the grid has to be resident (a tile waits for the other tiles of its
 // set): one CTA per SM, grid = number of SMs.
 int pmt_launch_reads_tc_long(const CallPlan& C, const float* weights, const PmtBatch* batch, const PmtOutputs* out,
-                             unsigned char* image_buf, unsigned char* long_buf, cudaStream_t st) {
+                             const FwdBuffers& W, cudaStream_t st) {
   const LongLayout& L = C.long_tc;
-  unsigned char* image = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(image_buf) + 1023) & ~uintptr_t(1023));
-  unsigned char* base = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(long_buf) + 255) & ~uintptr_t(255));
-  int* list = reinterpret_cast<int*>(base + L.list);
-  int* n_tiles = reinterpret_cast<int*>(base + L.n_tiles);
-  LongTile* tiles = reinterpret_cast<LongTile*>(base + L.tiles);
+  const LongBuffers& LB = W.lng;
   const long long* ro = reinterpret_cast<const long long*>(batch->ref_off);
   const long long* ao = reinterpret_cast<const long long*>(batch->alt_off);
-  PMT_CUDA(cudaMemsetAsync(list, 0, sizeof(int), st));
-  PMT_CUDA(cudaMemsetAsync(tiles, 0xFF, (size_t)L.max_tiles * sizeof(LongTile), st));
-  PMT_CUDA(cudaMemsetAsync(base + L.counters, 0, L.counters_bytes, st));
+  PMT_CUDA(cudaMemsetAsync(LB.list, 0, sizeof(int), st));
+  PMT_CUDA(cudaMemsetAsync(LB.tiles, 0xFF, (size_t)L.max_tiles * sizeof(LongTile), st));
+  PMT_CUDA(cudaMemsetAsync(LB.counters, 0, L.counters.bytes, st));
   int blocks = (batch->n_variants + 255) / 256;
   if (blocks > 4 * C.n_sm) blocks = 4 * C.n_sm;
-  long_list_kernel<<<blocks, 256, 0, st>>>(ro, ao, batch->n_variants, L.cap, list);
-  long_layout_kernel<<<1, 1024, 0, st>>>(ro, ao, list, L.cap, L.R, L.max_tiles, tiles, n_tiles);
+  long_list_kernel<<<blocks, 256, 0, st>>>(ro, ao, batch->n_variants, L.cap, LB.list);
+  long_layout_kernel<<<1, 1024, 0, st>>>(ro, ao, LB.list, L.cap, L.R, L.max_tiles, LB.tiles, LB.n_tiles);
   TcArgs A;
   memset(&A, 0, sizeof(A));
-  A.wflat = weights; A.image = image; A.tiles = nullptr; A.batch = *batch; A.out = *out;
+  A.wflat = weights; A.image = W.tc_image; A.tiles = nullptr; A.batch = *batch; A.out = *out;
   A.scratch = nullptr; A.tile_first = 0; A.tile_limit = 0x7fffffff;
-  A.lng.tiles = tiles; A.lng.n_tiles = n_tiles;
-  A.lng.mf_cnt = reinterpret_cast<int*>(base + L.counters);
-  A.lng.fin_cnt = reinterpret_cast<int*>(base + L.fin_cnt);
-  A.lng.mf_part = reinterpret_cast<float*>(base + L.mf_part);
-  A.lng.fin_part = reinterpret_cast<float*>(base + L.fin_part);
+  A.lng.tiles = LB.tiles; A.lng.n_tiles = LB.n_tiles;
+  A.lng.mf_cnt = LB.counters;
+  A.lng.fin_cnt = LB.fin_cnt;
+  A.lng.mf_part = LB.mf_part;
+  A.lng.fin_part = LB.fin_part;
   const int grid = L.R / 2;
   return C.passes == 1 ? launch_reads_tc<1, false, true>(C.P.d, C.T, A, grid, C.ring, st)
                        : launch_reads_tc<3, false, true>(C.P.d, C.T, A, grid, C.ring, st);

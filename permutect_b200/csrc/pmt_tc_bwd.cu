@@ -822,21 +822,7 @@ __global__ void unfold_kernel(const __grid_constant__ PmtModelDesc D, const __gr
 using namespace pmt;
 using namespace pmt::tc;
 
-// Tiles per recompute / backward pass: bounds the operand scratch (0.7 MB per tile: 5.9 GB).  The scratch is streamed through
-// HBM either way (it never was L2-sized), so fewer, longer passes only save launches -- the tile bound is an upper bound and most
-// passes beyond the first found nothing to do -- and the partly filled last round of every pass.
-static const int kChunkTiles = 8192;
-// measured: 9 GB (65 536 variants) wins 14 %, 27 GB (200 000) loses to the recompute
-static const size_t kTrainSavedBudget = (size_t)16 << 30;
-static const unsigned kTrainSavedMagic = 0x544d5031u;
-
-// claims of the training tile list (planned with PMT_PARTIAL_CTAS for the SM count, whatever the device)
-static int train_claims(int n_variants) {
-  const int cv = pmt_plan_claim_variants(n_variants, PMT_PARTIAL_CTAS);
-  return n_variants > 0 ? (n_variants + cv - 1) / cv : 0;
-}
-
-static long long tile_bound(const PmtBatch* batch, int n_claims) {
+long long pmt_train_tile_bound(const PmtBatch* batch, int n_claims) {
   // without a row count (n_rows <= 0) nothing bounds the rows per variant: a training tile holds at least one whole set
   if (batch->n_rows <= 0) return batch->n_variants < 1 ? 1 : batch->n_variants;
   const long long rows = batch->n_rows;
@@ -852,43 +838,7 @@ static long long tile_bound(const PmtBatch* batch, int n_claims) {
   return bound < 1 ? 1 : bound;
 }
 
-BwdLayout pmt_tc_bwd_layout(const TcPlan& T, const PmtBatch* batch, int max_chunk_tiles) {
-  BwdLayout L;
-  memset(&L, 0, sizeof(L));
-  const int B = batch ? batch->n_variants : 0;
-  size_t off = 1024;
-  L.image_f = off; off += (size_t)T.image_bytes + 2048;
-  L.image_t = off; off += (size_t)T.t_image_bytes + 2048;
-  L.tiles = off; off += pmt_tile_list_bytes(B) + 256;
-  L.claims = off; off += pmt_plan_claim_bytes(B, PMT_PARTIAL_CTAS) + 256;
-  L.partials = off; off += (size_t)2 * PMT_PARTIAL_CTAS * T.part_floats * sizeof(float);
-  L.reduced = off; off += (size_t)T.part_floats * sizeof(float) + 256;
-  off = (off + 1023) & ~(size_t)1023;
-  L.n_claims = train_claims(B);
-  const long long bound = batch ? tile_bound(batch, L.n_claims) : 1;
-  const int chunk_cap = max_chunk_tiles >= 1 ? max_chunk_tiles : kChunkTiles;
-  L.chunk_tiles = (int)(bound < chunk_cap ? bound : chunk_cap);
-  L.n_chunks = (int)((bound + L.chunk_tiles - 1) / L.chunk_tiles);
-  L.scratch = off; off += (size_t)L.chunk_tiles * T.tile_bytes;
-  L.total = off + 1024;
-  return L;
-}
-
-SavedLayout pmt_saved_layout(const CallPlan& C, const PmtBatch* batch) {
-  SavedLayout S;
-  memset(&S, 0, sizeof(S));
-  if (C.mode != PMT_PRECISION_TF32X3 || !batch || batch->n_variants <= 0 || !C.bwd_reads_tc || !C.bwd_cnn_tc) return S;
-  const int B = batch->n_variants;
-  S.bound = tile_bound(batch, train_claims(B));
-  S.tiles = 256;
-  S.scratch = (S.tiles + pmt_tile_list_bytes(B) + 256 + 1023) & ~(size_t)1023;
-  S.cnn = (S.scratch + (size_t)S.bound * C.T.tile_bytes + 1024 + 1023) & ~(size_t)1023;
-  const size_t total = S.cnn + ((size_t)B + C.C.G - 1) / C.C.G * C.CB.group_floats * sizeof(float) + 256 + 1024;
-  if (total <= kTrainSavedBudget) S.total = total;
-  return S;
-}
-
-// The operand scratch is sized from an upper bound of the tile count (tile_bound): should the planner ever produce more
+// The operand scratch is sized from an upper bound of the tile count (pmt_train_tile_bound): should the planner ever produce more
 // tiles than that, fail loudly instead of writing past the buffer.
 __global__ void check_tile_bound_kernel(const int* __restrict__ tiles, int bound) {
   if (tiles[0] > bound) {
@@ -910,26 +860,21 @@ Ring pmt_tc_bwd_ring(const TcPlan& T) {
 }
 
 // The training forward of the tile-sized sets: deterministic tile list, then the SAVE variant of the read kernel over ALL
-// tiles with the outputs switched on.  `image_buf`: the forward layout's tc_image region (weight images, packed here);
-// `claim_buf`: the forward layout's planner scratch.
-int pmt_tc_forward_train(const CallPlan& C, const float* weights, const PmtBatch* batch, const PmtOutputs* out, unsigned char* image_buf,
-                         unsigned char* claim_buf, unsigned char* saved, cudaStream_t st) {
+// tiles with the outputs switched on: the weight images are packed into W.tc_image, the tile list and the operands go to
+// the saved buffer.
+int pmt_tc_forward_train(const CallPlan& C, const float* weights, const PmtBatch* batch, const PmtOutputs* out, const FwdBuffers& W,
+                         const SavedBuffers& S, cudaStream_t st) {
   const TcPlan& T = C.T;
-  const SavedLayout& S = C.saved;
-  unsigned char* image = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(image_buf) + 1023) & ~uintptr_t(1023));
-  int* tiles = reinterpret_cast<int*>(saved + S.tiles);
-  int* claims = reinterpret_cast<int*>((reinterpret_cast<uintptr_t>(claim_buf) + 255) & ~uintptr_t(255));
+  const long long bound = C.saved.bound;
   int n_claims = 0;
-  if (pmt_plan_tiles(batch, BWD_MAXV, true, PMT_PARTIAL_CTAS, tiles, claims, &n_claims, st)) return 1;
-  check_tile_bound_kernel<<<1, 1, 0, st>>>(tiles, (int)S.bound);
-  if (pmt_launch_pack_tc(C.P, T, weights, image, st)) return 1;
-  const unsigned header[4] = {kTrainSavedMagic, (unsigned)batch->n_variants, (unsigned)S.bound, 0u};
-  PMT_CUDA(cudaMemcpyAsync(saved, header, sizeof(header), cudaMemcpyHostToDevice, st));
+  if (pmt_plan_tiles(batch, BWD_MAXV, true, PMT_PARTIAL_CTAS, S.tiles, W.claims, &n_claims, st)) return 1;
+  check_tile_bound_kernel<<<1, 1, 0, st>>>(S.tiles, (int)bound);
+  if (pmt_launch_pack_tc(C.P, T, weights, W.tc_image, st)) return 1;
   const int grid = pmt_tile_grid(batch, n_claims, C.n_sm < PMT_PARTIAL_CTAS ? C.n_sm : PMT_PARTIAL_CTAS);
   TcArgs F;
   memset(&F, 0, sizeof(F));
-  F.wflat = weights; F.image = image; F.tiles = tiles; F.perm = nullptr; F.batch = *batch; F.out = *out;
-  F.scratch = saved + S.scratch; F.tile_first = 0; F.tile_limit = (int)S.bound;
+  F.wflat = weights; F.image = W.tc_image; F.tiles = S.tiles; F.perm = nullptr; F.batch = *batch; F.out = *out;
+  F.scratch = S.scratch; F.tile_first = 0; F.tile_limit = (int)bound;
   pmt_profile_begin(st);
   const int rc = pmt_launch_reads_tc_save(C, F, grid, st);
   pmt_profile_end(st);
@@ -937,35 +882,27 @@ int pmt_tc_forward_train(const CallPlan& C, const float* weights, const PmtBatch
 }
 
 // Backward of the tile-sized read sets: writes d_info_seq for the variants of those sets and leaves the weight gradients
-// in the private buffers of the workspace; pmt_finish_reads_tc_backward adds them to d_weights.  `ws`: the backward
-// layout's tensor-core region (C.tc_bwd.total + 1024 bytes).
+// in the private buffers of the workspace; pmt_finish_reads_tc_backward adds them to d_weights.
 int pmt_launch_reads_tc_backward(const CallPlan& C, const float* weights, const PmtBatch* batch, const float* info_seq,
                                  const float* d_logits_bk, const float* d_alt_means, const float* d_ref_means, float* d_info_seq,
-                                 unsigned char* ws, size_t ws_bytes, int* grid_out, cudaStream_t st, const unsigned char* saved) {
+                                 const TcBwdBuffers& W, int* grid_out, cudaStream_t st, const SavedBuffers* saved) {
   const TcPlan& T = C.T;
   const BwdLayout& L = C.tc_bwd;
-  unsigned char* base = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 1023) & ~uintptr_t(1023));
-  PMT_CHECK((size_t)(base - ws) + L.total <= ws_bytes + 1024, "tensor-core backward: workspace too small (%zu < %zu)", ws_bytes, L.total);
-  unsigned char* image_f = base + L.image_f;
-  unsigned char* image_t = base + L.image_t;
-  int* tiles = reinterpret_cast<int*>(base + L.tiles);
-  int* claims = reinterpret_cast<int*>(base + L.claims);
-  float* partials = reinterpret_cast<float*>(base + L.partials);
-  unsigned char* scratch = base + L.scratch;
-
+  int* tiles = W.tiles;
+  unsigned char* scratch = W.scratch;
   int n_claims = 0;
   if (saved) {   // the training forward left the tile list and every tile's operands (pmt_tc_forward_train): no recompute
-    tiles = const_cast<int*>(reinterpret_cast<const int*>(saved + C.saved.tiles));
-    scratch = const_cast<unsigned char*>(saved + C.saved.scratch);
+    tiles = saved->tiles;
+    scratch = saved->scratch;
     n_claims = L.n_claims;
   } else {
-    if (pmt_plan_tiles(batch, BWD_MAXV, true, PMT_PARTIAL_CTAS, tiles, claims, &n_claims, st)) return 1;
-    if (pmt_launch_pack_tc(C.P, T, weights, image_f, st)) return 1;
+    if (pmt_plan_tiles(batch, BWD_MAXV, true, PMT_PARTIAL_CTAS, tiles, W.claims, &n_claims, st)) return 1;
+    if (pmt_launch_pack_tc(C.P, T, weights, W.image_f, st)) return 1;
   }
-  pack_tc_bwd_kernel<<<dim3(T.n_steps, 8), 256, 0, st>>>(C.P.d, T, weights, image_t);
+  pack_tc_bwd_kernel<<<dim3(T.n_steps, 8), 256, 0, st>>>(C.P.d, T, weights, W.image_t);
 
   const int grid = pmt_tile_grid(batch, n_claims, C.n_sm < PMT_PARTIAL_CTAS ? C.n_sm : PMT_PARTIAL_CTAS);
-  PMT_CUDA(cudaMemsetAsync(partials, 0, (size_t)2 * grid * T.part_floats * sizeof(float), st));
+  PMT_CUDA(cudaMemsetAsync(W.partials, 0, (size_t)2 * grid * T.part_floats * sizeof(float), st));
   const Ring& R = C.ring_bwd;
   PMT_CUDA(cudaFuncSetAttribute(reads_backward_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)R.smem));
 
@@ -973,10 +910,10 @@ int pmt_launch_reads_tc_backward(const CallPlan& C, const float* weights, const 
   memset(&no_out, 0, sizeof(no_out));
   no_out.info_seq_be = const_cast<float*>(info_seq);   // read by the first gated block's concat
   TcArgs F;
-  F.wflat = weights; F.image = image_f; F.tiles = tiles; F.perm = nullptr; F.batch = *batch; F.out = no_out; F.scratch = scratch;
+  F.wflat = weights; F.image = W.image_f; F.tiles = tiles; F.perm = nullptr; F.batch = *batch; F.out = no_out; F.scratch = scratch;
   TcBwdArgs Bk;
-  Bk.wflat = weights; Bk.image_t = image_t; Bk.tiles = tiles; Bk.batch = *batch; Bk.d_logits_bk = d_logits_bk;
-  Bk.d_alt_means = d_alt_means; Bk.d_ref_means = d_ref_means; Bk.d_info_seq = d_info_seq; Bk.scratch = scratch; Bk.partials = partials;
+  Bk.wflat = weights; Bk.image_t = W.image_t; Bk.tiles = tiles; Bk.batch = *batch; Bk.d_logits_bk = d_logits_bk;
+  Bk.d_alt_means = d_alt_means; Bk.d_ref_means = d_ref_means; Bk.d_info_seq = d_info_seq; Bk.scratch = scratch; Bk.partials = W.partials;
   pmt_profile_begin(st);
   for (int c = 0; c < L.n_chunks; ++c) {
     F.tile_first = Bk.tile_first = c * L.chunk_tiles;
@@ -994,13 +931,11 @@ int pmt_launch_reads_tc_backward(const CallPlan& C, const float* weights, const 
 
 // d_weights += the tile-sized sets' gradient (call after the other kernels' sums have been WRITTEN to d_weights and before
 // skip_fix_kernel: the last layer of a DenseSkipBlock is handed over un-scaled, as the SIMT kernels do).
-int pmt_finish_reads_tc_backward(const CallPlan& C, const float* weights, float* d_weights, unsigned char* ws, int grid, cudaStream_t st) {
+int pmt_finish_reads_tc_backward(const CallPlan& C, const float* weights, float* d_weights, const TcBwdBuffers& W, int grid,
+                                 cudaStream_t st) {
   const TcPlan& T = C.T;
-  unsigned char* base = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 1023) & ~uintptr_t(1023));
-  const float* partials = reinterpret_cast<const float*>(base + C.tc_bwd.partials);
-  float* reduced = reinterpret_cast<float*>(base + C.tc_bwd.reduced);
-  reduce_private_kernel<<<(T.part_floats + 255) / 256, 256, 0, st>>>(partials, 2 * grid, T.part_floats, reduced);
-  unfold_kernel<<<T.n_steps + C.P.d.n_blocks + 1, 256, 0, st>>>(C.P.d, T, weights, reduced, d_weights);
+  reduce_private_kernel<<<(T.part_floats + 255) / 256, 256, 0, st>>>(W.partials, 2 * grid, T.part_floats, W.reduced);
+  unfold_kernel<<<T.n_steps + C.P.d.n_blocks + 1, 256, 0, st>>>(C.P.d, T, weights, W.reduced, d_weights);
   cudaError_t e = cudaGetLastError();
   PMT_CHECK(e == cudaSuccess, "tensor-core backward (unfold) launch failed: %s", cudaGetErrorString(e));
   return 0;

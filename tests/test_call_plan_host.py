@@ -75,6 +75,40 @@ def test_fp32_backward_refuses_before_any_cuda_call(shape):
     assert b"shared-memory plan" in lib.pmt_last_error(), lib.pmt_last_error()
 
 
+@pytest.mark.skipif(torch.cuda.is_available(), reason="placeholder pointers must never reach a device")
+@pytest.mark.parametrize("base_offset", [None, 4, 256], ids=["one_byte_short", "base+4", "base+256"])
+@pytest.mark.parametrize("mode", MODES)
+@pytest.mark.parametrize("shape", ALL_SHAPES, ids=lambda s: s.name)
+def test_buffers_are_resolved_before_any_cuda_call(shape, mode, base_offset):
+    """pmt_forward, pmt_forward_train and pmt_backward lay the call plan's maps over their buffers before their first CUDA
+    call.  One byte less than the size the library reports is refused with the size message.  At the exact size, from a
+    base that is not aligned, every region realigns inside its slack and the call gets past the bounds check to that CUDA
+    call, which fails on a machine without a GPU (unless the call plan refuses the call first)."""
+    desc = build_model(shape, CPU).descriptor()
+    lib = L.load()
+    L.set_precision(mode)
+    out = L.PmtOutputs(*([PLACEHOLDER] * len(L.PmtOutputs._fields_)))
+    grads = L.PmtOutGrads(*([PLACEHOLDER] * 3 + [None, None]))
+    short = 1 if base_offset is None else 0
+    ws = PLACEHOLDER + (base_offset or 0)
+    for batch in BATCHES[1:]:
+        pb = _batch(*batch)
+        fwd, bwd, saved = _sizes(lib, desc, batch)
+        args = (ctypes.byref(desc), PLACEHOLDER, ctypes.byref(pb))
+        calls = [lambda: lib.pmt_forward(*args, ctypes.byref(out), ws, fwd - short, None),
+                 lambda: lib.pmt_backward(*args, ctypes.byref(grads), PLACEHOLDER, ws, bwd - short, None)]
+        if saved:   # the saved buffer one byte short, or the workspace from the unaligned base
+            calls.append(lambda: lib.pmt_forward_train(*args, ctypes.byref(out), ws, fwd, PLACEHOLDER, saved - short, None))
+        for call in calls:
+            assert call() != 0
+            err = lib.pmt_last_error()
+            if short:
+                assert b"too small" in err, (batch, err)
+            else:
+                # past the resolver: the first CUDA call failed, or the plan refused the call after the buffers were resolved
+                assert b"too small" not in err and b"ends past" not in err, (batch, err)
+
+
 @pytest.mark.parametrize("mode", MODES)
 @pytest.mark.parametrize("shape", ALL_SHAPES, ids=lambda s: s.name)
 def test_sizes_and_backward_kernels_are_unchanged(shape, mode):

@@ -208,7 +208,7 @@ def test_tensor_core_shapes_gradients_against_float64(shape, n_variants, mode):
 
 @pytest.mark.parametrize("shape", [s for s in TC_SHAPES if s.trains and s.bwd_tc], ids=ids)
 def test_saved_forward_equals_recompute_at_other_step_programs(shape, monkeypatch):
-    """The saved-forward buffer (pmt_saved_layout) and the backward workspace (backward_layout) are sized from the step
+    """The saved-forward buffer and the backward workspace (their maps in pmt_call.cu) are sized from the step
     program: outputs and gradients of the saved forward are BITWISE those of the recompute, which here walks the tile list
     in several ranges, and both are bitwise reproducible."""
     monkeypatch.setenv("PMT_BWD_CHUNK_TILES", "64")
