@@ -405,6 +405,40 @@ int pmt_posterior_fit_pass(const PmtPosteriorDesc* desc, const float* params, fl
                            float* somatic_snv_totals_rrra, float* snv_context_totals_rrra, void* workspace,
                            size_t workspace_bytes, void* stream);
 
+/* The passes of many independent fits (a cohort's samples, each with its own model and records) in one launch: one CTA
+ * per problem, each running exactly pmt_posterior_fit_pass's pass on its own arguments, so problem i ends with the bits
+ * pmt_posterior_fit_pass gives for it alone.  A sample's fit is a sequential chain of Adam steps and keeps one SM busy;
+ * a launch of n problems keeps min(n, SM count) SMs busy, more problems than SMs run in waves.  Problems may differ in
+ * every field: K, het_beta, no-germline mode, context priors, record count, batch size, fp16 / fp32 floats and strides,
+ * learning rate, which totals are NULL.  Every argument check of pmt_posterior_fit_pass applies to every problem, all
+ * before anything is enqueued; a refusal names the problem's index.  `h_problems` is a HOST array of n_problems >= 1;
+ * the call copies it into the workspace (stream-ordered, the host array may be reused once the call returns).
+ * workspace: pmt_posterior_fit_pass_many_workspace_size(n_problems, largest K of the problems) bytes (0 for
+ * n_problems < 1 or a K outside 1..PMT_POSTERIOR_MAX_COMPONENTS): the problem table and each problem's context scratch. */
+typedef struct PmtPosteriorFitProblem {
+  PmtPosteriorDesc desc;
+  const float* params;
+  float* raw_params;
+  float* adam_m;
+  float* adam_v;
+  int64_t* adam_step;
+  double learning_rate;
+  const int16_t* int_array;
+  int64_t int_stride;
+  const void* float_array;
+  int32_t float_kind;
+  int64_t float_stride;
+  int64_t n_records;
+  int32_t batch_size;
+  float* batch_losses_out;
+  float* posterior_totals_tc;               /* these three may be NULL, as for pmt_posterior_fit_pass */
+  float* somatic_snv_totals_rrra;
+  float* snv_context_totals_rrra;
+} PmtPosteriorFitProblem;
+size_t pmt_posterior_fit_pass_many_workspace_size(int32_t n_problems, int32_t max_components);
+int pmt_posterior_fit_pass_many(const PmtPosteriorFitProblem* h_problems, int32_t n_problems, void* workspace, size_t workspace_bytes,
+                                void* stream);
+
 /* ---- batch assembly from the dataset memory maps ----------------------------------------------------
  * Replaces the row re-stacking of Batch.__init__ (batch.py:41-62) for batches cut from a MemoryMappedData
  * (memory_mapped_data.py:36-58, reads_dataset.py:109-196): the reads memory map holds, variant after variant, the ref

@@ -7,7 +7,8 @@ posterior model fitted by the reference loads here and ``log_posterior_and_ingre
 ``learn_priors_and_spectra`` (posterior_model.py:101-165) runs its E step -- negative log evidence, its gradient w.r.t.
 the spectra, the posterior totals -- as pmt_posterior_fit_step and the optimiser / M step on the host; with its records
 resident on the model's device (``PosteriorRecords``) every pass of the batch loop, E steps and Adam steps, is one
-launch of pmt_posterior_fit_pass and only the M step stays on the host.  Context-dependent
+launch of pmt_posterior_fit_pass and only the M step stays on the host.  ``learn_priors_and_spectra_together`` fits many
+samples' models side by side, a pass of all of them per launch of pmt_posterior_fit_pass_many.  Context-dependent
 SNV priors are switched on for the second half of the iterations as in the reference (:125-127); its M step for them, a
 PyMC ADVI fit (posterior_model_priors.py:157-203), is replaced by a deterministic fit of the same model and variational
 family (architecture/snv_context_priors.py; pymc is absent from the image, so that one step has no reference golden).
@@ -15,7 +16,8 @@ family (architecture/snv_context_priors.py; pymc is absent from the image, so th
 drawn.  There is no CPU path for the model itself.
 """
 import ctypes as C
-from typing import Optional, Tuple
+import os
+from typing import List, Optional, Sequence, Tuple, Union
 
 import torch
 from torch import Tensor, nn
@@ -23,7 +25,7 @@ from torch.nn import Parameter
 from torch.nn.utils import parametrize
 
 from permutect_b200.architecture.layers import BoundedNumber, LogWeights, PositiveNumber
-from permutect_b200.architecture.snv_context_priors import context_m_step
+from permutect_b200.architecture.snv_context_priors import ContextFitPool, context_fit_inputs, fit_mutation_rates_sc, write_log_rates
 from permutect_b200.data.datum import HAPLOTYPES_START_IDX
 from permutect_b200.engine import library as L
 from permutect_b200.utils.enums import Variation
@@ -218,6 +220,15 @@ class PosteriorModel(nn.Module):
         """posterior_model_priors.py:141-224.  With context-dependent SNV priors switched on and both rrra totals given,
         ``somatic_snv_log_priors_rrra`` gets the log mutation rates of the hierarchical substitution x context model
         (snv_context_priors.context_m_step); otherwise it is filled with the SNV somatic log prior (:223-225)."""
+        fit_inputs = self._m_step_before_context_fit(posterior_totals_vc, ignored_to_non_ignored_ratio, somatic_snv_totals_rrra,
+                                                     snv_context_totals_rrra)
+        if fit_inputs is not None:
+            write_log_rates(self.priors.somatic_snv_log_priors_rrra, fit_mutation_rates_sc(*fit_inputs))
+
+    def _m_step_before_context_fit(self, posterior_totals_vc: Tensor, ignored_to_non_ignored_ratio: float,
+                                   somatic_snv_totals_rrra: Optional[Tensor], snv_context_totals_rrra: Optional[Tensor]):
+        """update_priors_m_step up to its context fit: returns that fit's inputs (snv_context_priors.context_fit_inputs) when
+        the context-dependent SNV priors are on, else None with the M step done."""
         total_nonignored = torch.sum(posterior_totals_vc)
         overall_total = (1 + ignored_to_non_ignored_ratio) * total_nonignored
         with torch.no_grad():
@@ -229,10 +240,9 @@ class PosteriorModel(nn.Module):
                 if somatic_snv_totals_rrra is None or snv_context_totals_rrra is None:
                     raise ValueError("context-dependent SNV priors are on: the M step needs both rrra totals")
                 total_ignored_per_context = float(ignored_to_non_ignored_ratio * total_nonignored) / 64      # :150-153
-                context_m_step(pri.somatic_snv_log_priors_rrra, somatic_snv_totals_rrra, snv_context_totals_rrra,
-                               total_ignored_per_context)
-            else:
-                pri.somatic_snv_log_priors_rrra.fill_(pri.log_priors_vc[int(Variation.SNV), CALL_SOMATIC])
+                return context_fit_inputs(somatic_snv_totals_rrra, snv_context_totals_rrra, total_ignored_per_context)
+            pri.somatic_snv_log_priors_rrra.fill_(pri.log_priors_vc[int(Variation.SNV), CALL_SOMATIC])
+            return None
 
     def learn_priors_and_spectra(self, posterior_loader, num_iterations, ignored_to_non_ignored_ratio: float, summary_writer=None,
                                  learning_rate: float = 0.001):
@@ -279,45 +289,143 @@ class PosteriorModel(nn.Module):
         """learn_priors_and_spectra with one pmt_posterior_fit_pass per iteration: the batches of ``records`` in order,
         each an E step and an Adam step of the raw spectra (the loop's fresh optimiser: zero moments, step 0, in flat
         device buffers for the call), then the same M step.  The raw parameters go back into the module after every pass."""
-        dev = records.device
         lib = L.load()
-        K = self.spectra.somatic_spectrum.K
-        raws = self._raw_spectra_tensors()
-        with torch.no_grad():
-            raw = torch.cat([t.detach().reshape(-1) for t in raws]).to(torch.float32).contiguous()
-        adam_m, adam_v = torch.zeros_like(raw), torch.zeros_like(raw)
-        adam_step = torch.zeros(1, dtype=torch.int64, device=dev)
-        ws = torch.empty(int(lib.pmt_posterior_fit_pass_workspace_size(K)), dtype=torch.uint8, device=dev)
-        it, ft = records.int_tensor, records.float_tensor
-        n_batches = len(records)
-        losses = torch.empty(n_batches, dtype=torch.float32, device=dev)
-        sizes = torch.full((n_batches,), float(records.batch_size), dtype=torch.float64, device=dev)
-        sizes[-1] = records.size() - (n_batches - 1) * records.batch_size
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        self.priors.disable_context_dependent_snv_priors()
-        history = []
+        fit = _DeviceFit(self, records, learning_rate)
+        ws = torch.empty(int(lib.pmt_posterior_fit_pass_workspace_size(self.spectra.somatic_spectrum.K)), dtype=torch.uint8,
+                         device=records.device)
+        stream = torch.cuda.current_stream(records.device).cuda_stream
         for epoch in range(1, num_iterations + 1):
-            if epoch > (num_iterations / 2):
-                self.priors.enable_context_dependent_snv_priors()
-            totals_tc = torch.zeros((len(Variation), NUM_CALLS), device=dev)
-            somatic_snv_rrra = torch.zeros((5, 5, 5, 5), device=dev)
-            snv_context_rrra = torch.zeros((5, 5, 5, 5), device=dev)
-            _, _, desc, flat = self._inputs(records)
-            L.check(lib.pmt_posterior_fit_pass(C.byref(desc), flat.data_ptr(), raw.data_ptr(), adam_m.data_ptr(), adam_v.data_ptr(),
-                                               adam_step.data_ptr(), float(learning_rate), it.data_ptr(), it.stride(0), ft.data_ptr(),
-                                               L.F16 if ft.dtype == torch.float16 else L.F32, ft.stride(0), records.size(),
-                                               records.batch_size, losses.data_ptr(), totals_tc.data_ptr(), somatic_snv_rrra.data_ptr(),
-                                               snv_context_rrra.data_ptr(), ws.data_ptr(), ws.numel(), stream))
-            with torch.no_grad():
-                off = 0
-                for t in raws:
-                    t.copy_(raw[off:off + t.numel()].view_as(t))
-                    off += t.numel()
-            self.update_priors_m_step(totals_tc, ignored_to_non_ignored_ratio, somatic_snv_rrra, snv_context_rrra)
-            history.append(float((losses.double() * sizes).sum()) / records.size())
-            if summary_writer is not None:
-                summary_writer.add_scalar("spectrum negative log evidence", history[-1], epoch)
-        return history
+            p = fit.begin_pass(epoch, num_iterations)
+            L.check(lib.pmt_posterior_fit_pass(C.byref(p.desc), p.params, p.raw_params, p.adam_m, p.adam_v, p.adam_step, p.learning_rate,
+                                               p.int_array, p.int_stride, p.float_array, p.float_kind, p.float_stride, p.n_records,
+                                               p.batch_size, p.batch_losses_out, p.posterior_totals_tc, p.somatic_snv_totals_rrra,
+                                               p.snv_context_totals_rrra, ws.data_ptr(), ws.numel(), stream))
+            fit.end_pass()
+            self.update_priors_m_step(fit.totals_tc, ignored_to_non_ignored_ratio, fit.somatic_snv_rrra, fit.snv_context_rrra)
+            fit.record(epoch, summary_writer)
+        return fit.history
+
+
+class _DeviceFit:
+    """One model's fit on a ``PosteriorRecords`` on its device, as ``pmt_posterior_fit_pass`` and
+    ``pmt_posterior_fit_pass_many`` run it: the raw spectra and the fresh optimiser's state (zero moments, step 0) in flat
+    device buffers carried from pass to pass, each pass's E-step totals, and the host steps around a pass."""
+
+    def __init__(self, model: PosteriorModel, records: "PosteriorRecords", learning_rate: float):
+        dev = records.device
+        self.model, self.records, self.learning_rate = model, records, float(learning_rate)
+        self.raws = model._raw_spectra_tensors()
+        with torch.no_grad():
+            self.raw = torch.cat([t.detach().reshape(-1) for t in self.raws]).to(torch.float32).contiguous()
+        self.adam_m, self.adam_v = torch.zeros_like(self.raw), torch.zeros_like(self.raw)
+        self.adam_step = torch.zeros(1, dtype=torch.int64, device=dev)
+        n_batches = len(records)
+        self.losses = torch.empty(n_batches, dtype=torch.float32, device=dev)
+        self.sizes = torch.full((n_batches,), float(records.batch_size), dtype=torch.float64, device=dev)
+        self.sizes[-1] = records.size() - (n_batches - 1) * records.batch_size
+        self.history = []
+        model.priors.disable_context_dependent_snv_priors()
+
+    def begin_pass(self, epoch: int, num_iterations: int) -> L.PmtPosteriorFitProblem:
+        """Context-dependent SNV priors from the second half of the iterations on (:125-127), zeroed totals; returns the
+        pass's arguments, valid until the next begin_pass."""
+        if epoch > (num_iterations / 2):
+            self.model.priors.enable_context_dependent_snv_priors()
+        dev = self.records.device
+        self.totals_tc = torch.zeros((len(Variation), NUM_CALLS), device=dev)
+        self.somatic_snv_rrra = torch.zeros((5, 5, 5, 5), device=dev)
+        self.snv_context_rrra = torch.zeros((5, 5, 5, 5), device=dev)
+        it, ft, desc, self.flat = self.model._inputs(self.records)
+        return L.PmtPosteriorFitProblem(desc, self.flat.data_ptr(), self.raw.data_ptr(), self.adam_m.data_ptr(), self.adam_v.data_ptr(),
+                                        self.adam_step.data_ptr(), self.learning_rate, it.data_ptr(), it.stride(0), ft.data_ptr(),
+                                        L.F16 if ft.dtype == torch.float16 else L.F32, ft.stride(0), self.records.size(),
+                                        self.records.batch_size, self.losses.data_ptr(), self.totals_tc.data_ptr(),
+                                        self.somatic_snv_rrra.data_ptr(), self.snv_context_rrra.data_ptr())
+
+    def end_pass(self) -> None:
+        """The pass's raw parameters back into the module."""
+        with torch.no_grad():
+            off = 0
+            for t in self.raws:
+                t.copy_(self.raw[off:off + t.numel()].view_as(t))
+                off += t.numel()
+
+    def record(self, epoch: int, summary_writer) -> None:
+        self.history.append(float((self.losses.double() * self.sizes).sum()) / self.records.size())
+        if summary_writer is not None:
+            summary_writer.add_scalar("spectrum negative log evidence", self.history[-1], epoch)
+
+
+def _per_model(value, n: int, what: str) -> List[float]:
+    if isinstance(value, (int, float)):
+        return [float(value)] * n
+    values = [float(v) for v in value]
+    if len(values) != n:
+        raise ValueError(f"{what}: {len(values)} values for {n} models")
+    return values
+
+
+def _usable_cpus() -> int:
+    return len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
+
+
+def learn_priors_and_spectra_together(models: Sequence[PosteriorModel], records: Sequence["PosteriorRecords"], num_iterations: int,
+                                      ignored_to_non_ignored_ratio: Union[float, Sequence[float]], summary_writers=None,
+                                      learning_rate: Union[float, Sequence[float]] = 0.001) -> List[List[float]]:
+    """``models[i].learn_priors_and_spectra(records[i], ...)`` for every i, the fits side by side: a cohort's samples
+    (tumour / normal pairs, the folds of an evaluation) each have their own model and records, and each fit is a chain of
+    Adam steps that keeps one SM busy, so every pass over all models is ONE pmt_posterior_fit_pass_many launch with a CTA
+    per model.  Between passes each model takes the M step of ``_learn_on_device``; the float64 context fits of the
+    second half run in a pool of worker processes (snv_context_priors.ContextFitPool) when there are several models.
+    Every model ends with the parameters, and every history equals the history, of its own ``learn_priors_and_spectra``.
+
+    ``records[i]`` is a ``PosteriorRecords`` (its own batch size); all models and records on one CUDA device.
+    ``ignored_to_non_ignored_ratio`` and ``learning_rate``: one value for all or one per model; ``summary_writers``: None
+    or one writer (or None) per model.  Returns one history per model."""
+    models, records = list(models), list(records)
+    n = len(models)
+    if n == 0:
+        raise ValueError("learn_priors_and_spectra_together: no models")
+    if len(records) != n:
+        raise ValueError(f"learn_priors_and_spectra_together: {n} models but {len(records)} record sets")
+    ratios = _per_model(ignored_to_non_ignored_ratio, n, "ignored_to_non_ignored_ratio")
+    rates = _per_model(learning_rate, n, "learning_rate")
+    writers = [None] * n if summary_writers is None else list(summary_writers)
+    if len(writers) != n:
+        raise ValueError(f"summary_writers: {len(writers)} writers for {n} models")
+    dev = records[0].device if isinstance(records[0], PosteriorRecords) else None
+    for i, (m, r) in enumerate(zip(models, records)):
+        if not isinstance(r, PosteriorRecords):
+            raise TypeError(f"records[{i}] is a {type(r).__name__}, not a PosteriorRecords")
+        if not (_same_device(r.device, dev) and _same_device(m._device, dev)):
+            raise RuntimeError(f"model {i} ({m._device}) and its records ({r.device}) must be on the device of records[0] ({dev})")
+    lib = L.load()
+    fits = [_DeviceFit(m, r, lr) for m, r, lr in zip(models, records, rates)]
+    max_k = max(m.spectra.somatic_spectrum.K for m in models)
+    ws = torch.empty(int(lib.pmt_posterior_fit_pass_many_workspace_size(n, max_k)), dtype=torch.uint8, device=dev)
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    workers = min(n, _usable_cpus())
+    pool = ContextFitPool(workers) if workers > 1 else None
+    try:
+        for epoch in range(1, num_iterations + 1):
+            problems = (L.PmtPosteriorFitProblem * n)(*[f.begin_pass(epoch, num_iterations) for f in fits])
+            L.check(lib.pmt_posterior_fit_pass_many(problems, n, ws.data_ptr(), ws.numel(), stream))
+            fit_inputs = []
+            for f, ratio in zip(fits, ratios):
+                f.end_pass()
+                fit_inputs.append(f.model._m_step_before_context_fit(f.totals_tc, ratio, f.somatic_snv_rrra, f.snv_context_rrra))
+            pending = [(f, x) for f, x in zip(fits, fit_inputs) if x is not None]
+            if pending:
+                inputs = [x for _, x in pending]
+                fitted = pool.map(inputs) if pool is not None and len(inputs) > 1 else [fit_mutation_rates_sc(*x) for x in inputs]
+                for (f, _), rates_sc in zip(pending, fitted):
+                    write_log_rates(f.model.priors.somatic_snv_log_priors_rrra, rates_sc)
+            for f, w in zip(fits, writers):
+                f.record(epoch, w)
+    finally:
+        if pool is not None:
+            pool.close()
+    return [f.history for f in fits]
 
 
 def _same_device(a, b) -> bool:

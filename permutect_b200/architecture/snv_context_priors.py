@@ -24,7 +24,9 @@ Host side (float64, 194 variational means + 194 scales), like the PyMC fit it re
 5x5x5x5 totals is the CUDA kernel ``pmt_posterior_fit_step``.
 """
 import math
-from typing import Tuple
+import multiprocessing
+from concurrent.futures import ProcessPoolExecutor
+from typing import List, Sequence, Tuple
 
 import torch
 from torch import Tensor
@@ -121,13 +123,58 @@ def fit_mutation_rates_sc(total_sc: Tensor, snv_sc: Tensor, max_iter: int = 300)
         return rate.mean(0)
 
 
+def context_fit_inputs(somatic_snv_totals_rrra: Tensor, snv_context_totals_rrra: Tensor,
+                       total_ignored_per_context: float) -> Tuple[Tensor, Tensor]:
+    """(total_sc, snv_sc): the E-step totals rounded as the reference rounds them for its Binomial (:158-159)."""
+    total_sc = torch.round(convert_rrra_tensor_to_sc(snv_context_totals_rrra.detach().double().cpu()) + total_ignored_per_context)
+    snv_sc = torch.round(convert_rrra_tensor_to_sc(somatic_snv_totals_rrra.detach().double().cpu()))
+    return total_sc, snv_sc
+
+
+def write_log_rates(somatic_snv_log_priors_rrra: Tensor, rates_sc: Tensor) -> None:
+    with torch.no_grad():
+        scatter_sc_to_rrra(torch.log(rates_sc), somatic_snv_log_priors_rrra)
+
+
 def context_m_step(somatic_snv_log_priors_rrra: Tensor, somatic_snv_totals_rrra: Tensor, snv_context_totals_rrra: Tensor,
                    total_ignored_per_context: float) -> Tensor:
     """posterior_model_priors.py:157-222: rounds the totals as the reference does, fits the rates and writes their logs
     into ``somatic_snv_log_priors_rrra`` in place.  Returns the fitted rates [12, 16]."""
-    total_sc = torch.round(convert_rrra_tensor_to_sc(snv_context_totals_rrra.detach().double().cpu()) + total_ignored_per_context)
-    snv_sc = torch.round(convert_rrra_tensor_to_sc(somatic_snv_totals_rrra.detach().double().cpu()))
-    rates_sc = fit_mutation_rates_sc(total_sc, snv_sc)
-    with torch.no_grad():
-        scatter_sc_to_rrra(torch.log(rates_sc), somatic_snv_log_priors_rrra)
+    rates_sc = fit_mutation_rates_sc(*context_fit_inputs(somatic_snv_totals_rrra, snv_context_totals_rrra, total_ignored_per_context))
+    write_log_rates(somatic_snv_log_priors_rrra, rates_sc)
     return rates_sc
+
+
+def _init_fit_worker() -> None:
+    torch.set_num_threads(1)
+    fit_mutation_rates_sc(torch.ones(NUM_SUBSTITUTIONS, NUM_CONTEXTS), torch.zeros(NUM_SUBSTITUTIONS, NUM_CONTEXTS), max_iter=1)
+
+
+def _started() -> None:
+    pass
+
+
+def _fit_arrays(total_sc, snv_sc):
+    return fit_mutation_rates_sc(torch.from_numpy(total_sc), torch.from_numpy(snv_sc)).numpy()
+
+
+class ContextFitPool:
+    """``fit_mutation_rates_sc`` for the totals of many independent models at once, in spawned worker processes.  The fit
+    is an L-BFGS loop of small float64 tensor operations whose time goes to Python, so threads would serialise on the GIL;
+    each worker runs one torch thread.  Every fit is deterministic CPU work on fixed Sobol draws: each result is bit for
+    bit what the in-process call gives.  The workers start, and load torch's lazily imported optimiser code, as soon as
+    the pool is created; ``close()`` ends them."""
+
+    def __init__(self, n_workers: int):
+        self._pool = ProcessPoolExecutor(n_workers, mp_context=multiprocessing.get_context("spawn"), initializer=_init_fit_worker)
+        for _ in range(n_workers):           # a process per task submitted while none is idle: start them all now
+            self._pool.submit(_started)
+
+    def map(self, inputs: Sequence[Tuple[Tensor, Tensor]]) -> List[Tensor]:
+        """[fit_mutation_rates_sc(total_sc, snv_sc) for (total_sc, snv_sc) in inputs], the fits spread over the workers."""
+        totals = [t.detach().double().cpu().numpy() for t, _ in inputs]
+        snvs = [s.detach().double().cpu().numpy() for _, s in inputs]
+        return [torch.from_numpy(r) for r in self._pool.map(_fit_arrays, totals, snvs)]
+
+    def close(self) -> None:
+        self._pool.shutdown()

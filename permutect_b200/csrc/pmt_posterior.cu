@@ -6,10 +6,14 @@
 // logit.  The reference builds ~25 [B] or [B, K, 100] temporaries per call; here a variant's 5 x 100 binomial terms of
 // the somatic mixture live in registers and nothing but the requested [B, 5] tables touches HBM.
 // fit_pass_kernel runs a whole pass of the fit's batch loop (E step, parametrisation VJP, Adam) in one CTA on the same
-// per-record device functions.
+// per-record device functions; fit_pass_many_kernel runs the passes of independent problems (one per sample) a CTA each.
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <math.h>
+
+#include <algorithm>
+#include <cstdio>
+#include <vector>
 
 #include "../../include/permutect_b200.h"
 #include "pmt_host.h"
@@ -438,8 +442,8 @@ struct LaneMix {
 
 __device__ __forceinline__ float sigmoidf(float x) { return 1.f / (1.f + expf(-x)); }   // torch.sigmoid
 
-__global__ void __launch_bounds__(PASS_THREADS, 1) fit_pass_kernel(const FitPassArgs A) {
-  extern __shared__ float smem[];
+// One problem's pass on the calling CTA; smem: fit_pass_smem(K) bytes or more
+__device__ __forceinline__ void fit_pass(const FitPassArgs& A, float* smem) {
   const PmtPosteriorDesc& D = A.D;
   const int K = D.n_components, n_small = small_count(K), n_slots = slot_count(K), n_grad = n_slots - 1 - N_TYPES * N_CALLS;
   const int row_w = n_slots + 2;                 // slots, then the record's context cell (-1: none) and SOMATIC posterior
@@ -568,6 +572,23 @@ __global__ void __launch_bounds__(PASS_THREADS, 1) fit_pass_kernel(const FitPass
   }
 }
 
+__global__ void __launch_bounds__(PASS_THREADS, 1) fit_pass_kernel(const FitPassArgs A) {
+  extern __shared__ float smem[];
+  fit_pass(A, smem);
+}
+
+// A CTA per problem: problem blockIdx.x's arguments come from a table in global memory and are copied to shared memory
+// first (the pass reads them throughout, and its own global writes would otherwise force re-loads)
+__global__ void __launch_bounds__(PASS_THREADS, 1) fit_pass_many_kernel(const FitPassArgs* __restrict__ table) {
+  extern __shared__ float smem[];
+  __shared__ FitPassArgs A;
+  static_assert(sizeof(FitPassArgs) % sizeof(int) == 0 && sizeof(FitPassArgs) / sizeof(int) <= PASS_THREADS, "a word per thread");
+  if (threadIdx.x < sizeof(FitPassArgs) / sizeof(int))
+    reinterpret_cast<int*>(&A)[threadIdx.x] = reinterpret_cast<const int*>(table + blockIdx.x)[threadIdx.x];
+  __syncthreads();
+  fit_pass(A, smem);
+}
+
 size_t fit_pass_smem(int K) {
   return (size_t)(small_count(MAXK) + 2 * MAXK + 70 + PASS_WARPS * 2 * MAXK * 32 + PASS_ROWS * (slot_count(K) + 2)) * sizeof(float);
 }
@@ -633,32 +654,86 @@ extern "C" size_t pmt_posterior_fit_pass_workspace_size(int32_t n_components) {
   return 2 * post::CONTEXT_CELLS * sizeof(float) + 256;
 }
 
+// The refusals of one fit-pass problem (`who` names the call, and the problem of a many-launch); on success *out holds
+// the kernel's arguments with context_ws as the problem's context scratch
+static int fit_pass_args(const PmtPosteriorFitProblem& p, const char* who, float* context_ws, post::FitPassArgs* out) {
+  const PmtPosteriorDesc& d = p.desc;
+  PMT_CHECK(p.params && p.raw_params && p.adam_m && p.adam_v && p.adam_step && p.int_array && p.float_array && p.batch_losses_out,
+            "%s: null argument", who);
+  PMT_CHECK(d.n_components >= 1 && d.n_components <= PMT_POSTERIOR_MAX_COMPONENTS, "%s: somatic spectrum components %d outside 1..%d",
+            who, d.n_components, PMT_POSTERIOR_MAX_COMPONENTS);
+  PMT_CHECK(p.batch_size >= 1, "%s: batch_size %d < 1", who, p.batch_size);
+  PMT_CHECK(p.float_kind == PMT_F16 || p.float_kind == PMT_F32, "%s: float_kind must be PMT_F16 or PMT_F32", who);
+  PMT_CHECK(p.n_records > 0, "%s: no records", who);
+  const int64_t n_batches = (p.n_records + p.batch_size - 1) / p.batch_size;
+  PMT_CHECK(n_batches <= INT32_MAX, "%s: %lld batches exceed the int32 range", who, (long long)n_batches);
+  PMT_CHECK((!p.somatic_snv_totals_rrra && !p.snv_context_totals_rrra) || d.hap_len >= 3,
+            "%s: SNV context totals need haplotypes of >= 3 bases", who);
+  PMT_CHECK(!d.use_context_dependent_snv_priors || d.hap_len >= 3, "%s: context-dependent SNV priors need haplotypes of >= 3 bases", who);
+  *out = post::FitPassArgs{d, p.params, p.raw_params, p.adam_m, p.adam_v, reinterpret_cast<long long*>(p.adam_step), p.learning_rate,
+                           p.int_array, p.int_stride, p.float_array, p.float_kind, p.float_stride, p.n_records, p.batch_size,
+                           (int)n_batches, p.batch_losses_out, p.posterior_totals_tc, p.somatic_snv_totals_rrra,
+                           p.snv_context_totals_rrra, context_ws};
+  return 0;
+}
+
 extern "C" int pmt_posterior_fit_pass(const PmtPosteriorDesc* desc, const float* params, float* raw_params, float* adam_m, float* adam_v,
                                       int64_t* adam_step, double learning_rate, const int16_t* int_array, int64_t int_stride,
                                       const void* float_array, int32_t float_kind, int64_t float_stride, int64_t n_records,
                                       int32_t batch_size, float* batch_losses_out, float* posterior_totals_tc,
                                       float* somatic_snv_totals_rrra, float* snv_context_totals_rrra, void* workspace,
                                       size_t workspace_bytes, void* stream) {
-  PMT_CHECK(desc && params && raw_params && adam_m && adam_v && adam_step && int_array && float_array && batch_losses_out && workspace,
-            "pmt_posterior_fit_pass: null argument");
-  PMT_CHECK(desc->n_components >= 1 && desc->n_components <= PMT_POSTERIOR_MAX_COMPONENTS, "somatic spectrum components %d outside 1..%d",
-            desc->n_components, PMT_POSTERIOR_MAX_COMPONENTS);
-  PMT_CHECK(batch_size >= 1, "pmt_posterior_fit_pass: batch_size %d < 1", batch_size);
-  PMT_CHECK(float_kind == PMT_F16 || float_kind == PMT_F32, "float_kind must be PMT_F16 or PMT_F32");
-  PMT_CHECK(n_records > 0, "no records");
-  const int64_t n_batches = (n_records + batch_size - 1) / batch_size;
-  PMT_CHECK(n_batches <= INT32_MAX, "pmt_posterior_fit_pass: %lld batches exceed the int32 range", (long long)n_batches);
+  PMT_CHECK(desc && workspace, "pmt_posterior_fit_pass: null argument");
+  const PmtPosteriorFitProblem p{*desc, params, raw_params, adam_m, adam_v, adam_step, learning_rate, int_array, int_stride, float_array,
+                                 float_kind, float_stride, n_records, batch_size, batch_losses_out, posterior_totals_tc,
+                                 somatic_snv_totals_rrra, snv_context_totals_rrra};
+  post::FitPassArgs A;
+  if (fit_pass_args(p, "pmt_posterior_fit_pass", reinterpret_cast<float*>(workspace), &A)) return 1;
   PMT_CHECK(workspace_bytes >= pmt_posterior_fit_pass_workspace_size(desc->n_components), "workspace too small: %zu bytes, need %zu",
             workspace_bytes, pmt_posterior_fit_pass_workspace_size(desc->n_components));
-  PMT_CHECK((!somatic_snv_totals_rrra && !snv_context_totals_rrra) || desc->hap_len >= 3, "SNV context totals need haplotypes of >= 3 bases");
-  PMT_CHECK(!desc->use_context_dependent_snv_priors || desc->hap_len >= 3, "context-dependent SNV priors need haplotypes of >= 3 bases");
-  post::FitPassArgs A{*desc, params, raw_params, adam_m, adam_v, reinterpret_cast<long long*>(adam_step), learning_rate, int_array,
-                      int_stride, float_array, float_kind, float_stride, n_records, batch_size, (int)n_batches, batch_losses_out,
-                      posterior_totals_tc, somatic_snv_totals_rrra, snv_context_totals_rrra, reinterpret_cast<float*>(workspace)};
   const size_t smem = post::fit_pass_smem(desc->n_components);
   PMT_CUDA(cudaFuncSetAttribute(post::fit_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   post::fit_pass_kernel<<<1, post::PASS_THREADS, smem, reinterpret_cast<cudaStream_t>(stream)>>>(A);
   cudaError_t e = cudaGetLastError();
   PMT_CHECK(e == cudaSuccess, "pmt_posterior_fit_pass launch failed: %s", cudaGetErrorString(e));
+  return 0;
+}
+
+// Workspace of a many-launch: the device copy of the problem table (256-byte aligned), then [n_problems][2][625] floats
+// of context scratch; the extra 256 bytes realign a caller's buffer
+static size_t fit_pass_many_table_bytes(int32_t n_problems) {
+  return ((size_t)n_problems * sizeof(post::FitPassArgs) + 255) & ~(size_t)255;
+}
+
+extern "C" size_t pmt_posterior_fit_pass_many_workspace_size(int32_t n_problems, int32_t max_components) {
+  if (n_problems < 1 || max_components < 1 || max_components > PMT_POSTERIOR_MAX_COMPONENTS) return 0;
+  return fit_pass_many_table_bytes(n_problems) + (size_t)n_problems * 2 * post::CONTEXT_CELLS * sizeof(float) + 256;
+}
+
+extern "C" int pmt_posterior_fit_pass_many(const PmtPosteriorFitProblem* h_problems, int32_t n_problems, void* workspace,
+                                           size_t workspace_bytes, void* stream) {
+  PMT_CHECK(h_problems && workspace, "pmt_posterior_fit_pass_many: null argument");
+  PMT_CHECK(n_problems >= 1, "pmt_posterior_fit_pass_many: n_problems %d < 1", n_problems);
+  unsigned char* base = pmt_align_up(workspace, 256);
+  float* context_ws = reinterpret_cast<float*>(base + fit_pass_many_table_bytes(n_problems));
+  std::vector<post::FitPassArgs> table((size_t)n_problems);
+  int max_k = 1;
+  for (int32_t i = 0; i < n_problems; ++i) {
+    char who[64];
+    snprintf(who, sizeof(who), "pmt_posterior_fit_pass_many: problem %d", i);
+    if (fit_pass_args(h_problems[i], who, context_ws + (size_t)i * 2 * post::CONTEXT_CELLS, &table[i])) return 1;
+    max_k = std::max(max_k, (int)h_problems[i].desc.n_components);
+  }
+  const size_t need = pmt_posterior_fit_pass_many_workspace_size(n_problems, max_k);
+  PMT_CHECK(workspace_bytes >= need, "pmt_posterior_fit_pass_many: workspace too small: %zu bytes, need %zu", workspace_bytes, need);
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  auto* d_table = reinterpret_cast<post::FitPassArgs*>(base);
+  // from pageable memory: the call returns once `table` has been staged, so it may go out of scope
+  PMT_CUDA(cudaMemcpyAsync(d_table, table.data(), table.size() * sizeof(post::FitPassArgs), cudaMemcpyHostToDevice, st));
+  const size_t smem = post::fit_pass_smem(max_k);
+  PMT_CUDA(cudaFuncSetAttribute(post::fit_pass_many_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  post::fit_pass_many_kernel<<<n_problems, post::PASS_THREADS, smem, st>>>(d_table);
+  cudaError_t e = cudaGetLastError();
+  PMT_CHECK(e == cudaSuccess, "pmt_posterior_fit_pass_many launch failed: %s", cudaGetErrorString(e));
   return 0;
 }
