@@ -395,8 +395,10 @@ int pmt_posterior_fit_step(const PmtPosteriorDesc* desc, const float* params, co
  * pmt_posterior_fit_step's grads_out; adam_step[1] (in / out) += the number of batches.  batch_losses_out[number of
  * batches] = every batch's loss.  posterior_totals_tc, somatic_snv_totals_rrra, snv_context_totals_rrra += the pass's
  * E-step totals, as pmt_posterior_fit_step adds them (any may be NULL).  Every sum has a fixed order and no atomics:
- * the pass is bitwise reproducible.  One CTA walks the batches; workspace: pmt_posterior_fit_pass_workspace_size(K)
- * bytes (0 for a K outside 1..PMT_POSTERIOR_MAX_COMPONENTS). */
+ * the pass is bitwise reproducible.  A cluster of up to 16 CTAs, so up to 16 SMs, walks the batches, its CTAs sharing
+ * each batch's records through distributed shared memory; every width gives the same bits (pmt_posterior_fit_ctas
+ * reports the width).  workspace: pmt_posterior_fit_pass_workspace_size(K) bytes (0 for a K outside
+ * 1..PMT_POSTERIOR_MAX_COMPONENTS). */
 size_t pmt_posterior_fit_pass_workspace_size(int32_t n_components);
 int pmt_posterior_fit_pass(const PmtPosteriorDesc* desc, const float* params, float* raw_params, float* adam_m, float* adam_v,
                            int64_t* adam_step, double learning_rate, const int16_t* int_array, int64_t int_stride,
@@ -405,10 +407,11 @@ int pmt_posterior_fit_pass(const PmtPosteriorDesc* desc, const float* params, fl
                            float* somatic_snv_totals_rrra, float* snv_context_totals_rrra, void* workspace,
                            size_t workspace_bytes, void* stream);
 
-/* The passes of many independent fits (a cohort's samples, each with its own model and records) in one launch: one CTA
- * per problem, each running exactly pmt_posterior_fit_pass's pass on its own arguments, so problem i ends with the bits
- * pmt_posterior_fit_pass gives for it alone.  A sample's fit is a sequential chain of Adam steps and keeps one SM busy;
- * a launch of n problems keeps min(n, SM count) SMs busy, more problems than SMs run in waves.  Problems may differ in
+/* The passes of many independent fits (a cohort's samples, each with its own model and records) in one launch: one
+ * cluster of CTAs per problem (up to 16 SMs each), each running exactly pmt_posterior_fit_pass's pass on its own
+ * arguments, so problem i ends with the bits pmt_posterior_fit_pass gives for it alone.  A sample's fit is a sequential
+ * chain of Adam steps; the clusters are as wide as lets every problem's cluster be resident at once (one CTA each from
+ * as many problems as SMs on, more problems than SMs run in waves).  Problems may differ in
  * every field: K, het_beta, no-germline mode, context priors, record count, batch size, fp16 / fp32 floats and strides,
  * learning rate, which totals are NULL.  Every argument check of pmt_posterior_fit_pass applies to every problem, all
  * before anything is enqueued; a refusal names the problem's index.  `h_problems` is a HOST array of n_problems >= 1;
@@ -438,6 +441,14 @@ typedef struct PmtPosteriorFitProblem {
 size_t pmt_posterior_fit_pass_many_workspace_size(int32_t n_problems, int32_t max_components);
 int pmt_posterior_fit_pass_many(const PmtPosteriorFitProblem* h_problems, int32_t n_problems, void* workspace, size_t workspace_bytes,
                                 void* stream);
+/* The cluster width (CTAs per problem: 1, 2, 4, 8 or 16) with which pmt_posterior_fit_pass_many runs these n_problems
+ * problems, or pmt_posterior_fit_pass a single one: the largest width that gives every CTA at least 16 records of the
+ * largest batch (a warp each) and lets every problem's cluster be resident at once, and 1 from as many problems as SMs
+ * on.  The width never changes a result.  The environment variable PMT_POSTERIOR_CTAS=n (tests and measurements) forces
+ * the width n of both passes; any other value than the five widths makes them, and this query, refuse.  Returns 0 with
+ * pmt_last_error() on a refusal: the fit-pass checks of every problem apply (the problem's index is named), and the
+ * query needs the device the passes would run on. */
+int pmt_posterior_fit_ctas(const PmtPosteriorFitProblem* h_problems, int32_t n_problems);
 
 /* ---- batch assembly from the dataset memory maps ----------------------------------------------------
  * Replaces the row re-stacking of Batch.__init__ (batch.py:41-62) for batches cut from a MemoryMappedData

@@ -374,8 +374,8 @@ def learn_priors_and_spectra_together(models: Sequence[PosteriorModel], records:
                                       learning_rate: Union[float, Sequence[float]] = 0.001) -> List[List[float]]:
     """``models[i].learn_priors_and_spectra(records[i], ...)`` for every i, the fits side by side: a cohort's samples
     (tumour / normal pairs, the folds of an evaluation) each have their own model and records, and each fit is a chain of
-    Adam steps that keeps one SM busy, so every pass over all models is ONE pmt_posterior_fit_pass_many launch with a CTA
-    per model.  Between passes each model takes the M step of ``_learn_on_device``; the float64 context fits of the
+    Adam steps that keeps at most 16 SMs busy, so every pass over all models is ONE pmt_posterior_fit_pass_many launch with
+    a cluster of CTAs per model (one CTA each from as many models as SMs on).  Between passes each model takes the M step of ``_learn_on_device``; the float64 context fits of the
     second half run in a pool of worker processes (snv_context_priors.ContextFitPool) when there are several models.
     Every model ends with the parameters, and every history equals the history, of its own ``learn_priors_and_spectra``.
 

@@ -785,6 +785,17 @@ static Overrides read_overrides() {
   return {get("PMT_CNN_SINGLE"), get("PMT_TC_PACKED"), get("PMT_LONG_SIMT"), get("PMT_BWD_CHUNK_TILES")};
 }
 
+// The posterior fit passes take no call plan; their override is read here, by its only reader:
+//   PMT_POSTERIOR_CTAS=n   every problem of pmt_posterior_fit_pass / _many runs on a cluster of n CTAs (n = 1: the one-SM pass)
+// -1 when unset, 0 when set to anything but 1, 2, 4, 8 or 16 (the callers refuse that).
+int pmt_posterior_ctas_override() {
+  const char* e = getenv("PMT_POSTERIOR_CTAS");
+  if (!e) return -1;
+  char* end = nullptr;
+  const long n = strtol(e, &end, 10);
+  return end != e && *end == '\0' && (n == 1 || n == 2 || n == 4 || n == 8 || n == 16) ? (int)n : 0;
+}
+
 // Batches below this size keep the sequential planner: packing saves ~5.5 % of the read kernel (1.13 ns per read), the packed
 // planner costs ~0.1 ms more than the sequential one (one lane per claim places 512 sets), so it pays from ~2 M reads.
 static const long long kPackedPlannerMinRows = 2000000;

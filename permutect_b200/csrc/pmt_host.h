@@ -40,3 +40,4 @@ size_t pmt_image_bytes(const pmt::Plan& P, const pmt::CnnGeom& G);
 void pmt_profile_begin(cudaStream_t st);
 void pmt_profile_end(cudaStream_t st);
 int pmt_precision_mode();
+int pmt_posterior_ctas_override();

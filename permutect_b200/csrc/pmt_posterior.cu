@@ -5,8 +5,10 @@
 // normal_artifact_spectrum.py:38-58, germline :18-58), the matched-normal table, and their sum with the cached artifact
 // logit.  The reference builds ~25 [B] or [B, K, 100] temporaries per call; here a variant's 5 x 100 binomial terms of
 // the somatic mixture live in registers and nothing but the requested [B, 5] tables touches HBM.
-// fit_pass_kernel runs a whole pass of the fit's batch loop (E step, parametrisation VJP, Adam) in one CTA on the same
-// per-record device functions; fit_pass_many_kernel runs the passes of independent problems (one per sample) a CTA each.
+// fit_pass_kernel runs a whole pass of the fit's batch loop (E step, parametrisation VJP, Adam) on one cluster of up to 16
+// CTAs on the same per-record device functions; fit_pass_many_kernel runs the passes of independent problems (one per
+// sample) a cluster each.
+#include <cooperative_groups.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <math.h>
@@ -384,12 +386,17 @@ __global__ void fit_reduce_kernel(const float* __restrict__ partials, int n_bloc
 }
 
 
-// ---- one pass of the fit (learn_priors_and_spectra's batch loop, posterior_model.py:128-151) in one CTA ----------------
+// ---- one pass of the fit (learn_priors_and_spectra's batch loop, posterior_model.py:128-151) on a cluster of CTAs ------
 // A warp per record: lane l takes the interpolation points j = l, l + 32, ... of every mixture component and the warp
 // merges the 32 streaming states; the rest of the record's math runs on every lane (identical values).  A record's slot
-// terms go to a row of shared memory; the rows of up to PASS_ROWS records are summed slot by slot in record order, so
-// the pass is bitwise reproducible without atomics.
+// terms go to a row of shared memory; the rows are summed slot by slot in record order, so the pass is bitwise
+// reproducible without atomics.  A cluster of C CTAs (ranks) takes a batch's records in chunks of up to C * PASS_ROWS,
+// rank r a contiguous range of at most PASS_ROWS of them in its own shared memory.  Every rank then sums every rank's
+// rows, in rank order through distributed shared memory, and runs the VJP and Adam itself: the sums see the rows in
+// record order whatever C is, so each rank holds the bits of the one-CTA pass (C = 1) and no second exchange of the
+// results is needed.  Rank 0 alone writes to global memory.
 constexpr int PASS_WARPS = 16, PASS_THREADS = PASS_WARPS * 32, PASS_ROWS = 64;
+constexpr int MAX_CLUSTER = 16;
 constexpr int CONTEXT_CELLS = 625;
 static_assert(PASS_THREADS >= 1 + 2 * MAXK + 4 * N_DEPTH_BINS * N_TYPES + 2 * N_TYPES + N_TYPES * N_CALLS, "a thread per slot");
 static_assert(2 * PASS_THREADS >= CONTEXT_CELLS, "two context cells per thread");
@@ -442,8 +449,17 @@ struct LaneMix {
 
 __device__ __forceinline__ float sigmoidf(float x) { return 1.f / (1.f + expf(-x)); }   // torch.sigmoid
 
-// One problem's pass on the calling CTA; smem: fit_pass_smem(K) bytes or more
+// One problem's pass on the calling cluster (a lone CTA: C = 1); smem: fit_pass_smem(K) bytes or more per CTA
 __device__ __forceinline__ void fit_pass(const FitPassArgs& A, float* smem) {
+  namespace cg = cooperative_groups;
+  const cg::cluster_group cluster = cg::this_cluster();
+  const int n_ranks = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
+  const bool lead = rank == 0;
+  // C = 1 keeps the CTA barrier; a cluster barrier also orders the ranks' shared-memory writes before the others' reads
+  auto pass_sync = [&]() {
+    if (n_ranks == 1) __syncthreads();
+    else cluster.sync();
+  };
   const PmtPosteriorDesc& D = A.D;
   const int K = D.n_components, n_small = small_count(K), n_slots = slot_count(K), n_grad = n_slots - 1 - N_TYPES * N_CALLS;
   const int row_w = n_slots + 2;                 // slots, then the record's context cell (-1: none) and SOMATIC posterior
@@ -459,7 +475,8 @@ __device__ __forceinline__ void fit_pass(const FitPassArgs& A, float* smem) {
   const int si = tid < 2 * K ? tid : tid + 4;
   if (tid < n_grad) { raw = A.raw[tid]; m1 = A.adam_m[tid]; m2 = A.adam_v[tid]; }
   const long long step0 = *A.adam_step;
-  const bool context = A.somatic_snv_totals_rrra || A.snv_context_totals_rrra;
+  const bool row_cells = A.somatic_snv_totals_rrra || A.snv_context_totals_rrra;   // rows carry their context cells
+  const bool context = lead && row_cells;        // rank 0 keeps the context totals
   // context cells c0 = tid and c1 = tid + PASS_THREADS are this thread's, for the whole pass
   const int c0 = tid, c1 = tid + PASS_THREADS;
   if (context) {
@@ -475,45 +492,55 @@ __device__ __forceinline__ void fit_pass(const FitPassArgs& A, float* smem) {
     const long long r0 = (long long)b * A.batch_size;
     const int nb = (int)min((long long)A.batch_size, A.n_records - r0);
     float acc = 0.f;                             // thread s < n_slots: slot s summed over the batch
-    for (int q0 = 0; q0 < nb; q0 += PASS_ROWS) {
-      const int nq = min(PASS_ROWS, nb - q0);
+    for (int q0 = 0; q0 < nb; q0 += n_ranks * PASS_ROWS) {
+      const int nq = min(n_ranks * PASS_ROWS, nb - q0);
+      const int per = (nq + n_ranks - 1) / n_ranks;   // rank r's records: [r * per, (r + 1) * per) of the chunk's nq
+      const int lo = min(nq, rank * per), hi = min(nq, lo + per);
       float ctx[4] = {0.f, 0.f, 0.f, 0.f};        // the context cells' running values (hidden behind the E step)
       if (context) {
         if (c0 < CONTEXT_CELLS) { ctx[0] = A.context_ws[c0]; ctx[1] = A.context_ws[CONTEXT_CELLS + c0]; }
         if (c1 < CONTEXT_CELLS) { ctx[2] = A.context_ws[c1]; ctx[3] = A.context_ws[CONTEXT_CELLS + c1]; }
       }
-      for (int q = warp; q < nq; q += PASS_WARPS) {
+      for (int q = lo + warp; q < hi; q += PASS_WARPS) {
         const Record R = load_record(A.ints, A.int_stride, A.floats, A.float_kind, A.float_stride, r0 + q0 + q);
         float pri[N_CALLS], spec[N_CALLS], norm[N_CALLS], post[N_CALLS], r[N_CALLS];
         Ingredients I;
         record_tables<true>(D, S, snv_rrra, R, lane, 32, WarpMerge{}, mix_term, mix_dcf, pri, spec, norm, post, I);
-        float* row = rows + q * row_w;
+        float* row = rows + (q - lo) * row_w;
         evidence_terms(S, K, R, I, mix_term, mix_dcf, post, 1.f, r, [&](int slot, float val) {
           if ((slot & 31) == lane) row[slot] = val;
         });
         if (lane == 0) {
-          row[n_slots] = __int_as_float(context && R.vt == 0 ? snv_context_cell(D, R.ir) : -1);
+          row[n_slots] = __int_as_float(row_cells && R.vt == 0 ? snv_context_cell(D, R.ir) : -1);
           row[n_slots + 1] = r[SOMATIC];
         }
       }
-      __syncthreads();
-      if (tid < n_slots)
-        for (int q = 0; q < nq; ++q) acc += rows[q * row_w + tid];
-      if (context) {
-        bool hit0 = false, hit1 = false;
-        for (int q = 0; q < nq; ++q) {
-          const int cell = __float_as_int(rows[q * row_w + n_slots]);
-          if (cell == c0) { ctx[0] += rows[q * row_w + n_slots + 1]; ctx[1] += 1.f; hit0 = true; }
-          else if (cell == c1) { ctx[2] += rows[q * row_w + n_slots + 1]; ctx[3] += 1.f; hit1 = true; }
+      pass_sync();
+      // the rows of n records from `src`, next in record order
+      bool hit0 = false, hit1 = false;
+      auto take_rows = [&](const float* src, int n) {
+        if (tid < n_slots)
+          for (int q = 0; q < n; ++q) acc += src[q * row_w + tid];
+        if (context)
+          for (int q = 0; q < n; ++q) {
+            const int cell = __float_as_int(src[q * row_w + n_slots]);
+            if (cell == c0) { ctx[0] += src[q * row_w + n_slots + 1]; ctx[1] += 1.f; hit0 = true; }
+            else if (cell == c1) { ctx[2] += src[q * row_w + n_slots + 1]; ctx[3] += 1.f; hit1 = true; }
+          }
+      };
+      if (n_ranks == 1) take_rows(rows, nq);
+      else
+        for (int rr = 0; rr < n_ranks; ++rr) {
+          const int rlo = min(nq, rr * per);
+          take_rows(rr == rank ? rows : cluster.map_shared_rank(rows, rr), min(nq, rlo + per) - rlo);
         }
-        if (hit0) { A.context_ws[c0] = ctx[0]; A.context_ws[CONTEXT_CELLS + c0] = ctx[1]; }
-        if (hit1) { A.context_ws[c1] = ctx[2]; A.context_ws[CONTEXT_CELLS + c1] = ctx[3]; }
-      }
-      __syncthreads();
+      if (hit0) { A.context_ws[c0] = ctx[0]; A.context_ws[CONTEXT_CELLS + c0] = ctx[1]; }
+      if (hit1) { A.context_ws[c1] = ctx[2]; A.context_ws[CONTEXT_CELLS + c1] = ctx[3]; }
+      pass_sync();                               // no rank overwrites its rows while another still reads them
     }
     // ---- loss and gradient w.r.t. the constrained spectra (fit_reduce_kernel's -1/B) ----
     const float inv_b = 1.f / (float)nb;
-    if (tid == 0) A.batch_losses[b] = -acc * inv_b;
+    if (tid == 0) { if (lead) A.batch_losses[b] = -acc * inv_b; }
     else if (tid <= n_grad) gsh[tid - 1] = -acc * inv_b;
     else if (tid < n_slots) pass_total += acc;
     __syncthreads();
@@ -561,6 +588,7 @@ __device__ __forceinline__ void fit_pass(const FitPassArgs& A, float* smem) {
     __syncthreads();
   }
   // ---- the pass's results ----
+  if (!lead) return;
   if (tid < n_grad) { A.raw[tid] = raw; A.adam_m[tid] = m1; A.adam_v[tid] = m2; }
   if (tid == 0) *A.adam_step = step0 + A.n_batches;
   if (A.totals_tc && tid > n_grad && tid < n_slots) A.totals_tc[tid - 1 - n_grad] += pass_total;
@@ -577,14 +605,15 @@ __global__ void __launch_bounds__(PASS_THREADS, 1) fit_pass_kernel(const FitPass
   fit_pass(A, smem);
 }
 
-// A CTA per problem: problem blockIdx.x's arguments come from a table in global memory and are copied to shared memory
-// first (the pass reads them throughout, and its own global writes would otherwise force re-loads)
+// A cluster per problem: every rank of cluster i copies problem i's arguments from a table in global memory to its shared
+// memory first (the pass reads them throughout, and its own global writes would otherwise force re-loads)
 __global__ void __launch_bounds__(PASS_THREADS, 1) fit_pass_many_kernel(const FitPassArgs* __restrict__ table) {
   extern __shared__ float smem[];
   __shared__ FitPassArgs A;
   static_assert(sizeof(FitPassArgs) % sizeof(int) == 0 && sizeof(FitPassArgs) / sizeof(int) <= PASS_THREADS, "a word per thread");
+  const unsigned problem = blockIdx.x / cooperative_groups::this_cluster().num_blocks();
   if (threadIdx.x < sizeof(FitPassArgs) / sizeof(int))
-    reinterpret_cast<int*>(&A)[threadIdx.x] = reinterpret_cast<const int*>(table + blockIdx.x)[threadIdx.x];
+    reinterpret_cast<int*>(&A)[threadIdx.x] = reinterpret_cast<const int*>(table + problem)[threadIdx.x];
   __syncthreads();
   fit_pass(A, smem);
 }
@@ -677,6 +706,56 @@ static int fit_pass_args(const PmtPosteriorFitProblem& p, const char* who, float
   return 0;
 }
 
+// The cluster launch of a fit-pass kernel: n_clusters clusters of `ctas` CTAs; `attr` holds the cluster dimension
+static cudaLaunchConfig_t fit_pass_config(int n_clusters, int ctas, size_t smem, cudaStream_t st, cudaLaunchAttribute* attr) {
+  attr->id = cudaLaunchAttributeClusterDimension;
+  attr->val.clusterDim.x = (unsigned)ctas;
+  attr->val.clusterDim.y = attr->val.clusterDim.z = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)(n_clusters * ctas));
+  cfg.blockDim = dim3(post::PASS_THREADS);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  return cfg;
+}
+
+// The cluster width C of a fit-pass launch of `kernel` (smem bytes of dynamic shared memory per CTA) over n_problems
+// problems whose largest batch is max_batch records, into *ctas; sets the kernel attributes the launch needs.
+// PMT_POSTERIOR_CTAS when set, otherwise the largest C of 16, 8, 4 and 2 such that
+//   - C <= ceil(max_batch / 16): a rank gives each record a warp, and a rank with fewer records than warps idles;
+//   - every problem's cluster is resident at once (cudaOccupancyMaxActiveClusters), so no cluster waits for a second wave;
+//   - there are fewer problems than SMs: from there on one CTA per problem fills the GPU by itself;
+// and C = 1 (a CTA per problem) when none is.
+static int fit_pass_ctas(const void* kernel, int n_problems, long long max_batch, size_t smem, const char* who, int* ctas) {
+  const int forced = pmt_posterior_ctas_override();
+  PMT_CHECK(forced != 0, "%s: PMT_POSTERIOR_CTAS must be 1, 2, 4, 8 or 16", who);
+  PMT_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  PMT_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+  if (forced > 0) {
+    *ctas = forced;
+    return 0;
+  }
+  int dev = 0, n_sm = 0;
+  PMT_CUDA(cudaGetDevice(&dev));
+  PMT_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
+  *ctas = 1;
+  if (n_problems >= n_sm) return 0;
+  for (int c = post::MAX_CLUSTER; c > 1; c /= 2) {
+    if (16LL * (c - 1) >= max_batch) continue;                     // c > ceil(max_batch / 16)
+    cudaLaunchAttribute attr;
+    const cudaLaunchConfig_t cfg = fit_pass_config(1, c, smem, nullptr, &attr);
+    int resident = 0;
+    PMT_CUDA(cudaOccupancyMaxActiveClusters(&resident, kernel, &cfg));
+    if (n_problems <= resident) {
+      *ctas = c;
+      return 0;
+    }
+  }
+  return 0;
+}
+
 extern "C" int pmt_posterior_fit_pass(const PmtPosteriorDesc* desc, const float* params, float* raw_params, float* adam_m, float* adam_v,
                                       int64_t* adam_step, double learning_rate, const int16_t* int_array, int64_t int_stride,
                                       const void* float_array, int32_t float_kind, int64_t float_stride, int64_t n_records,
@@ -692,9 +771,13 @@ extern "C" int pmt_posterior_fit_pass(const PmtPosteriorDesc* desc, const float*
   PMT_CHECK(workspace_bytes >= pmt_posterior_fit_pass_workspace_size(desc->n_components), "workspace too small: %zu bytes, need %zu",
             workspace_bytes, pmt_posterior_fit_pass_workspace_size(desc->n_components));
   const size_t smem = post::fit_pass_smem(desc->n_components);
-  PMT_CUDA(cudaFuncSetAttribute(post::fit_pass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  post::fit_pass_kernel<<<1, post::PASS_THREADS, smem, reinterpret_cast<cudaStream_t>(stream)>>>(A);
-  cudaError_t e = cudaGetLastError();
+  int ctas = 1;
+  if (fit_pass_ctas((const void*)post::fit_pass_kernel, 1, std::min<long long>(batch_size, n_records), smem, "pmt_posterior_fit_pass",
+                    &ctas))
+    return 1;
+  cudaLaunchAttribute attr;
+  const cudaLaunchConfig_t cfg = fit_pass_config(1, ctas, smem, reinterpret_cast<cudaStream_t>(stream), &attr);
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, post::fit_pass_kernel, A);
   PMT_CHECK(e == cudaSuccess, "pmt_posterior_fit_pass launch failed: %s", cudaGetErrorString(e));
   return 0;
 }
@@ -710,30 +793,61 @@ extern "C" size_t pmt_posterior_fit_pass_many_workspace_size(int32_t n_problems,
   return fit_pass_many_table_bytes(n_problems) + (size_t)n_problems * 2 * post::CONTEXT_CELLS * sizeof(float) + 256;
 }
 
+// The refusals of a many-launch's problems (`who` names the call); on success table[i] (when table is not null) holds
+// problem i's kernel arguments with its share of context_ws, *max_k the largest K and *max_batch the largest batch
+static int fit_pass_many_args(const PmtPosteriorFitProblem* h_problems, int32_t n_problems, const char* who, float* context_ws,
+                              post::FitPassArgs* table, int* max_k, long long* max_batch) {
+  PMT_CHECK(h_problems, "%s: null argument", who);
+  PMT_CHECK(n_problems >= 1, "%s: n_problems %d < 1", who, n_problems);
+  *max_k = 1;
+  *max_batch = 1;
+  for (int32_t i = 0; i < n_problems; ++i) {
+    char problem[96];
+    snprintf(problem, sizeof(problem), "%s: problem %d", who, i);
+    post::FitPassArgs A;
+    float* ws = context_ws ? context_ws + (size_t)i * 2 * post::CONTEXT_CELLS : nullptr;
+    if (fit_pass_args(h_problems[i], problem, ws, table ? &table[i] : &A)) return 1;
+    *max_k = std::max(*max_k, (int)h_problems[i].desc.n_components);
+    *max_batch = std::max(*max_batch, std::min<long long>(h_problems[i].batch_size, h_problems[i].n_records));
+  }
+  return 0;
+}
+
+extern "C" int pmt_posterior_fit_ctas(const PmtPosteriorFitProblem* h_problems, int32_t n_problems) {
+  const char* who = "pmt_posterior_fit_ctas";
+  int max_k = 1, ctas = 0;
+  long long max_batch = 1;
+  if (fit_pass_many_args(h_problems, n_problems, who, nullptr, nullptr, &max_k, &max_batch)) return 0;
+  // the kernel of the entry that would run these problems (both hold one CTA per SM)
+  const void* kernel = n_problems == 1 ? (const void*)post::fit_pass_kernel : (const void*)post::fit_pass_many_kernel;
+  if (fit_pass_ctas(kernel, n_problems, max_batch, post::fit_pass_smem(max_k), who, &ctas)) return 0;
+  return ctas;
+}
+
 extern "C" int pmt_posterior_fit_pass_many(const PmtPosteriorFitProblem* h_problems, int32_t n_problems, void* workspace,
                                            size_t workspace_bytes, void* stream) {
-  PMT_CHECK(h_problems && workspace, "pmt_posterior_fit_pass_many: null argument");
-  PMT_CHECK(n_problems >= 1, "pmt_posterior_fit_pass_many: n_problems %d < 1", n_problems);
+  const char* who = "pmt_posterior_fit_pass_many";
+  PMT_CHECK(h_problems && workspace, "%s: null argument", who);
+  PMT_CHECK(n_problems >= 1, "%s: n_problems %d < 1", who, n_problems);
   unsigned char* base = pmt_align_up(workspace, 256);
-  float* context_ws = reinterpret_cast<float*>(base + fit_pass_many_table_bytes(n_problems));
   std::vector<post::FitPassArgs> table((size_t)n_problems);
   int max_k = 1;
-  for (int32_t i = 0; i < n_problems; ++i) {
-    char who[64];
-    snprintf(who, sizeof(who), "pmt_posterior_fit_pass_many: problem %d", i);
-    if (fit_pass_args(h_problems[i], who, context_ws + (size_t)i * 2 * post::CONTEXT_CELLS, &table[i])) return 1;
-    max_k = std::max(max_k, (int)h_problems[i].desc.n_components);
-  }
+  long long max_batch = 1;
+  if (fit_pass_many_args(h_problems, n_problems, who, reinterpret_cast<float*>(base + fit_pass_many_table_bytes(n_problems)),
+                         table.data(), &max_k, &max_batch))
+    return 1;
   const size_t need = pmt_posterior_fit_pass_many_workspace_size(n_problems, max_k);
   PMT_CHECK(workspace_bytes >= need, "pmt_posterior_fit_pass_many: workspace too small: %zu bytes, need %zu", workspace_bytes, need);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   auto* d_table = reinterpret_cast<post::FitPassArgs*>(base);
+  const size_t smem = post::fit_pass_smem(max_k);
+  int ctas = 1;
+  if (fit_pass_ctas((const void*)post::fit_pass_many_kernel, n_problems, max_batch, smem, who, &ctas)) return 1;
   // from pageable memory: the call returns once `table` has been staged, so it may go out of scope
   PMT_CUDA(cudaMemcpyAsync(d_table, table.data(), table.size() * sizeof(post::FitPassArgs), cudaMemcpyHostToDevice, st));
-  const size_t smem = post::fit_pass_smem(max_k);
-  PMT_CUDA(cudaFuncSetAttribute(post::fit_pass_many_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  post::fit_pass_many_kernel<<<n_problems, post::PASS_THREADS, smem, st>>>(d_table);
-  cudaError_t e = cudaGetLastError();
+  cudaLaunchAttribute attr;
+  const cudaLaunchConfig_t cfg = fit_pass_config(n_problems, ctas, smem, st, &attr);
+  const cudaError_t e = cudaLaunchKernelEx(&cfg, post::fit_pass_many_kernel, (const post::FitPassArgs*)d_table);
   PMT_CHECK(e == cudaSuccess, "pmt_posterior_fit_pass_many launch failed: %s", cudaGetErrorString(e));
   return 0;
 }
