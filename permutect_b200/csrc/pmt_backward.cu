@@ -14,10 +14,7 @@
 
 // The per-row phases are written for NPART = NTHREADS / TILE threads per tile row.  Measured on B200 (65 536 variants,
 // profiles/r1_tensor_core_kernels.md): 256 threads 30.4 ms, 384 threads 31.6 ms, 512 threads 32.5 ms (register cap 128,
-// spills), so the default of two threads per row stays.
-#ifndef PMT_NTHREADS
-#define PMT_NTHREADS 256
-#endif
+// spills), so NTHREADS stays at 256: two threads per row.
 #include "pmt_cnn.cuh"
 #include "pmt_call.h"
 #include "pmt_tile.cuh"

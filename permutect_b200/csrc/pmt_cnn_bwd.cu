@@ -24,17 +24,6 @@
 namespace pmt {
 namespace cnnbwd {
 
-__device__ __forceinline__ float rna(float v) {
-  unsigned r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(v));
-  return __uint_as_float(r);
-}
-__device__ __forceinline__ void mma_tf32(float* c, const float* a, float b0, float b1) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-               : "r"(__float_as_uint(a[0])), "r"(__float_as_uint(a[1])), "r"(__float_as_uint(a[2])), "r"(__float_as_uint(a[3])),
-                 "r"(__float_as_uint(b0)), "r"(__float_as_uint(b1)));
-}
 __host__ __device__ __forceinline__ int w_index(const BLayer& Ly, int co, int ci, int t) {
   if (Ly.is_linear) return Ly.w_off + co * Ly.op_in_ch + (Ly.flat_len > 1 ? ci * Ly.flat_len + t : ci);
   return Ly.w_off + (co * Ly.op_in_ch + ci) * Ly.ks + t;
@@ -52,13 +41,8 @@ __global__ void pack_cnn_bwd_kernel(const __grid_constant__ BPlan BP, const floa
     const int m = frag % Ly.Mt_d, kc = (frag / Ly.Mt_d) % Ly.Cout8, t = frag / (Ly.Mt_d * Ly.Cout8);
     const int co = kc * 8 + (lane & 3) + ((r & 2) ? 4 : 0), ci = m * 16 + (lane >> 2) + ((r & 1) ? 8 : 0);
     const float v = (co < Ly.Cout && ci < Ly.Cin) ? w[w_index(Ly, co, ci, t)] : 0.f;
-    image[Ly.img_off + idx] = rna(v);
+    image[Ly.img_off + idx] = rna_tf32(v);
   }
-}
-
-// cp.async of 16 bytes of which the first src_bytes come from global memory (the rest is zero-filled)
-__device__ __forceinline__ void cp_async16_zfill(void* smem, const void* gmem, int src_bytes) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(smem_addr(smem)), "l"(gmem), "r"(src_bytes));
 }
 
 // What a weight-gradient unit needs from its layer, in registers
@@ -154,7 +138,7 @@ __device__ __forceinline__ void make_dY(float* __restrict__ dY, const float* __r
         val += g * (a > 0.f ? sc : fmaf(sa, a, sb));
       }
     }
-    dY[co * ldy + v * lpg + x] = rna(val);
+    dY[co * ldy + v * lpg + x] = rna_tf32(val);
     co += dco; v += dv; x += dx;
     if (x >= lpg) { x -= lpg; v += 1; }
     if (v >= VT) { v -= VT; co += 1; }

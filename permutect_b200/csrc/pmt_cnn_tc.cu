@@ -29,25 +29,6 @@ namespace cnntc {
 
 using namespace pmt::tc;
 
-// Shared-memory matrix descriptor, K-major, no swizzle.  Low word: start address >> 4 | (LBO >> 4) << 16 with LBO = the
-// distance between K-adjacent core matrices; high word (constant): SBO = 128 B between 8-row groups, descriptor version 1.
-constexpr unsigned DESC_HI = 8u | (1u << 14);
-__device__ __forceinline__ unsigned desc_lo(unsigned addr, unsigned lbo_bytes) { return ((addr >> 4) & 0x3FFFu) | ((lbo_bytes >> 4) << 16); }
-template <unsigned IDESC>
-__device__ __forceinline__ void mma_ss(unsigned tmem_d, unsigned a_lo32, unsigned b_lo32, unsigned accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-      "setp.ne.b32 p, %3, 0;\n\t"
-      "mov.b64 da, {%1, %4};\n\t"
-      "mov.b64 db, {%2, %4};\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], da, db, %5, p;\n\t}" ::"r"(tmem_d),
-      "r"(a_lo32), "r"(b_lo32), "r"(accumulate), "n"(DESC_HI), "n"(IDESC)
-      : "memory");
-}
-__host__ __device__ constexpr unsigned make_idesc(int N) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((unsigned)(N >> 3) << 17) | ((128u >> 4) << 24);
-}
-
 // Split-precision scheme (PASSES == 3): the weight image stacks [W_hi ; W_lo] along N, so ONE MMA of width 2N computes
 // A_hi.W_hi (columns [0, N)) and A_hi.W_lo (columns [N, 2N)) from a single read of the A rows -- operand fetch from shared
 // memory, not the tensor pipe, bounds these small-N MMAs -- and a second MMA of width N adds A_lo.W_hi to columns [0, N).
@@ -66,10 +47,10 @@ __device__ __forceinline__ void issue_shifted(int taps, unsigned d, unsigned a_h
       const unsigned bo = (unsigned)(2 * ks * R);
       const unsigned acc = (ks == 0) ? (t > 0 ? 1u : 0u) : 1u;
       if (PASSES == 3) {
-        mma_ss<make_idesc(64)>(d, a_hi + ao, b + bo, acc);
-        mma_ss<make_idesc(32)>(d, a_lo + ao, b + bo, 1u);
+        mma_ss_desc_lo<make_idesc(64)>(d, a_hi + ao, b + bo, acc);
+        mma_ss_desc_lo<make_idesc(32)>(d, a_lo + ao, b + bo, 1u);
       } else {
-        mma_ss<make_idesc(32)>(d, a_hi + ao, b + bo, acc);
+        mma_ss_desc_lo<make_idesc(32)>(d, a_hi + ao, b + bo, acc);
       }
     }
     a_hi += 1; a_lo += 1; b += 8 * R;
@@ -84,7 +65,7 @@ __device__ __forceinline__ void issue_first(int ksteps, unsigned d, unsigned a, 
   for (int ks = 0; ks < 8; ++ks) {
     if (ks < ksteps) {
       const unsigned ao = (unsigned)(2 * ks * (PLANE_BYTES / 16)), bo = (unsigned)(2 * ks * R);
-      mma_ss<idesc>(d, a + ao, b + bo, ks != 0 ? 1u : 0u);
+      mma_ss_desc_lo<idesc>(d, a + ao, b + bo, ks != 0 ? 1u : 0u);
     }
   }
 }
@@ -109,6 +90,7 @@ struct Bars {
   unsigned tmem_base;
   int pad_;
 };
+constexpr int CNN_TMEM_COLS = MAX_CHUNKS * CHUNK_COLS;   // one accumulator per chunk
 
 template <int PASSES, bool SAVE>
 __global__ void __launch_bounds__(THREADS, 1)
@@ -131,7 +113,7 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
   if (tid == 0) {
     for (int i = 0; i <= n_items; ++i) mbar_init(smem_addr(&S->done_bar[i]), EPI_WARPS);
     for (int i = 0; i < n_items; ++i) mbar_init(smem_addr(&S->acc_bar[i]), 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   // resident weight images (no-swizzle K-major planes, built by pack_cnn_tc_kernel) and biases
   for (int i = tid; i < TP.image_bytes / 16; i += THREADS)
@@ -141,11 +123,8 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
     const int n = i % 32, b_off = D.cnn_ops[Ly.op].b_off;
     bias_s[i] = (n < Ly.out_ch && b_off >= 0) ? __ldg(wflat + b_off + n) : 0.f;
   }
-  if (warp == MMA_WARP) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_addr(&S->tmem_base)), "r"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-  }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  if (warp == MMA_WARP) tmem_alloc<CNN_TMEM_COLS>(smem_addr(&S->tmem_base));
+  fence_proxy_async();
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -252,7 +231,7 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
           sts_f32(t_row[k] + (col >> 2) * PLANE_BYTES + (col & 3) * 4, 1.f);
         }
       }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      fence_proxy_async();
       __syncwarp();
       if (lane == 0) mbar_arrive(smem_addr(&S->done_bar[0]));
       fetch_codes(g + gridDim.x);
@@ -326,11 +305,7 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
             float* sg = save + (size_t)g * SL.group_floats;
             float* dstg = sg + save_a + (cq * 8) * cols + col;
 #pragma unroll
-            for (int i = 0; i < 8; ++i) {   // rounded to TF32: the backward's MMAs read them as they lie
-              unsigned rb;
-              asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(rb) : "f"(x[i]));
-              dstg[i * cols] = __uint_as_float(rb);
-            }
+            for (int i = 0; i < 8; ++i) dstg[i * cols] = rna_tf32(x[i]);   // rounded to TF32: the backward's MMAs read them as they lie
             if (save_bits >= 0) reinterpret_cast<unsigned char*>(sg + save_bits)[cq * cols + col] = (unsigned char)win;
           }
           if (!SAVE && (flags & F_TAIL)) {   // the split forward: fp32 into the tail kernel's A layout (pmt_cnn_tc.cuh)
@@ -351,7 +326,7 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
               sts128(dst + BUF_BYTES + PLANE_BYTES, make_float4(x[4], x[5], x[6], x[7]));
             }
           }
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          fence_proxy_async();
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(smem_addr(&S->done_bar[1 + it]));
@@ -360,7 +335,7 @@ hap_cnn_tc_kernel(const __grid_constant__ Plan TP, const unsigned char* __restri
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == MMA_WARP) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
+  if (warp == MMA_WARP) tmem_dealloc<CNN_TMEM_COLS>(tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -395,10 +370,10 @@ __device__ __forceinline__ void issue_dense(unsigned d, unsigned a_hi, unsigned 
     const unsigned ao = (unsigned)(2 * ks * (TAIL_PLANE / 16)), bo = (unsigned)(2 * ks * R);
     const unsigned acc = (first && ks == 0) ? 0u : 1u;
     if (PASSES == 3) {
-      mma_ss<make_idesc(2 * N)>(d, a_hi + ao, b + bo, acc);
-      mma_ss<make_idesc(N)>(d, a_lo + ao, b + bo, 1u);
+      mma_ss_desc_lo<make_idesc(2 * N)>(d, a_hi + ao, b + bo, acc);
+      mma_ss_desc_lo<make_idesc(N)>(d, a_lo + ao, b + bo, 1u);
     } else {
-      mma_ss<make_idesc(N)>(d, a_hi + ao, b + bo, acc);
+      mma_ss_desc_lo<make_idesc(N)>(d, a_hi + ao, b + bo, acc);
     }
   }
 }
@@ -436,7 +411,7 @@ hap_cnn_tail_kernel(const __grid_constant__ TailPlan TT, const unsigned char* __
     for (int t = 0; t < MAX_TAIL; ++t) mbar_init(smem_addr(&S->acc[t]), 1);
     mbar_init(smem_addr(&S->mid), TAIL_EPI_WARPS);
     mbar_init(smem_addr(&S->free0), TAIL_EPI_WARPS);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
   for (int i = tid; i < TT.image_bytes / 16; i += TAIL_THREADS)
     reinterpret_cast<uint4*>(img_s)[i] = __ldg(reinterpret_cast<const uint4*>(image) + i);
@@ -445,11 +420,8 @@ hap_cnn_tail_kernel(const __grid_constant__ TailPlan TT, const unsigned char* __
     const int n = i % 32, b_off = D.cnn_ops[Ly.op].b_off;
     bias_s[i] = (n < Ly.out_ch && b_off >= 0) ? __ldg(wflat + b_off + n) : 0.f;
   }
-  if (warp == TAIL_EPI_WARPS) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_addr(&S->tmem_base)), "r"(TAIL_TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-  }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+  if (warp == TAIL_EPI_WARPS) tmem_alloc<TAIL_TMEM_COLS>(smem_addr(&S->tmem_base));
+  fence_proxy_async();
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -528,7 +500,7 @@ hap_cnn_tail_kernel(const __grid_constant__ TailPlan TT, const unsigned char* __
             v.w -= __uint_as_float(__float_as_uint(v.w) & 0xFFFFE000u);
             sts128(hi + TAIL_STAGE_BYTES + o, v);
           }
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          fence_proxy_async();
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(smem_addr(&S->full[s]));
@@ -594,7 +566,7 @@ hap_cnn_tail_kernel(const __grid_constant__ TailPlan TT, const unsigned char* __
               sts128(dst + TAIL_STAGE_BYTES, make_float4(x[i], x[i + 1], x[i + 2], x[i + 3]));
             }
           }
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          fence_proxy_async();
           __syncwarp();
           if (lane == 0) mbar_arrive(smem_addr(&S->mid));
         }
@@ -603,7 +575,7 @@ hap_cnn_tail_kernel(const __grid_constant__ TailPlan TT, const unsigned char* __
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == TAIL_EPI_WARPS) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TAIL_TMEM_COLS));
+  if (warp == TAIL_EPI_WARPS) tmem_dealloc<TAIL_TMEM_COLS>(tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -632,9 +604,7 @@ __global__ void pack_cnn_tc_kernel(const __grid_constant__ PmtModelDesc D, const
   for (int idx = blockIdx.y * blockDim.x + threadIdx.x; idx < taps * chunks * R * 4; idx += gridDim.y * blockDim.x) {
     const int e = idx & 3, r = (idx >> 2) % R, ch = (idx >> 2) / R % chunks, tap = (idx >> 2) / R / chunks;
     const float v = cnn_weight(D, Ly, w, tap, r % N, ch * 4 + e);
-    unsigned hb;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(v));
-    const float hi = __uint_as_float(hb);
+    const float hi = rna_tf32(v);
     *reinterpret_cast<float*>(image + (size_t)Ly.img_off + (size_t)idx * 4) = r < N ? hi : v - hi;
   }
 }
@@ -649,9 +619,7 @@ __global__ void pack_cnn_tail_kernel(const __grid_constant__ PmtModelDesc D, con
     const int e = idx & 3, r = (idx >> 2) % R, ch = (idx >> 2) / R;
     const int kk = ch * 4 + e, n = r % N, tap = (kk >> 5) - (n >> 5);
     const float v = tap >= 0 && tap < Ly.taps ? cnn_weight(D, Ly, w, tap, n & 31, kk & 31) : 0.f;
-    unsigned hb;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(v));
-    const float hi = __uint_as_float(hb);
+    const float hi = rna_tf32(v);
     *reinterpret_cast<float*>(image + (size_t)Ly.img_off + (size_t)idx * 4) = r < N ? hi : v - hi;
   }
 }

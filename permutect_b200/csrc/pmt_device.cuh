@@ -16,10 +16,7 @@ namespace pmt {
 
 constexpr int TILE = PMT_TILE_ROWS;  // rows (reads, or variants in the per-variant kernels) per CTA tile
 constexpr int LD = TILE + 4;         // row stride of the feature-major activation buffers (floats)
-#ifndef PMT_NTHREADS
-#define PMT_NTHREADS 256   // a translation unit may compile its kernels for more warps (pmt_backward.cu: 512)
-#endif
-constexpr int NTHREADS = PMT_NTHREADS;
+constexpr int NTHREADS = 256;
 constexpr int NWARPS = NTHREADS / 32;
 constexpr int NPART = NTHREADS / TILE;   // threads per tile row; thread (row, part) = (tid % TILE, tid / TILE)
 // Part `part` of a per-row loop over n items covers [part_lo(n, part), part_lo(n, part + 1)).
@@ -91,6 +88,7 @@ __device__ __forceinline__ float selu(float x) {
 __device__ __forceinline__ float selu_grad_from_out(float y) {
   return y > 0.f ? SELU_SCALE : y + SELU_SCALE * SELU_ALPHA;
 }
+__device__ __forceinline__ float sigmoidf(float x) { return 1.f / (1.f + expf(-x)); }   // torch.sigmoid
 __device__ __forceinline__ unsigned smem_addr(const void* p) { return static_cast<unsigned>(__cvta_generic_to_shared(p)); }
 __device__ __forceinline__ float4 lds128(unsigned a) {
   float4 v;
@@ -105,8 +103,33 @@ __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
   unsigned s = static_cast<unsigned>(__cvta_generic_to_shared(smem));
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem));
 }
+// cp.async of 16 bytes of which the first src_bytes come from global memory (the rest is zero-filled)
+__device__ __forceinline__ void cp_async16_zfill(void* smem, const void* gmem, int src_bytes) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(smem_addr(smem)), "l"(gmem), "r"(src_bytes));
+}
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;\n" ::: "memory"); }
+
+__device__ __forceinline__ int ld_acquire_gpu(const int* p) {
+  int v;
+  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
+
+// fp32 -> TF32 rounded to nearest: the operand precision of the TF32 tensor-core instructions
+__device__ __forceinline__ float rna_tf32(float v) {
+  unsigned r;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(v));
+  return __uint_as_float(r);
+}
+// c += a b: one warp-level m16n8k8 TF32 MMA (mma.sync), fp32 accumulators
+__device__ __forceinline__ void mma_tf32(float* c, const float* a, float b0, float b1) {
+  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
+               : "r"(__float_as_uint(a[0])), "r"(__float_as_uint(a[1])), "r"(__float_as_uint(a[2])), "r"(__float_as_uint(a[3])),
+                 "r"(__float_as_uint(b0)), "r"(__float_as_uint(b1)));
+}
 
 // Double-buffered weight stage.  All control flow is CTA-uniform.  Keys: g for the forward image of
 // GemmOp g, MAX_GEMM + g for its transposed image.
@@ -257,11 +280,7 @@ __device__ __forceinline__ void gemm_tile_T(const float* dY, const GemmOp& op, c
 // Fire-and-forget accumulation into a CTA-private gradient buffer: a reduction does not wait for the old value the way
 // a load-add-store does.  Every address is only ever updated by one thread of one CTA, in program order, so the result
 // is still bitwise reproducible.
-#ifdef PMT_EXPERIMENT_NO_RED   // timing experiment only (gradients are wrong): how much of the backward is the accumulation traffic
-__device__ __forceinline__ void red_add(float* p, float v) { if (v == 123.456f) *p = v; }
-#else
 __device__ __forceinline__ void red_add(float* p, float v) { asm volatile("red.global.add.f32 [%0], %1;" ::"l"(p), "f"(v) : "memory"); }
-#endif
 
 // Weight gradient: part[n*K + k] += sum_{r in [r_lo, r_hi)} dY[n][r] * A[k][r]   (r_lo, r_hi multiples of 4).
 // `part` is this CTA's private gradient buffer, so the read-modify-write needs no atomics and the

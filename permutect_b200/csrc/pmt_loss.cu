@@ -21,7 +21,6 @@ constexpr int MAXW = PMT_MAX_HEAD_DIM;
 constexpr int MAXOPS = PMT_MAX_MLP_OPS;
 
 __device__ __forceinline__ float softplus(float x) { return fmaxf(x, 0.f) + log1pf(expf(-fabsf(x))); }
-__device__ __forceinline__ float sigmoidf(float x) { return 1.f / (1.f + expf(-x)); }
 // BCEWithLogitsLoss(reduction='none')
 __device__ __forceinline__ float bce_logits(float x, float y) { return fmaxf(x, 0.f) - x * y + log1pf(expf(-fabsf(x))); }
 

@@ -447,8 +447,6 @@ struct LaneMix {
   __device__ __forceinline__ float& operator[](int k) const { return p[k * 32]; }
 };
 
-__device__ __forceinline__ float sigmoidf(float x) { return 1.f / (1.f + expf(-x)); }   // torch.sigmoid
-
 // One problem's pass on the calling cluster (a lone CTA: C = 1); smem: fit_pass_smem(K) bytes or more per CTA
 __device__ __forceinline__ void fit_pass(const FitPassArgs& A, float* smem) {
   namespace cg = cooperative_groups;
@@ -573,7 +571,7 @@ __device__ __forceinline__ void fit_pass(const FitPassArgs& A, float* smem) {
     if (tid < n_grad) {
       float w;
       if (tid < K || (tid >= 2 * K + 4 * N_DEPTH_BINS * N_TYPES && tid < 2 * K + 4 * N_DEPTH_BINS * N_TYPES + N_TYPES)) {
-        w = sigmoidf(raw);
+        w = pmt::sigmoidf(raw);
       } else if (tid < 2 * K) {
         float mx = -INFINITY;
         for (int k = 0; k < K; ++k) mx = fmaxf(mx, gsh[K + k]);

@@ -31,11 +31,6 @@
 namespace pmt {
 namespace tc {
 
-__device__ __forceinline__ float rna_tf32(float v) {
-  unsigned r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(v));
-  return __uint_as_float(r);
-}
 // Training recompute: operand columns [col0, col0 + NC) of `row`, rounded to TF32, into the step's panels (pmt_tc.cuh).
 template <int NC>
 __device__ __forceinline__ void save_operand(unsigned char* op, int row, int col0, const float* v) {
@@ -43,12 +38,6 @@ __device__ __forceinline__ void save_operand(unsigned char* op, int row, int col
   for (int i = 0; i < NC / 4; ++i)
     *reinterpret_cast<float4*>(op + panel_off(row, col0 / 4 + i)) =
         make_float4(rna_tf32(v[4 * i]), rna_tf32(v[4 * i + 1]), rna_tf32(v[4 * i + 2]), rna_tf32(v[4 * i + 3]));
-}
-
-__device__ __forceinline__ int ld_acquire_gpu(const int* p) {
-  int v;
-  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
 }
 
 template <int PASSES, bool SAVE, bool LONG>
@@ -81,7 +70,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
       for (int b = 0; b < 2; ++b) { mbar_init(smem_addr(&S->meta_full[s][b]), 1); mbar_init(smem_addr(&S->meta_free[s][b]), 8); }
     }
     for (int i = 0; i < n_stages; ++i) { mbar_init(smem_addr(&S->wfull[i]), 1); mbar_init(smem_addr(&S->wfree[i]), 2); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
     head_constants(D, W, HC);
     for (int e = 0; e < MAXE; ++e) HCT->inv_sigma[e] = e < D.d_feat ? 1.f / HC->sigma[e] : 0.f;
     for (int s = 0; s < TP.n_steps; ++s) p[FWD_STEPS + s] = (unsigned char)(TP.step[s].epi | TP.step[s].blk << 4);
@@ -107,10 +96,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
     else if (c == BC_REGW) v = W[BO.reg_weight] + 0.25f;   // gated_mlp.py:237
     blkc[i] = v;
   }
-  if (warp == MMA_WARP) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_addr(&S->tmem_base)), "r"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-  }
+  if (warp == MMA_WARP) tmem_alloc<TMEM_COLS>(smem_addr(&S->tmem_base));
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -175,7 +161,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
           for (int q = 0; q < 4; ++q) TB->m.rowvar[q * 32 + lane] = (q * 32 + lane < nr_tot + na_tot) ? (unsigned char)0 : (unsigned char)255;
           if (nv && lane == 0 && A.out.info_seq_be) {
             const char* e = reinterpret_cast<const char*>(A.out.info_seq_be + (long long)v0 * DIS);
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(e));
+            prefetch_l2(e);
           }
         } else {
           if (t < n_tiles) { v0 = __ldg(A.tiles + 2 + 2 * (tile_first + t)); nv = __ldg(A.tiles + 3 + 2 * (tile_first + t)); }
@@ -194,8 +180,8 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
               rc[k] = (int)(__ldg(A.batch.ref_off + var[k] + 1) - r0[k]); ac[k] = (int)(__ldg(A.batch.alt_off + var[k] + 1) - a0[k]);
               if (A.out.info_seq_be) {   // the concat step's embedding rows: towards L2
                 const char* e = reinterpret_cast<const char*>(A.out.info_seq_be + (long long)var[k] * DIS);
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(e));
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(e + DIS * 4 - 4));
+                prefetch_l2(e);
+                prefetch_l2(e + DIS * 4 - 4);
               }
             }
             rsum += rc[k]; asum += ac[k];
@@ -890,9 +876,7 @@ reads_forward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_con
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == MMA_WARP) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
-  }
+  if (warp == MMA_WARP) tmem_dealloc<TMEM_COLS>(tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1200,9 +1184,7 @@ __global__ void pack_tc_kernel(const __grid_constant__ PmtModelDesc D, const __g
     const int kb = idx / (o.N * 32), rem = idx % (o.N * 32), n = rem / 32, kk = rem % 32;
     const int k = kb * 32 + kk;
     const float v = k < K ? tc_weight(D, o, w, n, k) : 0.f;
-    unsigned hb;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hb) : "f"(v));
-    const float hi = __uint_as_float(hb);
+    const float hi = rna_tf32(v);
     const float lo = v - hi;
     const unsigned L = (unsigned)n * 128u + (unsigned)kk * 4u;
     const unsigned phys = L ^ (((L >> 7) & 7u) << 4);

@@ -16,6 +16,7 @@ constexpr int META_WARP = 19, FWD_THREADS = 640;   // forward only: one more war
 constexpr int SUMS_FLOATS = 2 * TILE * 11;   // per slot: [segment][MAXH]
 constexpr int MAX_STEPS = 64;
 constexpr int COL_X = 0, COL_Z = 64, COL_AHI = 128, COL_ALO = 192, SLOT_COLS = 256;
+constexpr int TMEM_COLS = 2 * SLOT_COLS;   // TMEM columns of the forward and the backward CTA: both slots
 constexpr int MAXH = 11;    // d_ffn / 2: the proj2 operand [t_ref | t_alt | is_ref, is_alt] must fit 24 columns
 constexpr int NP1 = 24;     // padded width of one proj1 weight set (>= 2 * MAXH)
 constexpr int MAXE = 16;    // final feature dimension

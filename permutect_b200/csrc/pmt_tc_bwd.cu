@@ -44,24 +44,6 @@ struct SharedB {
   SlotMeta slot[2];
 };
 
-// SWIZZLE_128B_BASE32B descriptor of an MN-major tf32 operand made of panels: MN atoms (32 features) one panel apart,
-// K atoms (4 rows) 512 bytes apart (profiles/microbench/wgrad_probe.cu)
-__device__ __forceinline__ uint64_t desc_panels(unsigned addr) {
-  return (uint64_t)((addr >> 4) & 0x3FFF) | ((uint64_t)(PANEL_BYTES >> 4) << 16) | ((uint64_t)(512 >> 4) << 32) | (1ull << 46) | (1ull << 61);
-}
-__device__ __forceinline__ void mma_ss(unsigned tmem_d, uint64_t adesc, uint64_t bdesc, unsigned idesc, unsigned accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ float rna(float v) {
-  unsigned r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(v));
-  return __uint_as_float(r);
-}
 __device__ __forceinline__ float du(float a) { return a > 0.f ? 1.f : a + SELU_ALPHA; }   // u'(x) from a = u(x)
 
 template <int NC>
@@ -139,7 +121,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
       mbar_init(smem_addr(&S->act_full[s]), 1); mbar_init(smem_addr(&S->act_free[s]), 9);
     }
     for (int i = 0; i < n_stages; ++i) { mbar_init(smem_addr(&S->wfull[i]), 1); mbar_init(smem_addr(&S->wfree[i]), 2); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
     head_constants(D, W, HC);
   }
   for (int i = tid; i < D.n_blocks * BC_STRIDE; i += THREADS) {
@@ -157,10 +139,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
     else if (c == BC_REGW) v = W[BO.reg_weight] + 0.25f;   // gated_mlp.py:237
     blkc[i] = v;
   }
-  if (warp == MMA_WARP) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_addr(&S->tmem_base)), "r"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-  }
+  if (warp == MMA_WARP) tmem_alloc<TMEM_COLS>(smem_addr(&S->tmem_base));
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -210,7 +189,8 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
     const unsigned tb = tmem_base + s * SLOT_COLS;
     const unsigned bar_a = smem_addr(&S->bar_a[s]), bar_d = smem_addr(&S->bar_d[s]), bar_w = smem_addr(&S->bar_w[s]);
     const unsigned act_full = smem_addr(&S->act_full[s]), act_free = smem_addr(&S->act_free[s]);
-    const uint64_t a_desc = desc_panels(opbuf + s * OPBUF_BYTES), b_desc = desc_panels(opbuf + s * OPBUF_BYTES + 2 * PANEL_BYTES);
+    const uint64_t a_desc = desc_panels(opbuf + s * OPBUF_BYTES, PANEL_BYTES);
+    const uint64_t b_desc = desc_panels(opbuf + s * OPBUF_BYTES + 2 * PANEL_BYTES, PANEL_BYTES);
     int stage = 0;
     unsigned wparity = 0, aparity = 0, fparity = 0;
     for (int round = 0; round < rounds; ++round) {
@@ -245,7 +225,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
           const unsigned idesc = (1u << 4) | (2u << 7) | (2u << 10) | (1u << 15) | (1u << 16) | ((unsigned)(oN >> 3) << 17) | ((128u >> 4) << 24);
 #pragma unroll
           for (int ks = 0; ks < TILE / 8; ++ks)
-            mma_ss(tb + COL_DW, a_desc + (uint64_t)(ks * 64), b_desc + (uint64_t)(ks * 64), idesc, ks > 0 ? 1u : 0u);
+            mma_ss_desc64(tb + COL_DW, a_desc + (uint64_t)(ks * 64), b_desc + (uint64_t)(ks * 64), idesc, ks > 0 ? 1u : 0u);
           mma_commit(bar_w);
           mma_commit(act_free);
         }
@@ -351,7 +331,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
               warp_reduce_red<MAXE>(cs, scal + PMT_MAX_BLOCKS * SCAL_BLOCK, lane);
               named_barrier(pair_bar, 64);
 #pragma unroll
-              for (int e = 0; e < MAXE; ++e) dy[e] = (e < E && real) ? rna(dy[e] + lds_f32(xch + (e * XCH_LD + row) * 4)) : 0.f;
+              for (int e = 0; e < MAXE; ++e) dy[e] = (e < E && real) ? rna_tf32(dy[e] + lds_f32(xch + (e * XCH_LD + row) * 4)) : 0.f;
             } else {
               float dfb[MAXE];
 #pragma unroll
@@ -399,7 +379,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
             load_cols<32>(t_d + half * 32, v);
             unsigned r[32];
 #pragma unroll
-            for (int i = 0; i < 32; ++i) { v[i] = (real && i < n_half) ? v[i] : 0.f; r[i] = __float_as_uint(v[i]); dy[i] = rna(v[i]); }
+            for (int i = 0; i < 32; ++i) { v[i] = (real && i < n_half) ? v[i] : 0.f; r[i] = __float_as_uint(v[i]); dy[i] = rna_tf32(v[i]); }
             tmem_st32(t_g + half * 32, r);
           } break;
           case BE_DZ64:
@@ -420,7 +400,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
                 tmem_st16(t_g + half * 32 + c * 16, r);
               }
 #pragma unroll
-              for (int i = 0; i < 16; ++i) dy[c * 16 + i] = rna(v[i]);
+              for (int i = 0; i < 16; ++i) dy[c * 16 + i] = rna_tf32(v[i]);
             }
           } break;
           case BE_DZ32:
@@ -448,7 +428,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
               }
             }
 #pragma unroll
-            for (int i = 0; i < 16; ++i) dy[i] = rna(v[i]);
+            for (int i = 0; i < 16; ++i) dy[i] = rna_tf32(v[i]);
           } break;
           case BE_LN64:
           case BE_LN_EMBED: {   // LayerNorm of gated block `blk` in reverse (gated_mlp.py:185), added to the residual gradient
@@ -506,7 +486,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
               }
             }
 #pragma unroll
-            for (int i = 0; i < 32; ++i) dy[i] = rna(dy[i]);
+            for (int i = 0; i < 32; ++i) dy[i] = rna_tf32(dy[i]);
           } break;
           case BE_GATE: {   // spatial gating unit in reverse (gated_mlp.py:186-190, 228-251); this thread owns hidden units [k0, k0 + 6)
             const int blk = TP.step[step].blk;
@@ -605,7 +585,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
             for (int j = 0; j < 6; ++j) {
               const bool ok = real && k0 + j < H;
               const float dz2 = ok ? rstd2 * (dxh2[j] - m1 - xh2[j] * m2) * ds2[j] : 0.f;
-              const float a = rna(dz1[j]), b = rna(dz2);
+              const float a = rna_tf32(dz1[j]), b = rna_tf32(dz2);
               dy[j] = is_alt ? 0.f : a; dy[6 + j] = is_alt ? 0.f : b;
               dy[12 + j] = is_alt ? a : 0.f; dy[18 + j] = is_alt ? b : 0.f;
             }
@@ -633,7 +613,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
           default: store_dy<32>(t_dy, dy_s, row, half * 32, dy); break;
         }
         tmem_wait_st();
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(bar_a);
@@ -642,9 +622,7 @@ reads_backward_tc_kernel(const __grid_constant__ PmtModelDesc D, const __grid_co
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == MMA_WARP) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512));
-  }
+  if (warp == MMA_WARP) tmem_dealloc<TMEM_COLS>(tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -671,7 +649,7 @@ __global__ void pack_tc_bwd_kernel(const __grid_constant__ PmtModelDesc D, const
     }
     const unsigned L = (unsigned)n * 128u + (unsigned)kk * 4u;
     const unsigned phys = L ^ (((L >> 7) & 7u) << 4);
-    *reinterpret_cast<float*>(image + (size_t)o.t_img_off + (size_t)kb * o.Nd * 128 + phys) = rna(v);
+    *reinterpret_cast<float*>(image + (size_t)o.t_img_off + (size_t)kb * o.Nd * 128 + phys) = rna_tf32(v);
   }
 }
 

@@ -1,4 +1,5 @@
-// PTX wrappers for the tcgen05 / TMEM / mbarrier / bulk-copy instructions used by the tensor-core kernels (sm_100a).
+// PTX wrappers for the tcgen05 / TMEM / mbarrier / fence / bulk-copy instructions used by the tensor-core kernels, and the
+// shared-memory descriptors of their MMA operands (sm_100a).
 #pragma once
 #include <cstdint>
 
@@ -11,6 +12,9 @@ namespace tc {
 __device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
 }
+__device__ __forceinline__ void fence_mbar_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+// generic-proxy shared-memory writes -> visible to the async proxy (tcgen05.mma operands, bulk copies)
+__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void mbar_arrive(unsigned bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
@@ -42,10 +46,61 @@ __device__ __forceinline__ bool elect_one() {
   asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
   return pred != 0;
 }
+// TMEM allocation of COLS columns for the CTA, written to shared memory at `slot`; called by one whole warp, which also
+// deallocates.  Alloc and dealloc must name the same COLS.
+template <int COLS>
+__device__ __forceinline__ void tmem_alloc(unsigned slot) {
+  static_assert(COLS >= 32 && COLS <= 512 && (COLS & (COLS - 1)) == 0, "TMEM allocations are a power of two, 32 to 512 columns");
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(slot), "r"(COLS));
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
+}
+template <int COLS>
+__device__ __forceinline__ void tmem_dealloc(unsigned base) {
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(COLS));
+}
+
+// ---------------------------------------------------------------- shared-memory descriptors
 __device__ __forceinline__ uint64_t smem_desc(unsigned addr) {
   // K-major, SWIZZLE_128B: 8-row groups 1024 B apart, descriptor version 1 (sm_100)
   return (uint64_t)((addr >> 4) & 0x3FFF) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
 }
+// K-major, no swizzle.  Low word: start address >> 4 | (LBO >> 4) << 16 with LBO = the distance between K-adjacent core
+// matrices; high word (constant): SBO = 128 B between 8-row groups, descriptor version 1.
+constexpr unsigned DESC_HI = 8u | (1u << 14);
+__device__ __forceinline__ unsigned desc_lo(unsigned addr, unsigned lbo_bytes) { return ((addr >> 4) & 0x3FFFu) | ((lbo_bytes >> 4) << 16); }
+// MN-major tf32 operand made of panels, SWIZZLE_128B_BASE32B: MN atoms (32 features) panel_bytes apart, K atoms (4 rows)
+// 512 bytes apart (profiles/microbench/wgrad_probe.cu)
+__device__ __forceinline__ uint64_t desc_panels(unsigned addr, unsigned panel_bytes) {
+  return (uint64_t)((addr >> 4) & 0x3FFF) | ((uint64_t)(panel_bytes >> 4) << 16) | ((uint64_t)(512 >> 4) << 32) | (1ull << 46) | (1ull << 61);
+}
+// Instruction descriptor of kind::tf32, M = 128, N columns: fp32 accumulator, both operands K-major
+__host__ __device__ constexpr unsigned make_idesc(int N) {
+  return (1u << 4) | (2u << 7) | (2u << 10) | ((unsigned)(N >> 3) << 17) | ((128u >> 4) << 24);
+}
+
+// ---------------------------------------------------------------- MMAs (kind::tf32, accumulate into TMEM unless accumulate == 0)
+// A and B in shared memory, given by the low words of no-swizzle descriptors (desc_lo; high word DESC_HI)
+template <unsigned IDESC>
+__device__ __forceinline__ void mma_ss_desc_lo(unsigned tmem_d, unsigned a_lo32, unsigned b_lo32, unsigned accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
+      "setp.ne.b32 p, %3, 0;\n\t"
+      "mov.b64 da, {%1, %4};\n\t"
+      "mov.b64 db, {%2, %4};\n\t"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], da, db, %5, p;\n\t}" ::"r"(tmem_d),
+      "r"(a_lo32), "r"(b_lo32), "r"(accumulate), "n"(DESC_HI), "n"(IDESC)
+      : "memory");
+}
+// A and B in shared memory, given by full 64-bit descriptors
+__device__ __forceinline__ void mma_ss_desc64(unsigned tmem_d, uint64_t adesc, uint64_t bdesc, unsigned idesc, unsigned accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+// A in TMEM, B in shared memory (64-bit descriptor)
 __device__ __forceinline__ void mma_ts(unsigned tmem_d, unsigned tmem_a, uint64_t bdesc, unsigned idesc, unsigned accumulate) {
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
