@@ -450,6 +450,24 @@ int pmt_posterior_fit_pass_many(const PmtPosteriorFitProblem* h_problems, int32_
  * query needs the device the passes would run on. */
 int pmt_posterior_fit_ctas(const PmtPosteriorFitProblem* h_problems, int32_t n_problems);
 
+/* The context-dependent SNV-prior fit of the posterior model's M step (architecture/snv_context_priors.py,
+ * fit_mutation_rates_sc) for n independent problems in one launch, one CTA each, float64 throughout: the mean-field fit
+ * of the hierarchical substitution x context model to problem i's rounded totals by the algorithm of torch.optim.LBFGS
+ * (strong-Wolfe line search, max_iter 300) over the sample-average ELBO of the 64 draws `elbo_draws`, then
+ * rates_out[i][12][16] = E_q[rate_sc], the mean over the 1000 draws `mean_draws`.  total_sc, snv_sc: contiguous
+ * [n][12][16] (snv is clamped to total, as the host fit does); elbo_draws [64][194] and mean_draws [1000][194]: the
+ * standard-normal tables of the host fit (_sobol_normal(64, 194, 1234) and _sobol_normal(1000, 194, 4321)).  Optional
+ * outputs (may be NULL): mu_out, log_sigma_out [n][194], the fitted variational parameters; n_iter_out,
+ * func_evals_out [n], the optimiser's iteration and objective-evaluation counts.  Every reduction has a fixed order and
+ * problems do not interact: problem i gives the same bits whatever else is in the launch.  workspace:
+ * pmt_snv_context_fit_workspace_size(n) bytes (0 for n < 1), the problems' L-BFGS histories.  Refused before anything
+ * is enqueued: n < 1, a NULL required pointer, a short workspace. */
+size_t pmt_snv_context_fit_workspace_size(int32_t n);
+int pmt_snv_context_fit_many(int32_t n, const double* total_sc, const double* snv_sc, const double* elbo_draws,
+                             const double* mean_draws, double* rates_out, double* mu_out, double* log_sigma_out,
+                             int32_t* n_iter_out, int32_t* func_evals_out, void* workspace, size_t workspace_bytes,
+                             void* stream);
+
 /* ---- batch assembly from the dataset memory maps ----------------------------------------------------
  * Replaces the row re-stacking of Batch.__init__ (batch.py:41-62) for batches cut from a MemoryMappedData
  * (memory_mapped_data.py:36-58, reads_dataset.py:109-196): the reads memory map holds, variant after variant, the ref

@@ -11,7 +11,8 @@ launch of pmt_posterior_fit_pass and only the M step stays on the host.  ``learn
 samples' models side by side, a pass of all of them per launch of pmt_posterior_fit_pass_many.  Context-dependent
 SNV priors are switched on for the second half of the iterations as in the reference (:125-127); its M step for them, a
 PyMC ADVI fit (posterior_model_priors.py:157-203), is replaced by a deterministic fit of the same model and variational
-family (architecture/snv_context_priors.py; pymc is absent from the image, so that one step has no reference golden).
+family (architecture/snv_context_priors.py; pymc is absent from the image, so that one step has no reference golden),
+on the host by default or, with ``context_fit="device"``, as one kernel launch for all models of an iteration.
 ``calculate_probability_thresholds`` (posterior_model.py:171-264) returns the same thresholds; its ROC plots are not
 drawn.  There is no CPU path for the model itself.
 """
@@ -25,7 +26,8 @@ from torch.nn import Parameter
 from torch.nn.utils import parametrize
 
 from permutect_b200.architecture.layers import BoundedNumber, LogWeights, PositiveNumber
-from permutect_b200.architecture.snv_context_priors import ContextFitPool, context_fit_inputs, fit_mutation_rates_sc, write_log_rates
+from permutect_b200.architecture.snv_context_priors import (ContextFitPool, context_fit_inputs, fit_mutation_rates_sc,
+                                                            fit_mutation_rates_sc_on_device, write_log_rates)
 from permutect_b200.data.datum import HAPLOTYPES_START_IDX
 from permutect_b200.engine import library as L
 from permutect_b200.utils.enums import Variation
@@ -216,19 +218,26 @@ class PosteriorModel(nn.Module):
         return _EvidenceLoss.apply(loss, grads, *self._spectra_tensors())
 
     def update_priors_m_step(self, posterior_totals_vc: Tensor, ignored_to_non_ignored_ratio: float,
-                             somatic_snv_totals_rrra: Optional[Tensor] = None, snv_context_totals_rrra: Optional[Tensor] = None):
+                             somatic_snv_totals_rrra: Optional[Tensor] = None, snv_context_totals_rrra: Optional[Tensor] = None,
+                             context_fit: str = "host"):
         """posterior_model_priors.py:141-224.  With context-dependent SNV priors switched on and both rrra totals given,
         ``somatic_snv_log_priors_rrra`` gets the log mutation rates of the hierarchical substitution x context model
-        (snv_context_priors.context_m_step); otherwise it is filled with the SNV somatic log prior (:223-225)."""
+        (snv_context_priors.context_m_step; ``context_fit="device"`` fits it on the totals' device); otherwise it is
+        filled with the SNV somatic log prior (:223-225)."""
+        _check_context_fit(context_fit)
+        on_device = context_fit == "device"
         fit_inputs = self._m_step_before_context_fit(posterior_totals_vc, ignored_to_non_ignored_ratio, somatic_snv_totals_rrra,
-                                                     snv_context_totals_rrra)
+                                                     snv_context_totals_rrra, on_device)
         if fit_inputs is not None:
-            write_log_rates(self.priors.somatic_snv_log_priors_rrra, fit_mutation_rates_sc(*fit_inputs))
+            rates_sc = (fit_mutation_rates_sc_on_device([fit_inputs], fit_inputs[0].device)[0] if on_device
+                        else fit_mutation_rates_sc(*fit_inputs))
+            write_log_rates(self.priors.somatic_snv_log_priors_rrra, rates_sc)
 
     def _m_step_before_context_fit(self, posterior_totals_vc: Tensor, ignored_to_non_ignored_ratio: float,
-                                   somatic_snv_totals_rrra: Optional[Tensor], snv_context_totals_rrra: Optional[Tensor]):
-        """update_priors_m_step up to its context fit: returns that fit's inputs (snv_context_priors.context_fit_inputs) when
-        the context-dependent SNV priors are on, else None with the M step done."""
+                                   somatic_snv_totals_rrra: Optional[Tensor], snv_context_totals_rrra: Optional[Tensor],
+                                   on_device: bool = False):
+        """update_priors_m_step up to its context fit: returns that fit's inputs (snv_context_priors.context_fit_inputs, on
+        the totals' device with ``on_device``) when the context-dependent SNV priors are on, else None with the M step done."""
         total_nonignored = torch.sum(posterior_totals_vc)
         overall_total = (1 + ignored_to_non_ignored_ratio) * total_nonignored
         with torch.no_grad():
@@ -240,18 +249,22 @@ class PosteriorModel(nn.Module):
                 if somatic_snv_totals_rrra is None or snv_context_totals_rrra is None:
                     raise ValueError("context-dependent SNV priors are on: the M step needs both rrra totals")
                 total_ignored_per_context = float(ignored_to_non_ignored_ratio * total_nonignored) / 64      # :150-153
-                return context_fit_inputs(somatic_snv_totals_rrra, snv_context_totals_rrra, total_ignored_per_context)
+                return context_fit_inputs(somatic_snv_totals_rrra, snv_context_totals_rrra, total_ignored_per_context, on_device)
             pri.somatic_snv_log_priors_rrra.fill_(pri.log_priors_vc[int(Variation.SNV), CALL_SOMATIC])
             return None
 
     def learn_priors_and_spectra(self, posterior_loader, num_iterations, ignored_to_non_ignored_ratio: float, summary_writer=None,
-                                 learning_rate: float = 0.001):
+                                 learning_rate: float = 0.001, context_fit: str = "host"):
         """posterior_model.py:101-165: Adam on the spectra against the negative log evidence (E step, one kernel per
         batch), then the priors' M step; context-dependent SNV priors from the second half of the iterations on.
         ``posterior_loader`` yields batches of posterior records on the model's device; a ``PosteriorRecords`` there has
-        every pass run as one kernel (``_learn_on_device``).  Returns the mean loss of every iteration."""
+        every pass run as one kernel (``_learn_on_device``).  ``context_fit``: where the M step's context fit runs,
+        "host" (float64 L-BFGS on the CPU) or "device" (pmt_snv_context_fit_many on the records' device; the same method,
+        fitted rates equal to rounding).  Returns the mean loss of every iteration."""
+        _check_context_fit(context_fit)
         if isinstance(posterior_loader, PosteriorRecords) and _same_device(posterior_loader.device, self._device):
-            return self._learn_on_device(posterior_loader, num_iterations, ignored_to_non_ignored_ratio, summary_writer, learning_rate)
+            return self._learn_on_device(posterior_loader, num_iterations, ignored_to_non_ignored_ratio, summary_writer, learning_rate,
+                                         context_fit)
         optimizer = torch.optim.Adam(self.spectra.parameters(), lr=learning_rate)
         self.priors.disable_context_dependent_snv_priors()
         history = []
@@ -270,7 +283,7 @@ class PosteriorModel(nn.Module):
                 optimizer.step()
                 loss_sum += loss.detach() * batch.size()
                 count += batch.size()
-            self.update_priors_m_step(totals_tc, ignored_to_non_ignored_ratio, somatic_snv_rrra, snv_context_rrra)
+            self.update_priors_m_step(totals_tc, ignored_to_non_ignored_ratio, somatic_snv_rrra, snv_context_rrra, context_fit)
             history.append(float(loss_sum) / max(count, 1))
             if summary_writer is not None:
                 summary_writer.add_scalar("spectrum negative log evidence", history[-1], epoch)
@@ -285,7 +298,7 @@ class PosteriorModel(nn.Module):
                 na.parametrizations.mean_multiplier_v.original, na.parametrizations.concentration_v.original]
 
     def _learn_on_device(self, records: "PosteriorRecords", num_iterations, ignored_to_non_ignored_ratio: float, summary_writer,
-                         learning_rate: float):
+                         learning_rate: float, context_fit: str = "host"):
         """learn_priors_and_spectra with one pmt_posterior_fit_pass per iteration: the batches of ``records`` in order,
         each an E step and an Adam step of the raw spectra (the loop's fresh optimiser: zero moments, step 0, in flat
         device buffers for the call), then the same M step.  The raw parameters go back into the module after every pass."""
@@ -301,7 +314,8 @@ class PosteriorModel(nn.Module):
                                                p.batch_size, p.batch_losses_out, p.posterior_totals_tc, p.somatic_snv_totals_rrra,
                                                p.snv_context_totals_rrra, ws.data_ptr(), ws.numel(), stream))
             fit.end_pass()
-            self.update_priors_m_step(fit.totals_tc, ignored_to_non_ignored_ratio, fit.somatic_snv_rrra, fit.snv_context_rrra)
+            self.update_priors_m_step(fit.totals_tc, ignored_to_non_ignored_ratio, fit.somatic_snv_rrra, fit.snv_context_rrra,
+                                      context_fit)
             fit.record(epoch, summary_writer)
         return fit.history
 
@@ -365,23 +379,31 @@ def _per_model(value, n: int, what: str) -> List[float]:
     return values
 
 
+def _check_context_fit(context_fit) -> None:
+    if context_fit not in ("host", "device"):
+        raise ValueError(f'context_fit must be "host" or "device", got {context_fit!r}')
+
+
 def _usable_cpus() -> int:
     return len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
 
 
 def learn_priors_and_spectra_together(models: Sequence[PosteriorModel], records: Sequence["PosteriorRecords"], num_iterations: int,
                                       ignored_to_non_ignored_ratio: Union[float, Sequence[float]], summary_writers=None,
-                                      learning_rate: Union[float, Sequence[float]] = 0.001) -> List[List[float]]:
+                                      learning_rate: Union[float, Sequence[float]] = 0.001, context_fit: str = "host") -> List[List[float]]:
     """``models[i].learn_priors_and_spectra(records[i], ...)`` for every i, the fits side by side: a cohort's samples
     (tumour / normal pairs, the folds of an evaluation) each have their own model and records, and each fit is a chain of
     Adam steps that keeps at most 16 SMs busy, so every pass over all models is ONE pmt_posterior_fit_pass_many launch with
     a cluster of CTAs per model (one CTA each from as many models as SMs on).  Between passes each model takes the M step of ``_learn_on_device``; the float64 context fits of the
-    second half run in a pool of worker processes (snv_context_priors.ContextFitPool) when there are several models.
+    second half run in a pool of worker processes (snv_context_priors.ContextFitPool) when there are several models, or
+    with ``context_fit="device"`` as one pmt_snv_context_fit_many launch per iteration for every model that needs one.
     Every model ends with the parameters, and every history equals the history, of its own ``learn_priors_and_spectra``.
 
     ``records[i]`` is a ``PosteriorRecords`` (its own batch size); all models and records on one CUDA device.
     ``ignored_to_non_ignored_ratio`` and ``learning_rate``: one value for all or one per model; ``summary_writers``: None
     or one writer (or None) per model.  Returns one history per model."""
+    _check_context_fit(context_fit)
+    on_device = context_fit == "device"
     models, records = list(models), list(records)
     n = len(models)
     if n == 0:
@@ -404,7 +426,7 @@ def learn_priors_and_spectra_together(models: Sequence[PosteriorModel], records:
     max_k = max(m.spectra.somatic_spectrum.K for m in models)
     ws = torch.empty(int(lib.pmt_posterior_fit_pass_many_workspace_size(n, max_k)), dtype=torch.uint8, device=dev)
     stream = torch.cuda.current_stream(dev).cuda_stream
-    workers = min(n, _usable_cpus())
+    workers = 1 if on_device else min(n, _usable_cpus())
     pool = ContextFitPool(workers) if workers > 1 else None
     try:
         for epoch in range(1, num_iterations + 1):
@@ -413,11 +435,17 @@ def learn_priors_and_spectra_together(models: Sequence[PosteriorModel], records:
             fit_inputs = []
             for f, ratio in zip(fits, ratios):
                 f.end_pass()
-                fit_inputs.append(f.model._m_step_before_context_fit(f.totals_tc, ratio, f.somatic_snv_rrra, f.snv_context_rrra))
+                fit_inputs.append(f.model._m_step_before_context_fit(f.totals_tc, ratio, f.somatic_snv_rrra, f.snv_context_rrra,
+                                                                     on_device))
             pending = [(f, x) for f, x in zip(fits, fit_inputs) if x is not None]
             if pending:
                 inputs = [x for _, x in pending]
-                fitted = pool.map(inputs) if pool is not None and len(inputs) > 1 else [fit_mutation_rates_sc(*x) for x in inputs]
+                if on_device:
+                    fitted = fit_mutation_rates_sc_on_device(inputs, dev)
+                elif pool is not None and len(inputs) > 1:
+                    fitted = pool.map(inputs)
+                else:
+                    fitted = [fit_mutation_rates_sc(*x) for x in inputs]
                 for (f, _), rates_sc in zip(pending, fitted):
                     write_log_rates(f.model.priors.somatic_snv_log_priors_rrra, rates_sc)
             for f, w in zip(fits, writers):

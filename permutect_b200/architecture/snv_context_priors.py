@@ -21,7 +21,9 @@ tests hold it to the model's own limits (large counts: rate -> snv / total; empt
 mean) and to the reference's index conventions (``convert_rrra_tensor_to_sc``, :39-60; the write-back loop :210-222).
 
 Host side (float64, 194 variational means + 194 scales), like the PyMC fit it replaces: the E step that produces the two
-5x5x5x5 totals is the CUDA kernel ``pmt_posterior_fit_step``.
+5x5x5x5 totals is the CUDA kernel ``pmt_posterior_fit_step``.  ``fit_mutation_rates_sc_on_device`` runs the same method
+-- same start, same draws, the same L-BFGS algorithm with a hand-written gradient -- for many models in one launch of
+pmt_snv_context_fit_many (csrc/pmt_context_fit.cu); its results agree with the host fit's to rounding.
 """
 import math
 import multiprocessing
@@ -90,12 +92,27 @@ def _log_joint(z: Tensor, total_sc: Tensor, snv_sc: Tensor) -> Tuple[Tensor, Ten
     return lp, torch.exp(log_rate)
 
 
+DIM = 3 + (NUM_SUBSTITUTIONS - 1) + NUM_SUBSTITUTIONS * (NUM_CONTEXTS - 1)   # 194 unconstrained coordinates
+_ELBO_SEED, _MEAN_SEED = 1234, 4321
+
+
+def _clamped_inputs(total_sc: Tensor, snv_sc: Tensor) -> Tuple[Tensor, Tensor]:
+    total = total_sc.detach().double().cpu().reshape(NUM_SUBSTITUTIONS, NUM_CONTEXTS)
+    return total, torch.minimum(snv_sc.detach().double().cpu().reshape(NUM_SUBSTITUTIONS, NUM_CONTEXTS), total)
+
+
 def fit_mutation_rates_sc(total_sc: Tensor, snv_sc: Tensor, max_iter: int = 300) -> Tensor:
     """E_q[rate_sc] [12, 16] (float64, CPU) of the mean-field fit described in the module docstring.  ``total_sc`` and
     ``snv_sc`` are the integer-rounded totals the reference hands to its Binomial (:158-159)."""
-    total = total_sc.detach().double().cpu().reshape(NUM_SUBSTITUTIONS, NUM_CONTEXTS)
-    snv = torch.minimum(snv_sc.detach().double().cpu().reshape(NUM_SUBSTITUTIONS, NUM_CONTEXTS), total)
-    dim = 3 + (NUM_SUBSTITUTIONS - 1) + NUM_SUBSTITUTIONS * (NUM_CONTEXTS - 1)
+    mu, log_sigma, _, _ = fit_variational_sc(total_sc, snv_sc, max_iter)
+    return mean_rates_sc(mu, log_sigma, total_sc, snv_sc)
+
+
+def fit_variational_sc(total_sc: Tensor, snv_sc: Tensor, max_iter: int = 300) -> Tuple[Tensor, Tensor, int, int]:
+    """The host fit's variational parameters (mu [194], log_sigma [194], float64) and its L-BFGS iteration and
+    objective-evaluation counts."""
+    total, snv = _clamped_inputs(total_sc, snv_sc)
+    dim = DIM
     # start at the smoothed maximum-likelihood point
     overall = float((snv.sum() + 1.0) / (total.sum() + 1e6))
     ts = (snv.sum(1) + 1.0) / (snv.sum() + NUM_SUBSTITUTIONS)
@@ -104,7 +121,7 @@ def fit_mutation_rates_sc(total_sc: Tensor, snv_sc: Tensor, max_iter: int = 300)
     mu = torch.cat([torch.tensor([math.log(overall) - math.log1p(-overall), 0.0, 0.0], dtype=torch.float64),
                     simplex_fwd(ts), simplex_fwd(tsc).reshape(-1)]).requires_grad_(True)
     log_sigma = torch.full((dim,), -2.0, dtype=torch.float64, requires_grad=True)
-    eps = _sobol_normal(_ELBO_DRAWS, dim, seed=1234)
+    eps = _sobol_normal(_ELBO_DRAWS, dim, seed=_ELBO_SEED)
     opt = torch.optim.LBFGS([mu, log_sigma], lr=1.0, max_iter=max_iter, tolerance_grad=1e-9, tolerance_change=1e-12,
                             history_size=100, line_search_fn="strong_wolfe")
 
@@ -117,17 +134,26 @@ def fit_mutation_rates_sc(total_sc: Tensor, snv_sc: Tensor, max_iter: int = 300)
         return loss
 
     opt.step(closure)
+    state = opt.state[mu]
+    return mu.detach(), log_sigma.detach(), int(state["n_iter"]), int(state["func_evals"])
+
+
+def mean_rates_sc(mu: Tensor, log_sigma: Tensor, total_sc: Tensor, snv_sc: Tensor) -> Tensor:
+    """E_q[rate_sc] [12, 16]: the mean of rate_sc over the 1000 fixed draws from the Gaussian (mu, exp(log_sigma))."""
+    total, snv = _clamped_inputs(total_sc, snv_sc)
     with torch.no_grad():
-        z = mu + torch.exp(log_sigma) * _sobol_normal(_MEAN_DRAWS, dim, seed=4321)
+        z = mu.detach().double().cpu() + torch.exp(log_sigma.detach().double().cpu()) * _sobol_normal(_MEAN_DRAWS, DIM, seed=_MEAN_SEED)
         _, rate = _log_joint(z, total, snv)
         return rate.mean(0)
 
 
 def context_fit_inputs(somatic_snv_totals_rrra: Tensor, snv_context_totals_rrra: Tensor,
-                       total_ignored_per_context: float) -> Tuple[Tensor, Tensor]:
-    """(total_sc, snv_sc): the E-step totals rounded as the reference rounds them for its Binomial (:158-159)."""
-    total_sc = torch.round(convert_rrra_tensor_to_sc(snv_context_totals_rrra.detach().double().cpu()) + total_ignored_per_context)
-    snv_sc = torch.round(convert_rrra_tensor_to_sc(somatic_snv_totals_rrra.detach().double().cpu()))
+                       total_ignored_per_context: float, on_device: bool = False) -> Tuple[Tensor, Tensor]:
+    """(total_sc, snv_sc): the E-step totals rounded as the reference rounds them for its Binomial (:158-159).  On the
+    CPU, or with ``on_device`` on the totals' device: the same float64 add and rounding, so the same bits either way."""
+    where = (lambda t: t) if on_device else (lambda t: t.cpu())
+    total_sc = torch.round(convert_rrra_tensor_to_sc(where(snv_context_totals_rrra.detach().double())) + total_ignored_per_context)
+    snv_sc = torch.round(convert_rrra_tensor_to_sc(where(somatic_snv_totals_rrra.detach().double())))
     return total_sc, snv_sc
 
 
@@ -178,3 +204,54 @@ class ContextFitPool:
 
     def close(self) -> None:
         self._pool.shutdown()
+
+
+_DRAW_TABLES = {}
+
+
+def draw_tables(device) -> Tuple[Tensor, Tensor]:
+    """The host fit's two standard-normal tables, [64, 194] for the ELBO and [1000, 194] for the rates' mean, as
+    contiguous float64 on ``device``; computed once per device."""
+    device = torch.device(device)
+    if device.type == "cuda" and device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    if device not in _DRAW_TABLES:
+        _DRAW_TABLES[device] = (_sobol_normal(_ELBO_DRAWS, DIM, seed=_ELBO_SEED).to(device).contiguous(),
+                                _sobol_normal(_MEAN_DRAWS, DIM, seed=_MEAN_SEED).to(device).contiguous())
+    return _DRAW_TABLES[device]
+
+
+def fit_context_models_on_device(total_sc: Tensor, snv_sc: Tensor, device=None) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """The fits of n models' totals ([n, 12, 16] each) in one launch of pmt_snv_context_fit_many on ``device`` (default:
+    the totals' device).  Returns, on that device, rates [n, 12, 16] (E_q[rate_sc]), mu and log_sigma [n, 194], and the
+    L-BFGS iteration and objective-evaluation counts [n] (int32)."""
+    from permutect_b200.engine import library as L
+    dev = torch.device(device) if device is not None else total_sc.device
+    if dev.type != "cuda":
+        raise RuntimeError("the device context fit runs on a CUDA device (the host fit is fit_mutation_rates_sc)")
+    total = total_sc.detach().to(device=dev, dtype=torch.float64).reshape(-1, NUM_SUBSTITUTIONS, NUM_CONTEXTS).contiguous()
+    snv = snv_sc.detach().to(device=dev, dtype=torch.float64).reshape(-1, NUM_SUBSTITUTIONS, NUM_CONTEXTS).contiguous()
+    if total.shape != snv.shape:
+        raise ValueError(f"total_sc {tuple(total.shape)} and snv_sc {tuple(snv.shape)} differ")
+    n = total.shape[0]
+    elbo, mean = draw_tables(dev)
+    rates = torch.empty((n, NUM_SUBSTITUTIONS, NUM_CONTEXTS), dtype=torch.float64, device=dev)
+    mu, log_sigma = (torch.empty((n, DIM), dtype=torch.float64, device=dev) for _ in range(2))
+    n_iter, func_evals = (torch.empty(n, dtype=torch.int32, device=dev) for _ in range(2))
+    lib = L.load()
+    ws = torch.empty(int(lib.pmt_snv_context_fit_workspace_size(max(n, 1))), dtype=torch.uint8, device=dev)
+    L.check(lib.pmt_snv_context_fit_many(n, total.data_ptr(), snv.data_ptr(), elbo.data_ptr(), mean.data_ptr(), rates.data_ptr(),
+                                         mu.data_ptr(), log_sigma.data_ptr(), n_iter.data_ptr(), func_evals.data_ptr(),
+                                         ws.data_ptr(), ws.numel(), torch.cuda.current_stream(dev).cuda_stream))
+    return rates, mu, log_sigma, n_iter, func_evals
+
+
+def fit_mutation_rates_sc_on_device(inputs: Sequence[Tuple[Tensor, Tensor]], device) -> List[Tensor]:
+    """[E_q[rate_sc] of (total_sc, snv_sc) for (total_sc, snv_sc) in inputs] -- the contract of ContextFitPool.map, float64
+    [12, 16] CPU tensors -- from one launch of the device fit on ``device``."""
+    if len(inputs) == 0:
+        return []
+    total = torch.stack([t.detach().to(device=device, dtype=torch.float64).reshape(NUM_SUBSTITUTIONS, NUM_CONTEXTS) for t, _ in inputs])
+    snv = torch.stack([s.detach().to(device=device, dtype=torch.float64).reshape(NUM_SUBSTITUTIONS, NUM_CONTEXTS) for _, s in inputs])
+    rates = fit_context_models_on_device(total, snv, device)[0].cpu()
+    return list(rates.unbind(0))

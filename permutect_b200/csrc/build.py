@@ -8,7 +8,7 @@ import subprocess
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-SOURCES = ["pmt_call.cu", "pmt_forward.cu", "pmt_backward.cu", "pmt_loader.cu", "pmt_tc.cu", "pmt_tc_bwd.cu", "pmt_cnn_tc.cu", "pmt_cnn_bwd.cu", "pmt_head_bwd.cu", "pmt_loss.cu", "pmt_optim.cu", "pmt_posterior.cu"]
+SOURCES = ["pmt_call.cu", "pmt_forward.cu", "pmt_backward.cu", "pmt_loader.cu", "pmt_tc.cu", "pmt_tc_bwd.cu", "pmt_cnn_tc.cu", "pmt_cnn_bwd.cu", "pmt_head_bwd.cu", "pmt_loss.cu", "pmt_optim.cu", "pmt_posterior.cu", "pmt_context_fit.cu"]
 HEADERS = ["pmt_device.cuh", "pmt_tile.cuh", "pmt_cnn.cuh", "pmt_host.h", "pmt_tc_ptx.cuh", "pmt_tc.cuh", "pmt_cnn_tc.cuh", "pmt_call.h", os.path.join("..", "..", "include", "permutect_b200.h")]
 OUTPUT = os.path.join(HERE, "libpermutect_b200.so")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-shared",

@@ -96,7 +96,7 @@ EXPORTED_SYMBOLS = ["pmt_posterior_fit_step", "pmt_posterior_fit_workspace_size"
                     "pmt_posterior_fit_pass_workspace_size", "pmt_posterior_fit_pass_many", "pmt_posterior_fit_pass_many_workspace_size",
                     "pmt_posterior_fit_ctas", "pmt_orthogonal_forward", "pmt_orthogonal_backward", "pmt_posterior_param_count", "pmt_posterior_log_posteriors", "pmt_dataset_read_indices", "pmt_pack_posterior", "pmt_adamw_step", "pmt_adamw_workspace_size", "pmt_losses_forward", "pmt_losses_backward", "pmt_losses_workspace_size", "pmt_last_error", "pmt_abi_version", "pmt_workspace_size", "pmt_forward", "pmt_forward_prepared", "pmt_backward",
                     "pmt_decode_reads", "pmt_set_profile_events", "pmt_downsample_counts", "pmt_downsample_fill", "pmt_set_precision", "pmt_get_precision", "pmt_constraints_forward", "pmt_constraints_backward", "pmt_backward_kernels", "pmt_train_saved_bytes", "pmt_forward_train",
-                    "pmt_head_backward_workspace_size", "pmt_head_backward"]
+                    "pmt_head_backward_workspace_size", "pmt_head_backward", "pmt_snv_context_fit_many", "pmt_snv_context_fit_workspace_size"]
 
 class PmtPosteriorDesc(C.Structure):
     _fields_ = [("n_components", C.c_int32), ("hap_start", C.c_int32), ("hap_len", C.c_int32), ("no_germline_mode", C.c_int32),
@@ -211,6 +211,11 @@ def load():
     lib.pmt_posterior_fit_pass_many.argtypes = [C.POINTER(PmtPosteriorFitProblem), C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]
     lib.pmt_posterior_fit_ctas.restype = C.c_int
     lib.pmt_posterior_fit_ctas.argtypes = [C.POINTER(PmtPosteriorFitProblem), C.c_int32]
+    lib.pmt_snv_context_fit_workspace_size.restype = C.c_size_t
+    lib.pmt_snv_context_fit_workspace_size.argtypes = [C.c_int32]
+    lib.pmt_snv_context_fit_many.restype = C.c_int
+    lib.pmt_snv_context_fit_many.argtypes = [C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
     lib.pmt_posterior_param_count.restype = C.c_int
     lib.pmt_posterior_param_count.argtypes = [C.c_int32]
     lib.pmt_posterior_log_posteriors.restype = C.c_int
