@@ -1,6 +1,7 @@
 """CPU restatement of PosteriorModel.log_posterior_and_ingredients (test infrastructure; SURVEY §8 f3).
 
-Follows, in torch float32 on the CPU:
+Follows, in torch float32 on the CPU (or in float64 with ``dtype=torch.float64``: the parameters and the float block,
+fp16 or fp32, are widened exactly and every constant and intermediate is float64):
   permutect/architecture/posterior_model.py:69-99            log posteriors = priors + spectra + normal + artifact logit
   permutect/architecture/posterior_model_priors.py:22-31,121-139   context-dependent log priors, log_softmax over calls
   permutect/architecture/spectra/posterior_model_spectra.py:18-124  germline likelihood, assembly of the [B, 5] tables
@@ -35,16 +36,16 @@ def beta_binomial_log_lk(n, k, alpha, beta):                                   #
             - lgamma(alpha) - lgamma(beta))
 
 
-def uniform_binomial_log_lk(n, k, x1, x2):                                     # stats_utils.py:181-198
-    interp = torch.arange(start=0.001, end=0.999, step=0.01)
+def uniform_binomial_log_lk(n, k, x1, x2, dtype=torch.float32):                # stats_utils.py:181-198
+    interp = torch.arange(start=0.001, end=0.999, step=0.01, dtype=dtype)
     p = x2.unsqueeze(-1) * interp + x1.unsqueeze(-1) * (1 - interp)
     lk = binomial_log_lk(n.unsqueeze(-1), k.unsqueeze(-1), p)
     return torch.logsumexp(lk, dim=-1) - math.log(len(interp))
 
 
-def constrained(sd: Dict[str, Tensor]) -> Dict[str, Tensor]:
+def constrained(sd: Dict[str, Tensor], dtype=torch.float32) -> Dict[str, Tensor]:
     """The tensors the reference's forward sees: parametrisations applied (parameterizations.py)."""
-    g = lambda k: sd[k].float() if isinstance(sd[k], Tensor) else torch.as_tensor(np.asarray(sd[k]), dtype=torch.float32)
+    g = lambda k: sd[k].to(dtype) if isinstance(sd[k], Tensor) else torch.as_tensor(np.asarray(sd[k]), dtype=dtype)
     s = "spectra."
     return dict(
         cf_k=torch.sigmoid(g(s + "somatic_spectrum.parametrizations.cf_k.original")),                  # BoundedNumber(0, 1)
@@ -64,7 +65,7 @@ def depth_bins(depths):                                                         
     return (depths >= 10).long() + (depths >= 20).long()
 
 
-def germline_log_likelihood(afs, mafs, alt, depths, het_beta):                  # posterior_model_spectra.py:18-58
+def germline_log_likelihood(afs, mafs, alt, depths, het_beta, dtype=torch.float32):   # posterior_model_spectra.py:18-58
     het_probs = 2 * afs * (1 - afs)
     hom_probs = afs * afs
     het_prop = het_probs / (het_probs + hom_probs)
@@ -75,16 +76,18 @@ def germline_log_likelihood(afs, mafs, alt, depths, het_beta):                  
         minor = comb + alt * torch.log(mafs) + ref * torch.log(1 - mafs)
         major = comb + ref * torch.log(mafs) + alt * torch.log(1 - mafs)
     else:
-        hb = torch.tensor([het_beta])
+        hb = torch.tensor([het_beta], dtype=dtype)
         minor = major = beta_binomial_log_lk(depths, alt, hb, hb)
     half = torch.log(het_prop / 2)
-    hom = torch.log(hom_prop) + beta_binomial_log_lk(depths, alt, torch.tensor([98.0]), torch.tensor([2.0]))
+    hom = torch.log(hom_prop) + beta_binomial_log_lk(depths, alt, torch.tensor([98.0], dtype=dtype),
+                                                         torch.tensor([2.0], dtype=dtype))
     return torch.logsumexp(torch.vstack((half + minor, half + major, hom)), dim=0)
 
 
 def log_posterior_and_ingredients(sd, int_array: np.ndarray, float_array: np.ndarray, no_germline_mode: bool = False,
-                                  het_beta=None, use_context_dependent_snv_priors: bool = True):
-    return tables(constrained(sd), int_array, float_array, no_germline_mode, het_beta, use_context_dependent_snv_priors)
+                                  het_beta=None, use_context_dependent_snv_priors: bool = True, dtype=torch.float32):
+    return tables(constrained(sd, dtype), int_array, float_array, no_germline_mode, het_beta, use_context_dependent_snv_priors,
+                  dtype)
 
 
 SPECTRA_RAW = {"cf_k": "spectra.somatic_spectrum.parametrizations.cf_k.original",
@@ -98,17 +101,17 @@ SPECTRA_RAW = {"cf_k": "spectra.somatic_spectrum.parametrizations.cf_k.original"
 
 
 def negative_log_evidence_and_grads(sd, int_array, float_array, no_germline_mode=False, het_beta=None,
-                                    use_context_dependent_snv_priors=True):
+                                    use_context_dependent_snv_priors=True, dtype=torch.float32):
     """The loss of learn_priors_and_spectra (posterior_model.py:139-146: -mean logsumexp of the log posteriors) with its
     gradients by autograd through this restatement: (loss, d/d constrained tensor, d/d raw parameter = what
     ``loss.backward()`` leaves in ``.grad`` of the spectra parameters)."""
-    leaf = {k: (torch.as_tensor(np.asarray(v), dtype=torch.float32).clone().requires_grad_(k in SPECTRA_RAW.values())
-                if not isinstance(v, Tensor) else v.detach().float().clone().requires_grad_(k in SPECTRA_RAW.values()))
+    leaf = {k: (torch.as_tensor(np.asarray(v), dtype=dtype).clone().requires_grad_(k in SPECTRA_RAW.values())
+                if not isinstance(v, Tensor) else v.detach().to(dtype).clone().requires_grad_(k in SPECTRA_RAW.values()))
             for k, v in sd.items()}
-    P = constrained(leaf)
+    P = constrained(leaf, dtype)
     for k in SPECTRA_RAW:
         P[k].retain_grad()
-    out = tables(P, int_array, float_array, no_germline_mode, het_beta, use_context_dependent_snv_priors)
+    out = tables(P, int_array, float_array, no_germline_mode, het_beta, use_context_dependent_snv_priors, dtype)
     loss = -torch.mean(torch.logsumexp(out["log_posteriors_bc"], dim=1))
     loss.backward()
     zero = lambda t: torch.zeros_like(t)
@@ -117,13 +120,14 @@ def negative_log_evidence_and_grads(sd, int_array, float_array, no_germline_mode
 
 
 def tables(P, int_array: np.ndarray, float_array: np.ndarray, no_germline_mode: bool = False,
-           het_beta=None, use_context_dependent_snv_priors: bool = True):
+           het_beta=None, use_context_dependent_snv_priors: bool = True, dtype=torch.float32):
     it = torch.as_tensor(np.asarray(int_array)).long()
-    ft = torch.as_tensor(np.asarray(float_array), dtype=torch.float32)
+    ft = torch.as_tensor(np.asarray(float_array), dtype=torch.float32).to(dtype)   # fp16 / fp32 as the kernel reads them
     B = len(it)
     vt = it[:, IDX["VARIANT_TYPE"]]
-    depth, alt = it[:, IDX["ORIGINAL_DEPTH"]], it[:, IDX["ORIGINAL_ALT_COUNT"]]
-    ndepth, nalt = it[:, IDX["ORIGINAL_NORMAL_DEPTH"]], it[:, IDX["ORIGINAL_NORMAL_ALT_COUNT"]]
+    # the counts as `dtype` (exact: int16 values); integer tensors would put lgamma and friends in the default float32
+    depth, alt = it[:, IDX["ORIGINAL_DEPTH"]].to(dtype), it[:, IDX["ORIGINAL_ALT_COUNT"]].to(dtype)
+    ndepth, nalt = it[:, IDX["ORIGINAL_NORMAL_DEPTH"]].to(dtype), it[:, IDX["ORIGINAL_NORMAL_ALT_COUNT"]].to(dtype)
     af, maf, nmaf = ft[:, FIDX["ALLELE_FREQUENCY"]], ft[:, FIDX["MAF"]], ft[:, FIDX["NORMAL_MAF"]]
     logit = ft[:, FIDX["CACHED_ARTIFACT_LOGIT"]]
 
@@ -136,7 +140,7 @@ def tables(P, int_array: np.ndarray, float_array: np.ndarray, no_germline_mode: 
         c = (L - 1) // 2
         hap = it[:, HAP_START:]
         ctx = P["snv_log_priors_rrra"][hap[:, c - 1], hap[:, c], hap[:, c + 1], hap[:, c + L]]
-        is_snv = (vt == 0).float()
+        is_snv = (vt == 0).to(dtype)
         pri[:, SOMATIC] = is_snv * ctx + (1 - is_snv) * pri[:, SOMATIC]
     pri = torch.log_softmax(pri, dim=-1)
 
@@ -145,7 +149,7 @@ def tables(P, int_array: np.ndarray, float_array: np.ndarray, no_germline_mode: 
     mafs_bk = torch.clamp(maf, max=0.49).view(-1, 1)
     cf = P["cf_k"].view(1, -1)
     ub = uniform_binomial_log_lk(depth.view(-1, 1).expand(-1, cf.shape[1]), alt.view(-1, 1).expand(-1, cf.shape[1]),
-                                 mafs_bk * cf, (1 - mafs_bk) * cf)
+                                 mafs_bk * cf, (1 - mafs_bk) * cf, dtype)
     non_bg = torch.logsumexp(P["log_weights_k"].view(1, -1) + ub, dim=-1)
     bg = beta_binomial_log_lk(depth, alt, P["bg_alpha"], P["bg_beta"])
     spec_cols[SOMATIC] = torch.logaddexp(P["log_non_bg"] + non_bg, P["log_bg"] + bg)          # math_utils.add_in_log_space
@@ -158,18 +162,18 @@ def tables(P, int_array: np.ndarray, float_array: np.ndarray, no_germline_mode: 
     b_b = torch.clamp(conc - a_b, min=0.001)
     spec_cols[NORMAL_ARTIFACT] = beta_binomial_log_lk(depth, alt, a_b, b_b)
     spec_cols[SEQ_ERROR] = ft[:, FIDX["SEQ_ERROR_LOG_LK"]]
-    spec_cols[GERMLINE] = germline_log_likelihood(af, maf, alt, depth, het_beta)
+    spec_cols[GERMLINE] = germline_log_likelihood(af, maf, alt, depth, het_beta, dtype)
     spec = torch.stack(spec_cols, dim=1)          # (the reference fills a zeros tensor column by column: same values)
 
     nse = ft[:, FIDX["NORMAL_SEQ_ERROR_LOG_LK"]]
-    norm_cols = [nse, nse, nse, germline_log_likelihood(af, nmaf, nalt, ndepth, het_beta),
-                 torch.where(nalt < 1, torch.tensor(-9999.0), na_normal)]
+    norm_cols = [nse, nse, nse, germline_log_likelihood(af, nmaf, nalt, ndepth, het_beta, dtype),
+                 torch.where(nalt < 1, torch.tensor(-9999.0, dtype=dtype), na_normal)]
     norm = torch.stack(norm_cols, dim=1)
 
     post_cols = list((pri + spec + norm).unbind(dim=1))
     post_cols[ARTIFACT] = post_cols[ARTIFACT] + logit
     post_cols[NORMAL_ARTIFACT] = post_cols[NORMAL_ARTIFACT] + logit
-    post_cols[ARTIFACT] = torch.where(logit < 0, torch.tensor(-9999.0), post_cols[ARTIFACT])  # posterior_model.py:90-93
+    post_cols[ARTIFACT] = torch.where(logit < 0, torch.tensor(-9999.0, dtype=dtype), post_cols[ARTIFACT])  # posterior_model.py:90-93
     post = torch.stack(post_cols, dim=1)
     return dict(log_priors_bc=pri, spectra_log_lks_bc=spec, normal_log_lks_bc=norm, log_posteriors_bc=post,
                 posterior_probabilities_bc=torch.softmax(post, dim=1),
